@@ -16,6 +16,12 @@ every input already resident in HBM; `e2e` is the same step through the public A
 buffers (pinned), host<->device copies inside the timed region.  Other BASELINE.json configs are
 selectable with --workload (configs[1] = ml1m_item_pearson_k40).
 
+--steps K times exactly K steps of each kind (device and e2e).  --dump-outputs DIR writes what the last
+timed device step computed (predictions, similarity rows, neighbour lists; seeded samples where larger
+than the 64 MB budget; NaN and infinities as a separate mask, see dump_outputs) as .npy files of finite
+numbers: the inputs are generated from fixed seeds, so two builds run with the same arguments can be
+compared output for output.
+
 N > 1 (torchrun, one rank per GPU): STRONG scaling of that ONE matrix.  The exact sparse path runs as
 cyclic row shards — every pair is computed once across the ranks, the other triangle of a rank's rows is
 pulled from the peers' matrices over NVLink, each rank predicts the test pairs whose left row it owns and
@@ -273,6 +279,65 @@ def pinned_like(a):
 
 _KEEP = []
 
+# --dump-outputs: all files together stay under 64 MB (DUMP_BYTES leaves room for the .npy headers); larger
+# outputs are sampled, with the same seeded rows or entries on every run, so that two builds can be compared
+# array by array.  Every file holds finite numbers only: a NaN or infinite value (an unset similarity, a
+# prediction without neighbours) is written as 0.0 in <name>.npy and its kind in <name>_nonfinite.npy
+# (float32, same shape: 0 finite, 1 NaN, 2 +inf, 3 -inf), so the budgets count 8 + 4 bytes per value.
+DUMP_BYTES = 63_000_000
+DUMP_PRED_BYTES = 48_000_000      # the predictions' share: all 4 M of the MovieLens-20M test set
+DUMP_SEED = 0
+
+
+def _dump_sample(n, cap):
+    """Positions 0..n-1, or a sorted seeded sample of `cap` of them."""
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, cap, replace=False))
+
+
+def dump_outputs(out_dir, h, d_pred, lists, n_pred, store_matrix):
+    """Writes what one step of the timed path returned as out_dir/<name>.npy, float64 throughout (ids too):
+    predictions.npy, in test-set order (predictions_index.npy: which test pairs, when sampled);
+    matrix.npy, rows matrix_rows.npy of the similarity matrix the handle holds; topk_index.npy (-1: no
+    neighbour) and topk_sims.npy, rows topk_rows.npy of the neighbour lists; <name>_nonfinite.npy beside
+    an output that had NaN or infinite values."""
+    import torch
+
+    out_dir.mkdir(parents=True, exist_ok=True)
+
+    def save(name, a):
+        a = np.asarray(a, dtype=np.float64)
+        bad = ~np.isfinite(a)
+        if bad.any():
+            kind = np.where(np.isnan(a), 1, np.where(a > 0, 2, 3)) * bad
+            np.save(out_dir / f"{name}_nonfinite.npy", kind.astype(np.float32))
+            a = np.where(bad, 0.0, a)
+        np.save(out_dir / f"{name}.npy", np.ascontiguousarray(a))
+
+    left = DUMP_BYTES
+    if d_pred is not None:
+        full = n_pred * 12 <= DUMP_PRED_BYTES
+        per = 12 if full else 20                                   # value + kind (+ index when sampled)
+        sel = _dump_sample(n_pred, DUMP_PRED_BYTES // per)
+        save("predictions", d_pred[torch.from_numpy(sel).to(d_pred.device)].cpu().numpy())
+        if not full:
+            save("predictions_index", sel)
+        left -= len(sel) * per
+    share = left // max(1, int(store_matrix) + int(lists is not None))
+    if store_matrix:
+        owned = h.owned_rows()
+        rows = owned[_dump_sample(len(owned), share // (12 * h.n_left + 8))]
+        save("matrix", np.concatenate([h.sims_rows(int(r), 1) for r in rows]))
+        save("matrix_rows", rows)
+    if lists is not None:
+        idx, sims = lists
+        rows = _dump_sample(idx.shape[0], share // (20 * idx.shape[1] + 8))
+        d_rows = torch.from_numpy(rows).to(idx.device)
+        save("topk_index", idx[d_rows].cpu().numpy())
+        save("topk_sims", sims[d_rows].cpu().numpy())
+        save("topk_rows", rows)
+
 
 def run_ours(args, rank, world, local_rank):
     import torch
@@ -358,6 +423,8 @@ def run_ours(args, rank, world, local_rank):
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)  # > 126 MB L2
 
     def step_device():
+        """One step; returns what a caller of the path receives besides the similarity matrix that stays in
+        `h`: (predictions, neighbour lists), None where the workload has none."""
         h.fit_device(d_left.data_ptr(), d_right.data_ptr(), d_rating.data_ptr(), len(left), n_left, n_right,
                      train.GlobalMean, d_lb.data_ptr() if d_lb is not None else 0,
                      d_rb.data_ptr() if d_rb is not None else 0, global_bias)
@@ -366,17 +433,17 @@ def run_ours(args, rank, world, local_rank):
         if cyc:
             h.predict_batch_sharded_device(d_tl.data_ptr(), d_tr.data_ptr(), n_pred, d_out.data_ptr())
             dist.all_reduce(d_out.view(torch.int64), op=dist.ReduceOp.SUM)
-            return d_out
+            return d_out, None
         if n_pred:
             h.predict_batch_device(d_tl.data_ptr(), d_tr.data_ptr(), n_pred, d_out.data_ptr())
+        lists = None
         if shard:
             h.topk_device(k, d_tk_i.data_ptr(), d_tk_s.data_ptr())
-            allgather_topk(d_tk_i, d_tk_s, n_left, k)
+            lists = allgather_topk(d_tk_i, d_tk_s, n_left, k)
         if sym:
             h.topk_device(k, d_tk_i.data_ptr(), d_tk_s.data_ptr())
-            if multi:
-                return union_topk_device(*allgather_partial_topk(d_tk_i, d_tk_s))
-            return d_tk_i, d_tk_s
+            lists = union_topk_device(*allgather_partial_topk(d_tk_i, d_tk_s)) if multi else (d_tk_i, d_tk_s)
+        return (d_out if n_pred else None), lists
 
     def barrier():
         if world > 1:
@@ -395,7 +462,7 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     for s in range(args.steps):
         ev[s][0].record(stream)
-        step_device()
+        result = step_device()
         ev[s][1].record(stream)
         flush.fill_(s & 0xff)  # L2 flush between timed iterations (outside the event pairs)
     barrier()
@@ -403,6 +470,8 @@ def run_ours(args, rank, world, local_rank):
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = sum(step_ms)
     prof = h.profile()
+    if args.dump_outputs and rank == 0:     # before the e2e steps, which reuse the neighbour-list buffers
+        dump_outputs(Path(args.dump_outputs), h, *result, n_pred, store_matrix=not sym)
 
     # ---- e2e: public API, host (pinned) buffers in, host predictions out ----
     train.innerUsers = pinned_like(train.innerUsers)
@@ -447,7 +516,7 @@ def run_ours(args, rank, world, local_rank):
     # every e2e step is timed on its own (wall clock around the public API call, which ends with the
     # device->host read of the result); the MEDIAN step is reported: the host part (Python, id maps,
     # pinned copies) is exposed to noisy neighbours on these shared boxes, the device part is not
-    e2e_steps = max(1, min(args.steps, 10))
+    e2e_steps = args.steps
     step_e2e()
     barrier()
     e2e_times = []
@@ -655,7 +724,11 @@ def main():
     ap.add_argument("--pearson-mode", default="exact", choices=["exact", "sums"])
     ap.add_argument("--sim-path", default="auto", choices=["auto", "tensor", "stream"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64, under 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -24,11 +24,24 @@ def _built():
         g.build()
 
 
+def load_ml100k():
+    """The reference's data fixture (core/data/ml-100k), see tests/golden/make_golden.py: "u_data" and the
+    fixed folds "u1_base" .. "u5_test" as int64 (n, 3) arrays of (user, item, rating).  A fold's files are
+    the rows of u.data sorted by (user, item): u{f}_test those stored with fold f, u{f}_base the others."""
+    g = np.load(ROOT / "tests" / "golden" / "ml100k.npz")
+    u_data, fold = np.stack([g["user"], g["item"], g["rating"]], axis=1).astype(np.int64), g["fold"]
+    order = np.lexsort((u_data[:, 1], u_data[:, 0]))
+    out = {"u_data": u_data}
+    for f in range(1, 6):
+        test = fold[order] == f
+        out[f"u{f}_base"] = u_data[order[~test]]
+        out[f"u{f}_test"] = u_data[order[test]]
+    return out
+
+
 @pytest.fixture(scope="session")
 def ml100k():
-    """The reference's data fixture (core/data/ml-100k), see tests/golden/make_golden.py."""
-    g = np.load(ROOT / "tests" / "golden" / "ml100k.npz")
-    return {k: g[k].astype(np.int64) for k in g.files}
+    return load_ml100k()
 
 
 def split(a):

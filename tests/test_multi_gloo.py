@@ -10,6 +10,8 @@ from pathlib import Path
 import numpy as np
 import pytest
 
+from conftest import load_ml100k
+
 ROOT = Path(__file__).resolve().parent.parent
 
 
@@ -32,9 +34,9 @@ def _worker(rank, world, port, out_dir):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
-    g = np.load(ROOT / "tests" / "golden" / "ml100k.npz")
-    tr = g["u1_base"].astype(np.int64)[:30000]
-    te = g["u1_test"].astype(np.int64)[:3000]
+    g = load_ml100k()
+    tr = g["u1_base"][:30000]
+    te = g["u1_test"][:3000]
     ts = ob.TrainSet(tr[:, 0], tr[:, 1], tr[:, 2].astype(float))
     n = ts.user_count
     b, e = shard_rows(n, world, rank, align=16)
@@ -104,8 +106,8 @@ def _worker_symmetric(rank, world, port, out_dir):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
-    g = np.load(ROOT / "tests" / "golden" / "ml100k.npz")
-    tr = g["u1_base"].astype(np.int64)[:20000]
+    g = load_ml100k()
+    tr = g["u1_base"][:20000]
     ts = ob.TrainSet(tr[:, 0], tr[:, 1], tr[:, 2].astype(float))
     full = ob.KNN(sim="msd", k=10, user_based=True).fit(ts)
     S = full.sims()
@@ -162,9 +164,9 @@ def _worker_cyclic(rank, world, port, out_dir):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
-    g = np.load(ROOT / "tests" / "golden" / "ml100k.npz")
-    tr = g["u1_base"].astype(np.int64)[:30000]
-    te = g["u1_test"].astype(np.int64)[:3000]
+    g = load_ml100k()
+    tr = g["u1_base"][:30000]
+    te = g["u1_test"][:3000]
     ts = ob.TrainSet(tr[:, 0], tr[:, 1], tr[:, 2].astype(float))
     full = ob.KNN(sim="pearson", knn_type="centered", k=10, user_based=True).fit(ts)
     S = full.sims()
