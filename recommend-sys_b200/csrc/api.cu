@@ -684,6 +684,7 @@ int32_t rs_knn_predict_neighbors(rs_knn *h, int32_t left, int32_t right, int32_t
     RS_CUDA(cudaMemsetAsync(dcnt, 0, 4, h->stream));
     RS_TRY(rs_predict_launch(h, (const int32_t *)dl, (const int32_t *)dr, 1, (double *)dout, (int32_t *)dids,
                              (double *)dsims, (int32_t *)dcnt, cap));
+    RS_TRY(rs_nb_cells_launch(h, (const int32_t *)dl, (const int32_t *)dids, (const int32_t *)dcnt, (double *)dsims));
     int32_t cnt = 0;
     RS_CUDA(cudaMemcpyAsync(&cnt, dcnt, 4, cudaMemcpyDeviceToHost, h->stream));
     RS_CUDA(cudaStreamSynchronize(h->stream));

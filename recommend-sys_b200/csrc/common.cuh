@@ -226,6 +226,8 @@ bool rs_tensor_topk_fused(const rs_knn *h);
 // ---- predict.cu ----
 int32_t rs_predict_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_right, int64_t n, double *d_out,
                           int32_t *d_nb_ids, double *d_nb_sims, int32_t *d_nb_count, int32_t nb_cap, int32_t foreign_zero = 0);
+int32_t rs_nb_cells_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_nb_ids, const int32_t *d_nb_count,
+                           double *d_nb_sims);
 int32_t rs_topk_launch(rs_knn *h, int32_t k, int32_t *d_idx, double *d_sim);
 int32_t rs_slope_predict_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_right, int64_t n, double *d_out);
 int32_t rs_topk_slab_launch(rs_knn *h, int64_t g0, int32_t m, double *tbuf, int64_t ld_t, int32_t k);

@@ -508,7 +508,7 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) predict_select_kernel(PredArgs
                 else if (a.knn_type == RS_KNN_BASELINE) rating -= a.bias[id];
                 w_s[e] = s;
                 w_a[e] = rating;
-                if (a.nb_ids && e < a.nb_cap) { a.nb_ids[e] = id; a.nb_sims[e] = s; }
+                if (a.nb_ids && e < a.nb_cap) { a.nb_ids[e] = id; a.nb_sims[e] = s; }   // +-0 as +0: see nb_cells_kernel
             }
         }
         __syncwarp();
@@ -534,6 +534,18 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) predict_select_kernel(PredArgs
 
 
 // ---------------- per-row top-k from the resident matrix ----------------
+// +-0 share one key: they tie and are ordered by id, as the reference's float comparison does.  The block
+// top-k kernels carry the sign of a zero in bit 31 of the id word, so that a list reports the exact
+// similarity (-0.0 included) while the order stays that of (key, id).
+constexpr uint32_t NEG0 = 0x80000000u;
+__device__ __forceinline__ uint32_t neg0_bit(double s) {
+    return (unsigned long long)__double_as_longlong(s) == 0x8000000000000000ull ? NEG0 : 0u;
+}
+__device__ __forceinline__ bool ent_before(uint64_t ka, uint32_t pa, uint64_t kb, uint32_t pb) {
+    return rec_before(ka, pa & ~NEG0, kb, pb & ~NEG0);
+}
+__device__ __forceinline__ double ent_sim(uint64_t k, uint32_t p) { return (p & NEG0) ? -0.0 : rs_key_sim(k); }
+
 constexpr int TOPK_THREADS = 256;
 constexpr int TOPK_CAP = 2048;
 
@@ -547,7 +559,7 @@ __device__ void block_bitonic(uint64_t *keys, uint32_t *pos, int n_pad) {
                 bool up = ((lo & size) == 0);
                 uint64_t ka = keys[lo], kb = keys[hi];
                 uint32_t pa = pos[lo], pb = pos[hi];
-                bool swap = up ? rec_before(kb, pb, ka, pa) : rec_before(ka, pa, kb, pb);
+                bool swap = up ? ent_before(kb, pb, ka, pa) : ent_before(ka, pa, kb, pb);
                 if (swap) { keys[lo] = kb; keys[hi] = ka; pos[lo] = pb; pos[hi] = pa; }
             }
         }
@@ -572,17 +584,19 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_rows_kernel(const double *_
         const int32_t j = base + threadIdx.x;
         bool take = false;
         uint64_t key = 0;
+        uint32_t neg0 = 0;
         if (j < n) {
             const double s = row[j];
             if (s == s) {
                 key = rs_sim_key(s);
-                take = !have_thr || rec_before(key, (uint32_t)j, s_thr_key, s_thr_pos);
+                take = !have_thr || ent_before(key, (uint32_t)j, s_thr_key, s_thr_pos);
+                neg0 = neg0_bit(s);
             }
         }
         if (take) {
             int slot = atomicAdd(&s_have, 1);
             keys[slot] = key;
-            pos[slot] = (uint32_t)j;
+            pos[slot] = (uint32_t)j | neg0;
         }
         __syncthreads();
         // every thread must see the SAME count: read it, then a second barrier before anybody's next
@@ -609,7 +623,7 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_rows_kernel(const double *_
     block_bitonic(keys, pos, n_pad);
     for (int t = threadIdx.x; t < k; t += blockDim.x) {
         const int64_t o = r * k + t;
-        if (t < have) { idx[o] = (int32_t)pos[t]; sim[o] = rs_key_sim(keys[t]); }
+        if (t < have) { idx[o] = (int32_t)(pos[t] & ~NEG0); sim[o] = ent_sim(keys[t], pos[t]); }
         else { idx[o] = -1; sim[o] = __longlong_as_double(0x7ff8000000000001ll); }
     }
 }
@@ -649,7 +663,7 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_merge_kernel(const double *
         if (id >= 0) {
             const int slot = atomicAdd(&s_have, 1);
             keys[slot] = rs_sim_key(sim[g * k + t]);
-            pos[slot] = (uint32_t)id;
+            pos[slot] = (uint32_t)id | neg0_bit(sim[g * k + t]);
         }
     }
     bool have_thr = idx[g * k + (k - 1)] >= 0;
@@ -662,17 +676,19 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_merge_kernel(const double *
         const int32_t j = base + threadIdx.x;
         bool take = false;
         uint64_t key = 0;
+        uint32_t neg0 = 0;
         if (j < chi) {
             const double s = row[j];
             if (s == s) {
                 key = rs_sim_key(s);
-                take = !have_thr || rec_before(key, (uint32_t)j + id_off, s_thr_key, s_thr_pos);
+                take = !have_thr || ent_before(key, (uint32_t)j + id_off, s_thr_key, s_thr_pos);
+                neg0 = neg0_bit(s);
             }
         }
         if (take) {
             int slot = atomicAdd(&s_have, 1);
             keys[slot] = key;
-            pos[slot] = (uint32_t)j + id_off;
+            pos[slot] = ((uint32_t)j + id_off) | neg0;
         }
         __syncthreads();
         // every thread must see the SAME count: read it, then a second barrier before anybody's next
@@ -699,7 +715,7 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_merge_kernel(const double *
     block_bitonic(keys, pos, n_pad);
     for (int t = threadIdx.x; t < k; t += blockDim.x) {
         const int64_t o = g * k + t;
-        if (t < have) { idx[o] = (int32_t)pos[t]; sim[o] = rs_key_sim(keys[t]); }
+        if (t < have) { idx[o] = (int32_t)(pos[t] & ~NEG0); sim[o] = ent_sim(keys[t], pos[t]); }
         else { idx[o] = -1; sim[o] = __longlong_as_double(0x7ff8000000000001ll); }
     }
 }
@@ -728,7 +744,7 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_compact_kernel(
     for (int t = threadIdx.x; t < k; t += blockDim.x) {
         const int32_t id = idx[g * k + t];
         keys[t] = id >= 0 ? rs_sim_key(sim[g * k + t]) : 0ull;
-        pos[t] = id >= 0 ? (uint32_t)id : 0xffffffffu;
+        pos[t] = id >= 0 ? (uint32_t)id | neg0_bit(sim[g * k + t]) : 0xffffffffu;
     }
     __syncthreads();
     // number of list entries (prefix length)
@@ -741,7 +757,7 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_compact_kernel(
     have = s_have;
     for (int t = threadIdx.x; t < cnt; t += blockDim.x) {
         keys[have + t] = rs_sim_key(cand_sim[g * cap + t]);
-        pos[have + t] = (uint32_t)cand_id[g * cap + t];
+        pos[have + t] = (uint32_t)cand_id[g * cap + t] | neg0_bit(cand_sim[g * cap + t]);
     }
     const int total = have + cnt;
     int n_pad = 32;
@@ -752,7 +768,7 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_compact_kernel(
     if (!over) {
         for (int t = threadIdx.x; t < k; t += blockDim.x) {
             const int64_t o = g * k + t;
-            if (t < total) { idx[o] = (int32_t)pos[t]; sim[o] = rs_key_sim(keys[t]); }
+            if (t < total) { idx[o] = (int32_t)(pos[t] & ~NEG0); sim[o] = ent_sim(keys[t], pos[t]); }
             else { idx[o] = -1; sim[o] = __longlong_as_double(0x7ff8000000000001ll); }
         }
     }
@@ -761,7 +777,7 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_compact_kernel(
         // the buffer is discarded, so the k-th best of (list U buffer) itself — a real entry that may belong
         // to the final list — and everything above it must be admitted again: threshold = just below it
         // (same key, id + 1).
-        if (total >= k) { thr_key[g] = keys[k - 1]; thr_id[g] = (int32_t)pos[k - 1] + (over ? 1 : 0); }
+        if (total >= k) { thr_key[g] = keys[k - 1]; thr_id[g] = (int32_t)(pos[k - 1] & ~NEG0) + (over ? 1 : 0); }
         else { thr_key[g] = 0ull; thr_id[g] = -1; }            // list not full: accept every valid similarity
         cand_cnt[g] = 0;
         row_flag[g] = over ? 1 : 0;
@@ -816,7 +832,7 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_union_kernel(const int32_t 
         if (id >= 0) {
             const int slot = atomicAdd(&s_have, 1);
             keys[slot] = rs_sim_key(sim_all[o]);
-            pos[slot] = (uint32_t)id;
+            pos[slot] = (uint32_t)id | neg0_bit(sim_all[o]);
         }
     }
     __syncthreads();
@@ -827,7 +843,7 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_union_kernel(const int32_t 
     block_bitonic(keys, pos, n_pad);
     for (int t = threadIdx.x; t < k; t += blockDim.x) {
         const int64_t o = g * k + t;
-        if (t < have) { idx[o] = (int32_t)pos[t]; sim[o] = rs_key_sim(keys[t]); }
+        if (t < have) { idx[o] = (int32_t)(pos[t] & ~NEG0); sim[o] = ent_sim(keys[t], pos[t]); }
         else { idx[o] = -1; sim[o] = __longlong_as_double(0x7ff8000000000001ll); }
     }
 }
@@ -1024,6 +1040,26 @@ int32_t rs_predict_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_rig
     else RS_TRY(launch_select<8>(a, (unsigned)blocks, smem, scap, h->stream));
     h->prof.predict_launches++;
     h->prof.total_launches += 1;
+    RS_CUDA(cudaGetLastError());
+    return RS_OK;
+}
+
+// The neighbour report of a single prediction (rs_knn_predict_neighbors): the selection kernel writes the
+// similarity its record was sorted by, where -0.0 has become +0.0; the list reports the matrix cells themselves.
+__global__ void nb_cells_kernel(const double *__restrict__ sims, int64_t ld_s, int64_t row_begin, int32_t cyc_R,
+                                const int32_t *__restrict__ left, const int32_t *__restrict__ nb_ids,
+                                const int32_t *__restrict__ nb_count, double *__restrict__ nb_sims) {
+    const int32_t l = *left, cnt = *nb_count;
+    if (cnt <= 0) return;                                     // cold start / mink: nothing was reported
+    const double *row = sims + (cyc_R > 1 ? rs_cyc_local(l, cyc_R) : l - row_begin) * ld_s;
+    for (int e = threadIdx.x; e < cnt; e += blockDim.x) nb_sims[e] = row[nb_ids[e]];
+}
+
+int32_t rs_nb_cells_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_nb_ids, const int32_t *d_nb_count,
+                           double *d_nb_sims) {
+    nb_cells_kernel<<<1, 256, 0, h->stream>>>(h->sims, h->ld_s, h->row_begin, h->cyc_R, d_left, d_nb_ids, d_nb_count,
+                                              d_nb_sims);
+    h->prof.total_launches++;
     RS_CUDA(cudaGetLastError());
     return RS_OK;
 }

@@ -425,7 +425,8 @@ __global__ void right_means_kernel(const int64_t *__restrict__ r_ptr, const doub
 
 static int32_t rs_stream_jc(int32_t n_left) {
     int32_t jc = n_left < 8192 ? 128 : 256;
-    if (const char *e = getenv("RS_KNN_STREAM_JC")) { const int v = atoi(e); jc = v == 128 ? 128 : v == 512 ? 512 : 256; }
+    // the stream kernel is instantiated for 128 and 256 columns only (launch_stream_sym): anything else takes 256
+    if (const char *e = getenv("RS_KNN_STREAM_JC")) jc = atoi(e) == 128 ? 128 : 256;
     return jc;
 }
 

@@ -335,8 +335,9 @@ def test_continuous_ratings_bit_exact(ml100k, sim, knn_type):
     assert bits_equal(rs.NewRawSet(tu, ti, np.zeros(len(tu))).Predict(est), ref.predict_batch(tu, ti, n_threads=8))
 
 
-# ---- both chunk widths of the stream kernel (128 for small matrices, 256 for large ones) ----
-@pytest.mark.parametrize("jc", ["128", "256"])
+# ---- both chunk widths of the stream kernel (128 for small matrices, 256 for large ones); any other request
+# ("512") takes 256 ----
+@pytest.mark.parametrize("jc", ["128", "256", "512"])
 @pytest.mark.parametrize("sim", ["cosine", "msd", "pearson"])
 def test_sims_bit_exact_both_chunk_widths(ml100k, sim, jc, monkeypatch):
     monkeypatch.setenv("RS_KNN_STREAM_JC", jc)
