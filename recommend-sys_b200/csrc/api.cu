@@ -56,9 +56,8 @@ void free_fit_state(rs_knn *h) {
     h->row_heavy = nullptr;
     h->n_heavy = 0;
     h->n_pop = h->pop_ld = 0;
-    h->pop_idx = h->pop_items = nullptr;
+    h->rank = h->lab_row = h->pop_items = nullptr;
     h->pop_dense = nullptr;
-    h->pop_blk = nullptr;
     h->w_ptr = nullptr;
     h->w_col = nullptr;
     h->w_dev = nullptr;

@@ -146,13 +146,13 @@ struct rs_knn {
     double *right_means = nullptr;
 
     // stream path: b-side term of every rating in right-CSR order (value, value - row mean, ...),
-    // chunk pointers cp[right][Q+1] into each right row, and l2r: left-CSR entry -> right-CSR index
+    // chunk pointers cp[right][Q+1] into each right row, and l2r: left-CSR entry -> right-CSR (or walk-CSR) index
     double *r_dev = nullptr;
     int32_t *cp = nullptr;
     int32_t n_chunks = 0;
     int32_t stream_jc = 256;
     bool stream_lower = false;     // full-matrix stream Fit computes j < i (else j > i); chosen per Fit from the lookup counts
-    double inc_upper = 0.0, inc_lower = 0.0;   // (entry, chunk) lookups of the two triangles
+    double inc_upper = 0.0, inc_lower = 0.0;   // (entry, chunk) lookups of the two triangles (in label space with popular columns)
     int64_t *l2r = nullptr;
     int32_t *perm_lr = nullptr, *perm_rl = nullptr, *perm_tmp = nullptr;  // CSR position -> input row (arena, valid until the next Fit)
     int32_t *row_order = nullptr;  // left rows sorted by descending length
@@ -162,14 +162,17 @@ struct rs_knn {
     // taken out of the right CSR the column walk reads (walk CSR: w_ptr / w_col / w_dev, `cp` and `l2r` refer to
     // it) and kept as a dense table pop_dense[n_right][pop_ld] instead (one byte per cell when every rating is a
     // small integer, else the b-side double; 0 / NaN = no rating).
+    // Every row has a RANK, its position in the stable longest-first order of all rows: ranks below n_pop are the
+    // popular list, and the other rows are the walk's columns under the LABEL rank - n_pop (the walk CSR holds
+    // labels, ascending within each right row), so the long rows have the small labels.
     int32_t n_pop = 0, pop_ld = 0;
     bool pop_u8 = false;
-    int32_t *pop_idx = nullptr;    // [n_left] index in the popular list or -1
+    int32_t *rank = nullptr;       // [n_left] position in the longest-first order
+    int32_t *lab_row = nullptr;    // [n_left - n_pop] the row of each label
     int32_t *pop_items = nullptr;  // [pop_ld] row id (-1 beyond n_pop)
-    uint8_t *pop_blk = nullptr;    // [ceil(n_left / 32)] the block of 32 rows holds a popular row
     void *pop_dense = nullptr;
     int64_t *w_ptr = nullptr;
-    int32_t *w_col = nullptr;
+    int32_t *w_col = nullptr;      // labels
     double *w_dev = nullptr;
     int32_t *row_all = nullptr;    // every row of the shard, longest first (the dense pass visits them all)
     int64_t n_all_rows = 0;

@@ -253,68 +253,69 @@ __global__ void pop_count_kernel(const int32_t *__restrict__ len_sorted, int32_t
     }
     *out = lo < cap ? lo : cap;
 }
-// pop_idx[row] = position in the popular list (-1 elsewhere: the array is preset to 0xFF), pop_items = the list
-__global__ void pop_index_kernel(const int32_t *__restrict__ sorted, int32_t n_pop, int32_t pop_ld,
-                                 int32_t *__restrict__ pop_idx, int32_t *__restrict__ pop_items,
-                                 uint8_t *__restrict__ pop_blk) {
+// pop_items = the popular list, -1 beyond it
+__global__ void pop_items_kernel(const int32_t *__restrict__ sorted, int32_t n_pop, int32_t pop_ld,
+                                 int32_t *__restrict__ pop_items) {
     const int32_t p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= pop_ld) return;
-    if (p < n_pop) { const int32_t i = sorted[p]; pop_idx[i] = p; pop_items[p] = i; pop_blk[i >> 5] = 1; }
-    else pop_items[p] = -1;
+    if (p < pop_ld) pop_items[p] = p < n_pop ? sorted[p] : -1;
 }
-// One warp per right row: its popular ratings go into the dense table (preset to "no rating"), the others are
-// counted (w_cnt[c]; the walk CSR's row pointers are the exclusive sums).
+// One warp per right row: its popular ratings go into the dense table (preset to "no rating").
 template <typename DT>
 __global__ void pop_scatter_kernel(const int64_t *__restrict__ r_ptr, const int32_t *__restrict__ r_col,
                                    const double *__restrict__ r_val, const double *__restrict__ r_dev,
-                                   int32_t n_right, const int32_t *__restrict__ pop_idx, int32_t pop_ld,
-                                   DT *__restrict__ dense, int64_t *__restrict__ w_cnt) {
-    const int32_t c = (int32_t)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
-    const int lane = threadIdx.x & 31;
-    if (c > n_right) return;
-    if (c == n_right) { if (lane == 0) w_cnt[c] = 0; return; }
-    int32_t light = 0;
-    for (int64_t x = r_ptr[c] + lane; x < r_ptr[c + 1]; x += 32) {
-        const int32_t p = pop_idx[r_col[x]];
-        if (p < 0) { light++; continue; }
-        if (sizeof(DT) == 1) dense[(int64_t)c * pop_ld + p] = (DT)((int)r_val[x] + RS_INT8_BIAS);            // the byte code of code_int8_kernel
-        else dense[(int64_t)c * pop_ld + p] = (DT)r_dev[x];
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) light += __shfl_xor_sync(0xffffffffu, light, o);
-    if (lane == 0) w_cnt[c] = light;
-}
-// One warp per right row: the other ratings, compacted in order into the walk CSR; pos[x] = where the entry went.
-__global__ void pop_compact_kernel(const int64_t *__restrict__ r_ptr, const int32_t *__restrict__ r_col,
-                                   const double *__restrict__ r_dev, int32_t n_right,
-                                   const int32_t *__restrict__ pop_idx, const int64_t *__restrict__ w_ptr,
-                                   int32_t *__restrict__ w_col, double *__restrict__ w_dev, int64_t *__restrict__ pos) {
+                                   int32_t n_right, const int32_t *__restrict__ rank, int32_t n_pop, int32_t pop_ld,
+                                   DT *__restrict__ dense) {
     const int32_t c = (int32_t)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
     const int lane = threadIdx.x & 31;
     if (c >= n_right) return;
-    const int64_t b = r_ptr[c], e = r_ptr[c + 1];
-    int64_t out = w_ptr[c];
-    for (int64_t x0 = b; x0 < e; x0 += 32) {
-        const int64_t x = x0 + lane;
-        int32_t j = -1;
-        bool keep = false;
-        if (x < e) { j = r_col[x]; keep = pop_idx[j] < 0; }
-        const unsigned m = __ballot_sync(0xffffffffu, keep);
-        if (x < e) {
-            const int64_t o = out + __popc(m & ((1u << lane) - 1u));
-            if (keep) { w_col[o] = j; w_dev[o] = r_dev[x]; pos[x] = o; }
-            else pos[x] = -1;
-        }
-        out += __popc(m);
+    for (int64_t x = r_ptr[c] + lane; x < r_ptr[c + 1]; x += 32) {
+        const int32_t p = rank[r_col[x]];
+        if (p >= n_pop) continue;
+        if (sizeof(DT) == 1) dense[(int64_t)c * pop_ld + p] = (DT)((int)r_val[x] + RS_INT8_BIAS);            // the byte code of code_int8_kernel
+        else dense[(int64_t)c * pop_ld + p] = (DT)r_dev[x];
     }
 }
-__global__ void pop_remap_l2r_kernel(int64_t *__restrict__ l2r, const int64_t *__restrict__ pos, int64_t n) {
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e < n) l2r[e] = pos[l2r[e]];      // -1 for the entries of popular rows, which are never walked
+// The walk CSR is the transpose of the walked rows taken in label order: one warp per rank lays out the entries of
+// the walked rows as (right id, left-CSR entry) pairs at the row's offset in label order (w_off), and notes the
+// entry's label; a stable sort by right id then leaves every right row's entries in ascending label.  The entries
+// of the popular rows are never walked: l2r = -1.
+__global__ void walk_seq_kernel(const int32_t *__restrict__ sorted, int32_t n_left, int32_t n_pop,
+                                const int64_t *__restrict__ l_ptr, const int32_t *__restrict__ l_col,
+                                const int64_t *__restrict__ w_off, int32_t *__restrict__ key, int32_t *__restrict__ ent,
+                                int32_t *__restrict__ ent_lab, int64_t *__restrict__ l2r) {
+    const int32_t p = (int32_t)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+    const int lane = threadIdx.x & 31;
+    if (p >= n_left) return;
+    const int32_t i = sorted[p];
+    const int64_t b = l_ptr[i], e = l_ptr[i + 1];
+    if (p < n_pop) {
+        for (int64_t x = b + lane; x < e; x += 32) l2r[x] = -1;
+        return;
+    }
+    const int32_t lab = p - n_pop;
+    const int64_t o = w_off[lab] - b;
+#pragma unroll 4
+    for (int64_t x = b + lane; x < e; x += 32) {
+        key[o + x] = l_col[x];
+        ent[o + x] = (int32_t)x;
+        ent_lab[x] = lab;
+    }
+}
+// walk CSR position o <- left-CSR entry x = ent[o]: its label, its b-side term, and l2r[x] = o
+__global__ void walk_gather_kernel(const int32_t *__restrict__ ent, const int32_t *__restrict__ ent_lab,
+                                   const double *__restrict__ r_dev, int64_t n, int32_t *__restrict__ w_col,
+                                   double *__restrict__ w_dev, int64_t *__restrict__ l2r) {
+    const int64_t o = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (o >= n) return;
+    const int32_t x = ent[o];
+    w_col[o] = ent_lab[x];
+    w_dev[o] = r_dev[l2r[x]];
+    l2r[x] = o;
 }
 struct PopLight {
-    const int32_t *pop_idx;
-    __host__ __device__ bool operator()(const int32_t &i) const { return pop_idx[i] < 0; }
+    const int32_t *rank;
+    int32_t n_pop;
+    __host__ __device__ bool operator()(const int32_t &i) const { return rank[i] >= n_pop; }
 };
 
 
@@ -390,13 +391,14 @@ __global__ void triples_kernel(const int64_t *__restrict__ r_ptr, int32_t nr, un
 }
 
 // (entry, chunk) lookups the stream kernel performs when it computes the upper (j > i) or the lower
-// (j < i) triangle: row i pays one lookup per entry and per column chunk it visits.
-__global__ void incidence_kernel(const int64_t *__restrict__ l_ptr, int32_t nl, int32_t jc,
-                                 unsigned long long *out) {
+// (j < i) triangle: row i pays one lookup per entry and per column chunk it visits.  Row i's length is
+// len[i], or taken from l_ptr when len is null.
+__global__ void incidence_kernel(const int64_t *__restrict__ l_ptr, const int32_t *__restrict__ len, int32_t nl,
+                                 int32_t jc, unsigned long long *out) {
     unsigned long long up = 0, lo = 0;
     const long long q_all = (nl + jc - 1) / jc;
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < nl; i += (int64_t)gridDim.x * blockDim.x) {
-        const unsigned long long d = (unsigned long long)(l_ptr[i + 1] - l_ptr[i]);
+        const unsigned long long d = (unsigned long long)(len ? (int64_t)len[i] : l_ptr[i + 1] - l_ptr[i]);
         const long long q = i / jc;
         up += d * (unsigned long long)(q_all - q);
         lo += d * (unsigned long long)(q + 1);
@@ -421,6 +423,12 @@ __global__ void right_means_kernel(const int64_t *__restrict__ r_ptr, const doub
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
     if (lane == 0) out[c] = s / (double)(r_ptr[c + 1] - r_ptr[c]);
+}
+
+// the cheaper triangle by the lookup counts inc_upper / inc_lower
+static void pick_triangle(rs_knn *h) {
+    h->stream_lower = h->inc_lower < h->inc_upper;
+    if (const char *e = getenv("RS_KNN_STREAM_TRI")) h->stream_lower = !strcmp(e, "lower");   // tests: force a triangle
 }
 
 static int32_t rs_stream_jc(int32_t n_left) {
@@ -486,7 +494,7 @@ int32_t rs_prep_build(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
     // keys_b = the left ids in ascending order: the left CSR's row pointers, and the (entry, chunk) lookups of
     // the two triangles of a stream Fit
     ptr_from_sorted_kernel<<<blocks_for(nnz + 1), T, 0, st>>>(keys_b, nnz, nl, h->l_ptr);
-    incidence_kernel<<<148, T, 0, st>>>(h->l_ptr, nl, h->stream_jc, reinterpret_cast<unsigned long long *>(h->d_flags + 8));
+    incidence_kernel<<<148, T, 0, st>>>(h->l_ptr, nullptr, nl, h->stream_jc, reinterpret_cast<unsigned long long *>(h->d_flags + 8));
     h->prof.total_launches += 4;
     // (right, left asc): stable sort by right of the (left, right asc) sequence
     gather_keys_kernel<<<blocks_for(nnz), T, 0, st>>>(d_right, perm_lr, nnz, keys_a);
@@ -563,8 +571,7 @@ int32_t rs_prep_build(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
     { unsigned long long t; memcpy(&t, fl8 + 6, 8); h->triples = (double)t; }
     h->max_right_len = fl8[15];
     { unsigned long long t[2]; memcpy(t, fl8 + 8, 16); h->inc_upper = (double)t[0]; h->inc_lower = (double)t[1]; }
-    h->stream_lower = h->inc_lower < h->inc_upper;
-    if (const char *e = getenv("RS_KNN_STREAM_TRI")) h->stream_lower = !strcmp(e, "lower");   // tests: force a triangle
+    pick_triangle(h);
     if (flags & FLAG_DUP) {
         rs_set_error("duplicate (left,right) rating pairs are not supported (the reference's merge-join "
                      "double-counts them)");
@@ -616,9 +623,11 @@ static int32_t split_heavy_rows(rs_knn *h, int32_t *order, int64_t n_rows, bool 
 }
 
 // Popular columns: the rows of >= min_len entries (at most RS_POP_MAX, the longest).  `sorted`: ALL rows, longest
-// first; `len_sorted`: their lengths; `order` / n_rows: the rows of this shard, longest first.  Splits their
-// ratings off the right CSR (walk CSR + dense table, see rs_knn::pop_*), builds `cp` and re-targets `l2r` for the
-// walk CSR, and leaves the rows the column walk visits (the others, same order) in h->row_order.
+// first (stable: ties by id), so a row's position in it is its rank; `len_sorted`: their lengths; `order` / n_rows:
+// the rows of this shard, longest first.  Splits the popular rows' ratings off the right CSR into the dense table,
+// builds the walk CSR over the other rows' labels (see rs_knn::rank) and re-targets `l2r` to it, picks the triangle
+// by the lookups in label space, and leaves the rows the column walk visits (the others, same order) in
+// h->row_order.  `cp` is built by the caller over the labels.
 constexpr int RS_POP_MAX = 512;
 
 static int32_t split_popular(rs_knn *h, const int32_t *sorted, const int32_t *len_sorted, int32_t *order, int64_t n_rows,
@@ -634,60 +643,89 @@ static int32_t split_popular(rs_knn *h, const int32_t *sorted, const int32_t *le
     RS_CUDA(cudaStreamSynchronize(st));
     h->prof.total_launches++;
     if (n_pop < 2) return RS_OK;                              // nothing to split off
-    const int32_t nr = h->n_right;
+    const int32_t nr = h->n_right, nl = h->n_left, n_walk = nl - n_pop;
     h->n_pop = n_pop;
     h->pop_ld = (n_pop + 31) / 32 * 32;
     h->pop_u8 = h->rating_class == RS_CLASS_INT8;
-    RS_TRY(rs_alloc(h, &h->pop_idx, (size_t)h->n_left));
+    h->lab_row = const_cast<int32_t *>(sorted) + n_pop;
+    RS_TRY(rs_alloc(h, &h->rank, (size_t)nl));
     RS_TRY(rs_alloc(h, &h->pop_items, (size_t)h->pop_ld));
-    RS_TRY(rs_alloc(h, &h->pop_blk, ((size_t)h->n_left + 31) / 32 + 1));
-    RS_CUDA(cudaMemsetAsync(h->pop_idx, 0xFF, (size_t)h->n_left * 4, st));
-    RS_CUDA(cudaMemsetAsync(h->pop_blk, 0, ((size_t)h->n_left + 31) / 32 + 1, st));
-    pop_index_kernel<<<blocks_for(h->pop_ld), T, 0, st>>>(sorted, n_pop, h->pop_ld, h->pop_idx, h->pop_items, h->pop_blk);
-    // dense table + walk CSR
+    invert_perm_kernel<<<blocks_for(nl), T, 0, st>>>(sorted, nl, h->rank);
+    pop_items_kernel<<<blocks_for(h->pop_ld), T, 0, st>>>(sorted, n_pop, h->pop_ld, h->pop_items);
+    // dense table
     const size_t cell = h->pop_u8 ? 1 : 8;
     RS_TRY(rs_dev_alloc(h, &h->pop_dense, (size_t)nr * h->pop_ld * cell));
     RS_CUDA(cudaMemsetAsync(h->pop_dense, h->pop_u8 ? 0 : 0xFF, (size_t)nr * h->pop_ld * cell, st));   // 0 / NaN = no rating
-    int64_t *w_cnt, *pos;
-    RS_TRY(rs_alloc(h, &w_cnt, (size_t)nr + 1));
-    RS_TRY(rs_alloc(h, &h->w_ptr, (size_t)nr + 1));
-    RS_TRY(rs_alloc(h, &h->w_col, (size_t)h->nnz));
-    RS_TRY(rs_alloc(h, &h->w_dev, (size_t)h->nnz));
-    RS_TRY(rs_alloc(h, &pos, (size_t)h->nnz));
     if (h->pop_u8)
-        pop_scatter_kernel<uint8_t><<<blocks_for(((int64_t)nr + 1) * 32), T, 0, st>>>(
-            h->r_ptr, h->r_col, h->r_val, h->r_dev, nr, h->pop_idx, h->pop_ld, static_cast<uint8_t *>(h->pop_dense), w_cnt);
+        pop_scatter_kernel<uint8_t><<<blocks_for((int64_t)nr * 32), T, 0, st>>>(
+            h->r_ptr, h->r_col, h->r_val, h->r_dev, nr, h->rank, n_pop, h->pop_ld, static_cast<uint8_t *>(h->pop_dense));
     else
-        pop_scatter_kernel<double><<<blocks_for(((int64_t)nr + 1) * 32), T, 0, st>>>(
-            h->r_ptr, h->r_col, h->r_val, h->r_dev, nr, h->pop_idx, h->pop_ld, static_cast<double *>(h->pop_dense), w_cnt);
-    size_t need = 0;
-    RS_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, need, w_cnt, h->w_ptr, nr + 1, st));
-    void *tmp;
-    RS_TRY(rs_dev_alloc(h, &tmp, need + 256));
-    RS_CUDA(cub::DeviceScan::ExclusiveSum(tmp, need, w_cnt, h->w_ptr, nr + 1, st));
-    pop_compact_kernel<<<blocks_for((int64_t)nr * 32), T, 0, st>>>(h->r_ptr, h->r_col, h->r_dev, nr, h->pop_idx, h->w_ptr,
-                                                                   h->w_col, h->w_dev, pos);
-    pop_remap_l2r_kernel<<<blocks_for(h->nnz), T, 0, st>>>(h->l2r, pos, h->nnz);
-    h->prof.total_launches += 5;
+        pop_scatter_kernel<double><<<blocks_for((int64_t)nr * 32), T, 0, st>>>(
+            h->r_ptr, h->r_col, h->r_val, h->r_dev, nr, h->rank, n_pop, h->pop_ld, static_cast<double *>(h->pop_dense));
+    h->prof.total_launches += 3;
+    // offsets of the walked rows in label order, and the (entry, chunk) lookups of both triangles over the labels
+    int64_t *w_off;
+    unsigned long long *d_inc;
+    RS_TRY(rs_alloc(h, &w_off, (size_t)n_walk + 1));
+    RS_TRY(rs_alloc(h, &d_inc, 2));
+    RS_CUDA(cudaMemsetAsync(w_off, 0, 8, st));
+    RS_CUDA(cudaMemsetAsync(d_inc, 0, 16, st));
+    if (n_walk > 0) {
+        size_t need = 0;
+        RS_CUDA(cub::DeviceScan::InclusiveSum(nullptr, need, len_sorted + n_pop, w_off + 1, n_walk, st));
+        void *tmp;
+        RS_TRY(rs_dev_alloc(h, &tmp, need + 256));
+        RS_CUDA(cub::DeviceScan::InclusiveSum(tmp, need, len_sorted + n_pop, w_off + 1, n_walk, st));
+    }
+    incidence_kernel<<<148, T, 0, st>>>(nullptr, len_sorted + n_pop, n_walk, h->stream_jc, d_inc);
+    h->prof.total_launches++;
     // the rows the column walk visits: the shard's rows that are not popular
     h->row_all = order;
     h->n_all_rows = n_rows;
     int32_t *rest;
     RS_TRY(rs_alloc(h, &rest, (size_t)(n_rows > 0 ? n_rows : 1)));
     h->row_order = rest;
-    h->n_work_rows = 0;
+    int32_t cnt = 0;
     if (n_rows > 0) {
-        PopLight light{h->pop_idx};
+        PopLight light{h->rank, n_pop};
         size_t need2 = 0;
         RS_CUDA(cub::DeviceSelect::If(nullptr, need2, order, rest, d_num, (int)n_rows, light, st));
         void *tmp2;
         RS_TRY(rs_dev_alloc(h, &tmp2, need2 + 256));
         RS_CUDA(cub::DeviceSelect::If(tmp2, need2, order, rest, d_num, (int)n_rows, light, st));
-        int32_t cnt = 0;
         RS_CUDA(cudaMemcpyAsync(&cnt, d_num, 4, cudaMemcpyDeviceToHost, st));
-        RS_CUDA(cudaStreamSynchronize(st));
-        h->n_work_rows = cnt;
     }
+    int64_t nnz_w = 0;
+    unsigned long long inc[2] = {0, 0};
+    RS_CUDA(cudaMemcpyAsync(&nnz_w, w_off + n_walk, 8, cudaMemcpyDeviceToHost, st));
+    RS_CUDA(cudaMemcpyAsync(inc, d_inc, 16, cudaMemcpyDeviceToHost, st));
+    RS_CUDA(cudaStreamSynchronize(st));
+    h->n_work_rows = cnt;
+    h->inc_upper = (double)inc[0];
+    h->inc_lower = (double)inc[1];
+    pick_triangle(h);
+    h->n_chunks = (int32_t)(((int64_t)n_walk + h->stream_jc - 1) / h->stream_jc);
+    // walk CSR: the walked entries in label order, stably sorted by right id
+    int32_t *key, *ent, *key_s, *ent_s, *ent_lab;
+    RS_TRY(rs_alloc(h, &h->w_ptr, (size_t)nr + 1));
+    RS_TRY(rs_alloc(h, &h->w_col, (size_t)nnz_w));
+    RS_TRY(rs_alloc(h, &h->w_dev, (size_t)nnz_w));
+    RS_TRY(rs_alloc(h, &key, (size_t)nnz_w));
+    RS_TRY(rs_alloc(h, &ent, (size_t)nnz_w));
+    RS_TRY(rs_alloc(h, &key_s, (size_t)nnz_w));
+    RS_TRY(rs_alloc(h, &ent_s, (size_t)nnz_w));
+    RS_TRY(rs_alloc(h, &ent_lab, (size_t)h->nnz));
+    walk_seq_kernel<<<blocks_for((int64_t)nl * 32), T, 0, st>>>(sorted, nl, n_pop, h->l_ptr, h->l_col, w_off, key, ent,
+                                                                ent_lab, h->l2r);
+    h->prof.total_launches++;
+    if (nnz_w > 0) {
+        SortTmp tmp;
+        RS_SORT_PAIRS(key, key_s, ent, ent_s, nnz_w, bits_for(nr));
+        walk_gather_kernel<<<blocks_for(nnz_w), T, 0, st>>>(ent_s, ent_lab, h->r_dev, nnz_w, h->w_col, h->w_dev, h->l2r);
+        h->prof.total_launches++;
+    }
+    ptr_from_sorted_kernel<<<blocks_for(nnz_w + 1), T, 0, st>>>(key_s, nnz_w, nr, h->w_ptr);
+    h->prof.total_launches++;
     return RS_OK;
 }
 

@@ -51,7 +51,11 @@ struct StreamArgs {
     int64_t n_rows;           // rows of row_order to walk
     int cyc_R;                // >= 2: cyclic row shards, the output row is rs_cyc_local(i)
     int symmetric;            // 0: full rows; 1: only columns j > i are computed; 2: only j < i (the mirror pass fills the rest)
-    const int32_t *pop_idx;   // popular columns (not in the CSR this walk reads; sim_pop_kernel writes their cells) or null
+    // popular columns split off (else null): the CSR this walk reads holds the other rows under their labels
+    // (rank - n_pop), so chunks, triangles and the diagonal are in label space and lab_row maps a label back
+    const int32_t *rank;
+    const int32_t *lab_row;
+    int32_t n_pop;
     unsigned long long *counter;
 };
 
@@ -85,12 +89,13 @@ __device__ __forceinline__ void stream_update(double *acc, int j, double ra, dou
 // No lookups, no gathers, no shared-memory read-modify-writes, and no item depends on another: a row of 78 k
 // entries is 10 items of 78 k pipelined steps.  Who computes which pair (the mirror passes copy the transposed
 // cell): a popular column's pairs with every other row belong to THAT row; two popular rows: to the one further
-// down the popular list (the shorter one); two other rows: the triangle rule of the column walk.
+// down the popular list (the shorter one); two other rows: the triangle rule of the column walk over their labels.
 
 struct PopArgs {
     const int32_t *rows;      // the shard's rows, longest first: the popular ones come first
     int64_t n_rows;
-    const int32_t *pop_idx;   // [n_left] index in the popular list or -1
+    const int32_t *rank;      // [n_left] position in the longest-first order: < n_pop is the index in the popular list
+    int32_t n_pop;
     const int32_t *pop_items; // [32 * n_blk] row id, -1 beyond the list
     int32_t n_blk, ld;        // blocks of 32 popular columns; row stride of the table
     const void *dense;
@@ -121,7 +126,7 @@ __device__ __forceinline__ void pop_item(const StreamArgs &a, const PopArgs &pa,
     const double nan_v = __longlong_as_double(0x7ff8000000000001ll);
     const int32_t i = pa.rows[item / pa.n_blk];
     const int b = (int)(item % pa.n_blk);
-    const int pi = pa.pop_idx[i];
+    const int pi = pa.rank[i] < pa.n_pop ? pa.rank[i] : -1;
     if (pi >= 0 && 32 * b > pi) return;                       // a popular row: only the columns above it in the list
     const int col = 32 * b + lane;
     const int32_t hcol = pa.pop_items[col];
@@ -257,6 +262,9 @@ __device__ __forceinline__ void pop_item(const StreamArgs &a, const PopArgs &pa,
 // column against the first version of this kernel (profiles/r01_stream_notes.md).
 // POP = 1 / 2: popular columns were split off (table of bytes / of doubles): the queue holds the dense items of the
 // shard's popular rows (the longest chains) first, then the column-walk items, then the dense items of the other rows.
+// The walk's columns are then the LABELS of the other rows, longest first (rs_knn::rank): chunk q covers labels
+// [q JC, (q + 1) JC), the triangle is taken in label space, so the lower one visits few chunks for the long rows,
+// and the epilogue scatters the chunk's cells to the rows lab_row[label].
 template <int SIM, bool SHRINK, int SYM, int JC, int POP>
 __global__ void __launch_bounds__(SW * 32, 4) sim_stream_kernel(StreamArgs a, PopArgs pa) {
     constexpr int NACC = SHRINK ? 4 : 3;
@@ -291,9 +299,10 @@ __global__ void __launch_bounds__(SW * 32, 4) sim_stream_kernel(StreamArgs a, Po
         // items are ordered longest row first, so the critical path starts early
         const int64_t q = (int64_t)item % Q;
         const int32_t i = a.row_order[(int64_t)item / Q];
+        const int32_t li = POP ? a.rank[i] - a.n_pop : i;   // i's own column
         const int j0 = (int)(q * JC);
-        if (SYM == 1 && j0 + JC <= i) continue;  // every column of the chunk is < i
-        if (SYM == 2 && j0 > i) continue;        // every column of the chunk is > i
+        if (SYM == 1 && j0 + JC <= li) continue;  // every column of the chunk is < li
+        if (SYM == 2 && j0 > li) continue;        // every column of the chunk is > li
 
         for (int x = lane; x < NACC * JC; x += 32) acc[x] = 0.0;
 
@@ -374,14 +383,11 @@ __global__ void __launch_bounds__(SW * 32, 4) sim_stream_kernel(StreamArgs a, Po
         }
         __syncwarp();
 
-        // epilogue: JC similarities of row i, coalesced
-        double *out = a.sims + (a.cyc_R > 1 ? rs_cyc_local(i, a.cyc_R) : (int64_t)(i - a.row_begin)) * a.ld_s + j0;
-        for (int j = lane; j < JC; j += 32) {
-            const int64_t col = (int64_t)j0 + j;
-            if (col >= a.n_left) break;
-            if (SYM == 1 && col < i) continue;                                    // mirror pass writes it
-            if (SYM == 2 && col > i) break;
-            if (a.pop_idx && a.pop_idx[col] >= 0) continue;                       // sim_pop_kernel writes it
+        // epilogue: the chunk's similarities of row i, coalesced (scattered by label with popular columns): the
+        // columns below n_cols and > li (SYM 1) or <= li (SYM 2).  The POP kernels test them per column, the others
+        // hoist the bounds: fewer spills in each (profiles/r03_walk_labels.md)
+        double *out = a.sims + (a.cyc_R > 1 ? rs_cyc_local(i, a.cyc_R) : (int64_t)(i - a.row_begin)) * a.ld_s + (POP ? 0 : j0);
+        auto emit = [&](int j, int64_t col) {
             double s;
             if (SIM == RS_SIM_MSD) s = 1.0 / (acc[j] / acc[JC + j] + 1.0);        // core/sim.go:43
             else s = acc[2 * JC + j] / (sqrt(acc[j]) * sqrt(acc[JC + j]));        // core/sim.go:24 / :80
@@ -389,8 +395,23 @@ __global__ void __launch_bounds__(SW * 32, 4) sim_stream_kernel(StreamArgs a, Po
                 const double cn = acc[3 * JC + j];
                 s = (cn - 1.0) / (cn - 1.0 + a.shrinkage) * s;
             }
-            if (col == (int64_t)i) s = nan_v;                                     // diagonal stays NaN
-            out[j] = s;
+            if (col == (int64_t)li) s = nan_v;                                    // diagonal stays NaN
+            out[POP ? a.lab_row[col] : j] = s;
+        };
+        if (POP) {
+            for (int j = lane; j < JC; j += 32) {
+                const int64_t col = (int64_t)j0 + j;
+                if (col >= a.n_left - a.n_pop) break;
+                if (SYM == 1 && col < li) continue;                                   // mirror pass writes it
+                if (SYM == 2 && col > li) break;
+                emit(j, col);
+            }
+        } else {
+            int j_end = a.n_left - j0;
+            if (SYM == 2 && li - j0 + 1 < j_end) j_end = li - j0 + 1;
+            if (j_end > JC) j_end = JC;
+            const int j_beg = SYM == 1 && li > j0 ? li - j0 : 0;
+            for (int j = j_beg + lane; j < j_end; j += 32) emit(j, j0 + j);
         }
         __syncwarp();
     }
@@ -629,12 +650,11 @@ __global__ void __launch_bounds__(HV_WARPS * 32, 1) sim_stream_heavy_kernel(Stre
     }
 }
 
-// does row r's own pass (column walk or sim_pop_kernel) compute cell (r, c)?  pr / pc: their popular indices or -1
-__device__ __forceinline__ bool pop_owns(int64_t r, int64_t c, int pr, int pc, int lower) {
-    if (pc >= 0 && pr < 0) return true;
-    if (pr >= 0 && pc < 0) return false;
-    if (pr >= 0) return pc < pr;
-    return lower ? c < r : c > r;
+// does row r's own pass (column walk or sim_pop_kernel) compute cell (r, c)?  rr / rc: the rows' ranks.  The row
+// further down the longest-first order owns the pair; with the upper triangle two walked rows swap.
+__device__ __forceinline__ bool pop_owns(int32_t rr, int32_t rc, int32_t n_pop, int lower) {
+    if (!lower && rr >= n_pop && rc >= n_pop) return rr < rc;
+    return rr > rc;
 }
 
 // Mirror the computed upper block-triangle into the lower one: the three similarities are
@@ -691,29 +711,18 @@ __global__ void mirror_kernel(MirrorArgs a) {
 }
 
 // The same two passes when popular columns were split off: which of the cells (r, c) / (c, r) was computed is
-// pop_owns(), cell by cell, so a pair of transposed tiles may exchange cells in both directions.
+// pop_owns() of the rows' ranks, cell by cell, so a pair of transposed tiles exchanges cells in both directions.
 __global__ void symmetrize_pop_kernel(double *__restrict__ s, int64_t ld, int32_t n, int lower,
-                                      const int32_t *__restrict__ pop_idx, const uint8_t *__restrict__ pop_blk) {
+                                      const int32_t *__restrict__ rank, int32_t n_pop) {
     __shared__ double ta[32][33], tb[32][33];
+    __shared__ int32_t rk_a[32], rk_b[32];
     const int64_t bi = blockIdx.y, bj = blockIdx.x;
     if (bj > bi) return;                                     // one block per unordered tile pair
-    if (!(pop_blk[bi] | pop_blk[bj])) {
-        // neither block of 32 rows holds a popular row (most of the matrix): the plain triangle rule of
-        // symmetrize_kernel, one tile read and one written
-        const int64_t di = lower ? bj : bi, dj = lower ? bi : bj;     // destination tile (rows di, cols dj)
-        const int64_t r0 = di * 32, c0 = dj * 32;
-        for (int y = threadIdx.y; y < 32; y += blockDim.y) {
-            const int64_t sr = c0 + y, sc = r0 + threadIdx.x;         // source = transposed position
-            ta[y][threadIdx.x] = (sr < n && sc < n) ? s[sr * ld + sc] : 0.0;
-        }
-        __syncthreads();
-        for (int y = threadIdx.y; y < 32; y += blockDim.y) {
-            const int64_t r = r0 + y, c = c0 + threadIdx.x;
-            if (r < n && c < n && (lower ? c > r : c < r)) s[r * ld + c] = ta[threadIdx.x][y];
-        }
-        return;
-    }
     const int64_t r0 = bi * 32, c0 = bj * 32;                // tile A = rows r0.., cols c0..; tile B = rows c0.., cols r0..
+    if (threadIdx.y == 0) {
+        rk_a[threadIdx.x] = r0 + threadIdx.x < n ? rank[r0 + threadIdx.x] : 0;
+        rk_b[threadIdx.x] = c0 + threadIdx.x < n ? rank[c0 + threadIdx.x] : 0;
+    }
     for (int y = threadIdx.y; y < 32; y += blockDim.y) {
         const int64_t ar = r0 + y, ac = c0 + threadIdx.x, br = c0 + y, bc = r0 + threadIdx.x;
         ta[y][threadIdx.x] = (ar < n && ac < n) ? s[ar * ld + ac] : 0.0;
@@ -722,14 +731,14 @@ __global__ void symmetrize_pop_kernel(double *__restrict__ s, int64_t ld, int32_
     __syncthreads();
     for (int y = threadIdx.y; y < 32; y += blockDim.y) {
         int64_t r = r0 + y, c = c0 + threadIdx.x;            // a cell of A takes B's transposed cell (c, r)
-        if (r < n && c < n && r != c && !pop_owns(r, c, pop_idx[r], pop_idx[c], lower)) s[r * ld + c] = tb[threadIdx.x][y];
+        if (r < n && c < n && r != c && !pop_owns(rk_a[y], rk_b[threadIdx.x], n_pop, lower)) s[r * ld + c] = tb[threadIdx.x][y];
         if (bi == bj) continue;
         r = c0 + y; c = r0 + threadIdx.x;                    // a cell of B takes A's transposed cell
-        if (r < n && c < n && !pop_owns(r, c, pop_idx[r], pop_idx[c], lower)) s[r * ld + c] = ta[threadIdx.x][y];
+        if (r < n && c < n && !pop_owns(rk_b[y], rk_a[threadIdx.x], n_pop, lower)) s[r * ld + c] = ta[threadIdx.x][y];
     }
 }
 
-__global__ void mirror_pop_kernel(MirrorArgs a, const int32_t *__restrict__ pop_idx) {
+__global__ void mirror_pop_kernel(MirrorArgs a, const int32_t *__restrict__ rank, int32_t n_pop) {
     __shared__ double tile[32][33];
     const int64_t bI = blockIdx.y;                           // own block (local index)
     const int64_t gI = bI * a.count + a.index, gJ = blockIdx.x;
@@ -739,7 +748,7 @@ __global__ void mirror_pop_kernel(MirrorArgs a, const int32_t *__restrict__ pop_
     for (int k = 0; k < 4; k++) {
         const int y = threadIdx.y + 8 * k;
         const int64_t r = gI * 32 + y, c = gJ * 32 + threadIdx.x;
-        need[k] = r < a.n && c < a.n && r != c && !pop_owns(r, c, pop_idx[r], pop_idx[c], a.lower);
+        need[k] = r < a.n && c < a.n && r != c && !pop_owns(rank[r], rank[c], n_pop, a.lower);
         any = any || need[k];
     }
     if (!__syncthreads_or(any)) return;                      // every cell of the tile is this shard's own work
@@ -769,7 +778,7 @@ static int32_t launch_stream_pop(rs_knn *h, const StreamArgs &s, const PopArgs &
 }
 template <int SIM, bool SHRINK, int SYM, int JC>
 static int32_t launch_stream_jc(rs_knn *h, const StreamArgs &s, const PopArgs &pa, int grid) {
-    if (SYM != 0 && s.pop_idx) {                              // popular columns exist only where a triangle is computed
+    if (SYM != 0 && s.rank) {                              // popular columns exist only where a triangle is computed
         if (h->pop_u8) return launch_stream_pop<SIM, SHRINK, SYM ? SYM : 1, JC, 1>(h, s, pa, grid);
         return launch_stream_pop<SIM, SHRINK, SYM ? SYM : 1, JC, 2>(h, s, pa, grid);
     }
@@ -844,9 +853,10 @@ int32_t rs_sim_stream_launch(rs_knn *h) {
             rs_set_error("popular columns were split off, but this Fit does not compute a triangle of the full matrix");
             return RS_ERR_INVALID;
         }
-        a.r_ptr = h->w_ptr; a.r_col = h->w_col; a.r_dev = h->w_dev; a.pop_idx = h->pop_idx;
+        a.r_ptr = h->w_ptr; a.r_col = h->w_col; a.r_dev = h->w_dev;
+        a.rank = h->rank; a.lab_row = h->lab_row; a.n_pop = h->n_pop;
         pa.rows = h->row_all; pa.n_rows = h->n_all_rows;
-        pa.pop_idx = h->pop_idx; pa.pop_items = h->pop_items;
+        pa.rank = h->rank; pa.n_pop = h->n_pop; pa.pop_items = h->pop_items;
         pa.n_blk = h->pop_ld / 32; pa.ld = h->pop_ld;
         pa.dense = h->pop_dense;
         pa.n_first = (h->n_all_rows - a.n_rows) * pa.n_blk;
@@ -901,7 +911,7 @@ int32_t rs_mirror_launch(rs_knn *h) {
     const int64_t own = (nblk - h->cyc_r + h->cyc_R - 1) / h->cyc_R;
     if (own <= 0) return RS_OK;
     dim3 grid((unsigned)nblk, (unsigned)own), block(32, 8);
-    if (h->n_pop > 0) mirror_pop_kernel<<<grid, block, 0, h->stream>>>(a, h->pop_idx);
+    if (h->n_pop > 0) mirror_pop_kernel<<<grid, block, 0, h->stream>>>(a, h->rank, h->n_pop);
     else mirror_kernel<<<grid, block, 0, h->stream>>>(a);
     h->prof.total_launches++;
     RS_CUDA(cudaGetLastError());
@@ -913,7 +923,7 @@ int32_t rs_symmetrize_launch(rs_knn *h) {
     if (!(h->row_begin == 0 && h->row_end == h->n_left)) return RS_OK;
     const unsigned t = (unsigned)((h->n_left + 31) / 32);
     dim3 grid(t, t), block(32, 8);
-    if (h->n_pop > 0) symmetrize_pop_kernel<<<grid, block, 0, h->stream>>>(h->sims, h->ld_s, h->n_left, h->stream_lower ? 1 : 0, h->pop_idx, h->pop_blk);
+    if (h->n_pop > 0) symmetrize_pop_kernel<<<grid, block, 0, h->stream>>>(h->sims, h->ld_s, h->n_left, h->stream_lower ? 1 : 0, h->rank, h->n_pop);
     else symmetrize_kernel<<<grid, block, 0, h->stream>>>(h->sims, h->ld_s, h->n_left, h->stream_lower ? 1 : 0);
     h->prof.total_launches++;
     RS_CUDA(cudaGetLastError());
