@@ -228,6 +228,30 @@ int32_t rs_baseline_als(int32_t device, const int32_t *users, const int32_t *ite
 int32_t rs_knn_topk_union_device(int32_t n_lists, int64_t n_rows, int32_t k, const int32_t *d_idx_all,
                                  const double *d_sim_all, int32_t *d_idx, double *d_sim, void *cuda_stream);
 
+/* TOP-N RECOMMENDATION.  A query is an inner id of one side; its TARGETS are all ids of the other side:
+ *   RS_SIDE_RIGHT query q: score(t) = Predict(left = t, right = q) — item-based mode, the user is the right side;
+ *   RS_SIDE_LEFT  query q: score(t) = Predict(left = q, right = t) — user-based mode.
+ * Every score is bit-identical to what rs_knn_predict_batch returns for the same pair with the current k / mink
+ * (rs_knn_set_k applies); NaN and +-Inf scores (sum of weights <= 0) are reproduced as they are.  Targets the query
+ * rated (its row of the left or right ratings) are excluded: their score is NaN.  A query of -1 (newID) scores
+ * GlobalMean everywhere.  The host variants refuse ids outside [-1, n_side) with RS_ERR_INVALID; the _device
+ * variants treat them as -1.
+ * Ranking: the top n_top targets by (score desc, target inner id asc) under the order-preserving key of the
+ * neighbour lists; NaN is never listed, +Inf ranks first and -Inf last, +-0 tie by id and -0.0 is reported as
+ * -0.0; unused slots are id -1 / score NaN.  A -1 query therefore lists the first n_top target ids.
+ * Limits: 1 <= n_top <= 512, k <= 256, n >= 0.  Only RS_STORE_MATRIX handles that hold all rows: RS_STORE_TOPK is
+ * refused like Predict refuses it, row shards (row_begin/row_end or shard_count >= 2) and RS_SIM_SLOPE_ONE with
+ * RS_ERR_UNSUPPORTED.  Queries are scored in batches into a device slab of full score rows (~256 MiB). */
+enum rs_side { RS_SIDE_LEFT = 0, RS_SIDE_RIGHT = 1 };
+/* Full score rows: out[n][n_targets] (n_targets = n_right for left queries, n_left for right queries). */
+int32_t rs_knn_score_all(rs_knn *h, int32_t side, const int32_t *queries, int64_t n, double *out);
+int32_t rs_knn_score_all_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n, double *d_out);
+/* The n_top best targets of each query: ids[n][n_top] (inner ids), scores[n][n_top]. */
+int32_t rs_knn_recommend(rs_knn *h, int32_t side, const int32_t *queries, int64_t n, int32_t n_top, int32_t *ids,
+                         double *scores);
+int32_t rs_knn_recommend_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n, int32_t n_top,
+                                int32_t *d_ids, double *d_scores);
+
 /* Parameters["k"] / ["mink"] are read at Predict time by the reference (core/knn.go:80-81): change
  * them on a fitted handle without refitting.  The predict kernel supports k <= 256. */
 int32_t rs_knn_set_k(rs_knn *h, int32_t k, int32_t min_k);

@@ -42,6 +42,7 @@ RS_KNN_TYPE = {"basic": 0, "centered": 1, "zscore": 2, "baseline": 3}
 RS_PEARSON_MODE = {"exact": 0, "sums": 1}
 RS_SIM_PATH = {"auto": 0, "tensor": 1, "stream": 2}
 RS_STORE = {"matrix": 0, "topk": 1}
+RS_SIDE = {"left": 0, "right": 1}
 
 basic, centered, zScore, baseline = "basic", "centered", "zscore", "baseline"  # core/knn.go:10-15
 
@@ -68,7 +69,7 @@ ABI_SYMBOLS = [
     "rs_knn_profile_reset", "rs_knn_synchronize", "rs_knn_trim_cache", "rs_baseline_als",
     "rs_knn_topk_union_device", "rs_knn_set_k", "rs_knn_peer_export", "rs_knn_peer_import",
     "rs_knn_peer_import_local", "rs_knn_mirror", "rs_knn_predict_batch_sharded_device", "rs_knn_host_alloc",
-    "rs_knn_host_free",
+    "rs_knn_host_free", "rs_knn_score_all", "rs_knn_score_all_device", "rs_knn_recommend", "rs_knn_recommend_device",
 ]
 
 _knn_lib = None
@@ -119,6 +120,10 @@ def knn_lib():
     L.rs_knn_predict_batch_sharded_device.argtypes = [vp, vp, vp, i64, vp]
     L.rs_knn_host_alloc.argtypes = [C.c_size_t, C.POINTER(vp)]
     L.rs_knn_host_free.argtypes = [vp]
+    L.rs_knn_score_all.argtypes = [vp, i32, vp, i64, vp]
+    L.rs_knn_score_all_device.argtypes = [vp, i32, vp, i64, vp]
+    L.rs_knn_recommend.argtypes = [vp, i32, vp, i64, i32, vp, vp]
+    L.rs_knn_recommend_device.argtypes = [vp, i32, vp, i64, i32, vp, vp]
     _knn_lib = L
     return L
 
@@ -586,7 +591,7 @@ class _Handle:
         self.params = p
         self.h = C.c_void_p()
         _check(L.rs_knn_create(C.byref(p), C.byref(self.h)))
-        self.n_left = 0
+        self.n_left = self.n_right = 0
         self.rows = (0, 0)
 
     def close(self):
@@ -610,10 +615,10 @@ class _Handle:
         _check(knn_lib().rs_knn_fit(self.h, _ptr(left), _ptr(right), _ptr(rating), len(rating), n_left, n_right,
                                     global_mean, None if lb is None else _ptr(lb),
                                     None if rb is None else _ptr(rb), global_bias))
-        self._after_fit(n_left)
+        self._after_fit(n_left, n_right)
 
-    def _after_fit(self, n_left):
-        self.n_left = n_left
+    def _after_fit(self, n_left, n_right):
+        self.n_left, self.n_right = n_left, n_right
         rb, re = self.params.row_begin, self.params.row_end
         self.rows = (0, n_left) if (rb == 0 and re == 0) else (rb, re)
 
@@ -622,7 +627,7 @@ class _Handle:
         """Arguments are raw device pointers (ints), e.g. torch tensors' data_ptr()."""
         _check(knn_lib().rs_knn_fit_device(self.h, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean,
                                            d_left_bias or None, d_right_bias or None, global_bias))
-        self._after_fit(n_left)
+        self._after_fit(n_left, n_right)
 
     def predict_batch(self, left, right):
         left = np.ascontiguousarray(left, dtype=np.int32)
@@ -688,6 +693,34 @@ class _Handle:
 
     def set_k(self, k, min_k):
         _check(knn_lib().rs_knn_set_k(self.h, int(k), int(min_k)))
+
+    def _n_targets(self, side):
+        return self.n_left if side == RS_SIDE["right"] else self.n_right
+
+    def score_all(self, side, queries):
+        """Full score rows [len(queries)][n_targets] of inner-id queries of `side` ("left" / "right"); rated
+        targets NaN (include/rs_knn.h rs_knn_score_all)."""
+        side = RS_SIDE[side]
+        q = np.ascontiguousarray(queries, dtype=np.int32)
+        out = np.empty((len(q), self._n_targets(side)), dtype=np.float64)
+        _check(knn_lib().rs_knn_score_all(self.h, side, _ptr(q), len(q), _ptr(out)))
+        return out
+
+    def score_all_device(self, side, d_queries, n, d_out):
+        _check(knn_lib().rs_knn_score_all_device(self.h, RS_SIDE[side], d_queries, n, d_out))
+
+    def recommend(self, side, queries, n_top):
+        """(ids[len(queries)][n_top], scores[len(queries)][n_top]): the n_top best unrated targets of each
+        inner-id query (include/rs_knn.h rs_knn_recommend)."""
+        side = RS_SIDE[side]
+        q = np.ascontiguousarray(queries, dtype=np.int32)
+        ids = np.empty((len(q), n_top), dtype=np.int32)
+        scores = np.empty((len(q), n_top), dtype=np.float64)
+        _check(knn_lib().rs_knn_recommend(self.h, side, _ptr(q), len(q), int(n_top), _ptr(ids), _ptr(scores)))
+        return ids, scores
+
+    def recommend_device(self, side, d_queries, n, n_top, d_ids, d_scores):
+        _check(knn_lib().rs_knn_recommend_device(self.h, RS_SIDE[side], d_queries, n, int(n_top), d_ids, d_scores))
 
     # ---- cyclic row shards (RS_STORE_MATRIX, shard_count >= 2): the exchange step ----
     def peer_export(self):
@@ -884,11 +917,7 @@ class KNN(Base):
         iu = self.Data.convert_users(userIDs, out=pinned_empty(len(userIDs), np.int32) if big else None)
         ii = self.Data.convert_items(itemIDs, out=pinned_empty(len(itemIDs), np.int32) if big else None)
         left, right = (iu, ii) if self._userBased else (ii, iu)
-        # core/knn.go:80-81 reads k / mink in Predict: SetParams after Fit takes effect here
-        k, mink = self.Params.GetInt("k", 40), self.Params.GetInt("mink", 1)
-        if (k, mink) != self._kk:
-            self._h.set_k(k, mink)
-            self._kk = (k, mink)
+        self._sync_k()
         return self._h.predict_batch(left, right)
 
     def Predict(self, userID, itemID):
@@ -906,6 +935,34 @@ class KNN(Base):
 
     def TopK(self, k):
         return self._h.topk(k)
+
+    def _sync_k(self):
+        # core/knn.go:80-81 reads k / mink in Predict: SetParams after Fit takes effect here
+        k, mink = self.Params.GetInt("k", 40), self.Params.GetInt("mink", 1)
+        if (k, mink) != self._kk:
+            self._h.set_k(k, mink)
+            self._kk = (k, mink)
+
+    def _user_queries(self, userIDs):
+        self._sync_k()
+        side = "left" if self._userBased else "right"
+        return side, self.Data.convert_users(np.asarray(userIDs, dtype=np.int64))
+
+    def ScoreAll(self, userIDs):
+        """The score of every item for each user, [len(userIDs)][ItemCount] in inner item order: Predict(user, item)
+        bit for bit, NaN for the items the user rated (an unknown user scores GlobalMean everywhere)."""
+        side, q = self._user_queries(userIDs)
+        return self._h.score_all(side, q)
+
+    def Recommend(self, userIDs, n):
+        """(items[len][n], scores[len][n]): the n best items each user has not rated, by (score desc, inner item id
+        asc), as raw item ids; unused slots are newID (-1) with score NaN."""
+        side, q = self._user_queries(userIDs)
+        ids, scores = self._h.recommend(side, q, n)
+        raw = np.empty(self.Data.ItemCount, dtype=np.int64)    # inner -> raw: the order of first appearance
+        raw[self.Data.innerItems] = self.Data.Items
+        items = np.where(ids >= 0, raw[np.maximum(ids, 0)], newID)
+        return items, scores
 
     def Profile(self):
         return self._h.profile()

@@ -165,7 +165,7 @@ int32_t init_handle(rs_knn *h) {
 extern "C" {
 
 const char *rs_last_error(void) { return g_err; }
-int32_t rs_knn_abi_version(void) { return 1; }
+int32_t rs_knn_abi_version(void) { return 2; }
 
 int32_t rs_knn_device_count(void) {
     int n = 0;
@@ -692,6 +692,125 @@ int32_t rs_knn_predict_neighbors(rs_knn *h, int32_t left, int32_t right, int32_t
         RS_CUDA(cudaMemcpy(sims, dsims, (size_t)cnt * 8, cudaMemcpyDeviceToHost));
     }
     *n_out = cnt;
+    return RS_OK;
+}
+
+// What every recommend entry point checks: the handle holds the whole matrix, the query side exists, k fits.
+static int32_t require_recommend(rs_knn *h, const char *who, int32_t side, int64_t n) {
+    if (!h->fitted) {
+        rs_set_error("%s: Fit has not been called", who);
+        return RS_ERR_INVALID;
+    }
+    if (h->p.store != RS_STORE_MATRIX) return require_matrix(h, who);
+    if (h->cyc_R > 1 || h->p.shard_count > 1 || h->row_begin != 0 || h->row_end != h->n_left) {
+        rs_set_error("%s needs a handle that holds every row (no row_begin/row_end shard, shard_count <= 1)", who);
+        return RS_ERR_UNSUPPORTED;
+    }
+    if (h->p.sim == RS_SIM_SLOPE_ONE) {
+        rs_set_error("%s: Slope One is not supported", who);
+        return RS_ERR_UNSUPPORTED;
+    }
+    if (side != RS_SIDE_LEFT && side != RS_SIDE_RIGHT) {
+        rs_set_error("%s: side must be RS_SIDE_LEFT or RS_SIDE_RIGHT (got %d)", who, side);
+        return RS_ERR_INVALID;
+    }
+    if (h->p.k > 256) {
+        rs_set_error("%s: k=%d exceeds the 256 neighbours the predict kernel supports", who, h->p.k);
+        return RS_ERR_UNSUPPORTED;
+    }
+    if (n < 0 || n >= (1ll << 31)) {
+        rs_set_error("%s: n=%lld outside [0, 2^31)", who, (long long)n);
+        return RS_ERR_INVALID;
+    }
+    return RS_OK;
+}
+
+static int32_t check_n_top(const char *who, int32_t n_top) {
+    if (n_top < 1 || n_top > 512) {
+        rs_set_error("%s: n_top=%d outside [1, 512]", who, n_top);
+        return RS_ERR_INVALID;
+    }
+    return RS_OK;
+}
+
+// host variants: ids outside [-1, n_side) are refused
+static int32_t check_queries(rs_knn *h, const char *who, int32_t side, const int32_t *q, int64_t n) {
+    const int32_t n_side = side == RS_SIDE_RIGHT ? h->n_right : h->n_left;
+    for (int64_t i = 0; i < n; i++) {
+        if (q[i] < -1 || q[i] >= n_side) {
+            rs_set_error("%s: query %lld = %d outside [-1, %d)", who, (long long)i, q[i], n_side);
+            return RS_ERR_INVALID;
+        }
+    }
+    return RS_OK;
+}
+
+static int64_t n_targets_of(const rs_knn *h, int32_t side) { return side == RS_SIDE_RIGHT ? h->n_left : h->n_right; }
+
+int32_t rs_knn_score_all_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n, double *d_out) {
+    RS_ENTER(h);
+    RS_TRY(require_recommend(h, "rs_knn_score_all", side, n));
+    if (n == 0) return RS_OK;
+    if (!d_queries || !d_out) {
+        rs_set_error("rs_knn_score_all: null argument");
+        return RS_ERR_INVALID;
+    }
+    return rs_score_all_launch(h, side, d_queries, n, d_out);
+}
+
+int32_t rs_knn_score_all(rs_knn *h, int32_t side, const int32_t *queries, int64_t n, double *out) {
+    RS_ENTER(h);
+    RS_TRY(require_recommend(h, "rs_knn_score_all", side, n));
+    if (n == 0) return RS_OK;
+    if (!queries || !out) {
+        rs_set_error("rs_knn_score_all: null argument");
+        return RS_ERR_INVALID;
+    }
+    RS_TRY(check_queries(h, "rs_knn_score_all", side, queries, n));
+    const size_t bytes = (size_t)n * n_targets_of(h, side) * 8;
+    void *dq, *dout;
+    RS_TRY(rs_scratch_get(h, 20, (size_t)n * 4, &dq));
+    RS_TRY(rs_scratch_get(h, 21, bytes, &dout));
+    RS_CUDA(cudaMemcpyAsync(dq, queries, (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
+    RS_TRY(rs_score_all_launch(h, side, (const int32_t *)dq, n, (double *)dout));
+    RS_CUDA(cudaMemcpyAsync(out, dout, bytes, cudaMemcpyDeviceToHost, h->stream));
+    RS_CUDA(cudaStreamSynchronize(h->stream));
+    return RS_OK;
+}
+
+int32_t rs_knn_recommend_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n, int32_t n_top,
+                                int32_t *d_ids, double *d_scores) {
+    RS_ENTER(h);
+    RS_TRY(require_recommend(h, "rs_knn_recommend", side, n));
+    RS_TRY(check_n_top("rs_knn_recommend", n_top));
+    if (n == 0) return RS_OK;
+    if (!d_queries || !d_ids || !d_scores) {
+        rs_set_error("rs_knn_recommend: null argument");
+        return RS_ERR_INVALID;
+    }
+    return rs_recommend_launch(h, side, d_queries, n, n_top, d_ids, d_scores);
+}
+
+int32_t rs_knn_recommend(rs_knn *h, int32_t side, const int32_t *queries, int64_t n, int32_t n_top, int32_t *ids,
+                         double *scores) {
+    RS_ENTER(h);
+    RS_TRY(require_recommend(h, "rs_knn_recommend", side, n));
+    RS_TRY(check_n_top("rs_knn_recommend", n_top));
+    if (n == 0) return RS_OK;
+    if (!queries || !ids || !scores) {
+        rs_set_error("rs_knn_recommend: null argument");
+        return RS_ERR_INVALID;
+    }
+    RS_TRY(check_queries(h, "rs_knn_recommend", side, queries, n));
+    void *dq, *di, *ds;
+    RS_TRY(rs_scratch_get(h, 20, (size_t)n * 4, &dq));
+    RS_TRY(rs_scratch_get(h, 21, (size_t)n * n_top * 4, &di));
+    RS_TRY(rs_scratch_get(h, 22, (size_t)n * n_top * 8, &ds));
+    RS_CUDA(cudaMemcpyAsync(dq, queries, (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
+    RS_TRY(rs_recommend_launch(h, side, (const int32_t *)dq, n, n_top, (int32_t *)di, (double *)ds));
+    RS_CUDA(cudaMemcpyAsync(ids, di, (size_t)n * n_top * 4, cudaMemcpyDeviceToHost, h->stream));
+    RS_CUDA(cudaMemcpyAsync(scores, ds, (size_t)n * n_top * 8, cudaMemcpyDeviceToHost, h->stream));
+    RS_CUDA(cudaStreamSynchronize(h->stream));
     return RS_OK;
 }
 

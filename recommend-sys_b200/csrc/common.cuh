@@ -236,6 +236,13 @@ int32_t rs_slope_predict_launch(rs_knn *h, const int32_t *d_left, const int32_t 
 int32_t rs_topk_slab_launch(rs_knn *h, int64_t g0, int32_t m, double *tbuf, int64_t ld_t, int32_t k);
 int32_t rs_topk_compact_launch(rs_knn *h, int32_t k, int32_t *d_overflow, int rerun);
 int32_t rs_topk_mask_launch(rs_knn *h, int32_t k, int restore);
+int32_t rs_topk_rows_launch(rs_knn *h, const double *src, int64_t ld, int32_t n, int64_t rows, int32_t k, int32_t *d_idx,
+                            double *d_sim);
+
+// ---- recommend.cu ----
+int32_t rs_score_all_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, double *d_out);
+int32_t rs_recommend_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, int32_t n_top, int32_t *d_ids,
+                            double *d_scores);
 
 // order-preserving map double -> uint64 (larger similarity = larger key); -0.0 folded to +0.0
 __host__ __device__ inline uint64_t rs_sim_key(double s) {

@@ -197,6 +197,24 @@ func (d *deviceKNN) predictBatch(left, right []int32) []float64 {
 	return out
 }
 
+// Query sides of rs_knn_recommend (enum rs_side).
+const (
+	sideLeft  = 0
+	sideRight = 1
+)
+
+// recommend: ids / scores are [len(queries)][nTop], row-major.
+func (d *deviceKNN) recommend(side int, queries []int32, nTop int) ([]int32, []float64) {
+	ids := make([]int32, len(queries)*nTop)
+	scores := make([]float64, len(queries)*nTop)
+	if len(queries) == 0 {
+		return ids, scores
+	}
+	check(C.rs_knn_recommend(d.h, C.int32_t(side), i32(queries), C.int64_t(len(queries)), C.int32_t(nTop), i32(ids),
+		f64(scores)))
+	return ids, scores
+}
+
 // pinnedInt32 / pinnedFloat64: page-locked host memory of the library's per-process cache (rs_knn_host_alloc) viewed
 // as a Go slice, for callers that stage large batches themselves: copies from and to such memory run at full PCIe
 // speed.  The memory is C memory (no Go pointers in it); release returns the block to the cache.

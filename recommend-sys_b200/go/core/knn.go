@@ -134,12 +134,49 @@ func (K *KNN) PredictBatch(userIDs, itemIDs []int) []float64 {
 			left[i], right[i] = it, u
 		}
 	}
-	// core/knn.go:80-81 reads k / mink in Predict: SetParams after Fit takes effect here
+	K.syncK()
+	return K.dev.predictBatch(left, right)
+}
+
+// syncK: core/knn.go:80-81 reads k / mink in Predict, so SetParams after Fit takes effect at the next call.
+func (K *KNN) syncK() {
 	if kk := [2]int{K.Params.GetInt("k", 40), K.Params.GetInt("mink", 1)}; kk != K.kk {
 		K.dev.setK(kk[0], kk[1])
 		K.kk = kk
 	}
-	return K.dev.predictBatch(left, right)
+}
+
+// Recommend returns, for each user, the n best items the user has not rated: items[u][x] are raw item ids ranked
+// by (score desc, inner item id asc), scores[u][x] the scores, which are Predict(user, item) bit for bit.
+// Unused slots are newID (-1) with score NaN; an unknown user scores GlobalMean everywhere.
+func (K *KNN) Recommend(userIDs []int, n int) ([][]int, [][]float64) {
+	q := make([]int32, len(userIDs))
+	for i, u := range userIDs {
+		q[i] = int32(K.Data.ConvertUserID(u))
+	}
+	K.syncK()
+	side := sideLeft // user-based: the users are the left side
+	if !K.userBased {
+		side = sideRight
+	}
+	ids, sc := K.dev.recommend(side, q, n)
+	raw := make([]int, K.Data.ItemCount) // inner -> raw: the order of first appearance
+	for _, it := range K.Data.Items {
+		raw[K.Data.ConvertItemID(it)] = it
+	}
+	items := make([][]int, len(userIDs))
+	scores := make([][]float64, len(userIDs))
+	for i := range userIDs {
+		items[i] = make([]int, n)
+		for x := 0; x < n; x++ {
+			items[i][x] = newID
+			if id := ids[i*n+x]; id >= 0 {
+				items[i][x] = raw[id]
+			}
+		}
+		scores[i] = sc[i*n : (i+1)*n]
+	}
+	return items, scores
 }
 
 // Predict replaces core/knn.go:75-141 (a one-element batch).

@@ -239,14 +239,28 @@ struct KNN : Estimator {
             l[j] = userBased_ ? iu : ii;
             r[j] = userBased_ ? ii : iu;
         }
-        // core/knn.go:80-81 reads k / mink in Predict: SetParams after Fit takes effect here
-        const int k = Params.GetInt("k", 40), minK = Params.GetInt("mink", 1);
-        if (k != k_ || minK != minK_) { rs_check(rs_knn_set_k(h_, k, minK)); k_ = k; minK_ = minK; }
+        SyncK();
         std::vector<double> out(users.size());
         rs_check(rs_knn_predict_batch(h_, l.data(), r.data(), (int64_t)l.size(), out.data()));
         return out;
     }
     double Predict(int64_t u, int64_t i) override { return PredictBatch({u}, {i})[0]; }  // core/knn.go:75-141
+
+    // The n best items each user has not rated, as raw item ids ranked by (score desc, inner item id asc) with their
+    // scores (Predict(user, item) bit for bit): [users.size()][n] row-major, unused slots newID with score NaN.
+    void Recommend(const std::vector<int64_t> &users, int n, std::vector<int64_t> &items, std::vector<double> &scores) {
+        std::vector<int32_t> q(users.size()), ids(users.size() * (size_t)n);
+        for (size_t j = 0; j < users.size(); j++) q[j] = Data->ConvertUserID(users[j]);
+        SyncK();
+        scores.assign(ids.size(), 0.0);
+        if (!users.empty())
+            rs_check(rs_knn_recommend(h_, userBased_ ? RS_SIDE_LEFT : RS_SIDE_RIGHT, q.data(), (int64_t)q.size(), n,
+                                      ids.data(), scores.data()));
+        std::vector<int64_t> raw(Data->ItemCount);          // inner -> raw: the order of first appearance
+        for (size_t j = 0; j < Data->Length(); j++) raw[Data->innerItems[j]] = Data->Items[j];
+        items.resize(ids.size());
+        for (size_t j = 0; j < ids.size(); j++) items[j] = ids[j] >= 0 ? raw[ids[j]] : newID;
+    }
 
     std::vector<double> SimsRows(int64_t row0, int64_t nrows) {  // backs KNN.Sims (core/knn.go:21)
         std::vector<double> out((size_t)nrows * nLeft_);
@@ -258,6 +272,12 @@ struct KNN : Estimator {
     std::unique_ptr<Estimator> Clone() const override { return std::make_unique<KNN>(KNNType, Params); }
 
   private:
+    // core/knn.go:80-81 reads k / mink in Predict: SetParams after Fit takes effect at the next call
+    void SyncK() {
+        const int k = Params.GetInt("k", 40), minK = Params.GetInt("mink", 1);
+        if (k != k_ || minK != minK_) { rs_check(rs_knn_set_k(h_, k, minK)); k_ = k; minK_ = minK; }
+    }
+
     rs_knn *h_ = nullptr;
     int k_ = 40, minK_ = 1;   // what the handle currently holds
     bool userBased_ = true;
