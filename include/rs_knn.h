@@ -251,6 +251,25 @@ int32_t rs_knn_recommend(rs_knn *h, int32_t side, const int32_t *queries, int64_
                          double *scores);
 int32_t rs_knn_recommend_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n, int32_t n_top,
                                 int32_t *d_ids, double *d_scores);
+/* TOP-N RECOMMENDATION ON ROW SHARDS (cyclic shards after rs_knn_mirror, or row_begin/row_end shards): every shard
+ * gets the SAME queries and answers the part it owns ("owns": the cyclic block rule, resp. [row_begin, row_end)):
+ *   RS_SIDE_RIGHT query q: the shard scores and lists only the targets (left rows) it owns; list ids are global inner
+ *     ids.  A -1 query (an id out of range) scores GlobalMean on the shard's own targets.
+ *   RS_SIDE_LEFT  query q: the owner of row q produces the whole list / row; every other shard an empty list (ids -1,
+ *     scores NaN) or a +0.0 row.  A -1 query is answered by the shard that owns left row 0 only (cyclic shard 0, the
+ *     contiguous shard with row_begin == 0), so that it is not listed twice.
+ * rs_knn_recommend_sharded_device writes each shard's PARTIAL lists ids[n][n_top], scores[n][n_top]: all-gather them
+ * and unite them with rs_knn_topk_union_device — in groups of at most 2048 / n_top lists, and the results again when
+ * there are more shards; every target is in at most one partial list.  rs_knn_score_all_sharded_device writes rows
+ * out[n][n_targets] in which the cells the shard does not answer are +0.0 (all bits zero) and its own rated targets
+ * NaN: an integer SUM all-reduce of the 64-bit patterns over the shards assembles rs_knn_score_all.  Either way the
+ * result is bit-identical to rs_knn_recommend / rs_knn_score_all on one handle of all rows at the same k / mink.
+ * Refused: a handle that is not a row shard or a cyclic shard before rs_knn_mirror (RS_ERR_INVALID), RS_STORE_TOPK,
+ * RS_SIM_SLOPE_ONE, and the limits of rs_knn_recommend.  The plain entry points keep refusing row shards. */
+int32_t rs_knn_recommend_sharded_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n,
+                                        int32_t n_top, int32_t *d_ids, double *d_scores);
+int32_t rs_knn_score_all_sharded_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n,
+                                        double *d_out);
 
 /* Parameters["k"] / ["mink"] are read at Predict time by the reference (core/knn.go:80-81): change
  * them on a fitted handle without refitting.  The predict kernel supports k <= 256. */

@@ -70,6 +70,7 @@ ABI_SYMBOLS = [
     "rs_knn_topk_union_device", "rs_knn_set_k", "rs_knn_peer_export", "rs_knn_peer_import",
     "rs_knn_peer_import_local", "rs_knn_mirror", "rs_knn_predict_batch_sharded_device", "rs_knn_host_alloc",
     "rs_knn_host_free", "rs_knn_score_all", "rs_knn_score_all_device", "rs_knn_recommend", "rs_knn_recommend_device",
+    "rs_knn_score_all_sharded_device", "rs_knn_recommend_sharded_device",
 ]
 
 _knn_lib = None
@@ -124,6 +125,8 @@ def knn_lib():
     L.rs_knn_score_all_device.argtypes = [vp, i32, vp, i64, vp]
     L.rs_knn_recommend.argtypes = [vp, i32, vp, i64, i32, vp, vp]
     L.rs_knn_recommend_device.argtypes = [vp, i32, vp, i64, i32, vp, vp]
+    L.rs_knn_score_all_sharded_device.argtypes = [vp, i32, vp, i64, vp]
+    L.rs_knn_recommend_sharded_device.argtypes = [vp, i32, vp, i64, i32, vp, vp]
     _knn_lib = L
     return L
 
@@ -722,6 +725,17 @@ class _Handle:
     def recommend_device(self, side, d_queries, n, n_top, d_ids, d_scores):
         _check(knn_lib().rs_knn_recommend_device(self.h, RS_SIDE[side], d_queries, n, int(n_top), d_ids, d_scores))
 
+    def score_all_sharded_device(self, side, d_queries, n, d_out):
+        """Row shards: the score rows of this shard, +0.0 in the cells it does not answer (include/rs_knn.h
+        rs_knn_score_all_sharded_device); an integer sum of the shards' bit patterns is rs_knn_score_all."""
+        _check(knn_lib().rs_knn_score_all_sharded_device(self.h, RS_SIDE[side], d_queries, n, d_out))
+
+    def recommend_sharded_device(self, side, d_queries, n, n_top, d_ids, d_scores):
+        """Row shards: the partial top-n_top lists of this shard, to be united across the shards
+        (shard.union_recommend_device)."""
+        _check(knn_lib().rs_knn_recommend_sharded_device(self.h, RS_SIDE[side], d_queries, n, int(n_top), d_ids,
+                                                         d_scores))
+
     # ---- cyclic row shards (RS_STORE_MATRIX, shard_count >= 2): the exchange step ----
     def peer_export(self):
         """(64-byte CUDA IPC handle, byte offset) of this shard's matrix."""
@@ -959,10 +973,13 @@ class KNN(Base):
         asc), as raw item ids; unused slots are newID (-1) with score NaN."""
         side, q = self._user_queries(userIDs)
         ids, scores = self._h.recommend(side, q, n)
+        return self._raw_items(ids), scores
+
+    def _raw_items(self, ids):
+        """Inner item ids -> raw item ids; -1 (an unused slot) -> newID."""
         raw = np.empty(self.Data.ItemCount, dtype=np.int64)    # inner -> raw: the order of first appearance
         raw[self.Data.innerItems] = self.Data.Items
-        items = np.where(ids >= 0, raw[np.maximum(ids, 0)], newID)
-        return items, scores
+        return np.where(ids >= 0, raw[np.maximum(ids, 0)], newID)
 
     def Profile(self):
         return self._h.profile()

@@ -165,7 +165,7 @@ int32_t init_handle(rs_knn *h) {
 extern "C" {
 
 const char *rs_last_error(void) { return g_err; }
-int32_t rs_knn_abi_version(void) { return 2; }
+int32_t rs_knn_abi_version(void) { return 3; }
 
 int32_t rs_knn_device_count(void) {
     int n = 0;
@@ -695,17 +695,24 @@ int32_t rs_knn_predict_neighbors(rs_knn *h, int32_t left, int32_t right, int32_t
     return RS_OK;
 }
 
-// What every recommend entry point checks: the handle holds the whole matrix, the query side exists, k fits.
-static int32_t require_recommend(rs_knn *h, const char *who, int32_t side, int64_t n) {
+// What every recommend entry point checks: the handle holds the whole matrix (the _sharded entry points: a row
+// shard, mirrored if cyclic), the query side exists, k fits.
+static int32_t require_recommend(rs_knn *h, const char *who, int32_t side, int64_t n, bool sharded = false) {
     if (!h->fitted) {
         rs_set_error("%s: Fit has not been called", who);
         return RS_ERR_INVALID;
     }
     if (h->p.store != RS_STORE_MATRIX) return require_matrix(h, who);
-    if (h->cyc_R > 1 || h->p.shard_count > 1 || h->row_begin != 0 || h->row_end != h->n_left) {
+    const bool row_shard = h->cyc_R > 1 || h->p.shard_count > 1 || h->row_begin != 0 || h->row_end != h->n_left;
+    if (!sharded && row_shard) {
         rs_set_error("%s needs a handle that holds every row (no row_begin/row_end shard, shard_count <= 1)", who);
         return RS_ERR_UNSUPPORTED;
     }
+    if (sharded && !row_shard) {
+        rs_set_error("%s: the handle holds every row, not a row shard (use the plain entry point)", who);
+        return RS_ERR_INVALID;
+    }
+    if (sharded) RS_TRY(require_matrix(h, who));
     if (h->p.sim == RS_SIM_SLOPE_ONE) {
         rs_set_error("%s: Slope One is not supported", who);
         return RS_ERR_UNSUPPORTED;
@@ -812,6 +819,31 @@ int32_t rs_knn_recommend(rs_knn *h, int32_t side, const int32_t *queries, int64_
     RS_CUDA(cudaMemcpyAsync(scores, ds, (size_t)n * n_top * 8, cudaMemcpyDeviceToHost, h->stream));
     RS_CUDA(cudaStreamSynchronize(h->stream));
     return RS_OK;
+}
+
+int32_t rs_knn_score_all_sharded_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n,
+                                        double *d_out) {
+    RS_ENTER(h);
+    RS_TRY(require_recommend(h, "rs_knn_score_all_sharded", side, n, true));
+    if (n == 0) return RS_OK;
+    if (!d_queries || !d_out) {
+        rs_set_error("rs_knn_score_all_sharded: null argument");
+        return RS_ERR_INVALID;
+    }
+    return rs_score_all_sharded_launch(h, side, d_queries, n, d_out);
+}
+
+int32_t rs_knn_recommend_sharded_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n, int32_t n_top,
+                                        int32_t *d_ids, double *d_scores) {
+    RS_ENTER(h);
+    RS_TRY(require_recommend(h, "rs_knn_recommend_sharded", side, n, true));
+    RS_TRY(check_n_top("rs_knn_recommend_sharded", n_top));
+    if (n == 0) return RS_OK;
+    if (!d_queries || !d_ids || !d_scores) {
+        rs_set_error("rs_knn_recommend_sharded: null argument");
+        return RS_ERR_INVALID;
+    }
+    return rs_recommend_sharded_launch(h, side, d_queries, n, n_top, d_ids, d_scores);
 }
 
 int32_t rs_knn_sims_rows(rs_knn *h, int64_t row0, int64_t nrows, double *out) {

@@ -60,6 +60,10 @@ __host__ __device__ inline int64_t rs_cyc_local(int64_t i, int count) {
 __host__ __device__ inline bool rs_cyc_owns(int64_t i, int count, int index) {
     return (i / RS_CYC_B) % count == index;
 }
+// Global id of local row `loc` of shard `index`: the inverse of rs_cyc_local on the rows the shard owns.
+__host__ __device__ inline int64_t rs_cyc_global(int64_t loc, int count, int index) {
+    return ((loc / RS_CYC_B) * count + index) * RS_CYC_B + loc % RS_CYC_B;
+}
 inline int64_t rs_cyc_rows(int64_t n, int count, int index) {
     const int64_t nblk = (n + RS_CYC_B - 1) / RS_CYC_B;
     int64_t rows = 0;
@@ -243,6 +247,9 @@ int32_t rs_topk_rows_launch(rs_knn *h, const double *src, int64_t ld, int32_t n,
 int32_t rs_score_all_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, double *d_out);
 int32_t rs_recommend_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, int32_t n_top, int32_t *d_ids,
                             double *d_scores);
+int32_t rs_score_all_sharded_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, double *d_out);
+int32_t rs_recommend_sharded_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, int32_t n_top,
+                                    int32_t *d_ids, double *d_scores);
 
 // order-preserving map double -> uint64 (larger similarity = larger key); -0.0 folded to +0.0
 __host__ __device__ inline uint64_t rs_sim_key(double s) {

@@ -13,20 +13,52 @@
 //     all gathers of the query come from ONE matrix row, S[q][.]; the scores are handed out query-major, so the
 //     warps in flight share that row in L2.
 // Rated targets are then overwritten with NaN and topk_rows_kernel (predict.cu) picks the N best of each row.
+//
+// Row shards (rs_knn_*_sharded_device): a shard holds complete rows of the similarity matrix and both CSRs.
+//   right queries: the targets are the left rows, so a shard scores the targets it owns (local row t, global id
+//     map.global(t)) for every query; the global top N is contained in the union of the shards' top-N lists.
+//   left queries: a query needs row S[q] only; the owner of q scores it completely (a -1 query: the owner of row 0).
+//     The queries the shard answers are compacted first, scored query-major as above, and their lists scattered back.
 #include <cstdlib>
+
+#include <cub/cub.cuh>
 
 #include "common.cuh"
 #include "select.cuh"
 
 namespace {
 
+// Which left rows the handle holds, and where.  A full handle (row_begin 0, row_end n_left, no cyclic shards) maps
+// every row to itself.
+struct RowMap {
+    int64_t row_begin, row_end;
+    int32_t cyc_R, cyc_r;
+    __host__ __device__ bool owns(int64_t i) const {
+        return i >= row_begin && i < row_end && (cyc_R < 2 || rs_cyc_owns(i, cyc_R, cyc_r));
+    }
+    __host__ __device__ int64_t local(int64_t i) const { return cyc_R > 1 ? rs_cyc_local(i, cyc_R) : i - row_begin; }
+    // Strictly increasing in `loc` under both schemes (cyclic: blocks of 32 dealt in order, rows in order inside a
+    // block; contiguous: an offset).  So an order on local ids (the tie break "id asc" of topk_rows_kernel on a slab of
+    // local columns) is the same order on global ids, and a shard's top-N list of its own targets is exactly the
+    // prefix of the full ranking restricted to those targets: the union of the shards' lists is the full list.
+    __host__ __device__ int64_t global(int64_t loc) const {
+        return cyc_R > 1 ? rs_cyc_global(loc, cyc_R, cyc_r) : row_begin + loc;
+    }
+};
+
+RowMap row_map(const rs_knn *h) { return RowMap{h->row_begin, h->row_end, h->cyc_R, h->cyc_r}; }
+
 struct RecArgs {
     const int32_t *queries;
+    const int32_t *rows;    // optional: the output row of query b (else b)
     int64_t nq;
     int32_t side;           // enum rs_side
     int32_t n_side;         // ids of the query side: a query outside [0, n_side) is treated as -1 (cold start)
-    int32_t n_targets;
-    double *out;            // [nq][ld_out]
+    int32_t n_targets;      // targets scored per query: every id of the other side, or, for right queries on a row
+                            // shard, the shard's own rows by local index
+    int32_t out_global;     // right queries on a row shard: local target t goes to column map.global(t) (else t)
+    RowMap map;
+    double *out;            // [rows][ld_out]
     int64_t ld_out;
     unsigned long long *work;
 };
@@ -50,16 +82,17 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) recommend_kernel(PredArgs a, R
         const int64_t b = left ? w / ra.n_targets : w % ra.nq;
         const int32_t t = (int32_t)(left ? w % ra.n_targets : w / ra.nq);
         const int32_t q = ra.queries[b];
-        double *dst = ra.out + b * ra.ld_out + t;
+        const int32_t tg = left ? t : (int32_t)ra.map.global(t);     // right queries: t is a local row
+        double *dst = ra.out + (ra.rows ? (int64_t)ra.rows[b] : b) * ra.ld_out + (ra.out_global ? tg : t);
         if (q < 0 || q >= ra.n_side) {                      // newID: GlobalMean (core/knn.go:89-91)
             if (lane == 0) *dst = a.global_mean;
             return false;
         }
-        const int32_t l = left ? q : t, r = left ? t : q;  // the pair Predict(left = l, right = r)
+        const int32_t l = left ? q : tg, r = left ? t : q;  // the pair Predict(left = l, right = r)
         c.l = l;
         c.cb = a.r_ptr[r];
         c.cnt = (int)(a.r_ptr[r + 1] - c.cb);
-        c.row = a.sims + (int64_t)l * a.ld_s;
+        c.row = a.sims + (left ? ra.map.local(q) : (int64_t)t) * a.ld_s;   // a left query is one the shard owns
         c.dst = dst;
         return true;
     };
@@ -67,15 +100,57 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) recommend_kernel(PredArgs a, R
                               s_av[warp], sbuf, gbuf, scap);
 }
 
-// Rated targets: the query's row of the right CSR (right queries) or of the left CSR (left queries) -> NaN.
-__global__ void recommend_exclude_kernel(const int32_t *__restrict__ queries, int32_t n_side,
-                                         const int64_t *__restrict__ ptr, const int32_t *__restrict__ col,
-                                         double *__restrict__ out, int64_t ld_out) {
+// Rated targets: the query's row of the right CSR (right queries) or of the left CSR (left queries) -> NaN.  Right
+// queries on a row shard: only the rated targets the shard owns, at their local or global column.
+__global__ void recommend_exclude_kernel(const RecArgs ra, const int64_t *__restrict__ ptr,
+                                         const int32_t *__restrict__ col) {
     const int64_t b = blockIdx.x;
-    const int32_t q = queries[b];
-    if (q < 0 || q >= n_side) return;
+    const int32_t q = ra.queries[b];
+    if (q < 0 || q >= ra.n_side) return;
+    const bool right = ra.side == RS_SIDE_RIGHT;
+    double *row = ra.out + (ra.rows ? (int64_t)ra.rows[b] : b) * ra.ld_out;
     const double nan_v = __longlong_as_double(0x7ff8000000000001ll);
-    for (int64_t e = ptr[q] + threadIdx.x; e < ptr[q + 1]; e += blockDim.x) out[b * ld_out + col[e]] = nan_v;
+    for (int64_t e = ptr[q] + threadIdx.x; e < ptr[q + 1]; e += blockDim.x) {
+        int64_t t = col[e];
+        if (right) {
+            if (!ra.map.owns(t)) continue;
+            if (!ra.out_global) t = ra.map.local(t);
+        }
+        row[t] = nan_v;
+    }
+}
+
+// Left queries on a row shard: the queries this shard answers.  Its own rows, and -1 (or an id out of range) on the
+// shard that owns row 0 only, so that a cold-start list is not produced twice.
+__global__ void own_query_kernel(const int32_t *__restrict__ q, int64_t n, int32_t n_side, RowMap map,
+                                 uint8_t *__restrict__ flag) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int32_t v = q[i];
+    flag[i] = map.owns(v >= 0 && v < n_side ? v : 0) ? 1 : 0;
+}
+
+// Empty lists: id -1, score NaN.
+__global__ void empty_lists_kernel(int32_t *__restrict__ ids, double *__restrict__ scores, int64_t cnt) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= cnt) return;
+    ids[i] = -1;
+    scores[i] = __longlong_as_double(0x7ff8000000000001ll);
+}
+
+// Sharded lists: list b of the staging buffer goes to row rows[b] (else row0 + b) of the output; slab columns are
+// local rows for right queries and become global ids here (the map keeps their order).
+__global__ void place_lists_kernel(const int32_t *__restrict__ src_ids, const double *__restrict__ src_scores,
+                                   int32_t n_top, const int32_t *__restrict__ rows, int64_t row0, int32_t map_ids,
+                                   RowMap map, int32_t *__restrict__ ids, double *__restrict__ scores) {
+    const int64_t b = blockIdx.x;
+    const int64_t o = (rows ? (int64_t)rows[b] : row0 + b) * n_top;
+    for (int t = threadIdx.x; t < n_top; t += blockDim.x) {
+        int32_t id = src_ids[b * n_top + t];
+        if (map_ids && id >= 0) id = (int32_t)map.global(id);
+        ids[o + t] = id;
+        scores[o + t] = src_scores[b * n_top + t];
+    }
 }
 
 template <int R>
@@ -86,19 +161,27 @@ int32_t launch_scores(const PredArgs &a, const RecArgs &ra, unsigned blocks, siz
     return RS_OK;
 }
 
-// Scores of the queries d_q[0 .. nq) into out[nq][ld_out], rated targets NaN.
-int32_t score_rows(rs_knn *h, int32_t side, const int32_t *d_q, int64_t nq, double *out, int64_t ld_out) {
+// Scores of every target of the queries d_q[0 .. nq) into out[nq][ld_out]; the fields that differ on row shards are
+// set by the caller.
+RecArgs rec_args(const rs_knn *h, int32_t side, const int32_t *d_q, int64_t nq, double *out, int64_t ld_out) {
+    RecArgs ra{};
+    ra.queries = d_q; ra.nq = nq; ra.side = side;
+    ra.n_side = side == RS_SIDE_RIGHT ? h->n_right : h->n_left;
+    ra.n_targets = side == RS_SIDE_RIGHT ? h->n_left : h->n_right;
+    ra.map = row_map(h);
+    ra.out = out; ra.ld_out = ld_out;
+    return ra;
+}
+
+// Runs the scores of `ra`, then sets the rated targets to NaN.
+int32_t score_rows(rs_knn *h, RecArgs ra) {
+    if (ra.nq <= 0 || ra.n_targets <= 0) return RS_OK;    // a shard without rows scores nothing
     PredArgs a{};
     a.r_ptr = h->r_ptr; a.r_col = h->r_col; a.r_val = h->r_val;
     a.sims = h->sims; a.ld_s = h->ld_s;
     a.means = h->means; a.stddevs = h->stddevs; a.bias = h->left_bias;
     a.global_mean = h->global_mean; a.n_right = h->n_right;
     a.k = h->p.k; a.min_k = h->p.min_k; a.knn_type = h->p.knn_type;
-    RecArgs ra{};
-    ra.queries = d_q; ra.nq = nq; ra.side = side;
-    ra.n_side = side == RS_SIDE_RIGHT ? h->n_right : h->n_left;
-    ra.n_targets = side == RS_SIDE_RIGHT ? h->n_left : h->n_right;
-    ra.out = out; ra.ld_out = ld_out;
     void *work;
     RS_TRY(rs_scratch_get(h, 16, 8, &work));
     RS_CUDA(cudaMemsetAsync(work, 0, 8, h->stream));
@@ -110,7 +193,7 @@ int32_t score_rows(rs_knn *h, int32_t side, const int32_t *d_q, int64_t nq, doub
     // the same per-warp stage as Predict (select.cuh): 256 keys in shared memory, the rest in a global slice
     const int scap = 256;
     const size_t smem = (size_t)SEL_WARPS * scap * sizeof(double);
-    const int64_t warps = nq * ra.n_targets;
+    const int64_t warps = ra.nq * ra.n_targets;
     int64_t blocks = (int64_t)sms * ((200 * 1024) / (int64_t)(smem + 16 * 1024));   // resident CTAs, as Predict sizes them
     if (blocks > (warps + SEL_WARPS - 1) / SEL_WARPS) blocks = (warps + SEL_WARPS - 1) / SEL_WARPS;
     const int64_t gcap = h->max_right_len > scap ? (((int64_t)h->max_right_len - scap + 31) / 32 * 32) : 32;
@@ -121,9 +204,90 @@ int32_t score_rows(rs_knn *h, int32_t side, const int32_t *d_q, int64_t nq, doub
     if (h->p.k <= 44) RS_TRY(launch_scores<2>(a, ra, (unsigned)blocks, smem, scap, h->stream));
     else if (h->p.k <= 104) RS_TRY(launch_scores<4>(a, ra, (unsigned)blocks, smem, scap, h->stream));
     else RS_TRY(launch_scores<8>(a, ra, (unsigned)blocks, smem, scap, h->stream));
-    recommend_exclude_kernel<<<(unsigned)nq, 128, 0, h->stream>>>(d_q, ra.n_side, side == RS_SIDE_RIGHT ? h->r_ptr : h->l_ptr,
-                                                                  side == RS_SIDE_RIGHT ? h->r_col : h->l_col, out, ld_out);
+    const bool right = ra.side == RS_SIDE_RIGHT;
+    recommend_exclude_kernel<<<(unsigned)ra.nq, 128, 0, h->stream>>>(ra, right ? h->r_ptr : h->l_ptr,
+                                                                     right ? h->r_col : h->l_col);
     h->prof.total_launches += 2;
+    RS_CUDA(cudaGetLastError());
+    return RS_OK;
+}
+
+// Top-N lists of the queries d_q[0 .. n): scored in batches into a bounded slab of `width`-column score rows, ~256 MiB,
+// and selected by topk_rows_kernel.  Sharded: the lists are staged and placed by place_lists_kernel (to row rows[b],
+// else b; right queries' slab columns are local rows).
+int32_t recommend_rows(rs_knn *h, int32_t side, const int32_t *d_q, const int32_t *rows, int64_t n, int64_t width,
+                       bool sharded, int32_t n_top, int32_t *d_ids, double *d_scores) {
+    if (n <= 0) return RS_OK;
+    int64_t batch = ((int64_t)256 << 20) / (width * 8);
+    if (const char *e = getenv("RS_KNN_REC_BATCH")) batch = atoll(e);   // tests: force several batches
+    if (batch < 1) batch = 1;
+    if (batch > n) batch = n;
+    void *slab, *st_ids = nullptr, *st_scores = nullptr;
+    RS_TRY(rs_scratch_get(h, 23, (size_t)batch * width * 8, &slab));
+    if (sharded) {
+        RS_TRY(rs_scratch_get(h, 24, (size_t)batch * n_top * 4, &st_ids));
+        RS_TRY(rs_scratch_get(h, 25, (size_t)batch * n_top * 8, &st_scores));
+    }
+    for (int64_t b0 = 0; b0 < n; b0 += batch) {
+        const int64_t nb = n - b0 < batch ? n - b0 : batch;
+        RecArgs ra = rec_args(h, side, d_q + b0, nb, (double *)slab, width);
+        ra.n_targets = (int32_t)width;
+        RS_TRY(score_rows(h, ra));
+        if (!sharded) {
+            RS_TRY(rs_topk_rows_launch(h, (const double *)slab, width, (int32_t)width, nb, n_top, d_ids + b0 * n_top,
+                                       d_scores + b0 * n_top));
+            continue;
+        }
+        RS_TRY(rs_topk_rows_launch(h, (const double *)slab, width, (int32_t)width, nb, n_top, (int32_t *)st_ids,
+                                   (double *)st_scores));
+        place_lists_kernel<<<(unsigned)nb, 128, 0, h->stream>>>((const int32_t *)st_ids, (const double *)st_scores,
+                                                                n_top, rows ? rows + b0 : nullptr, b0,
+                                                                side == RS_SIDE_RIGHT, row_map(h), d_ids, d_scores);
+        h->prof.total_launches++;
+        RS_CUDA(cudaGetLastError());
+    }
+    return RS_OK;
+}
+
+// Left queries on a row shard: the queries this shard answers (values and positions), compacted; their count is read
+// back to size the batches.
+int32_t own_queries(rs_knn *h, const int32_t *d_q, int64_t n, const int32_t **q_own, const int32_t **pos,
+                    int64_t *n_own) {
+    void *flag, *qo, *po, *cnt, *tmp;
+    RS_TRY(rs_scratch_get(h, 26, (size_t)n, &flag));
+    RS_TRY(rs_scratch_get(h, 27, (size_t)n * 4, &qo));
+    RS_TRY(rs_scratch_get(h, 28, (size_t)n * 4, &po));
+    RS_TRY(rs_scratch_get(h, 29, 8, &cnt));
+    const cub::CountingInputIterator<int32_t> iota(0);
+    size_t need_q = 0, need_p = 0;
+    RS_CUDA(cub::DeviceSelect::Flagged(nullptr, need_q, d_q, (const uint8_t *)flag, (int32_t *)qo, (int32_t *)cnt,
+                                       (int)n, h->stream));
+    RS_CUDA(cub::DeviceSelect::Flagged(nullptr, need_p, iota, (const uint8_t *)flag, (int32_t *)po, (int32_t *)cnt,
+                                       (int)n, h->stream));
+    const size_t need = need_q > need_p ? need_q : need_p;
+    RS_TRY(rs_scratch_get(h, 30, need + 256, &tmp));
+    own_query_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(d_q, n, h->n_left, row_map(h),
+                                                                          (uint8_t *)flag);
+    h->prof.total_launches++;
+    RS_CUDA(cudaGetLastError());
+    size_t t_bytes = need;
+    RS_CUDA(cub::DeviceSelect::Flagged(tmp, t_bytes, d_q, (const uint8_t *)flag, (int32_t *)qo, (int32_t *)cnt, (int)n,
+                                       h->stream));
+    t_bytes = need;
+    RS_CUDA(cub::DeviceSelect::Flagged(tmp, t_bytes, iota, (const uint8_t *)flag, (int32_t *)po, (int32_t *)cnt, (int)n,
+                                       h->stream));
+    int32_t c = 0;
+    RS_CUDA(cudaMemcpyAsync(&c, cnt, 4, cudaMemcpyDeviceToHost, h->stream));
+    RS_CUDA(cudaStreamSynchronize(h->stream));
+    *q_own = (const int32_t *)qo;
+    *pos = (const int32_t *)po;
+    *n_own = c;
+    return RS_OK;
+}
+
+int32_t empty_lists(rs_knn *h, int32_t *d_ids, double *d_scores, int64_t cnt) {
+    empty_lists_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, h->stream>>>(d_ids, d_scores, cnt);
+    h->prof.total_launches++;
     RS_CUDA(cudaGetLastError());
     return RS_OK;
 }
@@ -131,27 +295,43 @@ int32_t score_rows(rs_knn *h, int32_t side, const int32_t *d_q, int64_t nq, doub
 }  // namespace
 
 int32_t rs_score_all_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, double *d_out) {
-    if (n <= 0) return RS_OK;
     const int64_t n_targets = side == RS_SIDE_RIGHT ? h->n_left : h->n_right;
-    return score_rows(h, side, d_q, n, d_out, n_targets);
+    return score_rows(h, rec_args(h, side, d_q, n, d_out, n_targets));
 }
 
 int32_t rs_recommend_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, int32_t n_top, int32_t *d_ids,
                             double *d_scores) {
+    const int64_t n_targets = side == RS_SIDE_RIGHT ? h->n_left : h->n_right;
+    return recommend_rows(h, side, d_q, nullptr, n, n_targets, false, n_top, d_ids, d_scores);
+}
+
+// Row shards: every cell this shard does not answer is +0.0 (all bits zero), for an integer SUM all-reduce.
+int32_t rs_score_all_sharded_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, double *d_out) {
     if (n <= 0) return RS_OK;
     const int64_t n_targets = side == RS_SIDE_RIGHT ? h->n_left : h->n_right;
-    // queries are scored in batches into a bounded slab of full score rows, ~256 MiB
-    int64_t batch = ((int64_t)256 << 20) / (n_targets * 8);
-    if (const char *e = getenv("RS_KNN_REC_BATCH")) batch = atoll(e);   // tests: force several batches
-    if (batch < 1) batch = 1;
-    if (batch > n) batch = n;
-    void *slab;
-    RS_TRY(rs_scratch_get(h, 23, (size_t)batch * n_targets * 8, &slab));
-    for (int64_t b0 = 0; b0 < n; b0 += batch) {
-        const int64_t nb = n - b0 < batch ? n - b0 : batch;
-        RS_TRY(score_rows(h, side, d_q + b0, nb, (double *)slab, n_targets));
-        RS_TRY(rs_topk_rows_launch(h, (const double *)slab, n_targets, (int32_t)n_targets, nb, n_top,
-                                   d_ids + b0 * n_top, d_scores + b0 * n_top));
+    RS_CUDA(cudaMemsetAsync(d_out, 0, (size_t)n * n_targets * 8, h->stream));
+    RecArgs ra = rec_args(h, side, d_q, n, d_out, n_targets);
+    if (side == RS_SIDE_RIGHT) {
+        ra.n_targets = (int32_t)h->rows_local;
+        ra.out_global = 1;
+        return score_rows(h, ra);
     }
-    return RS_OK;
+    RS_TRY(own_queries(h, d_q, n, &ra.queries, &ra.rows, &ra.nq));
+    return score_rows(h, ra);
+}
+
+// Row shards: partial lists, to be united across the shards (rs_knn_topk_union_device).  Lists this shard does not
+// produce are empty.
+int32_t rs_recommend_sharded_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, int32_t n_top,
+                                    int32_t *d_ids, double *d_scores) {
+    if (n <= 0) return RS_OK;
+    if (side == RS_SIDE_RIGHT) {
+        if (h->rows_local == 0) return empty_lists(h, d_ids, d_scores, n * n_top);
+        return recommend_rows(h, side, d_q, nullptr, n, h->rows_local, true, n_top, d_ids, d_scores);
+    }
+    const int32_t *q_own, *pos;
+    int64_t n_own = 0;
+    RS_TRY(own_queries(h, d_q, n, &q_own, &pos, &n_own));
+    RS_TRY(empty_lists(h, d_ids, d_scores, n * n_top));
+    return recommend_rows(h, side, q_own, pos, n_own, h->n_right, true, n_top, d_ids, d_scores);
 }

@@ -191,6 +191,21 @@ func (d *deviceKNN) predictBatchShardedDevice(dLeft, dRight unsafe.Pointer, n in
 		(*C.double)(dOut)))
 }
 
+// recommendShardedDevice: every shard gets the same queries (device pointers) and writes its PARTIAL lists
+// ids[n][nTop] / scores[n][nTop]: the targets it owns for right queries, the whole list of the left queries whose row
+// it owns.  All-gather them and unite them with rs_knn_topk_union_device (groups of at most 2048 / nTop lists).
+func (d *deviceKNN) recommendShardedDevice(side int, dQueries unsafe.Pointer, n, nTop int, dIDs, dScores unsafe.Pointer) {
+	check(C.rs_knn_recommend_sharded_device(d.h, C.int32_t(side), (*C.int32_t)(dQueries), C.int64_t(n), C.int32_t(nTop),
+		(*C.int32_t)(dIDs), (*C.double)(dScores)))
+}
+
+// scoreAllShardedDevice: the score rows out[n][nTargets] of this shard, +0.0 in the cells it does not answer; an
+// int64 SUM all-reduce of the bit patterns over the shards assembles rs_knn_score_all.
+func (d *deviceKNN) scoreAllShardedDevice(side int, dQueries unsafe.Pointer, n int, dOut unsafe.Pointer) {
+	check(C.rs_knn_score_all_sharded_device(d.h, C.int32_t(side), (*C.int32_t)(dQueries), C.int64_t(n),
+		(*C.double)(dOut)))
+}
+
 func (d *deviceKNN) predictBatch(left, right []int32) []float64 {
 	out := make([]float64, len(left))
 	check(C.rs_knn_predict_batch(d.h, i32(left), i32(right), C.int64_t(len(left)), f64(out)))

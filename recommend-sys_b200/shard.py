@@ -84,6 +84,31 @@ def union_topk_device(all_i, all_s):
     return out_i, out_s
 
 
+UNION_CAP = 2048   # entries rs_knn_topk_union_device unites per row: n_lists * k <= 2048
+
+
+def union_recommend_device(all_i, all_s, unite=None):
+    """Unites stacked partial top-N lists (n_lists, n, n_top) — one list per row shard, from
+    rs_knn_recommend_sharded_device — into the final (n, n_top) lists.  A union call takes at most
+    UNION_CAP // n_top lists; more are united in groups of that many and the results again, a tree of the
+    same kernel (valid because every target is in at most one partial list).  `unite` replaces
+    union_topk_device (tests)."""
+    unite = unite or union_topk_device
+    n_lists, n, n_top = all_i.shape
+    if n == 0:
+        return all_i[0], all_s[0]
+    group = UNION_CAP // n_top
+    while True:
+        parts = [unite(all_i[g:g + group], all_s[g:g + group]) for g in range(0, n_lists, group)]
+        if len(parts) == 1:
+            return parts[0]
+        all_i = all_i.new_empty((len(parts), n, n_top))
+        all_s = all_s.new_empty((len(parts), n, n_top))
+        for p, (pi, ps) in enumerate(parts):
+            all_i[p], all_s[p] = pi, ps
+        n_lists = len(parts)
+
+
 def allgather_predictions(pred_local, counts, group=None):
     """All-gather per-rank prediction vectors of (known) lengths `counts` into one vector."""
     import torch
@@ -237,6 +262,50 @@ class ShardedKNN:
         import numpy as np
 
         return float(self.PredictBatch(np.array([userID]), np.array([itemID]))[0])
+
+    def _device_queries(self, userIDs):
+        """The query side and the inner-id queries on this rank's GPU (every rank passes the same users)."""
+        import numpy as np
+        import torch
+
+        self._finish_fit()
+        side, q = self.knn._user_queries(userIDs)
+        dev = torch.device("cuda", torch.cuda.current_device())
+        return side, torch.from_numpy(np.ascontiguousarray(q, dtype=np.int32)).to(dev)
+
+    def Recommend(self, userIDs, n):
+        """KNN.Recommend on the row shards: each rank lists the best targets it can score (its own items for an
+        item-based KNN, its own users' lists for a user-based one), the partial lists are all-gathered and
+        united.  The same (items, scores) on every rank, bit for bit those of one unsharded KNN."""
+        import numpy as np
+        import torch
+
+        side, d_q = self._device_queries(userIDs)
+        m = d_q.shape[0]
+        if m == 0:
+            return np.empty((0, n), dtype=np.int64), np.empty((0, n), dtype=np.float64)
+        ids = torch.empty((m, n), dtype=torch.int32, device=d_q.device)
+        scores = torch.empty((m, n), dtype=torch.float64, device=d_q.device)
+        self.knn._h.recommend_sharded_device(side, d_q.data_ptr(), m, n, ids.data_ptr(), scores.data_ptr())
+        all_i, all_s = allgather_partial_topk(ids, scores, self.group)
+        ui, us = union_recommend_device(all_i, all_s)
+        return self.knn._raw_items(ui.cpu().numpy()), us.cpu().numpy()
+
+    def ScoreAll(self, userIDs):
+        """KNN.ScoreAll on the row shards: each rank scores the cells it owns, +0.0 elsewhere, and an int64 SUM
+        all-reduce of the bit patterns assembles the rows, as PredictBatch does.  The full rows on every rank."""
+        import torch
+        import torch.distributed as dist
+
+        from . import core
+
+        side, d_q = self._device_queries(userIDs)
+        m = d_q.shape[0]
+        out = torch.empty((m, self.knn._h._n_targets(core.RS_SIDE[side])), dtype=torch.float64, device=d_q.device)
+        if m:
+            self.knn._h.score_all_sharded_device(side, d_q.data_ptr(), m, out.data_ptr())
+            dist.all_reduce(out.view(torch.int64), op=dist.ReduceOp.SUM, group=self.group)
+        return out.cpu().numpy()
 
     def Close(self):
         self.knn.Close()
