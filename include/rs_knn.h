@@ -270,6 +270,38 @@ int32_t rs_knn_recommend_sharded_device(rs_knn *h, int32_t side, const int32_t *
                                         int32_t n_top, int32_t *d_ids, double *d_scores);
 int32_t rs_knn_score_all_sharded_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n,
                                         double *d_out);
+/* TOP-N RECOMMENDATION FOR QUERIES GIVEN AS RATING LISTS ("fold-in"): users who signed up or rated after the Fit are
+ * scored against the fitted model without a refit.  Query b is the list ids[ptr[b] .. ptr[b+1]), vals[...] of inner
+ * ids of the TARGET side and their ratings, in the caller's order (it plays the role of the user's dataset order).
+ *   RS_SIDE_RIGHT (item-based; ids are left ids): score(t) = Predict(left = t, right = q*), q* a right row whose
+ *     ratings are the list.  The candidates are the list's entries in ascending id, their similarities row S[t], their
+ *     statistics (means, stddevs, bias) the fitted ones.  The order of the list does not matter; a list equal to right
+ *     row u's ratings gives rs_knn_score_all(RS_SIDE_RIGHT, u) bit for bit.
+ *   RS_SIDE_LEFT (user-based; ids are right ids): S*[v] = Sim(list sorted by id, left row v) for every fitted left row
+ *     v, with the reference's formulas, term order and IEEE operations (the exact sparse Fit's; Pearson's mean of the
+ *     list summed in ascending id, NaN without a co-rating); then score(t) = Predict(left = q*, right = t) with the
+ *     candidates R(t) weighted by S*.  The list's own mean / stddev (centered, z-score) are accumulated in the
+ *     caller's order as Fit's are.  A list equal to left row u's ratings in dataset order gives
+ *     rs_knn_score_all(RS_SIDE_LEFT, u) bit for bit.
+ * The list's ids are the query's rated targets: NaN in score rows, never listed.  An empty list scores GlobalMean
+ * everywhere (a -1 query).  Output layout, ranking rule, unused slots and n_top limits are rs_knn_score_all's /
+ * rs_knn_recommend's.  NOT A REFIT: the given ratings enter neither the similarities between fitted rows, nor the
+ * fitted means, nor GlobalMean.
+ * Refused: RS_ERR_INVALID for an id outside [0, n_targets), ptr not starting at >= 0 or not non-decreasing, a NaN
+ * rating; RS_ERR_DUPLICATE for an id twice in one list (the _device variants check on the device and read back a
+ * few bytes); RS_ERR_UNSUPPORTED for RS_STORE_TOPK, RS_SIM_SLOPE_ONE, row shards, and for RS_SIDE_LEFT
+ * RS_KNN_BASELINE / RS_SIM_PEARSON_BASELINE (no bias for the list's user) and Pearson in RS_PEARSON_SUMS mode (the
+ * matrix is not the exact replay S* is); plus the limits of rs_knn_recommend.  Lists are scored in batches; for left
+ * queries the S* rows share the ~256 MiB slab with the score rows. */
+int32_t rs_knn_score_all_given(rs_knn *h, int32_t side, const int64_t *ptr, const int32_t *ids, const double *vals,
+                               int64_t n, double *out);
+int32_t rs_knn_score_all_given_device(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids,
+                                      const double *d_vals, int64_t n, double *d_out);
+int32_t rs_knn_recommend_given(rs_knn *h, int32_t side, const int64_t *ptr, const int32_t *ids, const double *vals,
+                               int64_t n, int32_t n_top, int32_t *out_ids, double *out_scores);
+int32_t rs_knn_recommend_given_device(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids,
+                                      const double *d_vals, int64_t n, int32_t n_top, int32_t *d_out_ids,
+                                      double *d_out_scores);
 
 /* Parameters["k"] / ["mink"] are read at Predict time by the reference (core/knn.go:80-81): change
  * them on a fitted handle without refitting.  The predict kernel supports k <= 256. */

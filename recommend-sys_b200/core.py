@@ -70,7 +70,8 @@ ABI_SYMBOLS = [
     "rs_knn_topk_union_device", "rs_knn_set_k", "rs_knn_peer_export", "rs_knn_peer_import",
     "rs_knn_peer_import_local", "rs_knn_mirror", "rs_knn_predict_batch_sharded_device", "rs_knn_host_alloc",
     "rs_knn_host_free", "rs_knn_score_all", "rs_knn_score_all_device", "rs_knn_recommend", "rs_knn_recommend_device",
-    "rs_knn_score_all_sharded_device", "rs_knn_recommend_sharded_device",
+    "rs_knn_score_all_sharded_device", "rs_knn_recommend_sharded_device", "rs_knn_score_all_given",
+    "rs_knn_score_all_given_device", "rs_knn_recommend_given", "rs_knn_recommend_given_device",
 ]
 
 _knn_lib = None
@@ -127,6 +128,10 @@ def knn_lib():
     L.rs_knn_recommend_device.argtypes = [vp, i32, vp, i64, i32, vp, vp]
     L.rs_knn_score_all_sharded_device.argtypes = [vp, i32, vp, i64, vp]
     L.rs_knn_recommend_sharded_device.argtypes = [vp, i32, vp, i64, i32, vp, vp]
+    L.rs_knn_score_all_given.argtypes = [vp, i32, vp, vp, vp, i64, vp]
+    L.rs_knn_score_all_given_device.argtypes = [vp, i32, vp, vp, vp, i64, vp]
+    L.rs_knn_recommend_given.argtypes = [vp, i32, vp, vp, vp, i64, i32, vp, vp]
+    L.rs_knn_recommend_given_device.argtypes = [vp, i32, vp, vp, vp, i64, i32, vp, vp]
     _knn_lib = L
     return L
 
@@ -736,6 +741,41 @@ class _Handle:
         _check(knn_lib().rs_knn_recommend_sharded_device(self.h, RS_SIDE[side], d_queries, n, int(n_top), d_ids,
                                                          d_scores))
 
+    @staticmethod
+    def _given_lists(ptr, ids, vals):
+        ptr = np.ascontiguousarray(ptr, dtype=np.int64)
+        ids = np.ascontiguousarray(ids, dtype=np.int32)
+        vals = np.ascontiguousarray(vals, dtype=np.float64)
+        if len(ids) == 0:           # the library wants valid pointers even when every list is empty
+            ids, vals = np.zeros(1, np.int32), np.zeros(1, np.float64)
+        return ptr, ids, vals, len(ptr) - 1
+
+    def score_all_given(self, side, ptr, ids, vals):
+        """Full score rows [n][n_targets] of queries given as rating lists: list b is ids[ptr[b]:ptr[b+1]] (inner ids
+        of the target side) with ratings vals[...] (include/rs_knn.h rs_knn_score_all_given)."""
+        side = RS_SIDE[side]
+        ptr, ids, vals, n = self._given_lists(ptr, ids, vals)
+        out = np.empty((n, self._n_targets(side)), dtype=np.float64)
+        _check(knn_lib().rs_knn_score_all_given(self.h, side, _ptr(ptr), _ptr(ids), _ptr(vals), n, _ptr(out)))
+        return out
+
+    def score_all_given_device(self, side, d_ptr, d_ids, d_vals, n, d_out):
+        _check(knn_lib().rs_knn_score_all_given_device(self.h, RS_SIDE[side], d_ptr, d_ids, d_vals, n, d_out))
+
+    def recommend_given(self, side, ptr, ids, vals, n_top):
+        """(ids[n][n_top], scores[n][n_top]) of queries given as rating lists (rs_knn_recommend_given)."""
+        side = RS_SIDE[side]
+        ptr, ids, vals, n = self._given_lists(ptr, ids, vals)
+        top_ids = np.empty((n, n_top), dtype=np.int32)
+        top = np.empty((n, n_top), dtype=np.float64)
+        _check(knn_lib().rs_knn_recommend_given(self.h, side, _ptr(ptr), _ptr(ids), _ptr(vals), n, int(n_top),
+                                                _ptr(top_ids), _ptr(top)))
+        return top_ids, top
+
+    def recommend_given_device(self, side, d_ptr, d_ids, d_vals, n, n_top, d_top_ids, d_top_scores):
+        _check(knn_lib().rs_knn_recommend_given_device(self.h, RS_SIDE[side], d_ptr, d_ids, d_vals, n, int(n_top),
+                                                       d_top_ids, d_top_scores))
+
     # ---- cyclic row shards (RS_STORE_MATRIX, shard_count >= 2): the exchange step ----
     def peer_export(self):
         """(64-byte CUDA IPC handle, byte offset) of this shard's matrix."""
@@ -974,6 +1014,42 @@ class KNN(Base):
         side, q = self._user_queries(userIDs)
         ids, scores = self._h.recommend(side, q, n)
         return self._raw_items(ids), scores
+
+    def _given(self, dataSet):
+        """(users, ptr, ids, vals): the rows of `dataSet` grouped by raw user in order of first appearance, each
+        user's entries in dataset order, as lists of inner item ids.  Items the train set does not know are dropped:
+        they have no row or column of the model, so Predict could never use them (nor do they enter the list's mean
+        on the user-based side).  A user all of whose items are unknown keeps an empty list (GlobalMean)."""
+        users = np.asarray(dataSet.Users, dtype=np.int64)
+        uniq, first, inv = np.unique(users, return_index=True, return_inverse=True)
+        rank = np.empty(len(uniq), dtype=np.int64)
+        rank[np.argsort(first, kind="stable")] = np.arange(len(uniq))
+        grp = rank[inv.reshape(-1)]
+        inner = self.Data.convert_items(np.asarray(dataSet.Items, dtype=np.int64))
+        keep = inner >= 0
+        order = np.argsort(grp[keep], kind="stable")
+        ids = inner[keep][order]
+        vals = np.asarray(dataSet.Ratings, dtype=np.float64)[keep][order]
+        ptr = np.zeros(len(uniq) + 1, dtype=np.int64)
+        np.cumsum(np.bincount(grp[keep], minlength=len(uniq)), out=ptr[1:])
+        return uniq[np.argsort(first, kind="stable")], ptr, ids, vals
+
+    def ScoreAllGiven(self, dataSet):
+        """Fold-in: (users, scores[len(users)][ItemCount]) for users whose ratings are given in `dataSet` (raw user,
+        raw item, rating) instead of taken from the train set — users who may or may not be in it.  The scores are
+        those of ScoreAll for a user whose ratings are the given ones; the model is not refitted (the given ratings
+        enter neither the similarities between the train set's rows, nor its means, nor GlobalMean)."""
+        self._sync_k()
+        users, ptr, ids, vals = self._given(dataSet)
+        return users, self._h.score_all_given("left" if self._userBased else "right", ptr, ids, vals)
+
+    def RecommendGiven(self, dataSet, n):
+        """Fold-in: (users, items[len][n], scores[len][n]) — Recommend for users whose ratings are given in `dataSet`
+        (see ScoreAllGiven); the given items are never recommended."""
+        self._sync_k()
+        users, ptr, ids, vals = self._given(dataSet)
+        top_ids, top = self._h.recommend_given("left" if self._userBased else "right", ptr, ids, vals, n)
+        return users, self._raw_items(top_ids), top
 
     def _raw_items(self, ids):
         """Inner item ids -> raw item ids; -1 (an unused slot) -> newID."""

@@ -165,7 +165,7 @@ int32_t init_handle(rs_knn *h) {
 extern "C" {
 
 const char *rs_last_error(void) { return g_err; }
-int32_t rs_knn_abi_version(void) { return 3; }
+int32_t rs_knn_abi_version(void) { return 4; }
 
 int32_t rs_knn_device_count(void) {
     int n = 0;
@@ -844,6 +844,127 @@ int32_t rs_knn_recommend_sharded_device(rs_knn *h, int32_t side, const int32_t *
         return RS_ERR_INVALID;
     }
     return rs_recommend_sharded_launch(h, side, d_queries, n, n_top, d_ids, d_scores);
+}
+
+// Queries given as rating lists: what rs_knn_recommend accepts, less top-k-only handles, and for left queries the
+// models that need something of the query the lists do not give (a baseline bias) or whose matrix is not the exact
+// replay the lists' similarity rows are (Pearson sums).
+static int32_t require_given(rs_knn *h, const char *who, int32_t side, int64_t n, const void *ptr, const void *ids,
+                             const void *vals, const void *out0, const void *out1) {
+    if (h->fitted && h->p.store == RS_STORE_TOPK) {
+        rs_set_error("%s needs RS_STORE_MATRIX (the handle keeps top-k lists only)", who);
+        return RS_ERR_UNSUPPORTED;
+    }
+    RS_TRY(require_recommend(h, who, side, n));
+    if (side == RS_SIDE_LEFT) {
+        if (h->p.knn_type == RS_KNN_BASELINE || h->p.sim == RS_SIM_PEARSON_BASELINE) {
+            rs_set_error("%s: left queries have no baseline bias (RS_KNN_BASELINE / RS_SIM_PEARSON_BASELINE)", who);
+            return RS_ERR_UNSUPPORTED;
+        }
+        if (h->p.sim == RS_SIM_PEARSON && h->p.pearson_mode == RS_PEARSON_SUMS) {
+            rs_set_error("%s: left queries need the exact Pearson matrix (pearson_mode EXACT)", who);
+            return RS_ERR_UNSUPPORTED;
+        }
+        if ((int64_t)h->n_left + n >= (1ll << 31)) {
+            rs_set_error("%s: n_left + n = %lld (at most 2^31 - 1)", who, (long long)h->n_left + n);
+            return RS_ERR_UNSUPPORTED;
+        }
+    }
+    if (n > 0 && (!ptr || !ids || !vals || !out0 || !out1)) {
+        rs_set_error("%s: null argument", who);
+        return RS_ERR_INVALID;
+    }
+    return RS_OK;
+}
+
+int32_t rs_knn_score_all_given_device(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids,
+                                      const double *d_vals, int64_t n, double *d_out) {
+    RS_ENTER(h);
+    RS_TRY(require_given(h, "rs_knn_score_all_given", side, n, d_ptr, d_ids, d_vals, d_out, d_out));
+    if (n == 0) return RS_OK;
+    return rs_given_launch(h, side, d_ptr, d_ids, d_vals, n, d_out, 0, nullptr, nullptr);
+}
+
+int32_t rs_knn_recommend_given_device(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids,
+                                      const double *d_vals, int64_t n, int32_t n_top, int32_t *d_top_ids,
+                                      double *d_top_scores) {
+    RS_ENTER(h);
+    RS_TRY(require_given(h, "rs_knn_recommend_given", side, n, d_ptr, d_ids, d_vals, d_top_ids, d_top_scores));
+    RS_TRY(check_n_top("rs_knn_recommend_given", n_top));
+    if (n == 0) return RS_OK;
+    return rs_given_launch(h, side, d_ptr, d_ids, d_vals, n, nullptr, n_top, d_top_ids, d_top_scores);
+}
+
+// host variants: ptr is checked here (it sizes the copies), the entries on the device as in the _device variants
+static int32_t stage_given(rs_knn *h, const char *who, const int64_t *ptr, const int32_t *ids, const double *vals,
+                           int64_t n, const int64_t **d_ptr, const int32_t **d_ids, const double **d_vals) {
+    if (ptr[0] < 0) {
+        rs_set_error("%s: ptr[0] = %lld < 0", who, (long long)ptr[0]);
+        return RS_ERR_INVALID;
+    }
+    for (int64_t b = 0; b < n; b++) {
+        if (ptr[b + 1] < ptr[b]) {
+            rs_set_error("%s: ptr is not non-decreasing at list %lld", who, (long long)b);
+            return RS_ERR_INVALID;
+        }
+    }
+    const int64_t p0 = ptr[0], nnz = ptr[n] - p0;
+    if (nnz >= (1ll << 31)) {
+        rs_set_error("%s: %lld entries (at most 2^31 - 1 per call)", who, (long long)nnz);
+        return RS_ERR_UNSUPPORTED;
+    }
+    void *dp, *di, *dv;
+    RS_TRY(rs_scratch_get(h, 42, (size_t)(n + 1) * 8, &dp));
+    RS_TRY(rs_scratch_get(h, 43, (size_t)nnz * 4 + 4, &di));
+    RS_TRY(rs_scratch_get(h, 44, (size_t)nnz * 8 + 8, &dv));
+    RS_CUDA(cudaMemcpyAsync(dp, ptr, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, h->stream));
+    if (nnz > 0) {
+        RS_CUDA(cudaMemcpyAsync(di, ids + p0, (size_t)nnz * 4, cudaMemcpyHostToDevice, h->stream));
+        RS_CUDA(cudaMemcpyAsync(dv, vals + p0, (size_t)nnz * 8, cudaMemcpyHostToDevice, h->stream));
+    }
+    // the device copies hold the entries from ptr[0] on: index them from ptr[0]
+    *d_ptr = (const int64_t *)dp;
+    *d_ids = (const int32_t *)di - p0;
+    *d_vals = (const double *)dv - p0;
+    return RS_OK;
+}
+
+int32_t rs_knn_score_all_given(rs_knn *h, int32_t side, const int64_t *ptr, const int32_t *ids, const double *vals,
+                               int64_t n, double *out) {
+    RS_ENTER(h);
+    RS_TRY(require_given(h, "rs_knn_score_all_given", side, n, ptr, ids, vals, out, out));
+    if (n == 0) return RS_OK;
+    const int64_t *dp;
+    const int32_t *di;
+    const double *dv;
+    RS_TRY(stage_given(h, "rs_knn_score_all_given", ptr, ids, vals, n, &dp, &di, &dv));
+    const size_t bytes = (size_t)n * n_targets_of(h, side) * 8;
+    void *dout;
+    RS_TRY(rs_scratch_get(h, 45, bytes, &dout));
+    RS_TRY(rs_given_launch(h, side, dp, di, dv, n, (double *)dout, 0, nullptr, nullptr));
+    RS_CUDA(cudaMemcpyAsync(out, dout, bytes, cudaMemcpyDeviceToHost, h->stream));
+    RS_CUDA(cudaStreamSynchronize(h->stream));
+    return RS_OK;
+}
+
+int32_t rs_knn_recommend_given(rs_knn *h, int32_t side, const int64_t *ptr, const int32_t *ids, const double *vals,
+                               int64_t n, int32_t n_top, int32_t *top_ids, double *top_scores) {
+    RS_ENTER(h);
+    RS_TRY(require_given(h, "rs_knn_recommend_given", side, n, ptr, ids, vals, top_ids, top_scores));
+    RS_TRY(check_n_top("rs_knn_recommend_given", n_top));
+    if (n == 0) return RS_OK;
+    const int64_t *dp;
+    const int32_t *di;
+    const double *dv;
+    RS_TRY(stage_given(h, "rs_knn_recommend_given", ptr, ids, vals, n, &dp, &di, &dv));
+    void *d_i, *d_s;
+    RS_TRY(rs_scratch_get(h, 45, (size_t)n * n_top * 4, &d_i));
+    RS_TRY(rs_scratch_get(h, 46, (size_t)n * n_top * 8, &d_s));
+    RS_TRY(rs_given_launch(h, side, dp, di, dv, n, nullptr, n_top, (int32_t *)d_i, (double *)d_s));
+    RS_CUDA(cudaMemcpyAsync(top_ids, d_i, (size_t)n * n_top * 4, cudaMemcpyDeviceToHost, h->stream));
+    RS_CUDA(cudaMemcpyAsync(top_scores, d_s, (size_t)n * n_top * 8, cudaMemcpyDeviceToHost, h->stream));
+    RS_CUDA(cudaStreamSynchronize(h->stream));
+    return RS_OK;
 }
 
 int32_t rs_knn_sims_rows(rs_knn *h, int64_t row0, int64_t nrows, double *out) {

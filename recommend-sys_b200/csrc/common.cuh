@@ -218,6 +218,8 @@ inline int32_t rs_alloc(rs_knn *h, T **out, size_t count) {
 }
 int32_t rs_prep_rt(rs_knn *h);
 int32_t rs_prep_planes(rs_knn *h);
+int32_t rs_row_stats_launch(rs_knn *h, const int64_t *ptr, const double *ld_val, const double *l_val, int64_t n,
+                            int want_std, double *means, double *stddevs, double *pmeans);
 
 // ---- sim_stream.cu ----
 int32_t rs_sim_stream_launch(rs_knn *h);
@@ -250,6 +252,27 @@ int32_t rs_recommend_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t
 int32_t rs_score_all_sharded_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, double *d_out);
 int32_t rs_recommend_sharded_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, int32_t n_top,
                                     int32_t *d_ids, double *d_scores);
+// Queries given as rating lists (rs_knn_*_given): d_ptr / d_ids / d_vals are the caller's device arrays.  d_out set:
+// score rows; else the top-n_top lists.
+int32_t rs_given_launch(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids, const double *d_vals,
+                        int64_t n, double *d_out, int32_t n_top, int32_t *d_top_ids, double *d_top_scores);
+
+// ---- given.cu ----
+// The lists of rs_knn_*_given, validated and sorted: list b is entries ptr[b] .. ptr[b+1) of ids / vals (ascending id)
+// and of vals_in (the caller's order).
+struct rs_given_lists {
+    const int64_t *ptr;      // [n + 1], ptr[0] = 0
+    const int32_t *ids;
+    const double *vals;
+    const double *vals_in;
+    int64_t nnz;
+    int64_t max_len;         // the longest list
+};
+int32_t rs_given_prepare(rs_knn *h, int32_t n_targets, const int64_t *d_ptr, const int32_t *d_ids,
+                         const double *d_vals, int64_t n, rs_given_lists *out);
+// The similarity rows S*[b][v] = Sim(list b, left row v) of the lists ptr[0 .. nq) (ids: right ids), into out[nq][ld].
+int32_t rs_given_sims_launch(rs_knn *h, const int64_t *ptr, const int32_t *ids, const double *vals,
+                             const double *qpmeans, int64_t nq, double *out, int64_t ld);
 
 // order-preserving map double -> uint64 (larger similarity = larger key); -0.0 folded to +0.0
 __host__ __device__ inline uint64_t rs_sim_key(double s) {

@@ -357,6 +357,18 @@ int bits_for(int32_t n) {
 
 }  // namespace
 
+// Row statistics of `n` rows given as a CSR: the entries of row i are ptr[i] .. ptr[i+1) of ld_val (dataset order:
+// means, stddevs) and of l_val (ascending id: pmeans).  Fit's statistics, for the rating lists of rs_knn_*_given.
+int32_t rs_row_stats_launch(rs_knn *h, const int64_t *ptr, const double *ld_val, const double *l_val, int64_t n,
+                            int want_std, double *means, double *stddevs, double *pmeans) {
+    if (n <= 0) return RS_OK;
+    row_stats_ordered_kernel<<<blocks_for(n * 32), T, 0, h->stream>>>(ptr, ld_val, l_val, (int32_t)n, 1, want_std,
+                                                                      means, stddevs, pmeans);
+    h->prof.total_launches++;
+    RS_CUDA(cudaGetLastError());
+    return RS_OK;
+}
+
 #define RS_SORT_PAIRS(keys_in, keys_out, vals_in, vals_out, n, end_bit)                                      \
     do {                                                                                                     \
         size_t need_ = 0;                                                                                    \

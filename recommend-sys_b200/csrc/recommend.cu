@@ -19,6 +19,12 @@
 //     map.global(t)) for every query; the global top N is contained in the union of the shards' top-N lists.
 //   left queries: a query needs row S[q] only; the owner of q scores it completely (a -1 query: the owner of row 0).
 //     The queries the shard answers are compacted first, scored query-major as above, and their lists scattered back.
+//
+// Queries given as rating lists (rs_knn_*_given, lists prepared by given.cu): query b is list b of the call.
+//   right: the list, sorted by id, is the right row of the query: it replaces the handle's right CSR as the candidate
+//     CSR (a.r_ptr / r_col / r_val, r = b), and it is the query's rated targets.
+//   left: the gathered row is the query's row of S* (given_sims_kernel, in a slab beside the score slab), and the
+//     query's own mean / stddev follow the fitted rows' in one statistics array: Predict's left row is n_left + b.
 #include <cstdlib>
 
 #include <cub/cub.cuh>
@@ -57,6 +63,10 @@ struct RecArgs {
     int32_t n_targets;      // targets scored per query: every id of the other side, or, for right queries on a row
                             // shard, the shard's own rows by local index
     int32_t out_global;     // right queries on a row shard: local target t goes to column map.global(t) (else t)
+    int32_t given;          // queries given as rating lists: query b is list b (queries unused)
+    int32_t qstat;          // left given: the statistics of query b are entry qstat + b of a.means / a.stddevs
+    const double *gsims;    // left given: the similarity rows S*[b] of the batch
+    int64_t ld_g;
     RowMap map;
     double *out;            // [rows][ld_out]
     int64_t ld_out;
@@ -81,18 +91,19 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) recommend_kernel(PredArgs a, R
         const bool left = ra.side == RS_SIDE_LEFT;
         const int64_t b = left ? w / ra.n_targets : w % ra.nq;
         const int32_t t = (int32_t)(left ? w % ra.n_targets : w / ra.nq);
-        const int32_t q = ra.queries[b];
+        const int32_t q = ra.given ? (int32_t)b : ra.queries[b];
         const int32_t tg = left ? t : (int32_t)ra.map.global(t);     // right queries: t is a local row
         double *dst = ra.out + (ra.rows ? (int64_t)ra.rows[b] : b) * ra.ld_out + (ra.out_global ? tg : t);
-        if (q < 0 || q >= ra.n_side) {                      // newID: GlobalMean (core/knn.go:89-91)
+        if (!ra.given && (q < 0 || q >= ra.n_side)) {       // newID: GlobalMean (core/knn.go:89-91)
             if (lane == 0) *dst = a.global_mean;
             return false;
         }
         const int32_t l = left ? q : tg, r = left ? t : q;  // the pair Predict(left = l, right = r)
-        c.l = l;
+        c.l = left && ra.given ? ra.qstat + q : l;
         c.cb = a.r_ptr[r];
         c.cnt = (int)(a.r_ptr[r + 1] - c.cb);
-        c.row = a.sims + (left ? ra.map.local(q) : (int64_t)t) * a.ld_s;   // a left query is one the shard owns
+        if (left && ra.given) c.row = ra.gsims + b * ra.ld_g;
+        else c.row = a.sims + (left ? ra.map.local(q) : (int64_t)t) * a.ld_s;   // a left query is one the shard owns
         c.dst = dst;
         return true;
     };
@@ -101,12 +112,13 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) recommend_kernel(PredArgs a, R
 }
 
 // Rated targets: the query's row of the right CSR (right queries) or of the left CSR (left queries) -> NaN.  Right
-// queries on a row shard: only the rated targets the shard owns, at their local or global column.
+// queries on a row shard: only the rated targets the shard owns, at their local or global column.  Given lists: list
+// b of the given CSR.
 __global__ void recommend_exclude_kernel(const RecArgs ra, const int64_t *__restrict__ ptr,
                                          const int32_t *__restrict__ col) {
     const int64_t b = blockIdx.x;
-    const int32_t q = ra.queries[b];
-    if (q < 0 || q >= ra.n_side) return;
+    const int32_t q = ra.given ? (int32_t)b : ra.queries[b];
+    if (!ra.given && (q < 0 || q >= ra.n_side)) return;
     const bool right = ra.side == RS_SIDE_RIGHT;
     double *row = ra.out + (ra.rows ? (int64_t)ra.rows[b] : b) * ra.ld_out;
     const double nan_v = __longlong_as_double(0x7ff8000000000001ll);
@@ -173,13 +185,31 @@ RecArgs rec_args(const rs_knn *h, int32_t side, const int32_t *d_q, int64_t nq, 
     return ra;
 }
 
-// Runs the scores of `ra`, then sets the rated targets to NaN.
-int32_t score_rows(rs_knn *h, RecArgs ra) {
+// Given lists of one batch: the lists (right queries: the candidate CSR), and for left queries the S* rows and the
+// statistics arrays that hold the queries' own after the fitted rows'.
+struct GivenBatch {
+    const int64_t *ptr;
+    const int32_t *ids;
+    const double *vals;
+    int64_t max_len;
+    const double *means, *stddevs;
+};
+
+// Runs the scores of `ra`, then sets the rated targets to NaN.  g: the batch's given lists (ra.given).
+int32_t score_rows(rs_knn *h, RecArgs ra, const GivenBatch *g = nullptr) {
     if (ra.nq <= 0 || ra.n_targets <= 0) return RS_OK;    // a shard without rows scores nothing
+    const bool right = ra.side == RS_SIDE_RIGHT;
     PredArgs a{};
     a.r_ptr = h->r_ptr; a.r_col = h->r_col; a.r_val = h->r_val;
     a.sims = h->sims; a.ld_s = h->ld_s;
     a.means = h->means; a.stddevs = h->stddevs; a.bias = h->left_bias;
+    int64_t max_cand = h->max_right_len;
+    if (g && right) {                                     // the lists are the candidates
+        a.r_ptr = g->ptr; a.r_col = g->ids; a.r_val = g->vals;
+        max_cand = g->max_len;
+    } else if (g) {
+        a.means = g->means; a.stddevs = g->stddevs;
+    }
     a.global_mean = h->global_mean; a.n_right = h->n_right;
     a.k = h->p.k; a.min_k = h->p.min_k; a.knn_type = h->p.knn_type;
     void *work;
@@ -196,20 +226,29 @@ int32_t score_rows(rs_knn *h, RecArgs ra) {
     const int64_t warps = ra.nq * ra.n_targets;
     int64_t blocks = (int64_t)sms * ((200 * 1024) / (int64_t)(smem + 16 * 1024));   // resident CTAs, as Predict sizes them
     if (blocks > (warps + SEL_WARPS - 1) / SEL_WARPS) blocks = (warps + SEL_WARPS - 1) / SEL_WARPS;
-    const int64_t gcap = h->max_right_len > scap ? (((int64_t)h->max_right_len - scap + 31) / 32 * 32) : 32;
-    void *g;
-    RS_TRY(rs_scratch_get(h, 17, (size_t)blocks * SEL_WARPS * (size_t)gcap * 8, &g));
-    a.gstage = reinterpret_cast<uint64_t *>(g);
+    const int64_t gcap = max_cand > scap ? ((max_cand - scap + 31) / 32 * 32) : 32;
+    void *gst;
+    RS_TRY(rs_scratch_get(h, 17, (size_t)blocks * SEL_WARPS * (size_t)gcap * 8, &gst));
+    a.gstage = reinterpret_cast<uint64_t *>(gst);
     a.gcap = gcap;
     if (h->p.k <= 44) RS_TRY(launch_scores<2>(a, ra, (unsigned)blocks, smem, scap, h->stream));
     else if (h->p.k <= 104) RS_TRY(launch_scores<4>(a, ra, (unsigned)blocks, smem, scap, h->stream));
     else RS_TRY(launch_scores<8>(a, ra, (unsigned)blocks, smem, scap, h->stream));
-    const bool right = ra.side == RS_SIDE_RIGHT;
-    recommend_exclude_kernel<<<(unsigned)ra.nq, 128, 0, h->stream>>>(ra, right ? h->r_ptr : h->l_ptr,
-                                                                     right ? h->r_col : h->l_col);
+    if (g) recommend_exclude_kernel<<<(unsigned)ra.nq, 128, 0, h->stream>>>(ra, g->ptr, g->ids);
+    else recommend_exclude_kernel<<<(unsigned)ra.nq, 128, 0, h->stream>>>(ra, right ? h->r_ptr : h->l_ptr,
+                                                                          right ? h->r_col : h->l_col);
     h->prof.total_launches += 2;
     RS_CUDA(cudaGetLastError());
     return RS_OK;
+}
+
+// Rows per batch of a slab of `width` doubles per row: ~256 MiB.
+int64_t slab_batch(int64_t width, int64_t n) {
+    int64_t batch = ((int64_t)256 << 20) / (width * 8);
+    if (const char *e = getenv("RS_KNN_REC_BATCH")) batch = atoll(e);   // tests: force several batches
+    if (batch < 1) batch = 1;
+    if (batch > n) batch = n;
+    return batch;
 }
 
 // Top-N lists of the queries d_q[0 .. n): scored in batches into a bounded slab of `width`-column score rows, ~256 MiB,
@@ -218,10 +257,7 @@ int32_t score_rows(rs_knn *h, RecArgs ra) {
 int32_t recommend_rows(rs_knn *h, int32_t side, const int32_t *d_q, const int32_t *rows, int64_t n, int64_t width,
                        bool sharded, int32_t n_top, int32_t *d_ids, double *d_scores) {
     if (n <= 0) return RS_OK;
-    int64_t batch = ((int64_t)256 << 20) / (width * 8);
-    if (const char *e = getenv("RS_KNN_REC_BATCH")) batch = atoll(e);   // tests: force several batches
-    if (batch < 1) batch = 1;
-    if (batch > n) batch = n;
+    const int64_t batch = slab_batch(width, n);
     void *slab, *st_ids = nullptr, *st_scores = nullptr;
     RS_TRY(rs_scratch_get(h, 23, (size_t)batch * width * 8, &slab));
     if (sharded) {
@@ -334,4 +370,60 @@ int32_t rs_recommend_sharded_launch(rs_knn *h, int32_t side, const int32_t *d_q,
     RS_TRY(own_queries(h, d_q, n, &q_own, &pos, &n_own));
     RS_TRY(empty_lists(h, d_ids, d_scores, n * n_top));
     return recommend_rows(h, side, q_own, pos, n_own, h->n_right, true, n_top, d_ids, d_scores);
+}
+
+// Queries given as rating lists.  Validated and sorted by rs_given_prepare; left queries get their statistics (the
+// fitted rows' followed by the lists', one array) and, per batch, their S* rows.  The S* slab and the score slab
+// share the ~256 MiB budget.
+int32_t rs_given_launch(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids, const double *d_vals,
+                        int64_t n, double *d_out, int32_t n_top, int32_t *d_top_ids, double *d_top_scores) {
+    if (n <= 0) return RS_OK;
+    const bool left = side == RS_SIDE_LEFT;
+    const int64_t n_targets = left ? h->n_right : h->n_left;
+    rs_given_lists gl;
+    RS_TRY(rs_given_prepare(h, (int32_t)n_targets, d_ptr, d_ids, d_vals, n, &gl));
+    GivenBatch g{};
+    g.ids = gl.ids; g.vals = gl.vals; g.max_len = gl.max_len;
+    double *qpmeans = nullptr, *sslab = nullptr;
+    if (left) {
+        void *m, *sd, *pm;
+        const size_t rows = (size_t)h->n_left + (size_t)n;
+        RS_TRY(rs_scratch_get(h, 37, rows * 8, &m));
+        RS_TRY(rs_scratch_get(h, 38, rows * 8, &sd));
+        RS_TRY(rs_scratch_get(h, 39, (size_t)n * 8, &pm));
+        RS_CUDA(cudaMemcpyAsync(m, h->means, (size_t)h->n_left * 8, cudaMemcpyDeviceToDevice, h->stream));
+        RS_CUDA(cudaMemcpyAsync(sd, h->stddevs, (size_t)h->n_left * 8, cudaMemcpyDeviceToDevice, h->stream));
+        // core/knn.go:167-177 over the caller's order; Pearson's mean over ascending ids (core/sim.go:49-54)
+        RS_TRY(rs_row_stats_launch(h, gl.ptr, gl.vals_in, gl.vals, n, h->p.knn_type == RS_KNN_ZSCORE,
+                                   (double *)m + h->n_left, (double *)sd + h->n_left, (double *)pm));
+        g.means = (const double *)m; g.stddevs = (const double *)sd;
+        qpmeans = (double *)pm;
+    }
+    const int64_t width = n_targets + (left ? h->n_left : 0);
+    const int64_t batch = slab_batch(width, n);
+    void *slab = nullptr;
+    if (!d_out) RS_TRY(rs_scratch_get(h, 23, (size_t)batch * n_targets * 8, &slab));
+    if (left) {
+        void *ss;
+        RS_TRY(rs_scratch_get(h, 40, (size_t)batch * h->n_left * 8, &ss));
+        sslab = (double *)ss;
+    }
+    for (int64_t b0 = 0; b0 < n; b0 += batch) {
+        const int64_t nb = n - b0 < batch ? n - b0 : batch;
+        double *rows = d_out ? d_out + b0 * n_targets : (double *)slab;
+        RecArgs ra = rec_args(h, side, nullptr, nb, rows, n_targets);
+        ra.given = 1;
+        g.ptr = gl.ptr + b0;
+        if (left) {
+            RS_TRY(rs_given_sims_launch(h, g.ptr, gl.ids, gl.vals, qpmeans + b0, nb, sslab, h->n_left));
+            ra.gsims = sslab;
+            ra.ld_g = h->n_left;
+            ra.qstat = (int32_t)(h->n_left + b0);
+        }
+        RS_TRY(score_rows(h, ra, &g));
+        if (!d_out)
+            RS_TRY(rs_topk_rows_launch(h, rows, n_targets, (int32_t)n_targets, nb, n_top, d_top_ids + b0 * n_top,
+                                       d_top_scores + b0 * n_top));
+    }
+    return RS_OK;
 }

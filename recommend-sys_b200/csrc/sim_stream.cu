@@ -25,6 +25,7 @@
 #include <cstring>
 
 #include "common.cuh"
+#include "sim_terms.cuh"
 
 namespace {
 
@@ -60,20 +61,6 @@ struct StreamArgs {
 };
 
 constexpr int G = 8;   // columns whose first 32 raters are loaded together (must divide 32)
-
-template <int SIM, bool SHRINK, int JC>
-__device__ __forceinline__ void stream_update(double *acc, int j, double ra, double raa, double rb) {
-    if (SIM == RS_SIM_MSD) {
-        const double d = ra - rb;
-        acc[j] += d * d;                 // sum += (ir-jr)^2   core/sim.go:37
-        acc[JC + j] += 1.0;              // count++            core/sim.go:38
-    } else {
-        acc[j] += raa;                   // m += ..            core/sim.go:19 / :75
-        acc[JC + j] += rb * rb;          // n += rb*rb         core/sim.go:20 / :76
-        acc[2 * JC + j] += ra * rb;      // l += ra*rb         core/sim.go:21 / :77
-        if (SHRINK) acc[3 * JC + j] += 1.0;
-    }
-}
 
 // ---------------------------------------------------------------------------------------------
 // Popular columns.  The column walk below serialises a row's entries in ONE warp, so the few rows that a large
@@ -241,11 +228,8 @@ __device__ __forceinline__ void pop_item(const StreamArgs &a, const PopArgs &pa,
         if (pi >= 0 && col == pi) {
             out[hcol] = nan_v;                                                    // diagonal stays NaN
         } else if (want) {
-            double s;
-            if (SIM == RS_SIM_MSD) s = 1.0 / (acc0 / acc1 + 1.0);                              // core/sim.go:43
-            else s = acc2 / (sqrt(acc0) * sqrt(acc1));                                         // core/sim.go:24 / :80
-            if (SHRINK) s = (acc3 - 1.0) / (acc3 - 1.0 + a.shrinkage) * s;
-            out[hcol] = s;
+            const double acc_r[4] = {acc0, acc1, acc2, acc3};
+            out[hcol] = sim_value<SIM, SHRINK>(acc_r, 1, a.shrinkage);                        // core/sim.go:43 / :24 / :80
         }
     }
 }
@@ -388,13 +372,7 @@ __global__ void __launch_bounds__(SW * 32, 4) sim_stream_kernel(StreamArgs a, Po
         // hoist the bounds: fewer spills in each (profiles/r03_walk_labels.md)
         double *out = a.sims + (a.cyc_R > 1 ? rs_cyc_local(i, a.cyc_R) : (int64_t)(i - a.row_begin)) * a.ld_s + (POP ? 0 : j0);
         auto emit = [&](int j, int64_t col) {
-            double s;
-            if (SIM == RS_SIM_MSD) s = 1.0 / (acc[j] / acc[JC + j] + 1.0);        // core/sim.go:43
-            else s = acc[2 * JC + j] / (sqrt(acc[j]) * sqrt(acc[JC + j]));        // core/sim.go:24 / :80
-            if (SHRINK) {
-                const double cn = acc[3 * JC + j];
-                s = (cn - 1.0) / (cn - 1.0 + a.shrinkage) * s;
-            }
+            double s = sim_value<SIM, SHRINK>(acc + j, JC, a.shrinkage);                 // core/sim.go:43 / :24 / :80
             if (col == (int64_t)li) s = nan_v;                                    // diagonal stays NaN
             out[POP ? a.lab_row[col] : j] = s;
         };
@@ -557,13 +535,7 @@ __global__ void __launch_bounds__(HV_WARPS * 32, 1) sim_stream_heavy_kernel(Stre
                 if (col >= a.n_left) break;
                 if (a.symmetric == 1 && col < i) continue;                        // mirror pass writes it
                 if (a.symmetric == 2 && col > i) break;
-                double s;
-                if (SIM == RS_SIM_MSD) s = 1.0 / (acc[j] / acc[HV_JC + j] + 1.0);              // core/sim.go:43
-                else s = acc[2 * HV_JC + j] / (sqrt(acc[j]) * sqrt(acc[HV_JC + j]));           // core/sim.go:24 / :80
-                if (SHRINK) {
-                    const double cn = acc[3 * HV_JC + j];
-                    s = (cn - 1.0) / (cn - 1.0 + a.shrinkage) * s;
-                }
+                double s = sim_value<SIM, SHRINK>(acc + j, HV_JC, a.shrinkage);      // core/sim.go:43 / :24 / :80
                 if (col == (int64_t)i) s = nan_v;                                 // diagonal stays NaN
                 out[j] = s;
             }

@@ -230,6 +230,23 @@ func (d *deviceKNN) recommend(side int, queries []int32, nTop int) ([]int32, []f
 	return ids, scores
 }
 
+// recommendGiven: queries given as rating lists — list b is ids[ptr[b]:ptr[b+1]] (inner ids of the target side) with
+// ratings vals[...], in the caller's order (rs_knn_recommend_given).  ids / scores are [len(ptr)-1][nTop], row-major.
+func (d *deviceKNN) recommendGiven(side int, ptr []int64, ids []int32, vals []float64, nTop int) ([]int32, []float64) {
+	n := len(ptr) - 1
+	outIDs := make([]int32, n*nTop)
+	outScores := make([]float64, n*nTop)
+	if n <= 0 {
+		return outIDs, outScores
+	}
+	if len(ids) == 0 { // every list empty: the library still wants valid pointers
+		ids, vals = []int32{0}, []float64{0}
+	}
+	check(C.rs_knn_recommend_given(d.h, C.int32_t(side), (*C.int64_t)(unsafe.Pointer(&ptr[0])), i32(ids), f64(vals),
+		C.int64_t(n), C.int32_t(nTop), i32(outIDs), f64(outScores)))
+	return outIDs, outScores
+}
+
 // pinnedInt32 / pinnedFloat64: page-locked host memory of the library's per-process cache (rs_knn_host_alloc) viewed
 // as a Go slice, for callers that stage large batches themselves: copies from and to such memory run at full PCIe
 // speed.  The memory is C memory (no Go pointers in it); release returns the block to the cache.

@@ -179,6 +179,63 @@ func (K *KNN) Recommend(userIDs []int, n int) ([][]int, [][]float64) {
 	return items, scores
 }
 
+// RecommendGiven is Recommend for users whose ratings are given in dataSet (raw user, raw item, rating) instead of
+// taken from the train set: users who signed up or rated after Fit, or held-out ratings (core/eval.go NewAUC).  The
+// rows are grouped by user in order of first appearance, each user's ratings kept in dataset order; items the train
+// set does not know are dropped (they have no row or column of the model).  users[u] are the raw user ids, items /
+// scores as in Recommend; the given items are never listed.  The model is not refitted: the given ratings enter
+// neither the similarities between the train set's rows, nor its means, nor GlobalMean.
+func (K *KNN) RecommendGiven(dataSet DataSet, n int) ([]int, [][]int, [][]float64) {
+	group := map[int]int{}
+	var users []int
+	var lists [][]int
+	for j, u := range dataSet.Users {
+		g, ok := group[u]
+		if !ok {
+			g = len(users)
+			group[u] = g
+			users = append(users, u)
+			lists = append(lists, nil)
+		}
+		if K.Data.ConvertItemID(dataSet.Items[j]) != newID {
+			lists[g] = append(lists[g], j)
+		}
+	}
+	ptr := make([]int64, len(users)+1)
+	var ids []int32
+	var vals []float64
+	for g, rows := range lists {
+		for _, j := range rows {
+			ids = append(ids, int32(K.Data.ConvertItemID(dataSet.Items[j])))
+			vals = append(vals, dataSet.Ratings[j])
+		}
+		ptr[g+1] = int64(len(ids))
+	}
+	K.syncK()
+	side := sideLeft // user-based: the users are the left side, the lists hold right (item) ids
+	if !K.userBased {
+		side = sideRight
+	}
+	top, sc := K.dev.recommendGiven(side, ptr, ids, vals, n)
+	raw := make([]int, K.Data.ItemCount) // inner -> raw: the order of first appearance
+	for _, it := range K.Data.Items {
+		raw[K.Data.ConvertItemID(it)] = it
+	}
+	items := make([][]int, len(users))
+	scores := make([][]float64, len(users))
+	for i := range users {
+		items[i] = make([]int, n)
+		for x := 0; x < n; x++ {
+			items[i][x] = newID
+			if id := top[i*n+x]; id >= 0 {
+				items[i][x] = raw[id]
+			}
+		}
+		scores[i] = sc[i*n : (i+1)*n]
+	}
+	return users, items, scores
+}
+
 // Predict replaces core/knn.go:75-141 (a one-element batch).
 func (K *KNN) Predict(userID int, itemID int) float64 {
 	return K.PredictBatch([]int{userID}, []int{itemID})[0]

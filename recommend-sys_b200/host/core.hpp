@@ -262,6 +262,43 @@ struct KNN : Estimator {
         for (size_t j = 0; j < ids.size(); j++) items[j] = ids[j] >= 0 ? raw[ids[j]] : newID;
     }
 
+    // Recommend for users whose ratings are given in `given` (raw user, raw item, rating) instead of taken from the
+    // train set (rs_knn_recommend_given, not a refit): users in order of first appearance, each user's ratings in
+    // dataset order, items the train set does not know dropped; the given items are never listed.
+    void RecommendGiven(const DataSet &given, int n, std::vector<int64_t> &users, std::vector<int64_t> &items,
+                        std::vector<double> &scores) {
+        std::unordered_map<int64_t, size_t> group;
+        std::vector<std::vector<size_t>> rows;
+        users.clear();
+        for (size_t j = 0; j < given.Length(); j++) {
+            auto it = group.find(given.Users[j]);
+            if (it == group.end()) {
+                it = group.emplace(given.Users[j], users.size()).first;
+                users.push_back(given.Users[j]);
+                rows.emplace_back();
+            }
+            if (Data->ConvertItemID(given.Items[j]) != newID) rows[it->second].push_back(j);
+        }
+        std::vector<int64_t> ptr(1, 0);
+        std::vector<int32_t> ids;
+        std::vector<double> vals;
+        for (const auto &r : rows) {
+            for (size_t j : r) { ids.push_back(Data->ConvertItemID(given.Items[j])); vals.push_back(given.Ratings[j]); }
+            ptr.push_back((int64_t)ids.size());
+        }
+        if (ids.empty()) { ids.push_back(0); vals.push_back(0.0); }   // every list empty: valid pointers all the same
+        SyncK();
+        std::vector<int32_t> top(users.size() * (size_t)n);
+        scores.assign(top.size(), 0.0);
+        if (!users.empty())
+            rs_check(rs_knn_recommend_given(h_, userBased_ ? RS_SIDE_LEFT : RS_SIDE_RIGHT, ptr.data(), ids.data(),
+                                            vals.data(), (int64_t)users.size(), n, top.data(), scores.data()));
+        std::vector<int64_t> raw(Data->ItemCount);          // inner -> raw: the order of first appearance
+        for (size_t j = 0; j < Data->Length(); j++) raw[Data->innerItems[j]] = Data->Items[j];
+        items.resize(top.size());
+        for (size_t j = 0; j < top.size(); j++) items[j] = top[j] >= 0 ? raw[top[j]] : newID;
+    }
+
     std::vector<double> SimsRows(int64_t row0, int64_t nrows) {  // backs KNN.Sims (core/knn.go:21)
         std::vector<double> out((size_t)nrows * nLeft_);
         rs_check(rs_knn_sims_rows(h_, row0, nrows, out.data()));

@@ -3,6 +3,8 @@
 //
 //   recommend <ratings file: user<TAB>item<TAB>rating per line> <cosine|msd|pearson> <basic|centered|zscore|baseline>
 //             <userBased 0|1> <k> <n> <user> [<user> ...]
+//   recommend ... <k> <n> --given <ratings file>   (KNN::RecommendGiven: the users of the second file, with the
+//             ratings given there instead of the train set's; one line per user in order of first appearance)
 //
 // The estimator is fitted with k = 40 and `k` is set afterwards (Predict reads k at call time, core/knn.go:80-81).
 // One output line per user: the user id, then n pairs "item score", the score as the 16 hex digits of its bits.
@@ -47,10 +49,14 @@ int main(int argc, char **argv) {
     knn.Params.Set("k", std::atoi(argv[5]));
     const int n = std::atoi(argv[6]);
     std::vector<int64_t> users;
-    for (int a = 7; a < argc; a++) users.push_back(std::atoll(argv[a]));
     std::vector<int64_t> items;
     std::vector<double> scores;
-    knn.Recommend(users, n, items, scores);
+    if (!std::strcmp(argv[7], "--given") && argc == 9) {
+        knn.RecommendGiven(load_file(argv[8]), n, users, items, scores);
+    } else {
+        for (int a = 7; a < argc; a++) users.push_back(std::atoll(argv[a]));
+        knn.Recommend(users, n, items, scores);
+    }
     for (size_t u = 0; u < users.size(); u++) {
         std::printf("%" PRId64, users[u]);
         for (int x = 0; x < n; x++) {

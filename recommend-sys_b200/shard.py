@@ -307,5 +307,13 @@ class ShardedKNN:
             dist.all_reduce(out.view(torch.int64), op=dist.ReduceOp.SUM, group=self.group)
         return out.cpu().numpy()
 
+    def ScoreAllGiven(self, dataSet):
+        """KNN.ScoreAllGiven is not available on row shards yet (the library refuses them)."""
+        raise NotImplementedError("ScoreAllGiven: row-sharded handles are not supported; use an unsharded KNN")
+
+    def RecommendGiven(self, dataSet, n):
+        """KNN.RecommendGiven is not available on row shards yet (the library refuses them)."""
+        raise NotImplementedError("RecommendGiven: row-sharded handles are not supported; use an unsharded KNN")
+
     def Close(self):
         self.knn.Close()
