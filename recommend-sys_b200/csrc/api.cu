@@ -556,18 +556,18 @@ int32_t rs_knn_fit(rs_knn *h, const int32_t *left, const int32_t *right, const d
     }
     // persistent device staging (grow-only): a refit of the same size allocates nothing
     void *d_left, *d_right, *d_rating, *d_lb = nullptr, *d_rb = nullptr;
-    RS_TRY(rs_scratch_get(h, 7, (size_t)nnz * 4, &d_left));
-    RS_TRY(rs_scratch_get(h, 8, (size_t)nnz * 4, &d_right));
-    RS_TRY(rs_scratch_get(h, 9, (size_t)nnz * 8, &d_rating));
+    RS_TRY(rs_scratch_get(h, RS_SCR_FIT_LEFT, (size_t)nnz * 4, &d_left));
+    RS_TRY(rs_scratch_get(h, RS_SCR_FIT_RIGHT, (size_t)nnz * 4, &d_right));
+    RS_TRY(rs_scratch_get(h, RS_SCR_FIT_RATING, (size_t)nnz * 8, &d_rating));
     RS_CUDA(cudaMemcpyAsync(d_left, left, (size_t)nnz * 4, cudaMemcpyHostToDevice, h->stream));
     RS_CUDA(cudaMemcpyAsync(d_right, right, (size_t)nnz * 4, cudaMemcpyHostToDevice, h->stream));
     RS_CUDA(cudaMemcpyAsync(d_rating, rating, (size_t)nnz * 8, cudaMemcpyHostToDevice, h->stream));
     if (left_bias) {
-        RS_TRY(rs_scratch_get(h, 10, (size_t)n_left * 8, &d_lb));
+        RS_TRY(rs_scratch_get(h, RS_SCR_FIT_LEFT_BIAS, (size_t)n_left * 8, &d_lb));
         RS_CUDA(cudaMemcpyAsync(d_lb, left_bias, (size_t)n_left * 8, cudaMemcpyHostToDevice, h->stream));
     }
     if (right_bias) {
-        RS_TRY(rs_scratch_get(h, 11, (size_t)n_right * 8, &d_rb));
+        RS_TRY(rs_scratch_get(h, RS_SCR_FIT_RIGHT_BIAS, (size_t)n_right * 8, &d_rb));
         RS_CUDA(cudaMemcpyAsync(d_rb, right_bias, (size_t)n_right * 8, cudaMemcpyHostToDevice, h->stream));
     }
     RS_CUDA(cudaEventRecord(h->ev_in, h->stream));
@@ -652,9 +652,9 @@ int32_t rs_knn_predict_batch(rs_knn *h, const int32_t *left, const int32_t *righ
         return RS_ERR_INVALID;
     }
     void *dl, *dr, *dout;
-    RS_TRY(rs_scratch_get(h, 0, (size_t)n * 4, &dl));
-    RS_TRY(rs_scratch_get(h, 1, (size_t)n * 4, &dr));
-    RS_TRY(rs_scratch_get(h, 2, (size_t)n * 8, &dout));
+    RS_TRY(rs_scratch_get(h, RS_SCR_PRED_LEFT, (size_t)n * 4, &dl));
+    RS_TRY(rs_scratch_get(h, RS_SCR_PRED_RIGHT, (size_t)n * 4, &dr));
+    RS_TRY(rs_scratch_get(h, RS_SCR_PRED_OUT, (size_t)n * 8, &dout));
     RS_CUDA(cudaMemcpyAsync(dl, left, (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
     RS_CUDA(cudaMemcpyAsync(dr, right, (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
     RS_TRY(rs_knn_predict_batch_device(h, (const int32_t *)dl, (const int32_t *)dr, n, (double *)dout));
@@ -672,12 +672,12 @@ int32_t rs_knn_predict_neighbors(rs_knn *h, int32_t left, int32_t right, int32_t
         return RS_ERR_INVALID;
     }
     void *dl, *dr, *dout, *dids, *dsims, *dcnt;
-    RS_TRY(rs_scratch_get(h, 0, 4, &dl));
-    RS_TRY(rs_scratch_get(h, 1, 4, &dr));
-    RS_TRY(rs_scratch_get(h, 2, 8, &dout));
-    RS_TRY(rs_scratch_get(h, 3, (size_t)cap * 4, &dids));
-    RS_TRY(rs_scratch_get(h, 4, (size_t)cap * 8, &dsims));
-    RS_TRY(rs_scratch_get(h, 5, 4, &dcnt));
+    RS_TRY(rs_scratch_get(h, RS_SCR_PRED_LEFT, 4, &dl));
+    RS_TRY(rs_scratch_get(h, RS_SCR_PRED_RIGHT, 4, &dr));
+    RS_TRY(rs_scratch_get(h, RS_SCR_PRED_OUT, 8, &dout));
+    RS_TRY(rs_scratch_get(h, RS_SCR_HOST_IDS, (size_t)cap * 4, &dids));
+    RS_TRY(rs_scratch_get(h, RS_SCR_HOST_SIMS, (size_t)cap * 8, &dsims));
+    RS_TRY(rs_scratch_get(h, RS_SCR_NB_COUNT, 4, &dcnt));
     RS_CUDA(cudaMemcpyAsync(dl, &left, 4, cudaMemcpyHostToDevice, h->stream));
     RS_CUDA(cudaMemcpyAsync(dr, &right, 4, cudaMemcpyHostToDevice, h->stream));
     RS_CUDA(cudaMemsetAsync(dcnt, 0, 4, h->stream));
@@ -695,168 +695,48 @@ int32_t rs_knn_predict_neighbors(rs_knn *h, int32_t left, int32_t right, int32_t
     return RS_OK;
 }
 
-// What every recommend entry point checks: the handle holds the whole matrix (the _sharded entry points: a row
-// shard, mirrored if cyclic), the query side exists, k fits.
-static int32_t require_recommend(rs_knn *h, const char *who, int32_t side, int64_t n, bool sharded = false) {
+// Every check of the recommendation entry points, in the order they fire: the handle holds the whole matrix (the
+// _sharded entry points: a row shard, mirrored if cyclic), the query side exists, k fits, and for lists what
+// rs_knn_recommend accepts less top-k-only handles (checked first) and, for left queries, the models that need
+// something of the query the lists do not give (a baseline bias) or whose matrix is not the exact replay the lists'
+// similarity rows are (Pearson sums).  Pointers are checked only when n > 0.
+static int32_t check_recommend(rs_knn *h, const char *who, const rs_rec_call &c) {
+    if (c.given && h->fitted && h->p.store == RS_STORE_TOPK) {
+        rs_set_error("%s needs RS_STORE_MATRIX (the handle keeps top-k lists only)", who);
+        return RS_ERR_UNSUPPORTED;
+    }
     if (!h->fitted) {
         rs_set_error("%s: Fit has not been called", who);
         return RS_ERR_INVALID;
     }
     if (h->p.store != RS_STORE_MATRIX) return require_matrix(h, who);
     const bool row_shard = h->cyc_R > 1 || h->p.shard_count > 1 || h->row_begin != 0 || h->row_end != h->n_left;
-    if (!sharded && row_shard) {
+    if (!c.sharded && row_shard) {
         rs_set_error("%s needs a handle that holds every row (no row_begin/row_end shard, shard_count <= 1)", who);
         return RS_ERR_UNSUPPORTED;
     }
-    if (sharded && !row_shard) {
+    if (c.sharded && !row_shard) {
         rs_set_error("%s: the handle holds every row, not a row shard (use the plain entry point)", who);
         return RS_ERR_INVALID;
     }
-    if (sharded) RS_TRY(require_matrix(h, who));
+    if (c.sharded) RS_TRY(require_matrix(h, who));
     if (h->p.sim == RS_SIM_SLOPE_ONE) {
         rs_set_error("%s: Slope One is not supported", who);
         return RS_ERR_UNSUPPORTED;
     }
-    if (side != RS_SIDE_LEFT && side != RS_SIDE_RIGHT) {
-        rs_set_error("%s: side must be RS_SIDE_LEFT or RS_SIDE_RIGHT (got %d)", who, side);
+    if (c.side != RS_SIDE_LEFT && c.side != RS_SIDE_RIGHT) {
+        rs_set_error("%s: side must be RS_SIDE_LEFT or RS_SIDE_RIGHT (got %d)", who, c.side);
         return RS_ERR_INVALID;
     }
     if (h->p.k > 256) {
         rs_set_error("%s: k=%d exceeds the 256 neighbours the predict kernel supports", who, h->p.k);
         return RS_ERR_UNSUPPORTED;
     }
-    if (n < 0 || n >= (1ll << 31)) {
-        rs_set_error("%s: n=%lld outside [0, 2^31)", who, (long long)n);
+    if (c.n < 0 || c.n >= (1ll << 31)) {
+        rs_set_error("%s: n=%lld outside [0, 2^31)", who, (long long)c.n);
         return RS_ERR_INVALID;
     }
-    return RS_OK;
-}
-
-static int32_t check_n_top(const char *who, int32_t n_top) {
-    if (n_top < 1 || n_top > 512) {
-        rs_set_error("%s: n_top=%d outside [1, 512]", who, n_top);
-        return RS_ERR_INVALID;
-    }
-    return RS_OK;
-}
-
-// host variants: ids outside [-1, n_side) are refused
-static int32_t check_queries(rs_knn *h, const char *who, int32_t side, const int32_t *q, int64_t n) {
-    const int32_t n_side = side == RS_SIDE_RIGHT ? h->n_right : h->n_left;
-    for (int64_t i = 0; i < n; i++) {
-        if (q[i] < -1 || q[i] >= n_side) {
-            rs_set_error("%s: query %lld = %d outside [-1, %d)", who, (long long)i, q[i], n_side);
-            return RS_ERR_INVALID;
-        }
-    }
-    return RS_OK;
-}
-
-static int64_t n_targets_of(const rs_knn *h, int32_t side) { return side == RS_SIDE_RIGHT ? h->n_left : h->n_right; }
-
-int32_t rs_knn_score_all_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n, double *d_out) {
-    RS_ENTER(h);
-    RS_TRY(require_recommend(h, "rs_knn_score_all", side, n));
-    if (n == 0) return RS_OK;
-    if (!d_queries || !d_out) {
-        rs_set_error("rs_knn_score_all: null argument");
-        return RS_ERR_INVALID;
-    }
-    return rs_score_all_launch(h, side, d_queries, n, d_out);
-}
-
-int32_t rs_knn_score_all(rs_knn *h, int32_t side, const int32_t *queries, int64_t n, double *out) {
-    RS_ENTER(h);
-    RS_TRY(require_recommend(h, "rs_knn_score_all", side, n));
-    if (n == 0) return RS_OK;
-    if (!queries || !out) {
-        rs_set_error("rs_knn_score_all: null argument");
-        return RS_ERR_INVALID;
-    }
-    RS_TRY(check_queries(h, "rs_knn_score_all", side, queries, n));
-    const size_t bytes = (size_t)n * n_targets_of(h, side) * 8;
-    void *dq, *dout;
-    RS_TRY(rs_scratch_get(h, 20, (size_t)n * 4, &dq));
-    RS_TRY(rs_scratch_get(h, 21, bytes, &dout));
-    RS_CUDA(cudaMemcpyAsync(dq, queries, (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
-    RS_TRY(rs_score_all_launch(h, side, (const int32_t *)dq, n, (double *)dout));
-    RS_CUDA(cudaMemcpyAsync(out, dout, bytes, cudaMemcpyDeviceToHost, h->stream));
-    RS_CUDA(cudaStreamSynchronize(h->stream));
-    return RS_OK;
-}
-
-int32_t rs_knn_recommend_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n, int32_t n_top,
-                                int32_t *d_ids, double *d_scores) {
-    RS_ENTER(h);
-    RS_TRY(require_recommend(h, "rs_knn_recommend", side, n));
-    RS_TRY(check_n_top("rs_knn_recommend", n_top));
-    if (n == 0) return RS_OK;
-    if (!d_queries || !d_ids || !d_scores) {
-        rs_set_error("rs_knn_recommend: null argument");
-        return RS_ERR_INVALID;
-    }
-    return rs_recommend_launch(h, side, d_queries, n, n_top, d_ids, d_scores);
-}
-
-int32_t rs_knn_recommend(rs_knn *h, int32_t side, const int32_t *queries, int64_t n, int32_t n_top, int32_t *ids,
-                         double *scores) {
-    RS_ENTER(h);
-    RS_TRY(require_recommend(h, "rs_knn_recommend", side, n));
-    RS_TRY(check_n_top("rs_knn_recommend", n_top));
-    if (n == 0) return RS_OK;
-    if (!queries || !ids || !scores) {
-        rs_set_error("rs_knn_recommend: null argument");
-        return RS_ERR_INVALID;
-    }
-    RS_TRY(check_queries(h, "rs_knn_recommend", side, queries, n));
-    void *dq, *di, *ds;
-    RS_TRY(rs_scratch_get(h, 20, (size_t)n * 4, &dq));
-    RS_TRY(rs_scratch_get(h, 21, (size_t)n * n_top * 4, &di));
-    RS_TRY(rs_scratch_get(h, 22, (size_t)n * n_top * 8, &ds));
-    RS_CUDA(cudaMemcpyAsync(dq, queries, (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
-    RS_TRY(rs_recommend_launch(h, side, (const int32_t *)dq, n, n_top, (int32_t *)di, (double *)ds));
-    RS_CUDA(cudaMemcpyAsync(ids, di, (size_t)n * n_top * 4, cudaMemcpyDeviceToHost, h->stream));
-    RS_CUDA(cudaMemcpyAsync(scores, ds, (size_t)n * n_top * 8, cudaMemcpyDeviceToHost, h->stream));
-    RS_CUDA(cudaStreamSynchronize(h->stream));
-    return RS_OK;
-}
-
-int32_t rs_knn_score_all_sharded_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n,
-                                        double *d_out) {
-    RS_ENTER(h);
-    RS_TRY(require_recommend(h, "rs_knn_score_all_sharded", side, n, true));
-    if (n == 0) return RS_OK;
-    if (!d_queries || !d_out) {
-        rs_set_error("rs_knn_score_all_sharded: null argument");
-        return RS_ERR_INVALID;
-    }
-    return rs_score_all_sharded_launch(h, side, d_queries, n, d_out);
-}
-
-int32_t rs_knn_recommend_sharded_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n, int32_t n_top,
-                                        int32_t *d_ids, double *d_scores) {
-    RS_ENTER(h);
-    RS_TRY(require_recommend(h, "rs_knn_recommend_sharded", side, n, true));
-    RS_TRY(check_n_top("rs_knn_recommend_sharded", n_top));
-    if (n == 0) return RS_OK;
-    if (!d_queries || !d_ids || !d_scores) {
-        rs_set_error("rs_knn_recommend_sharded: null argument");
-        return RS_ERR_INVALID;
-    }
-    return rs_recommend_sharded_launch(h, side, d_queries, n, n_top, d_ids, d_scores);
-}
-
-// Queries given as rating lists: what rs_knn_recommend accepts, less top-k-only handles, and for left queries the
-// models that need something of the query the lists do not give (a baseline bias) or whose matrix is not the exact
-// replay the lists' similarity rows are (Pearson sums).
-static int32_t require_given(rs_knn *h, const char *who, int32_t side, int64_t n, const void *ptr, const void *ids,
-                             const void *vals, const void *out0, const void *out1) {
-    if (h->fitted && h->p.store == RS_STORE_TOPK) {
-        rs_set_error("%s needs RS_STORE_MATRIX (the handle keeps top-k lists only)", who);
-        return RS_ERR_UNSUPPORTED;
-    }
-    RS_TRY(require_recommend(h, who, side, n));
-    if (side == RS_SIDE_LEFT) {
+    if (c.given && c.side == RS_SIDE_LEFT) {
         if (h->p.knn_type == RS_KNN_BASELINE || h->p.sim == RS_SIM_PEARSON_BASELINE) {
             rs_set_error("%s: left queries have no baseline bias (RS_KNN_BASELINE / RS_SIM_PEARSON_BASELINE)", who);
             return RS_ERR_UNSUPPORTED;
@@ -865,106 +745,169 @@ static int32_t require_given(rs_knn *h, const char *who, int32_t side, int64_t n
             rs_set_error("%s: left queries need the exact Pearson matrix (pearson_mode EXACT)", who);
             return RS_ERR_UNSUPPORTED;
         }
-        if ((int64_t)h->n_left + n >= (1ll << 31)) {
-            rs_set_error("%s: n_left + n = %lld (at most 2^31 - 1)", who, (long long)h->n_left + n);
+        if ((int64_t)h->n_left + c.n >= (1ll << 31)) {
+            rs_set_error("%s: n_left + n = %lld (at most 2^31 - 1)", who, (long long)h->n_left + c.n);
             return RS_ERR_UNSUPPORTED;
         }
     }
-    if (n > 0 && (!ptr || !ids || !vals || !out0 || !out1)) {
+    if (c.lists && (c.n_top < 1 || c.n_top > 512)) {
+        rs_set_error("%s: n_top=%d outside [1, 512]", who, c.n_top);
+        return RS_ERR_INVALID;
+    }
+    const bool null_in = c.given ? !c.ptr || !c.ids || !c.vals : !c.queries;
+    const bool null_out = c.lists ? !c.top_ids || !c.top_scores : !c.rows;
+    if (c.n > 0 && (null_in || null_out)) {
         rs_set_error("%s: null argument", who);
         return RS_ERR_INVALID;
     }
     return RS_OK;
 }
 
-int32_t rs_knn_score_all_given_device(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids,
-                                      const double *d_vals, int64_t n, double *d_out) {
-    RS_ENTER(h);
-    RS_TRY(require_given(h, "rs_knn_score_all_given", side, n, d_ptr, d_ids, d_vals, d_out, d_out));
-    if (n == 0) return RS_OK;
-    return rs_given_launch(h, side, d_ptr, d_ids, d_vals, n, d_out, 0, nullptr, nullptr);
-}
-
-int32_t rs_knn_recommend_given_device(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids,
-                                      const double *d_vals, int64_t n, int32_t n_top, int32_t *d_top_ids,
-                                      double *d_top_scores) {
-    RS_ENTER(h);
-    RS_TRY(require_given(h, "rs_knn_recommend_given", side, n, d_ptr, d_ids, d_vals, d_top_ids, d_top_scores));
-    RS_TRY(check_n_top("rs_knn_recommend_given", n_top));
-    if (n == 0) return RS_OK;
-    return rs_given_launch(h, side, d_ptr, d_ids, d_vals, n, nullptr, n_top, d_top_ids, d_top_scores);
-}
-
-// host variants: ptr is checked here (it sizes the copies), the entries on the device as in the _device variants
-static int32_t stage_given(rs_knn *h, const char *who, const int64_t *ptr, const int32_t *ids, const double *vals,
-                           int64_t n, const int64_t **d_ptr, const int32_t **d_ids, const double **d_vals) {
-    if (ptr[0] < 0) {
-        rs_set_error("%s: ptr[0] = %lld < 0", who, (long long)ptr[0]);
+// Host variants: the queries to the device.  Ids outside [-1, n_side) are refused (the _device variants score them
+// as -1).  Of the lists, ptr is checked only as far as it sizes the copies; the device checks the rest as it does for
+// the _device variants.
+static int32_t stage_queries(rs_knn *h, const char *who, rs_rec_call &c) {
+    if (!c.given) {
+        const int32_t n_side = c.side == RS_SIDE_RIGHT ? h->n_right : h->n_left;
+        for (int64_t i = 0; i < c.n; i++) {
+            if (c.queries[i] < -1 || c.queries[i] >= n_side) {
+                rs_set_error("%s: query %lld = %d outside [-1, %d)", who, (long long)i, c.queries[i], n_side);
+                return RS_ERR_INVALID;
+            }
+        }
+        void *dq;
+        RS_TRY(rs_scratch_get(h, RS_SCR_REC_QUERIES, (size_t)c.n * 4, &dq));
+        RS_CUDA(cudaMemcpyAsync(dq, c.queries, (size_t)c.n * 4, cudaMemcpyHostToDevice, h->stream));
+        c.queries = (const int32_t *)dq;
+        return RS_OK;
+    }
+    const int64_t p0 = c.ptr[0], nnz = c.ptr[c.n] - p0;
+    if (p0 < 0 || nnz < 0) {
+        rs_set_error("%s: ptr[0] = %lld, ptr[n] = %lld (need 0 <= ptr[0] <= ptr[n])", who, (long long)p0,
+                     (long long)c.ptr[c.n]);
         return RS_ERR_INVALID;
     }
-    for (int64_t b = 0; b < n; b++) {
-        if (ptr[b + 1] < ptr[b]) {
-            rs_set_error("%s: ptr is not non-decreasing at list %lld", who, (long long)b);
-            return RS_ERR_INVALID;
-        }
-    }
-    const int64_t p0 = ptr[0], nnz = ptr[n] - p0;
     if (nnz >= (1ll << 31)) {
         rs_set_error("%s: %lld entries (at most 2^31 - 1 per call)", who, (long long)nnz);
         return RS_ERR_UNSUPPORTED;
     }
     void *dp, *di, *dv;
-    RS_TRY(rs_scratch_get(h, 42, (size_t)(n + 1) * 8, &dp));
-    RS_TRY(rs_scratch_get(h, 43, (size_t)nnz * 4 + 4, &di));
-    RS_TRY(rs_scratch_get(h, 44, (size_t)nnz * 8 + 8, &dv));
-    RS_CUDA(cudaMemcpyAsync(dp, ptr, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, h->stream));
+    RS_TRY(rs_scratch_get(h, RS_SCR_REC_PTR, (size_t)(c.n + 1) * 8, &dp));
+    RS_TRY(rs_scratch_get(h, RS_SCR_REC_IDS, (size_t)nnz * 4 + 4, &di));
+    RS_TRY(rs_scratch_get(h, RS_SCR_REC_VALS, (size_t)nnz * 8 + 8, &dv));
+    RS_CUDA(cudaMemcpyAsync(dp, c.ptr, (size_t)(c.n + 1) * 8, cudaMemcpyHostToDevice, h->stream));
     if (nnz > 0) {
-        RS_CUDA(cudaMemcpyAsync(di, ids + p0, (size_t)nnz * 4, cudaMemcpyHostToDevice, h->stream));
-        RS_CUDA(cudaMemcpyAsync(dv, vals + p0, (size_t)nnz * 8, cudaMemcpyHostToDevice, h->stream));
+        RS_CUDA(cudaMemcpyAsync(di, c.ids + p0, (size_t)nnz * 4, cudaMemcpyHostToDevice, h->stream));
+        RS_CUDA(cudaMemcpyAsync(dv, c.vals + p0, (size_t)nnz * 8, cudaMemcpyHostToDevice, h->stream));
     }
     // the device copies hold the entries from ptr[0] on: index them from ptr[0]
-    *d_ptr = (const int64_t *)dp;
-    *d_ids = (const int32_t *)di - p0;
-    *d_vals = (const double *)dv - p0;
+    c.ptr = (const int64_t *)dp;
+    c.ids = (const int32_t *)di - p0;
+    c.vals = (const double *)dv - p0;
     return RS_OK;
+}
+
+// The call descriptions of the ten shims.
+static rs_rec_call by_id(int32_t side, const int32_t *queries, int64_t n, bool sharded) {
+    rs_rec_call c{};
+    c.side = side; c.sharded = sharded; c.queries = queries; c.n = n;
+    return c;
+}
+
+static rs_rec_call by_lists(int32_t side, const int64_t *ptr, const int32_t *ids, const double *vals, int64_t n) {
+    rs_rec_call c{};
+    c.side = side; c.given = true; c.ptr = ptr; c.ids = ids; c.vals = vals; c.n = n;
+    return c;
+}
+
+static rs_rec_call with_rows(rs_rec_call c, double *out) {
+    c.rows = out;
+    return c;
+}
+
+static rs_rec_call with_lists(rs_rec_call c, int32_t n_top, int32_t *ids, double *scores) {
+    c.lists = true; c.n_top = n_top; c.top_ids = ids; c.top_scores = scores;
+    return c;
+}
+
+// The one entry of the ten: checks, then the driver; host variants stage their inputs and copy the outputs back.
+static int32_t recommend(rs_knn *h, const char *who, rs_rec_call c, bool host) {
+    RS_ENTER(h);
+    RS_TRY(check_recommend(h, who, c));
+    if (c.n == 0) return RS_OK;
+    if (!host) return rs_recommend_run(h, c);
+    RS_TRY(stage_queries(h, who, c));
+    const rs_rec_call caller = c;   // the host outputs
+    const size_t cells = c.lists ? (size_t)c.n * c.n_top : (size_t)c.n * rs_n_targets(h, c.side);
+    void *d_out, *d_scores = nullptr;
+    RS_TRY(rs_scratch_get(h, RS_SCR_REC_OUT, cells * (c.lists ? 4 : 8), &d_out));
+    if (c.lists) {
+        RS_TRY(rs_scratch_get(h, RS_SCR_REC_SCORES, cells * 8, &d_scores));
+        c = with_lists(c, c.n_top, (int32_t *)d_out, (double *)d_scores);
+    } else {
+        c = with_rows(c, (double *)d_out);
+    }
+    RS_TRY(rs_recommend_run(h, c));
+    if (c.lists) {
+        RS_CUDA(cudaMemcpyAsync(caller.top_ids, d_out, cells * 4, cudaMemcpyDeviceToHost, h->stream));
+        RS_CUDA(cudaMemcpyAsync(caller.top_scores, d_scores, cells * 8, cudaMemcpyDeviceToHost, h->stream));
+    } else {
+        RS_CUDA(cudaMemcpyAsync(caller.rows, d_out, cells * 8, cudaMemcpyDeviceToHost, h->stream));
+    }
+    RS_CUDA(cudaStreamSynchronize(h->stream));
+    return RS_OK;
+}
+
+int32_t rs_knn_score_all_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n, double *d_out) {
+    return recommend(h, "rs_knn_score_all", with_rows(by_id(side, d_queries, n, false), d_out), false);
+}
+
+int32_t rs_knn_score_all(rs_knn *h, int32_t side, const int32_t *queries, int64_t n, double *out) {
+    return recommend(h, "rs_knn_score_all", with_rows(by_id(side, queries, n, false), out), true);
+}
+
+int32_t rs_knn_recommend_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n, int32_t n_top,
+                                int32_t *d_ids, double *d_scores) {
+    return recommend(h, "rs_knn_recommend", with_lists(by_id(side, d_queries, n, false), n_top, d_ids, d_scores), false);
+}
+
+int32_t rs_knn_recommend(rs_knn *h, int32_t side, const int32_t *queries, int64_t n, int32_t n_top, int32_t *ids,
+                         double *scores) {
+    return recommend(h, "rs_knn_recommend", with_lists(by_id(side, queries, n, false), n_top, ids, scores), true);
+}
+
+int32_t rs_knn_score_all_sharded_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n,
+                                        double *d_out) {
+    return recommend(h, "rs_knn_score_all_sharded", with_rows(by_id(side, d_queries, n, true), d_out), false);
+}
+
+int32_t rs_knn_recommend_sharded_device(rs_knn *h, int32_t side, const int32_t *d_queries, int64_t n, int32_t n_top,
+                                        int32_t *d_ids, double *d_scores) {
+    return recommend(h, "rs_knn_recommend_sharded", with_lists(by_id(side, d_queries, n, true), n_top, d_ids, d_scores),
+                     false);
+}
+
+int32_t rs_knn_score_all_given_device(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids,
+                                      const double *d_vals, int64_t n, double *d_out) {
+    return recommend(h, "rs_knn_score_all_given", with_rows(by_lists(side, d_ptr, d_ids, d_vals, n), d_out), false);
+}
+
+int32_t rs_knn_recommend_given_device(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids,
+                                      const double *d_vals, int64_t n, int32_t n_top, int32_t *d_top_ids,
+                                      double *d_top_scores) {
+    return recommend(h, "rs_knn_recommend_given",
+                     with_lists(by_lists(side, d_ptr, d_ids, d_vals, n), n_top, d_top_ids, d_top_scores), false);
 }
 
 int32_t rs_knn_score_all_given(rs_knn *h, int32_t side, const int64_t *ptr, const int32_t *ids, const double *vals,
                                int64_t n, double *out) {
-    RS_ENTER(h);
-    RS_TRY(require_given(h, "rs_knn_score_all_given", side, n, ptr, ids, vals, out, out));
-    if (n == 0) return RS_OK;
-    const int64_t *dp;
-    const int32_t *di;
-    const double *dv;
-    RS_TRY(stage_given(h, "rs_knn_score_all_given", ptr, ids, vals, n, &dp, &di, &dv));
-    const size_t bytes = (size_t)n * n_targets_of(h, side) * 8;
-    void *dout;
-    RS_TRY(rs_scratch_get(h, 45, bytes, &dout));
-    RS_TRY(rs_given_launch(h, side, dp, di, dv, n, (double *)dout, 0, nullptr, nullptr));
-    RS_CUDA(cudaMemcpyAsync(out, dout, bytes, cudaMemcpyDeviceToHost, h->stream));
-    RS_CUDA(cudaStreamSynchronize(h->stream));
-    return RS_OK;
+    return recommend(h, "rs_knn_score_all_given", with_rows(by_lists(side, ptr, ids, vals, n), out), true);
 }
 
 int32_t rs_knn_recommend_given(rs_knn *h, int32_t side, const int64_t *ptr, const int32_t *ids, const double *vals,
                                int64_t n, int32_t n_top, int32_t *top_ids, double *top_scores) {
-    RS_ENTER(h);
-    RS_TRY(require_given(h, "rs_knn_recommend_given", side, n, ptr, ids, vals, top_ids, top_scores));
-    RS_TRY(check_n_top("rs_knn_recommend_given", n_top));
-    if (n == 0) return RS_OK;
-    const int64_t *dp;
-    const int32_t *di;
-    const double *dv;
-    RS_TRY(stage_given(h, "rs_knn_recommend_given", ptr, ids, vals, n, &dp, &di, &dv));
-    void *d_i, *d_s;
-    RS_TRY(rs_scratch_get(h, 45, (size_t)n * n_top * 4, &d_i));
-    RS_TRY(rs_scratch_get(h, 46, (size_t)n * n_top * 8, &d_s));
-    RS_TRY(rs_given_launch(h, side, dp, di, dv, n, nullptr, n_top, (int32_t *)d_i, (double *)d_s));
-    RS_CUDA(cudaMemcpyAsync(top_ids, d_i, (size_t)n * n_top * 4, cudaMemcpyDeviceToHost, h->stream));
-    RS_CUDA(cudaMemcpyAsync(top_scores, d_s, (size_t)n * n_top * 8, cudaMemcpyDeviceToHost, h->stream));
-    RS_CUDA(cudaStreamSynchronize(h->stream));
-    return RS_OK;
+    return recommend(h, "rs_knn_recommend_given", with_lists(by_lists(side, ptr, ids, vals, n), n_top, top_ids, top_scores),
+                     true);
 }
 
 int32_t rs_knn_sims_rows(rs_knn *h, int64_t row0, int64_t nrows, double *out) {
@@ -1022,8 +965,8 @@ int32_t rs_knn_topk(rs_knn *h, int32_t k, int32_t *idx, double *sim) {
     }
     const int64_t rows = h->p.store == RS_STORE_TOPK ? h->topk_rows : h->rows_local;
     void *di, *ds;
-    RS_TRY(rs_scratch_get(h, 3, (size_t)rows * k * 4, &di));
-    RS_TRY(rs_scratch_get(h, 4, (size_t)rows * k * 8, &ds));
+    RS_TRY(rs_scratch_get(h, RS_SCR_HOST_IDS, (size_t)rows * k * 4, &di));
+    RS_TRY(rs_scratch_get(h, RS_SCR_HOST_SIMS, (size_t)rows * k * 8, &ds));
     RS_TRY(rs_knn_topk_device(h, k, (int32_t *)di, (double *)ds));
     RS_CUDA(cudaMemcpyAsync(idx, di, (size_t)rows * k * 4, cudaMemcpyDeviceToHost, h->stream));
     RS_CUDA(cudaMemcpyAsync(sim, ds, (size_t)rows * k * 8, cudaMemcpyDeviceToHost, h->stream));
@@ -1045,7 +988,7 @@ int32_t rs_knn_cosums(rs_knn *h, int64_t row0, int64_t nrows, int32_t *out) {
     if (!h->planes) RS_TRY(rs_prep_planes(h));
     void *d;
     const size_t bytes = (size_t)nrows * (size_t)h->n_left * 6 * 4;
-    RS_TRY(rs_scratch_get(h, 6, bytes, &d));
+    RS_TRY(rs_scratch_get(h, RS_SCR_COSUMS, bytes, &d));
     RS_TRY(rs_sim_tensor_launch(h, (int32_t *)d, row0, nrows));
     RS_CUDA(cudaMemcpyAsync(out, d, bytes, cudaMemcpyDeviceToHost, h->stream));
     RS_CUDA(cudaStreamSynchronize(h->stream));

@@ -206,7 +206,67 @@ void rs_cached_free(int device, void *p, size_t bytes);
 void rs_cache_trim(void);
 
 // ---- api.cu: grow-only per-handle device scratch (slot-indexed) ----
+// A slot holds one buffer, and asking it for more bytes than it has frees that buffer and allocates a larger one.  So
+// two buffers that are live at the same time need two slots.  ABI calls on one handle are serialised and run on its
+// stream, so different calls may share a slot; the slots that are shared say so.
+enum rs_scratch_slot {
+    // api.cu: host arguments of rs_knn_predict_batch and rs_knn_predict_neighbors (one call at a time)
+    RS_SCR_PRED_LEFT,
+    RS_SCR_PRED_RIGHT,
+    RS_SCR_PRED_OUT,
+    RS_SCR_HOST_IDS,          // rs_knn_predict_neighbors' list, rs_knn_topk's lists
+    RS_SCR_HOST_SIMS,
+    RS_SCR_NB_COUNT,
+    RS_SCR_COSUMS,
+    RS_SCR_FIT_LEFT,          // rs_knn_fit's inputs
+    RS_SCR_FIT_RIGHT,
+    RS_SCR_FIT_RATING,
+    RS_SCR_FIT_LEFT_BIAS,
+    RS_SCR_FIT_RIGHT_BIAS,
+    // predict.cu: the pairs grouped by left row
+    RS_SCR_PRED_KEYS_IN,
+    RS_SCR_PRED_KEYS,
+    RS_SCR_PRED_IOTA,
+    RS_SCR_PRED_PERM,
+    RS_SCR_PRED_SORT_TMP,
+    RS_SCR_PRED_OWN_COUNT,
+    // the work counter and the per-warp key spill of a select.cuh kernel: Predict, Slope One's Predict and
+    // recommend_kernel share them.  A launch uses them alone; the next one zeroes the counter and sizes the spill after
+    // it on the same stream (a larger spill is allocated only after that stream has drained).
+    RS_SCR_WORK,
+    RS_SCR_KEY_SPILL,
+    // api.cu: host arguments of the recommendation entry points (by id or as lists; one call at a time)
+    RS_SCR_REC_QUERIES,
+    RS_SCR_REC_PTR,
+    RS_SCR_REC_IDS,
+    RS_SCR_REC_VALS,
+    RS_SCR_REC_OUT,           // the score rows, or the list ids
+    RS_SCR_REC_SCORES,        // the list scores
+    // recommend.cu
+    RS_SCR_REC_SLAB,          // a batch's score rows
+    RS_SCR_REC_STAGE_IDS,     // a shard's lists of a batch, before they are placed
+    RS_SCR_REC_STAGE_SCORES,
+    RS_SCR_OWN_FLAG,          // the left queries a shard answers
+    RS_SCR_OWN_QUERIES,
+    RS_SCR_OWN_POS,
+    RS_SCR_OWN_COUNT,
+    RS_SCR_OWN_TMP,
+    // given.cu and the given lists' statistics (recommend.cu)
+    RS_SCR_GIVEN_COUNTER,
+    RS_SCR_GIVEN_HDR,
+    RS_SCR_GIVEN_PTR,
+    RS_SCR_GIVEN_IDS,
+    RS_SCR_GIVEN_VALS,
+    RS_SCR_GIVEN_SORT_TMP,
+    RS_SCR_GIVEN_MEANS,
+    RS_SCR_GIVEN_STDDEVS,
+    RS_SCR_GIVEN_PMEANS,
+    RS_SCR_GIVEN_SIMS,        // a batch's S* rows
+};
 extern "C" int32_t rs_scratch_get(rs_knn *h, int slot, size_t bytes, void **out);
+
+// The targets of a query of `side`: every id of the other side.
+inline int64_t rs_n_targets(const rs_knn *h, int32_t side) { return side == RS_SIDE_RIGHT ? h->n_left : h->n_right; }
 
 // ---- prep.cu ----
 int32_t rs_prep_build(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
@@ -246,16 +306,23 @@ int32_t rs_topk_rows_launch(rs_knn *h, const double *src, int64_t ld, int32_t n,
                             double *d_sim);
 
 // ---- recommend.cu ----
-int32_t rs_score_all_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, double *d_out);
-int32_t rs_recommend_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, int32_t n_top, int32_t *d_ids,
-                            double *d_scores);
-int32_t rs_score_all_sharded_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, double *d_out);
-int32_t rs_recommend_sharded_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, int32_t n_top,
-                                    int32_t *d_ids, double *d_scores);
-// Queries given as rating lists (rs_knn_*_given): d_ptr / d_ids / d_vals are the caller's device arrays.  d_out set:
-// score rows; else the top-n_top lists.
-int32_t rs_given_launch(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids, const double *d_vals,
-                        int64_t n, double *d_out, int32_t n_top, int32_t *d_top_ids, double *d_top_scores);
+// One call of a recommendation entry point (include/rs_knn.h), checked by api.cu; every pointer is device memory.
+struct rs_rec_call {
+    int32_t side;                 // enum rs_side
+    bool sharded;                 // a row shard's part (rs_knn_*_sharded_device)
+    bool given;                   // the queries are rating lists (rs_knn_*_given), else inner ids
+    bool lists;                   // the top-n_top lists, else the score rows
+    const int32_t *queries;       // by id: [n]
+    const int64_t *ptr;           // given: list b is ids / vals [ptr[b], ptr[b+1])
+    const int32_t *ids;
+    const double *vals;
+    int64_t n;
+    double *rows;                 // score rows [n][n_targets]
+    int32_t n_top;                // lists [n][n_top]
+    int32_t *top_ids;
+    double *top_scores;
+};
+int32_t rs_recommend_run(rs_knn *h, const rs_rec_call &c);
 
 // ---- given.cu ----
 // The lists of rs_knn_*_given, validated and sorted: list b is entries ptr[b] .. ptr[b+1) of ids / vals (ascending id)

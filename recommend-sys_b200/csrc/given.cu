@@ -163,8 +163,8 @@ int32_t launch_given_sims(rs_knn *h, const GivenSimArgs &a) {
 int32_t rs_given_prepare(rs_knn *h, int32_t n_targets, const int64_t *d_ptr, const int32_t *d_ids,
                          const double *d_vals, int64_t n, rs_given_lists *out) {
     void *hdr, *gp, *flags;
-    RS_TRY(rs_scratch_get(h, 32, 64, &hdr));
-    RS_TRY(rs_scratch_get(h, 33, (size_t)(n + 1) * 8, &gp));
+    RS_TRY(rs_scratch_get(h, RS_SCR_GIVEN_HDR, 64, &hdr));
+    RS_TRY(rs_scratch_get(h, RS_SCR_GIVEN_PTR, (size_t)(n + 1) * 8, &gp));
     flags = (char *)hdr + 32;
     RS_CUDA(cudaMemsetAsync(hdr, 0, 64, h->stream));
     given_ptr_kernel<<<(unsigned)((n + 1 + 255) / 256), 256, 0, h->stream>>>(d_ptr, n, (int64_t *)gp,
@@ -192,13 +192,13 @@ int32_t rs_given_prepare(rs_knn *h, int32_t n_targets, const int64_t *d_ptr, con
     if (nnz == 0) return RS_OK;
     // sort each list by id (stable; plumbing, not the hot path), then check the sorted entries
     void *s_ids, *s_vals, *tmp;
-    RS_TRY(rs_scratch_get(h, 34, (size_t)nnz * 4, &s_ids));
-    RS_TRY(rs_scratch_get(h, 35, (size_t)nnz * 8, &s_vals));
+    RS_TRY(rs_scratch_get(h, RS_SCR_GIVEN_IDS, (size_t)nnz * 4, &s_ids));
+    RS_TRY(rs_scratch_get(h, RS_SCR_GIVEN_VALS, (size_t)nnz * 8, &s_vals));
     size_t need = 0;
     RS_CUDA(cub::DeviceSegmentedSort::StableSortPairs(nullptr, need, d_ids + p0, (int32_t *)s_ids, d_vals + p0,
                                                        (double *)s_vals, (int)nnz, (int)n, (const int64_t *)gp,
                                                        (const int64_t *)gp + 1, h->stream));
-    RS_TRY(rs_scratch_get(h, 36, need + 256, &tmp));
+    RS_TRY(rs_scratch_get(h, RS_SCR_GIVEN_SORT_TMP, need + 256, &tmp));
     RS_CUDA(cub::DeviceSegmentedSort::StableSortPairs(tmp, need, d_ids + p0, (int32_t *)s_ids, d_vals + p0,
                                                        (double *)s_vals, (int)nnz, (int)n, (const int64_t *)gp,
                                                        (const int64_t *)gp + 1, h->stream));
@@ -226,7 +226,7 @@ int32_t rs_given_sims_launch(rs_knn *h, const int64_t *ptr, const int32_t *ids, 
                              const double *qpmeans, int64_t nq, double *out, int64_t ld) {
     if (nq <= 0) return RS_OK;
     void *counter;
-    RS_TRY(rs_scratch_get(h, 31, 8, &counter));
+    RS_TRY(rs_scratch_get(h, RS_SCR_GIVEN_COUNTER, 8, &counter));
     RS_CUDA(cudaMemsetAsync(counter, 0, 8, h->stream));
     GivenSimArgs a{};
     a.ptr = ptr; a.ids = ids; a.vals = vals; a.qpmeans = qpmeans; a.nq = nq;

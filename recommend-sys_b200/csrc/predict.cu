@@ -508,15 +508,15 @@ int32_t rs_predict_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_rig
         // only visits the shard's own pairs, found — and grouped by left row — by ONE radix sort whose key puts
         // foreign pairs last (walking all positions to skip 7 of 8 cost 2.7 ms of a 4.8 ms launch at 8 shards)
         void *keys_in, *keys_out, *iota, *perm, *tmp, *cnt;
-        RS_TRY(rs_scratch_get(h, 18, (size_t)n * 4, &keys_in));
-        RS_TRY(rs_scratch_get(h, 12, (size_t)n * 4, &keys_out));
-        RS_TRY(rs_scratch_get(h, 13, (size_t)n * 4, &iota));
-        RS_TRY(rs_scratch_get(h, 14, (size_t)n * 4, &perm));
-        RS_TRY(rs_scratch_get(h, 19, 8, &cnt));
+        RS_TRY(rs_scratch_get(h, RS_SCR_PRED_KEYS_IN, (size_t)n * 4, &keys_in));
+        RS_TRY(rs_scratch_get(h, RS_SCR_PRED_KEYS, (size_t)n * 4, &keys_out));
+        RS_TRY(rs_scratch_get(h, RS_SCR_PRED_IOTA, (size_t)n * 4, &iota));
+        RS_TRY(rs_scratch_get(h, RS_SCR_PRED_PERM, (size_t)n * 4, &perm));
+        RS_TRY(rs_scratch_get(h, RS_SCR_PRED_OWN_COUNT, 8, &cnt));
         size_t need = 0;
         RS_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, need, (int32_t *)keys_in, (int32_t *)keys_out, (int32_t *)iota,
                                                 (int32_t *)perm, (int)n, 0, 31, h->stream));
-        RS_TRY(rs_scratch_get(h, 15, need + 256, &tmp));
+        RS_TRY(rs_scratch_get(h, RS_SCR_PRED_SORT_TMP, need + 256, &tmp));
         RS_CUDA(cudaMemsetAsync(cnt, 0, 8, h->stream));
         RS_CUDA(cudaMemsetAsync(d_out, 0, (size_t)n * 8, h->stream));
         own_key_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(d_left, n, h->cyc_R, h->cyc_r, (int32_t *)keys_in,
@@ -529,15 +529,15 @@ int32_t rs_predict_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_rig
     } else if (n >= 65536 && (size_t)h->rows_local * (size_t)h->ld_s * 8 > ((size_t)64 << 20) &&
         !getenv("RS_KNN_PRED_NOSORT")) {
         void *keys_out, *iota, *perm, *tmp;
-        RS_TRY(rs_scratch_get(h, 12, (size_t)n * 4, &keys_out));
-        RS_TRY(rs_scratch_get(h, 13, (size_t)n * 4, &iota));
-        RS_TRY(rs_scratch_get(h, 14, (size_t)n * 4, &perm));
+        RS_TRY(rs_scratch_get(h, RS_SCR_PRED_KEYS, (size_t)n * 4, &keys_out));
+        RS_TRY(rs_scratch_get(h, RS_SCR_PRED_IOTA, (size_t)n * 4, &iota));
+        RS_TRY(rs_scratch_get(h, RS_SCR_PRED_PERM, (size_t)n * 4, &perm));
         size_t need = 0;
         int bits = 1;
         while ((1ll << bits) < (long long)h->n_left && bits < 31) bits++;
         RS_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, need, d_left, (int32_t *)keys_out, (int32_t *)iota,
                                                 (int32_t *)perm, (int)n, 0, bits, h->stream));
-        RS_TRY(rs_scratch_get(h, 15, need + 256, &tmp));
+        RS_TRY(rs_scratch_get(h, RS_SCR_PRED_SORT_TMP, need + 256, &tmp));
         iota_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>((int32_t *)iota, (int32_t)n);
         RS_CUDA(cub::DeviceRadixSort::SortPairs(tmp, need, d_left, (int32_t *)keys_out, (int32_t *)iota,
                                                 (int32_t *)perm, (int)n, 0, bits, h->stream));
@@ -546,7 +546,7 @@ int32_t rs_predict_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_rig
     }
     {
         void *work;
-        RS_TRY(rs_scratch_get(h, 16, 8, &work));
+        RS_TRY(rs_scratch_get(h, RS_SCR_WORK, 8, &work));
         RS_CUDA(cudaMemsetAsync(work, 0, 8, h->stream));
         a.work = reinterpret_cast<unsigned long long *>(work);
     }
@@ -570,7 +570,7 @@ int32_t rs_predict_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_rig
         // global spill of the staged keys: one slice per resident warp, sized by the longest right row
         const int64_t gcap = h->max_right_len > scap ? (((int64_t)h->max_right_len - scap + 31) / 32 * 32) : 32;
         void *g;
-        RS_TRY(rs_scratch_get(h, 17, (size_t)blocks * SEL_WARPS * (size_t)gcap * 8, &g));
+        RS_TRY(rs_scratch_get(h, RS_SCR_KEY_SPILL, (size_t)blocks * SEL_WARPS * (size_t)gcap * 8, &g));
         a.gstage = reinterpret_cast<uint64_t *>(g);
         a.gcap = gcap;
     }
@@ -695,7 +695,7 @@ int32_t rs_slope_predict_launch(rs_knn *h, const int32_t *d_left, const int32_t 
         return RS_ERR_INVALID;
     }
     void *work;
-    RS_TRY(rs_scratch_get(h, 16, 8, &work));
+    RS_TRY(rs_scratch_get(h, RS_SCR_WORK, 8, &work));
     RS_CUDA(cudaMemsetAsync(work, 0, 8, h->stream));
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);

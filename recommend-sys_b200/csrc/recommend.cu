@@ -173,18 +173,6 @@ int32_t launch_scores(const PredArgs &a, const RecArgs &ra, unsigned blocks, siz
     return RS_OK;
 }
 
-// Scores of every target of the queries d_q[0 .. nq) into out[nq][ld_out]; the fields that differ on row shards are
-// set by the caller.
-RecArgs rec_args(const rs_knn *h, int32_t side, const int32_t *d_q, int64_t nq, double *out, int64_t ld_out) {
-    RecArgs ra{};
-    ra.queries = d_q; ra.nq = nq; ra.side = side;
-    ra.n_side = side == RS_SIDE_RIGHT ? h->n_right : h->n_left;
-    ra.n_targets = side == RS_SIDE_RIGHT ? h->n_left : h->n_right;
-    ra.map = row_map(h);
-    ra.out = out; ra.ld_out = ld_out;
-    return ra;
-}
-
 // Given lists of one batch: the lists (right queries: the candidate CSR), and for left queries the S* rows and the
 // statistics arrays that hold the queries' own after the fitted rows'.
 struct GivenBatch {
@@ -213,7 +201,7 @@ int32_t score_rows(rs_knn *h, RecArgs ra, const GivenBatch *g = nullptr) {
     a.global_mean = h->global_mean; a.n_right = h->n_right;
     a.k = h->p.k; a.min_k = h->p.min_k; a.knn_type = h->p.knn_type;
     void *work;
-    RS_TRY(rs_scratch_get(h, 16, 8, &work));
+    RS_TRY(rs_scratch_get(h, RS_SCR_WORK, 8, &work));
     RS_CUDA(cudaMemsetAsync(work, 0, 8, h->stream));
     ra.work = reinterpret_cast<unsigned long long *>(work);
     a.work = ra.work;
@@ -228,7 +216,7 @@ int32_t score_rows(rs_knn *h, RecArgs ra, const GivenBatch *g = nullptr) {
     if (blocks > (warps + SEL_WARPS - 1) / SEL_WARPS) blocks = (warps + SEL_WARPS - 1) / SEL_WARPS;
     const int64_t gcap = max_cand > scap ? ((max_cand - scap + 31) / 32 * 32) : 32;
     void *gst;
-    RS_TRY(rs_scratch_get(h, 17, (size_t)blocks * SEL_WARPS * (size_t)gcap * 8, &gst));
+    RS_TRY(rs_scratch_get(h, RS_SCR_KEY_SPILL, (size_t)blocks * SEL_WARPS * (size_t)gcap * 8, &gst));
     a.gstage = reinterpret_cast<uint64_t *>(gst);
     a.gcap = gcap;
     if (h->p.k <= 44) RS_TRY(launch_scores<2>(a, ra, (unsigned)blocks, smem, scap, h->stream));
@@ -251,49 +239,15 @@ int64_t slab_batch(int64_t width, int64_t n) {
     return batch;
 }
 
-// Top-N lists of the queries d_q[0 .. n): scored in batches into a bounded slab of `width`-column score rows, ~256 MiB,
-// and selected by topk_rows_kernel.  Sharded: the lists are staged and placed by place_lists_kernel (to row rows[b],
-// else b; right queries' slab columns are local rows).
-int32_t recommend_rows(rs_knn *h, int32_t side, const int32_t *d_q, const int32_t *rows, int64_t n, int64_t width,
-                       bool sharded, int32_t n_top, int32_t *d_ids, double *d_scores) {
-    if (n <= 0) return RS_OK;
-    const int64_t batch = slab_batch(width, n);
-    void *slab, *st_ids = nullptr, *st_scores = nullptr;
-    RS_TRY(rs_scratch_get(h, 23, (size_t)batch * width * 8, &slab));
-    if (sharded) {
-        RS_TRY(rs_scratch_get(h, 24, (size_t)batch * n_top * 4, &st_ids));
-        RS_TRY(rs_scratch_get(h, 25, (size_t)batch * n_top * 8, &st_scores));
-    }
-    for (int64_t b0 = 0; b0 < n; b0 += batch) {
-        const int64_t nb = n - b0 < batch ? n - b0 : batch;
-        RecArgs ra = rec_args(h, side, d_q + b0, nb, (double *)slab, width);
-        ra.n_targets = (int32_t)width;
-        RS_TRY(score_rows(h, ra));
-        if (!sharded) {
-            RS_TRY(rs_topk_rows_launch(h, (const double *)slab, width, (int32_t)width, nb, n_top, d_ids + b0 * n_top,
-                                       d_scores + b0 * n_top));
-            continue;
-        }
-        RS_TRY(rs_topk_rows_launch(h, (const double *)slab, width, (int32_t)width, nb, n_top, (int32_t *)st_ids,
-                                   (double *)st_scores));
-        place_lists_kernel<<<(unsigned)nb, 128, 0, h->stream>>>((const int32_t *)st_ids, (const double *)st_scores,
-                                                                n_top, rows ? rows + b0 : nullptr, b0,
-                                                                side == RS_SIDE_RIGHT, row_map(h), d_ids, d_scores);
-        h->prof.total_launches++;
-        RS_CUDA(cudaGetLastError());
-    }
-    return RS_OK;
-}
-
 // Left queries on a row shard: the queries this shard answers (values and positions), compacted; their count is read
 // back to size the batches.
 int32_t own_queries(rs_knn *h, const int32_t *d_q, int64_t n, const int32_t **q_own, const int32_t **pos,
                     int64_t *n_own) {
     void *flag, *qo, *po, *cnt, *tmp;
-    RS_TRY(rs_scratch_get(h, 26, (size_t)n, &flag));
-    RS_TRY(rs_scratch_get(h, 27, (size_t)n * 4, &qo));
-    RS_TRY(rs_scratch_get(h, 28, (size_t)n * 4, &po));
-    RS_TRY(rs_scratch_get(h, 29, 8, &cnt));
+    RS_TRY(rs_scratch_get(h, RS_SCR_OWN_FLAG, (size_t)n, &flag));
+    RS_TRY(rs_scratch_get(h, RS_SCR_OWN_QUERIES, (size_t)n * 4, &qo));
+    RS_TRY(rs_scratch_get(h, RS_SCR_OWN_POS, (size_t)n * 4, &po));
+    RS_TRY(rs_scratch_get(h, RS_SCR_OWN_COUNT, 8, &cnt));
     const cub::CountingInputIterator<int32_t> iota(0);
     size_t need_q = 0, need_p = 0;
     RS_CUDA(cub::DeviceSelect::Flagged(nullptr, need_q, d_q, (const uint8_t *)flag, (int32_t *)qo, (int32_t *)cnt,
@@ -301,7 +255,7 @@ int32_t own_queries(rs_knn *h, const int32_t *d_q, int64_t n, const int32_t **q_
     RS_CUDA(cub::DeviceSelect::Flagged(nullptr, need_p, iota, (const uint8_t *)flag, (int32_t *)po, (int32_t *)cnt,
                                        (int)n, h->stream));
     const size_t need = need_q > need_p ? need_q : need_p;
-    RS_TRY(rs_scratch_get(h, 30, need + 256, &tmp));
+    RS_TRY(rs_scratch_get(h, RS_SCR_OWN_TMP, need + 256, &tmp));
     own_query_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(d_q, n, h->n_left, row_map(h),
                                                                           (uint8_t *)flag);
     h->prof.total_launches++;
@@ -330,100 +284,99 @@ int32_t empty_lists(rs_knn *h, int32_t *d_ids, double *d_scores, int64_t cnt) {
 
 }  // namespace
 
-int32_t rs_score_all_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, double *d_out) {
-    const int64_t n_targets = side == RS_SIDE_RIGHT ? h->n_left : h->n_right;
-    return score_rows(h, rec_args(h, side, d_q, n, d_out, n_targets));
-}
-
-int32_t rs_recommend_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, int32_t n_top, int32_t *d_ids,
-                            double *d_scores) {
-    const int64_t n_targets = side == RS_SIDE_RIGHT ? h->n_left : h->n_right;
-    return recommend_rows(h, side, d_q, nullptr, n, n_targets, false, n_top, d_ids, d_scores);
-}
-
-// Row shards: every cell this shard does not answer is +0.0 (all bits zero), for an integer SUM all-reduce.
-int32_t rs_score_all_sharded_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, double *d_out) {
-    if (n <= 0) return RS_OK;
-    const int64_t n_targets = side == RS_SIDE_RIGHT ? h->n_left : h->n_right;
-    RS_CUDA(cudaMemsetAsync(d_out, 0, (size_t)n * n_targets * 8, h->stream));
-    RecArgs ra = rec_args(h, side, d_q, n, d_out, n_targets);
-    if (side == RS_SIDE_RIGHT) {
-        ra.n_targets = (int32_t)h->rows_local;
-        ra.out_global = 1;
-        return score_rows(h, ra);
+// Every recommendation entry point (api.cu, after its checks): resolve the queries, choose one batch size, then per
+// batch the S* rows of left lists, the scores, and for list outputs topk_rows_kernel, written directly or, on a row
+// shard, staged and placed.
+int32_t rs_recommend_run(rs_knn *h, const rs_rec_call &c) {
+    if (c.n <= 0) return RS_OK;
+    const bool left = c.side == RS_SIDE_LEFT;
+    const int64_t n_targets = rs_n_targets(h, c.side);
+    // 1. the queries: q[0 .. n) (a shard's left queries: the ones it answers, their rows pos[b]) or the lists gl, and
+    //    `width`, the targets scored per query
+    const int32_t *q = c.queries, *pos = nullptr;
+    int64_t n = c.n, width = n_targets;
+    if (c.sharded) {
+        // every cell this shard does not answer is +0.0 (all bits zero), for an integer SUM all-reduce; every list it
+        // does not produce is empty
+        if (!c.lists) RS_CUDA(cudaMemsetAsync(c.rows, 0, (size_t)n * n_targets * 8, h->stream));
+        if (left) {
+            RS_TRY(own_queries(h, c.queries, c.n, &q, &pos, &n));
+            if (c.lists) RS_TRY(empty_lists(h, c.top_ids, c.top_scores, c.n * c.n_top));
+        } else {
+            width = h->rows_local;
+            if (width == 0) return c.lists ? empty_lists(h, c.top_ids, c.top_scores, c.n * c.n_top) : RS_OK;
+        }
+        if (n == 0) return RS_OK;
     }
-    RS_TRY(own_queries(h, d_q, n, &ra.queries, &ra.rows, &ra.nq));
-    return score_rows(h, ra);
-}
-
-// Row shards: partial lists, to be united across the shards (rs_knn_topk_union_device).  Lists this shard does not
-// produce are empty.
-int32_t rs_recommend_sharded_launch(rs_knn *h, int32_t side, const int32_t *d_q, int64_t n, int32_t n_top,
-                                    int32_t *d_ids, double *d_scores) {
-    if (n <= 0) return RS_OK;
-    if (side == RS_SIDE_RIGHT) {
-        if (h->rows_local == 0) return empty_lists(h, d_ids, d_scores, n * n_top);
-        return recommend_rows(h, side, d_q, nullptr, n, h->rows_local, true, n_top, d_ids, d_scores);
-    }
-    const int32_t *q_own, *pos;
-    int64_t n_own = 0;
-    RS_TRY(own_queries(h, d_q, n, &q_own, &pos, &n_own));
-    RS_TRY(empty_lists(h, d_ids, d_scores, n * n_top));
-    return recommend_rows(h, side, q_own, pos, n_own, h->n_right, true, n_top, d_ids, d_scores);
-}
-
-// Queries given as rating lists.  Validated and sorted by rs_given_prepare; left queries get their statistics (the
-// fitted rows' followed by the lists', one array) and, per batch, their S* rows.  The S* slab and the score slab
-// share the ~256 MiB budget.
-int32_t rs_given_launch(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids, const double *d_vals,
-                        int64_t n, double *d_out, int32_t n_top, int32_t *d_top_ids, double *d_top_scores) {
-    if (n <= 0) return RS_OK;
-    const bool left = side == RS_SIDE_LEFT;
-    const int64_t n_targets = left ? h->n_right : h->n_left;
-    rs_given_lists gl;
-    RS_TRY(rs_given_prepare(h, (int32_t)n_targets, d_ptr, d_ids, d_vals, n, &gl));
+    rs_given_lists gl{};
     GivenBatch g{};
-    g.ids = gl.ids; g.vals = gl.vals; g.max_len = gl.max_len;
-    double *qpmeans = nullptr, *sslab = nullptr;
-    if (left) {
-        void *m, *sd, *pm;
-        const size_t rows = (size_t)h->n_left + (size_t)n;
-        RS_TRY(rs_scratch_get(h, 37, rows * 8, &m));
-        RS_TRY(rs_scratch_get(h, 38, rows * 8, &sd));
-        RS_TRY(rs_scratch_get(h, 39, (size_t)n * 8, &pm));
-        RS_CUDA(cudaMemcpyAsync(m, h->means, (size_t)h->n_left * 8, cudaMemcpyDeviceToDevice, h->stream));
-        RS_CUDA(cudaMemcpyAsync(sd, h->stddevs, (size_t)h->n_left * 8, cudaMemcpyDeviceToDevice, h->stream));
-        // core/knn.go:167-177 over the caller's order; Pearson's mean over ascending ids (core/sim.go:49-54)
-        RS_TRY(rs_row_stats_launch(h, gl.ptr, gl.vals_in, gl.vals, n, h->p.knn_type == RS_KNN_ZSCORE,
-                                   (double *)m + h->n_left, (double *)sd + h->n_left, (double *)pm));
-        g.means = (const double *)m; g.stddevs = (const double *)sd;
-        qpmeans = (double *)pm;
+    const double *qpmeans = nullptr;
+    if (c.given) {
+        RS_TRY(rs_given_prepare(h, (int32_t)n_targets, c.ptr, c.ids, c.vals, n, &gl));
+        g.ids = gl.ids; g.vals = gl.vals; g.max_len = gl.max_len;
+        if (left) {   // the statistics arrays: the fitted rows' followed by the lists'
+            void *m, *sd, *pm;
+            const size_t rows = (size_t)h->n_left + (size_t)n;
+            RS_TRY(rs_scratch_get(h, RS_SCR_GIVEN_MEANS, rows * 8, &m));
+            RS_TRY(rs_scratch_get(h, RS_SCR_GIVEN_STDDEVS, rows * 8, &sd));
+            RS_TRY(rs_scratch_get(h, RS_SCR_GIVEN_PMEANS, (size_t)n * 8, &pm));
+            RS_CUDA(cudaMemcpyAsync(m, h->means, (size_t)h->n_left * 8, cudaMemcpyDeviceToDevice, h->stream));
+            RS_CUDA(cudaMemcpyAsync(sd, h->stddevs, (size_t)h->n_left * 8, cudaMemcpyDeviceToDevice, h->stream));
+            // core/knn.go:167-177 over the caller's order; Pearson's mean over ascending ids (core/sim.go:49-54)
+            RS_TRY(rs_row_stats_launch(h, gl.ptr, gl.vals_in, gl.vals, n, h->p.knn_type == RS_KNN_ZSCORE,
+                                       (double *)m + h->n_left, (double *)sd + h->n_left, (double *)pm));
+            g.means = (const double *)m; g.stddevs = (const double *)sd;
+            qpmeans = (const double *)pm;
+        }
     }
-    const int64_t width = n_targets + (left ? h->n_left : 0);
-    const int64_t batch = slab_batch(width, n);
-    void *slab = nullptr;
-    if (!d_out) RS_TRY(rs_scratch_get(h, 23, (size_t)batch * n_targets * 8, &slab));
-    if (left) {
-        void *ss;
-        RS_TRY(rs_scratch_get(h, 40, (size_t)batch * h->n_left * 8, &ss));
-        sslab = (double *)ss;
+    // 2. the batch: score rows by id go to the caller's rows in one pass; everything else is scored in batches, into
+    //    a slab of `width` columns for lists and, for left lists, the S* slab beside it (~256 MiB together)
+    const int64_t batch = !c.lists && !c.given ? n : slab_batch(width + (c.given && left ? h->n_left : 0), n);
+    void *slab = nullptr, *st_ids = nullptr, *st_scores = nullptr, *sslab = nullptr;
+    if (c.lists) RS_TRY(rs_scratch_get(h, RS_SCR_REC_SLAB, (size_t)batch * width * 8, &slab));
+    if (c.lists && c.sharded) {
+        RS_TRY(rs_scratch_get(h, RS_SCR_REC_STAGE_IDS, (size_t)batch * c.n_top * 4, &st_ids));
+        RS_TRY(rs_scratch_get(h, RS_SCR_REC_STAGE_SCORES, (size_t)batch * c.n_top * 8, &st_scores));
     }
+    if (c.given && left) RS_TRY(rs_scratch_get(h, RS_SCR_GIVEN_SIMS, (size_t)batch * h->n_left * 8, &sslab));
+    // 3. one loop
     for (int64_t b0 = 0; b0 < n; b0 += batch) {
         const int64_t nb = n - b0 < batch ? n - b0 : batch;
-        double *rows = d_out ? d_out + b0 * n_targets : (double *)slab;
-        RecArgs ra = rec_args(h, side, nullptr, nb, rows, n_targets);
-        ra.given = 1;
-        g.ptr = gl.ptr + b0;
-        if (left) {
-            RS_TRY(rs_given_sims_launch(h, g.ptr, gl.ids, gl.vals, qpmeans + b0, nb, sslab, h->n_left));
-            ra.gsims = sslab;
-            ra.ld_g = h->n_left;
-            ra.qstat = (int32_t)(h->n_left + b0);
+        RecArgs ra{};
+        ra.queries = q ? q + b0 : nullptr; ra.nq = nb; ra.side = c.side;
+        ra.n_side = left ? h->n_left : h->n_right;
+        ra.n_targets = (int32_t)width;
+        ra.map = row_map(h);
+        ra.out = c.lists ? (double *)slab : c.rows + b0 * n_targets;
+        ra.ld_out = c.lists ? width : n_targets;
+        if (!c.lists && c.sharded) {       // a shard's rows: left queries to their rows, right targets to global columns
+            ra.rows = pos;
+            ra.out_global = !left;
         }
-        RS_TRY(score_rows(h, ra, &g));
-        if (!d_out)
-            RS_TRY(rs_topk_rows_launch(h, rows, n_targets, (int32_t)n_targets, nb, n_top, d_top_ids + b0 * n_top,
-                                       d_top_scores + b0 * n_top));
+        if (c.given) {
+            ra.given = 1;
+            g.ptr = gl.ptr + b0;
+            if (left) {
+                RS_TRY(rs_given_sims_launch(h, g.ptr, gl.ids, gl.vals, qpmeans + b0, nb, (double *)sslab, h->n_left));
+                ra.gsims = (const double *)sslab;
+                ra.ld_g = h->n_left;
+                ra.qstat = (int32_t)(h->n_left + b0);
+            }
+        }
+        RS_TRY(score_rows(h, ra, c.given ? &g : nullptr));
+        if (!c.lists) continue;
+        if (!c.sharded) {
+            RS_TRY(rs_topk_rows_launch(h, (const double *)slab, width, (int32_t)width, nb, c.n_top,
+                                       c.top_ids + b0 * c.n_top, c.top_scores + b0 * c.n_top));
+            continue;
+        }
+        RS_TRY(rs_topk_rows_launch(h, (const double *)slab, width, (int32_t)width, nb, c.n_top, (int32_t *)st_ids,
+                                   (double *)st_scores));
+        place_lists_kernel<<<(unsigned)nb, 128, 0, h->stream>>>((const int32_t *)st_ids, (const double *)st_scores,
+                                                                c.n_top, pos ? pos + b0 : nullptr, b0, !left,
+                                                                row_map(h), c.top_ids, c.top_scores);
+        h->prof.total_launches++;
+        RS_CUDA(cudaGetLastError());
     }
     return RS_OK;
 }
