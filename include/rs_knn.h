@@ -129,8 +129,8 @@ typedef struct rs_knn_profile {
     int64_t total_launches;    /* every kernel this library launched on the handle         */
     int32_t sim_path_used;     /* enum rs_sim_path actually taken by the last Fit          */
     int32_t reserved0;
-    double corated_triples;    /* sum over right rows of cnt*(cnt-1)/2 of the last Fit: the work of the
-                                * exact sparse path, input of the RS_PATH_AUTO model        */
+    double corated_triples;    /* sum over right rows of cnt*(cnt-1)/2 of the last Fit (rs_knn_update leaves it):
+                                * the work of the exact sparse path, input of the RS_PATH_AUTO model */
 } rs_knn_profile;
 
 /* Thread-local message of the last error on this thread ("" if none). */
@@ -302,6 +302,36 @@ int32_t rs_knn_recommend_given(rs_knn *h, int32_t side, const int64_t *ptr, cons
 int32_t rs_knn_recommend_given_device(rs_knn *h, int32_t side, const int64_t *d_ptr, const int32_t *d_ids,
                                       const double *d_vals, int64_t n, int32_t n_top, int32_t *d_out_ids,
                                       double *d_out_scores);
+
+/* ADDING RATINGS TO A FITTED MODEL (an extension: the reference has no incremental Fit).  The ratings left[i],
+ * right[i], rating[i] (inner ids, in call order) join the fitted ones, and the model becomes the one rs_knn_fit
+ * returns for the union — the fitted ratings in their dataset order followed by these — with n_left x n_right ids and
+ * GlobalMean global_mean, bit for bit: matrix, means, stddevs, Predict, recommendation and fold-in.  Only the
+ * similarity rows (and columns) of the TOUCHED left ids are recomputed: the ids these ratings name, and the new ids
+ * n_left_fitted .. n_left-1; a cell between two untouched rows keeps its value, which is the refit's (the same terms
+ * in the same order).  n_left / n_right are the counts after the update, at least the fitted ones (larger ones add
+ * ids; an id without ratings gets the empty row a Fit gives it).  nnz may be 0 (only new ids, or a new GlobalMean).
+ * Host pointers are consumed when the call returns; the _device variant reads its arrays on the handle's stream.
+ * The call returns once the ratings are validated and the work is queued; rs_knn_synchronize waits for it.
+ * Refused before anything of the model is written, leaving it exactly as it was:
+ *   RS_ERR_INVALID     the handle is not fitted, an id outside [0, n_left) x [0, n_right), a count smaller than the
+ *                      fitted one, a null pointer with nnz > 0;
+ *   RS_ERR_UNSUPPORTED a NaN rating; RS_STORE_TOPK; row shards (row_begin/row_end, shard_count >= 2);
+ *                      RS_SIM_SLOPE_ONE; RS_KNN_BASELINE and RS_SIM_PEARSON_BASELINE (their biases come from a global
+ *                      fit that every rating changes); Pearson in RS_PEARSON_SUMS mode (the recomputed rows are the
+ *                      exact replay); a non-integer rating for a model fitted on integer ratings in [-11, 11] (such a
+ *                      Fit keeps no dataset order of the values); more than 2^31-1 ratings in all;
+ *   RS_ERR_DUPLICATE   a (left, right) pair the model holds already, or twice among these ratings;
+ *   RS_ERR_OOM         the merged arrays or the grown matrix do not fit.
+ * Memory: the merged arrays live in two blocks per array with a quarter of slack (the one the model reads and the one
+ * the next update writes), so a sequence of updates stops allocating; a new left id grows the matrix in place while
+ * ld = ceil(n_left / 16) * 16 does not change, else into a new block.  The int8 planes of rs_knn_cosums are dropped
+ * and rebuilt for the union on its next call, into a block of their own that later rebuilds reuse while it is large
+ * enough; rs_knn_profile's corated_triples stays the last Fit's. */
+int32_t rs_knn_update(rs_knn *h, const int32_t *left, const int32_t *right, const double *rating, int64_t nnz,
+                      int32_t n_left, int32_t n_right, double global_mean);
+int32_t rs_knn_update_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
+                             int64_t nnz, int32_t n_left, int32_t n_right, double global_mean);
 
 /* Parameters["k"] / ["mink"] are read at Predict time by the reference (core/knn.go:80-81): change
  * them on a fitted handle without refitting.  The predict kernel supports k <= 256. */

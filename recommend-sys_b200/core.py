@@ -71,7 +71,8 @@ ABI_SYMBOLS = [
     "rs_knn_peer_import_local", "rs_knn_mirror", "rs_knn_predict_batch_sharded_device", "rs_knn_host_alloc",
     "rs_knn_host_free", "rs_knn_score_all", "rs_knn_score_all_device", "rs_knn_recommend", "rs_knn_recommend_device",
     "rs_knn_score_all_sharded_device", "rs_knn_recommend_sharded_device", "rs_knn_score_all_given",
-    "rs_knn_score_all_given_device", "rs_knn_recommend_given", "rs_knn_recommend_given_device",
+    "rs_knn_score_all_given_device", "rs_knn_recommend_given", "rs_knn_recommend_given_device", "rs_knn_update",
+    "rs_knn_update_device",
 ]
 
 _knn_lib = None
@@ -132,6 +133,8 @@ def knn_lib():
     L.rs_knn_score_all_given_device.argtypes = [vp, i32, vp, vp, vp, i64, vp]
     L.rs_knn_recommend_given.argtypes = [vp, i32, vp, vp, vp, i64, i32, vp, vp]
     L.rs_knn_recommend_given_device.argtypes = [vp, i32, vp, vp, vp, i64, i32, vp, vp]
+    L.rs_knn_update.argtypes = [vp, vp, vp, vp, i64, i32, i32, dbl]
+    L.rs_knn_update_device.argtypes = [vp, vp, vp, vp, i64, i32, i32, dbl]
     _knn_lib = L
     return L
 
@@ -396,6 +399,13 @@ class TrainSet(DataSet):
     def RatingRange(self):
         return float(self.Ratings.min()), float(self.Ratings.max())
 
+    def Extend(self, rowSet: DataSet) -> "TrainSet":
+        """The TrainSet of this one's rows followed by `rowSet`'s: NewTrainSet of the concatenation, so the inner ids
+        continue the order of first appearance (known ids keep theirs, new ones come after) and GlobalMean is that
+        TrainSet's, bit for bit."""
+        return TrainSet(DataSet(np.concatenate([self.Users, rowSet.Users]), np.concatenate([self.Items, rowSet.Items]),
+                                np.concatenate([self.Ratings, rowSet.Ratings])))
+
 
 class _HostBlock:
     """A page-locked host block of rs_knn_host_alloc; goes back to the library's cache with the last array on it."""
@@ -635,6 +645,19 @@ class _Handle:
         """Arguments are raw device pointers (ints), e.g. torch tensors' data_ptr()."""
         _check(knn_lib().rs_knn_fit_device(self.h, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean,
                                            d_left_bias or None, d_right_bias or None, global_bias))
+        self._after_fit(n_left, n_right)
+
+    def update(self, left, right, rating, n_left, n_right, global_mean):
+        """Adds ratings to the fitted model: it becomes the Fit of the union, bit for bit (rs_knn_update)."""
+        left = np.ascontiguousarray(left, dtype=np.int32)
+        right = np.ascontiguousarray(right, dtype=np.int32)
+        rating = np.ascontiguousarray(rating, dtype=np.float64)
+        _check(knn_lib().rs_knn_update(self.h, _ptr(left), _ptr(right), _ptr(rating), len(rating), n_left, n_right,
+                                       global_mean))
+        self._after_fit(n_left, n_right)
+
+    def update_device(self, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean):
+        _check(knn_lib().rs_knn_update_device(self.h, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean))
         self._after_fit(n_left, n_right)
 
     def predict_batch(self, left, right):
@@ -951,6 +974,24 @@ class KNN(Base):
         self._h = self._new_handle(sim)
         self._h.fit(left, right, trainSet.Ratings, n_left, n_right, trainSet.GlobalMean, left_bias, right_bias,
                     global_bias)
+        self._after_fit()
+
+    def Update(self, rowSet: DataSet):
+        """Adds the ratings of `rowSet` (raw user, raw item, rating; users and items may be new) to the fitted model
+        without a refit: the model becomes the Fit of Data.Extend(rowSet), bit for bit — similarities, Means, StdDevs,
+        GlobalMean, Predict and Recommend (rs_knn_update; only the rows of the users (items) the ratings touch are
+        recomputed).  A pair the model already holds is refused, as are models an update cannot extend exactly:
+        KNNBaseline, PearsonBaseline, Pearson in sums mode, row shards, top-k-only stores."""
+        data = self.Data.Extend(rowSet)
+        n0 = self.Data.Length()
+        iu, ii = data.innerUsers[n0:], data.innerItems[n0:]
+        if self._userBased:
+            left, right, n_left, n_right = iu, ii, data.UserCount, data.ItemCount
+        else:
+            left, right, n_left, n_right = ii, iu, data.ItemCount, data.UserCount
+        self._h.update(left, right, data.Ratings[n0:], n_left, n_right, data.GlobalMean)
+        self.Data = data
+        self.GlobalMean = data.GlobalMean
         self._after_fit()
 
     @property

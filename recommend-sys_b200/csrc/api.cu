@@ -75,6 +75,7 @@ void free_fit_state(rs_knn *h) {
     h->cand_sim = nullptr;
     h->row_flag = nullptr;
     h->d_flags = nullptr;
+    rs_update_release(h);
 }
 
 int32_t fold_profile(rs_knn *h) {
@@ -165,7 +166,7 @@ int32_t init_handle(rs_knn *h) {
 extern "C" {
 
 const char *rs_last_error(void) { return g_err; }
-int32_t rs_knn_abi_version(void) { return 4; }
+int32_t rs_knn_abi_version(void) { return 5; }
 
 int32_t rs_knn_device_count(void) {
     int n = 0;
@@ -586,6 +587,78 @@ int32_t rs_knn_fit(rs_knn *h, const int32_t *left, const int32_t *right, const d
         return RS_ERR_CUDA;
     }
     return RS_OK;
+}
+
+// Every check of rs_knn_update, in the order they fire: the handle is fitted; its model is one that an update can
+// extend exactly (a matrix of all rows, no Slope One, no bias of a global fit, the exact Pearson replay); the counts
+// do not shrink; the pointers are there when there are ratings.  The ratings themselves are checked on the device.
+static int32_t check_update(rs_knn *h, const int32_t *left, const int32_t *right, const double *rating, int64_t nnz,
+                            int32_t n_left, int32_t n_right) {
+    const char *who = "rs_knn_update";
+    if (!h->fitted) {
+        rs_set_error("%s: Fit has not been called", who);
+        return RS_ERR_INVALID;
+    }
+    if (h->p.store != RS_STORE_MATRIX) {
+        rs_set_error("%s needs RS_STORE_MATRIX (the handle keeps top-k lists only)", who);
+        return RS_ERR_UNSUPPORTED;
+    }
+    if (h->cyc_R > 1 || h->p.shard_count > 1 || h->row_begin != 0 || h->row_end != h->n_left) {
+        rs_set_error("%s needs a handle that holds every row (no row_begin/row_end shard, shard_count <= 1)", who);
+        return RS_ERR_UNSUPPORTED;
+    }
+    if (h->p.sim == RS_SIM_SLOPE_ONE) {
+        rs_set_error("%s: Slope One is not supported", who);
+        return RS_ERR_UNSUPPORTED;
+    }
+    if (h->p.knn_type == RS_KNN_BASELINE || h->p.sim == RS_SIM_PEARSON_BASELINE) {
+        rs_set_error("%s: the baseline biases come from a global fit that every rating changes "
+                     "(RS_KNN_BASELINE / RS_SIM_PEARSON_BASELINE): refit", who);
+        return RS_ERR_UNSUPPORTED;
+    }
+    if (h->p.sim == RS_SIM_PEARSON && h->p.pearson_mode == RS_PEARSON_SUMS) {
+        rs_set_error("%s: the recomputed rows are the exact Pearson replay (pearson_mode EXACT)", who);
+        return RS_ERR_UNSUPPORTED;
+    }
+    if (n_left < h->n_left || n_right < h->n_right || nnz < 0) {
+        rs_set_error("%s: n_left=%d n_right=%d nnz=%lld (the fitted counts are %d x %d)", who, n_left, n_right,
+                     (long long)nnz, h->n_left, h->n_right);
+        return RS_ERR_INVALID;
+    }
+    if (nnz > 0 && (!left || !right || !rating)) {
+        rs_set_error("%s: null argument", who);
+        return RS_ERR_INVALID;
+    }
+    if (h->nnz + nnz >= (1ll << 31)) {
+        rs_set_error("%s: %lld ratings in all exceed the 2^31-1 entries supported", who, (long long)(h->nnz + nnz));
+        return RS_ERR_UNSUPPORTED;
+    }
+    return RS_OK;
+}
+
+int32_t rs_knn_update_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
+                             int64_t nnz, int32_t n_left, int32_t n_right, double global_mean) {
+    RS_ENTER(h);
+    RS_TRY(check_update(h, d_left, d_right, d_rating, nnz, n_left, n_right));
+    return rs_update_run(h, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean);
+}
+
+int32_t rs_knn_update(rs_knn *h, const int32_t *left, const int32_t *right, const double *rating, int64_t nnz,
+                      int32_t n_left, int32_t n_right, double global_mean) {
+    RS_ENTER(h);
+    RS_TRY(check_update(h, left, right, rating, nnz, n_left, n_right));
+    void *d_left = nullptr, *d_right = nullptr, *d_rating = nullptr;
+    if (nnz > 0) {
+        RS_TRY(rs_scratch_get(h, RS_SCR_FIT_LEFT, (size_t)nnz * 4, &d_left));
+        RS_TRY(rs_scratch_get(h, RS_SCR_FIT_RIGHT, (size_t)nnz * 4, &d_right));
+        RS_TRY(rs_scratch_get(h, RS_SCR_FIT_RATING, (size_t)nnz * 8, &d_rating));
+        RS_CUDA(cudaMemcpyAsync(d_left, left, (size_t)nnz * 4, cudaMemcpyHostToDevice, h->stream));
+        RS_CUDA(cudaMemcpyAsync(d_right, right, (size_t)nnz * 4, cudaMemcpyHostToDevice, h->stream));
+        RS_CUDA(cudaMemcpyAsync(d_rating, rating, (size_t)nnz * 8, cudaMemcpyHostToDevice, h->stream));
+    }
+    // the update reads its inputs before its validation read-back: they are consumed when it returns
+    return rs_update_run(h, (const int32_t *)d_left, (const int32_t *)d_right, (const double *)d_rating, nnz, n_left,
+                         n_right, global_mean);
 }
 
 static int32_t require_matrix(rs_knn *h, const char *who) {

@@ -71,6 +71,12 @@ inline int64_t rs_cyc_rows(int64_t n, int count, int index) {
     return rows;
 }
 
+// The model arrays rs_knn_update rewrites (update.cu); rs_knn::upd holds their blocks.
+enum rs_upd_array {
+    RS_UPD_L_PTR, RS_UPD_L_COL, RS_UPD_L_VAL, RS_UPD_L_CODE, RS_UPD_LD_VAL, RS_UPD_R_PTR, RS_UPD_R_COL, RS_UPD_R_VAL,
+    RS_UPD_MEANS, RS_UPD_STDDEVS, RS_UPD_PMEANS, RS_UPD_ROW_CNT, RS_UPD_ROW_SUM, RS_UPD_ARRAYS
+};
+
 struct rs_knn {
     std::recursive_mutex mu;             // serialises the ABI calls on this handle (api.cu Guard)
     rs_knn_params p{};
@@ -191,6 +197,16 @@ struct rs_knn {
     double *topk_sim = nullptr;
 
     int32_t *d_flags = nullptr;  // small device scratch for validation flags
+    // rs_knn_update: the model arrays an update rewrote live in blocks of their own (the arena only grows until the
+    // next Fit), two per array: the model's, p[cur], and the spare the next update merges into.  cur = -1 while
+    // the model's array is the Fit's, in the arena.
+    struct UpdArray { void *p[2] = {nullptr, nullptr}; size_t bytes[2] = {0, 0}; int cur = -1; };
+    UpdArray upd[RS_UPD_ARRAYS];
+    void *upd_sims = nullptr;    // the matrix, once an update has grown it out of the arena
+    size_t upd_sims_bytes = 0;
+    bool updated = false;        // an update has run since the last Fit: rs_prep_planes builds into upd_planes
+    void *upd_planes = nullptr;
+    size_t upd_planes_bytes = 0;
     void *ovf = nullptr;         // predict: overflow list (count + indices)
     size_t ovf_bytes = 0;
     std::vector<void *> scratch;         // device staging of the host-pointer entry points
@@ -218,7 +234,7 @@ enum rs_scratch_slot {
     RS_SCR_HOST_SIMS,
     RS_SCR_NB_COUNT,
     RS_SCR_COSUMS,
-    RS_SCR_FIT_LEFT,          // rs_knn_fit's inputs
+    RS_SCR_FIT_LEFT,          // rs_knn_fit's and rs_knn_update's inputs
     RS_SCR_FIT_RIGHT,
     RS_SCR_FIT_RATING,
     RS_SCR_FIT_LEFT_BIAS,
@@ -262,6 +278,10 @@ enum rs_scratch_slot {
     RS_SCR_GIVEN_STDDEVS,
     RS_SCR_GIVEN_PMEANS,
     RS_SCR_GIVEN_SIMS,        // a batch's S* rows
+    // update.cu
+    RS_SCR_UPD_WORK,          // the added ratings sorted both ways, their row pointers, the touched rows
+    RS_SCR_UPD_SORT_TMP,
+    RS_SCR_UPD_SLAB,          // a batch's recomputed rows
 };
 extern "C" int32_t rs_scratch_get(rs_knn *h, int slot, size_t bytes, void **out);
 
@@ -280,6 +300,15 @@ int32_t rs_prep_rt(rs_knn *h);
 int32_t rs_prep_planes(rs_knn *h);
 int32_t rs_row_stats_launch(rs_knn *h, const int64_t *ptr, const double *ld_val, const double *l_val, int64_t n,
                             int want_std, double *means, double *stddevs, double *pmeans);
+int32_t rs_prep_stats(rs_knn *h);
+// Kernels of the CSR build that rs_knn_update runs on the added ratings as Fit runs them on all ratings.
+enum rs_prep_flag { FLAG_BAD_ID = 1, FLAG_NOT_INT8 = 2, FLAG_DUP = 4, FLAG_NAN = 8 };
+__global__ void ptr_from_sorted_kernel(const int32_t *__restrict__ keys, int64_t nnz, int32_t n_rows,
+                                       int64_t *__restrict__ ptr);
+__global__ void gather_keys_kernel(const int32_t *__restrict__ src, const int32_t *__restrict__ perm, int64_t n,
+                                   int32_t *__restrict__ out);
+__global__ void dup_check_kernel(const int32_t *__restrict__ row, const int32_t *__restrict__ col, int64_t nnz,
+                                 int32_t *__restrict__ flags);
 
 // ---- sim_stream.cu ----
 int32_t rs_sim_stream_launch(rs_knn *h);
@@ -323,6 +352,8 @@ struct rs_rec_call {
     double *top_scores;
 };
 int32_t rs_recommend_run(rs_knn *h, const rs_rec_call &c);
+// Rows per batch of a slab of `width` doubles per row: ~256 MiB (RS_KNN_REC_BATCH forces a size).
+int64_t slab_batch(int64_t width, int64_t n);
 
 // ---- given.cu ----
 // The lists of rs_knn_*_given, validated and sorted: list b is entries ptr[b] .. ptr[b+1) of ids / vals (ascending id)
@@ -338,8 +369,25 @@ struct rs_given_lists {
 int32_t rs_given_prepare(rs_knn *h, int32_t n_targets, const int64_t *d_ptr, const int32_t *d_ids,
                          const double *d_vals, int64_t n, rs_given_lists *out);
 // The similarity rows S*[b][v] = Sim(list b, left row v) of the lists ptr[0 .. nq) (ids: right ids), into out[nq][ld].
+// With `rows`, list b is list rows[b] of ptr and its Pearson mean qpmeans[rows[b]].
 int32_t rs_given_sims_launch(rs_knn *h, const int64_t *ptr, const int32_t *ids, const double *vals,
-                             const double *qpmeans, int64_t nq, double *out, int64_t ld);
+                             const double *qpmeans, int64_t nq, double *out, int64_t ld,
+                             const int32_t *rows = nullptr);
+
+// ---- update.cu ----
+int32_t rs_update_run(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating, int64_t nnz,
+                      int32_t n_left, int32_t n_right, double global_mean);
+void rs_update_release(rs_knn *h);
+
+// First position in [lo, hi) of an ascending id array whose id is >= v: the searches of given.cu and update.cu.
+__device__ __forceinline__ int64_t lower_bound_id(const int32_t *__restrict__ col, int64_t lo, int64_t hi, int32_t v) {
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (col[mid] < v) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
 
 // order-preserving map double -> uint64 (larger similarity = larger key); -0.0 folded to +0.0
 __host__ __device__ inline uint64_t rs_sim_key(double s) {

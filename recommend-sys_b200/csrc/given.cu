@@ -61,6 +61,7 @@ struct GivenSimArgs {
     const int32_t *ids;
     const double *vals;
     const double *qpmeans;    // Pearson: each list's own mean, summed in ascending id order (core/sim.go:49-54)
+    const int32_t *rows;      // list b is list rows[b] of ptr / qpmeans (null: list b)
     int64_t nq;
     const int64_t *r_ptr;
     const int32_t *r_col;
@@ -71,16 +72,6 @@ struct GivenSimArgs {
     int64_t ld;
     unsigned long long *counter;
 };
-
-// first position in [lo, hi) whose id is >= v (the ids ascend)
-__device__ __forceinline__ int64_t lower_bound_id(const int32_t *__restrict__ col, int64_t lo, int64_t hi, int32_t v) {
-    while (lo < hi) {
-        const int64_t mid = (lo + hi) >> 1;
-        if (col[mid] < v) lo = mid + 1;
-        else hi = mid;
-    }
-    return lo;
-}
 
 template <int SIM>
 __global__ void __launch_bounds__(GS_WARPS * 32) given_sims_kernel(GivenSimArgs a) {
@@ -99,8 +90,9 @@ __global__ void __launch_bounds__(GS_WARPS * 32) given_sims_kernel(GivenSimArgs 
         const int32_t v1 = v0 + GS_JC < a.n_left ? v0 + GS_JC : a.n_left;
         __syncwarp();                                 // the previous item has finished with acc
         for (int x = lane; x < 3 * GS_JC; x += 32) acc[x] = 0.0;
-        const double aq = SIM == RS_SIM_PEARSON ? a.qpmeans[b] : 0.0;
-        const int64_t eb = a.ptr[b], ee = a.ptr[b + 1];
+        const int64_t lb = a.rows ? a.rows[b] : b;
+        const double aq = SIM == RS_SIM_PEARSON ? a.qpmeans[lb] : 0.0;
+        const int64_t eb = a.ptr[lb], ee = a.ptr[lb + 1];
         for (int64_t x0 = eb; x0 < ee; x0 += 32) {
             // each lane prepares one entry (c, x) of the list: its a-side term and the slice of c's raters in [v0, v1)
             const int64_t e = x0 + lane;
@@ -223,13 +215,13 @@ int32_t rs_given_prepare(rs_knn *h, int32_t n_targets, const int64_t *d_ptr, con
 }
 
 int32_t rs_given_sims_launch(rs_knn *h, const int64_t *ptr, const int32_t *ids, const double *vals,
-                             const double *qpmeans, int64_t nq, double *out, int64_t ld) {
+                             const double *qpmeans, int64_t nq, double *out, int64_t ld, const int32_t *rows) {
     if (nq <= 0) return RS_OK;
     void *counter;
     RS_TRY(rs_scratch_get(h, RS_SCR_GIVEN_COUNTER, 8, &counter));
     RS_CUDA(cudaMemsetAsync(counter, 0, 8, h->stream));
     GivenSimArgs a{};
-    a.ptr = ptr; a.ids = ids; a.vals = vals; a.qpmeans = qpmeans; a.nq = nq;
+    a.ptr = ptr; a.ids = ids; a.vals = vals; a.qpmeans = qpmeans; a.rows = rows; a.nq = nq;
     a.r_ptr = h->r_ptr; a.r_col = h->r_col; a.r_val = h->r_val; a.pmeans = h->pmeans;
     a.n_left = h->n_left;
     a.n_blk = (h->n_left + GS_JC - 1) / GS_JC;

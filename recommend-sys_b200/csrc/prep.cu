@@ -44,8 +44,6 @@ namespace {
 constexpr int T = 256;
 inline unsigned blocks_for(int64_t n, int t = T) { return (unsigned)((n + t - 1) / t); }
 
-enum { FLAG_BAD_ID = 1, FLAG_NOT_INT8 = 2, FLAG_DUP = 4, FLAG_NAN = 8 };
-
 // (the per-row counts are NOT taken here: 40 M atomic increments were the largest kernel of the ML-20M prep,
 // 1.0 ms; the row pointers come out of the sorted key sequences instead, ptr_from_sorted_kernel)
 __global__ void iota_validate_kernel(const int32_t *__restrict__ left, const int32_t *__restrict__ right,
@@ -62,6 +60,8 @@ __global__ void iota_validate_kernel(const int32_t *__restrict__ left, const int
     if (!(v == rint(v) && fabs(v) <= 11.0)) f |= FLAG_NOT_INT8;
     if (f) atomicOr(flags, f);
 }
+
+}  // namespace
 
 // CSR row pointers from the ascending key sequence of a sort: ptr[k] = first position whose key is >= k
 // (k = 0 .. n_rows; empty rows included).  The entry that opens a new key closes every pointer in between.
@@ -99,6 +99,8 @@ __global__ void dup_check_kernel(const int32_t *__restrict__ row, const int32_t 
     if (i == 0 || i >= nnz) return;
     if (row[i] == row[i - 1] && col[i] == col[i - 1]) atomicOr(flags, FLAG_DUP);
 }
+
+namespace {
 
 __global__ void gather_val_kernel(const int32_t *__restrict__ perm, const double *__restrict__ rating, int64_t nnz,
                                   double *__restrict__ val) {
@@ -357,6 +359,27 @@ int bits_for(int32_t n) {
 
 }  // namespace
 
+// The statistics of every left row from the left CSR, into the buffers h points to: means, stddevs (z-score) and
+// pmeans, and for integer ratings row_cnt / row_sum.  Fit's, and rs_knn_update's for the merged rows.
+int32_t rs_prep_stats(rs_knn *h) {
+    cudaStream_t st = h->stream;
+    const int32_t nl = h->n_left;
+    const int want_std = h->p.knn_type == RS_KNN_ZSCORE;
+    if (h->rating_class == RS_CLASS_INT8) {
+        row_isum_kernel<<<blocks_for((int64_t)nl * 32), T, 0, st>>>(h->l_ptr, h->l_code, nl, h->row_cnt, h->row_sum);
+        means_from_isum_kernel<<<blocks_for(nl), T, 0, st>>>(h->row_cnt, h->row_sum, nl, h->means, h->pmeans);
+        h->prof.total_launches += 2;
+    }
+    if (h->rating_class != RS_CLASS_INT8 || want_std) {
+        row_stats_ordered_kernel<<<blocks_for((int64_t)nl * 32), T, 0, st>>>(
+            h->l_ptr, h->ld_val, h->l_val, nl, h->rating_class != RS_CLASS_INT8, want_std, h->means, h->stddevs,
+            h->pmeans);
+        h->prof.total_launches++;
+    }
+    RS_CUDA(cudaGetLastError());
+    return RS_OK;
+}
+
 // Row statistics of `n` rows given as a CSR: the entries of row i are ptr[i] .. ptr[i+1) of ld_val (dataset order:
 // means, stddevs) and of l_val (ascending id: pmeans).  Fit's statistics, for the rating lists of rs_knn_*_given.
 int32_t rs_row_stats_launch(rs_knn *h, const int64_t *ptr, const double *ld_val, const double *l_val, int64_t n,
@@ -547,20 +570,11 @@ int32_t rs_prep_build(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
     RS_TRY(rs_alloc(h, &h->means, (size_t)nl + 1));
     RS_TRY(rs_alloc(h, &h->stddevs, (size_t)nl + 1));
     RS_TRY(rs_alloc(h, &h->pmeans, (size_t)nl + 1));
-    const int want_std = h->p.knn_type == RS_KNN_ZSCORE;
     if (h->rating_class == RS_CLASS_INT8) {
         RS_TRY(rs_alloc(h, &h->row_cnt, (size_t)nl + 1));
         RS_TRY(rs_alloc(h, &h->row_sum, (size_t)nl + 1));
-        row_isum_kernel<<<blocks_for((int64_t)nl * 32), T, 0, st>>>(h->l_ptr, h->l_code, nl, h->row_cnt, h->row_sum);
-        means_from_isum_kernel<<<blocks_for(nl), T, 0, st>>>(h->row_cnt, h->row_sum, nl, h->means, h->pmeans);
-        h->prof.total_launches += 2;
     }
-    if (h->rating_class != RS_CLASS_INT8 || want_std) {
-        row_stats_ordered_kernel<<<blocks_for((int64_t)nl * 32), T, 0, st>>>(
-            h->l_ptr, h->ld_val, h->l_val, nl, h->rating_class != RS_CLASS_INT8, want_std, h->means, h->stddevs,
-            h->pmeans);
-        h->prof.total_launches++;
-    }
+    RS_TRY(rs_prep_stats(h));
 
     if (h->p.sim == RS_SIM_SLOPE_ONE) {
         RS_TRY(rs_alloc(h, &h->right_means, (size_t)nr + 1));
@@ -827,7 +841,20 @@ int32_t rs_prep_planes(rs_knn *h) {
     h->tc_npad = ((int64_t)h->n_left + RS_TC_BM - 1) / RS_TC_BM * RS_TC_BM;
     h->tc_kpad = ((int64_t)h->n_right + RS_TC_KBLK - 1) / RS_TC_KBLK * RS_TC_KBLK;
     size_t bytes = 3 * (size_t)h->tc_npad * (size_t)h->tc_kpad;
-    RS_TRY(rs_alloc(h, &h->planes, bytes));
+    if (h->updated) {
+        // after rs_knn_update: a block of their own, reused while it is large enough, so that updates alternating with
+        // rs_knn_cosums do not grow the arena.  The stream has drained since the block's last use (rs_knn_cosums ends
+        // with a synchronisation).
+        if (h->upd_planes_bytes < bytes) {
+            rs_cached_free(h->device, h->upd_planes, h->upd_planes_bytes);
+            h->upd_planes = nullptr;
+            h->upd_planes_bytes = 0;
+            RS_TRY(rs_cached_malloc(h->device, &h->upd_planes, bytes + bytes / 4 + 256, &h->upd_planes_bytes));
+        }
+        h->planes = static_cast<int8_t *>(h->upd_planes);
+    } else {
+        RS_TRY(rs_alloc(h, &h->planes, bytes));
+    }
     RS_CUDA(cudaMemsetAsync(h->planes, 0, bytes, st));
     scatter_planes_kernel<<<blocks_for((int64_t)h->n_left * 32), T, 0, st>>>(h->l_ptr, h->l_col, h->l_code,
                                                                             h->n_left, h->tc_npad, h->tc_kpad,

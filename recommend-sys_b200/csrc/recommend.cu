@@ -230,6 +230,8 @@ int32_t score_rows(rs_knn *h, RecArgs ra, const GivenBatch *g = nullptr) {
     return RS_OK;
 }
 
+}  // namespace
+
 // Rows per batch of a slab of `width` doubles per row: ~256 MiB.
 int64_t slab_batch(int64_t width, int64_t n) {
     int64_t batch = ((int64_t)256 << 20) / (width * 8);
@@ -238,6 +240,8 @@ int64_t slab_batch(int64_t width, int64_t n) {
     if (batch > n) batch = n;
     return batch;
 }
+
+namespace {
 
 // Left queries on a row shard: the queries this shard answers (values and positions), compacted; their count is read
 // back to size the batches.

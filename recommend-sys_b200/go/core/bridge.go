@@ -136,6 +136,15 @@ func (d *deviceKNN) fit(left, right []int32, rating []float64, nLeft, nRight int
 	runtime.KeepAlive(rating)
 }
 
+// update adds ratings (inner ids, in call order) to the fitted model: it becomes the Fit of the union (rs_knn_update).
+func (d *deviceKNN) update(left, right []int32, rating []float64, nLeft, nRight int, globalMean float64) {
+	check(C.rs_knn_update(d.h, i32(left), i32(right), f64(rating), C.int64_t(len(rating)), C.int32_t(nLeft),
+		C.int32_t(nRight), C.double(globalMean)))
+	runtime.KeepAlive(left)
+	runtime.KeepAlive(right)
+	runtime.KeepAlive(rating)
+}
+
 // baselineALS is the EXTENSION behind Parameters["baseline"] = "als" (BASELINE.json config 3): ALS
 // baseline estimates computed on the device instead of BaseLine.Fit's sequential SGD
 // (core/base.go:135-163).  Returns (userBias, itemBias); the global bias is the global mean.

@@ -120,6 +120,52 @@ func (K *KNN) Fit(trainSet TrainSet) {
 	}
 }
 
+// Update adds the ratings of rowSet (raw user, raw item, rating; users and items may be new) to the fitted model
+// without a refit (rs_knn_update, an extension: the reference has none).  The model becomes the Fit of NewTrainSet of
+// the training rows followed by rowSet's, bit for bit, and Data that TrainSet; only the rows of the users (items) the
+// ratings touch are recomputed.  A pair the model holds already, KNNBaseline, PearsonBaseline, Pearson in sums mode,
+// row shards and top-k-only stores are refused (a panic, as every refused call).
+func (K *KNN) Update(rowSet DataSet) {
+	n0 := K.Data.Length()
+	trainSet := NewTrainSet(DataSet{
+		Users:   append(append([]int{}, K.Data.Users...), rowSet.Users...),
+		Items:   append(append([]int{}, K.Data.Items...), rowSet.Items...),
+		Ratings: append(append([]float64{}, K.Data.Ratings...), rowSet.Ratings...),
+	})
+	n := trainSet.Length() - n0
+	left := make([]int32, n)
+	right := make([]int32, n)
+	for i := 0; i < n; i++ {
+		u := int32(trainSet.ConvertUserID(trainSet.Users[n0+i]))
+		it := int32(trainSet.ConvertItemID(trainSet.Items[n0+i]))
+		if K.userBased {
+			left[i], right[i] = u, it
+		} else {
+			left[i], right[i] = it, u
+		}
+	}
+	nLeft, nRight := trainSet.UserCount, trainSet.ItemCount
+	if !K.userBased {
+		nLeft, nRight = nRight, nLeft
+	}
+	K.dev.update(left, right, trainSet.Ratings[n0:], nLeft, nRight, trainSet.GlobalMean)
+	K.Data = trainSet
+	K.GlobalMean = trainSet.GlobalMean
+	if K.userBased {
+		K.LeftRatings, K.RightRatings = trainSet.UserRatings(), trainSet.ItemRatings()
+	} else {
+		K.LeftRatings, K.RightRatings = trainSet.ItemRatings(), trainSet.UserRatings()
+	}
+	sorts(K.LeftRatings)
+	K.nLeft = nLeft
+	if K.KNNType == centered || K.KNNType == zScore {
+		K.Means = K.dev.means(nLeft)
+	}
+	if K.KNNType == zScore {
+		K.StdDevs = K.dev.stddevs(nLeft)
+	}
+}
+
 // PredictBatch implements BatchPredictor: DataSet.Predict (core/data.go:98-105) hands the
 // whole test set over in one cgo call.
 func (K *KNN) PredictBatch(userIDs, itemIDs []int) []float64 {

@@ -102,6 +102,16 @@ inline TrainSet NewTrainSet(const DataSet &rowSet) {  // core/data.go:131-154
     return s;
 }
 
+// The TrainSet of t's rows followed by rowSet's: NewTrainSet of the concatenation (inner ids continue the order of
+// first appearance, GlobalMean is the concatenation's).
+inline TrainSet Extend(const TrainSet &t, const DataSet &rowSet) {
+    DataSet d = t;
+    d.Users.insert(d.Users.end(), rowSet.Users.begin(), rowSet.Users.end());
+    d.Items.insert(d.Items.end(), rowSet.Items.begin(), rowSet.Items.end());
+    d.Ratings.insert(d.Ratings.end(), rowSet.Ratings.begin(), rowSet.Ratings.end());
+    return NewTrainSet(d);
+}
+
 // core/data.go:49-70 — the reference's permutation is unseeded (SURVEY.md hazard 3); here mt19937_64(seed).
 inline void KFold(const DataSet &d, int k, int64_t seed, std::vector<TrainSet> &trains, std::vector<DataSet> &tests) {
     const size_t n = d.Length();
@@ -228,8 +238,26 @@ struct KNN : Estimator {
         minK_ = p.min_k;
         rs_check(rs_knn_fit(h_, left.data(), right.data(), t.Ratings.data(), (int64_t)t.Length(), nLeft_, nRight,
                             t.GlobalMean, lb, rb, gb));
-        if (KNNType == "centered" || KNNType == "zscore") { Means.resize(nLeft_); rs_check(rs_knn_means(h_, Means.data())); }
-        if (KNNType == "zscore") { StdDevs.resize(nLeft_); rs_check(rs_knn_stddevs(h_, StdDevs.data())); }
+        extended_.reset();
+        ReadStats();
+    }
+
+    // Adds the ratings of `rowSet` (raw user, raw item, rating; users and items may be new) to the fitted model
+    // without a refit (rs_knn_update): the model becomes the Fit of Extend(*Data, rowSet), bit for bit, and Data that
+    // TrainSet (owned by the estimator).
+    void Update(const DataSet &rowSet) {
+        auto t = std::make_shared<const TrainSet>(Extend(*Data, rowSet));
+        const size_t n0 = Data->Length();
+        const auto &left = userBased_ ? t->innerUsers : t->innerItems;
+        const auto &right = userBased_ ? t->innerItems : t->innerUsers;
+        const int nLeft = userBased_ ? t->UserCount : t->ItemCount, nRight = userBased_ ? t->ItemCount : t->UserCount;
+        rs_check(rs_knn_update(h_, left.data() + n0, right.data() + n0, t->Ratings.data() + n0,
+                               (int64_t)(t->Length() - n0), nLeft, nRight, t->GlobalMean));
+        extended_ = t;
+        Data = t.get();
+        GlobalMean = t->GlobalMean;
+        nLeft_ = nLeft;
+        ReadStats();
     }
 
     std::vector<double> PredictBatch(const std::vector<int64_t> &users, const std::vector<int64_t> &items) override {
@@ -309,6 +337,11 @@ struct KNN : Estimator {
     std::unique_ptr<Estimator> Clone() const override { return std::make_unique<KNN>(KNNType, Params); }
 
   private:
+    void ReadStats() {
+        if (KNNType == "centered" || KNNType == "zscore") { Means.resize(nLeft_); rs_check(rs_knn_means(h_, Means.data())); }
+        if (KNNType == "zscore") { StdDevs.resize(nLeft_); rs_check(rs_knn_stddevs(h_, StdDevs.data())); }
+    }
+
     // core/knn.go:80-81 reads k / mink in Predict: SetParams after Fit takes effect at the next call
     void SyncK() {
         const int k = Params.GetInt("k", 40), minK = Params.GetInt("mink", 1);
@@ -316,6 +349,7 @@ struct KNN : Estimator {
     }
 
     rs_knn *h_ = nullptr;
+    std::shared_ptr<const TrainSet> extended_;   // Data after an Update
     int k_ = 40, minK_ = 1;   // what the handle currently holds
     bool userBased_ = true;
     int nLeft_ = 0;

@@ -5,6 +5,8 @@
 //             <userBased 0|1> <k> <n> <user> [<user> ...]
 //   recommend ... <k> <n> --given <ratings file>   (KNN::RecommendGiven: the users of the second file, with the
 //             ratings given there instead of the train set's; one line per user in order of first appearance)
+//   recommend ... <k> <n> --update <ratings file> <user> [<user> ...]   (KNN::Update with the second file's ratings,
+//             then KNN::Recommend)
 //
 // The estimator is fitted with k = 40 and `k` is set afterwards (Predict reads k at call time, core/knn.go:80-81).
 // One output line per user: the user id, then n pairs "item score", the score as the 16 hex digits of its bits.
@@ -54,7 +56,12 @@ int main(int argc, char **argv) {
     if (!std::strcmp(argv[7], "--given") && argc == 9) {
         knn.RecommendGiven(load_file(argv[8]), n, users, items, scores);
     } else {
-        for (int a = 7; a < argc; a++) users.push_back(std::atoll(argv[a]));
+        int a = 7;
+        if (!std::strcmp(argv[7], "--update") && argc >= 10) {
+            knn.Update(load_file(argv[8]));
+            a = 9;
+        }
+        for (; a < argc; a++) users.push_back(std::atoll(argv[a]));
         knn.Recommend(users, n, items, scores);
     }
     for (size_t u = 0; u < users.size(); u++) {
