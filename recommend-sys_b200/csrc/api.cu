@@ -53,8 +53,6 @@ void free_fit_state(rs_knn *h) {
     h->cp = nullptr;
     h->l2r = nullptr;
     h->row_order = nullptr;
-    h->row_heavy = nullptr;
-    h->n_heavy = 0;
     h->n_pop = h->pop_ld = 0;
     h->rank = h->lab_row = h->pop_items = nullptr;
     h->pop_dense = nullptr;
@@ -150,8 +148,6 @@ int32_t init_handle(rs_knn *h) {
     RS_CUDA(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
     RS_CUDA(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
     RS_CUDA(cudaEventCreateWithFlags(&h->ev_in, cudaEventDisableTiming));
-    RS_CUDA(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-    RS_CUDA(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
     h->stream = h->own_stream;
     RS_CUDA(cudaEventCreate(&h->ev_a));
     RS_CUDA(cudaEventCreate(&h->ev_b));
@@ -256,8 +252,6 @@ int32_t rs_knn_destroy(rs_knn *h) {
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     if (h->aux_stream) cudaStreamDestroy(h->aux_stream);
     if (h->ev_in) cudaEventDestroy(h->ev_in);
-    if (h->ev_fork) cudaEventDestroy(h->ev_fork);
-    if (h->ev_join) cudaEventDestroy(h->ev_join);
     delete h;
     return RS_OK;
 }

@@ -85,7 +85,6 @@ struct rs_knn {
     cudaStream_t stream = nullptr;
     cudaStream_t aux_stream = nullptr;   // read-backs of Fit statistics that must not wait for the similarity kernel
     cudaEvent_t ev_in = nullptr;         // the host inputs of rs_knn_fit have been consumed
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;   // heavy-row kernel on aux_stream beside the column walk
     cudaEvent_t ev_a = nullptr, ev_b = nullptr, ev_c = nullptr, ev_d = nullptr, ev_e = nullptr;
     rs_knn_profile prof{};
     // pending event pairs whose elapsed time has not been folded into prof yet
@@ -166,12 +165,10 @@ struct rs_knn {
     int64_t *l2r = nullptr;
     int32_t *perm_lr = nullptr, *perm_rl = nullptr, *perm_tmp = nullptr;  // CSR position -> input row (arena, valid until the next Fit)
     int32_t *row_order = nullptr;  // left rows sorted by descending length
-    int32_t *row_heavy = nullptr;  // heavy rows split off that order (sim_stream.cu: sim_stream_heavy_kernel)
-    int32_t n_heavy = 0;
-    // popular columns (sim_stream.cu: sim_pop_kernel): the n_pop longest rows, longest first.  Their ratings are
-    // taken out of the right CSR the column walk reads (walk CSR: w_ptr / w_col / w_dev, `cp` and `l2r` refer to
-    // it) and kept as a dense table pop_dense[n_right][pop_ld] instead (one byte per cell when every rating is a
-    // small integer, else the b-side double; 0 / NaN = no rating).
+    // popular columns (sim_stream.cu: the dense items of sim_stream_kernel): the n_pop longest rows, longest first.
+    // Their ratings are taken out of the right CSR the column walk reads (walk CSR: w_ptr / w_col / w_dev, `cp` and
+    // `l2r` refer to it) and kept as a dense table pop_dense[n_right][pop_ld] instead (one byte per cell when every
+    // rating is a small integer, else the b-side double; 0 / NaN = no rating).
     // Every row has a RANK, its position in the stable longest-first order of all rows: ranks below n_pop are the
     // popular list, and the other rows are the walk's columns under the LABEL rank - n_pop (the walk CSR holds
     // labels, ascending within each right row), so the long rows have the small labels.

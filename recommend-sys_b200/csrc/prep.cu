@@ -244,7 +244,7 @@ __global__ void compose_l2r_kernel(const int32_t *__restrict__ perm_lr, const in
     if (e < n) l2r[e] = inv_rl[perm_lr[e]];
 }
 
-// ---- popular columns (sim_stream.cu: sim_pop_kernel) ----
+// ---- popular columns (sim_stream.cu: the dense items of sim_stream_kernel) ----
 // n_pop = rows of at least min_len entries (len_sorted is descending), at most cap
 __global__ void pop_count_kernel(const int32_t *__restrict__ len_sorted, int32_t n, int64_t min_len, int32_t cap,
                                  int32_t *__restrict__ out) {
@@ -607,47 +607,6 @@ int32_t rs_prep_build(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
     return RS_OK;
 }
 
-// Heavy rows (sim_stream.cu: sim_stream_heavy_kernel): rows of >= min_len entries are split off the
-// longest-first order and processed by producer / consumer CTAs.  `order`: the rows to process, longest
-// first.  Writes h->row_order (the other rows, same order), h->row_heavy and the counts.
-struct HeavyPred {
-    const int64_t *l_ptr;
-    int64_t min_len;
-    bool negate;
-    __host__ __device__ bool operator()(const int32_t &i) const { return ((l_ptr[i + 1] - l_ptr[i]) >= min_len) != negate; }
-};
-
-static int32_t split_heavy_rows(rs_knn *h, int32_t *order, int64_t n_rows, bool allow) {
-    cudaStream_t st = h->stream;
-    // On ONE GPU the serial walk of a blockbuster row hides under the other rows' work; under cyclic sharding the
-    // per-GPU work shrinks and that walk becomes the critical path (profiles/r02_stream_notes.md).
-    int64_t min_len = h->cyc_R > 1 ? 8192 : -1;
-    if (const char *e = getenv("RS_KNN_HEAVY_MIN")) min_len = atoll(e);      // tests: 0 = every row
-    h->n_heavy = 0;
-    h->row_heavy = nullptr;
-    h->row_order = order;
-    h->n_work_rows = n_rows;
-    if (n_rows <= 0 || !allow || min_len < 0 || h->stream_jc != 256) return RS_OK;
-    int32_t *rest, *d_num;
-    RS_TRY(rs_alloc(h, &h->row_heavy, (size_t)n_rows));
-    RS_TRY(rs_alloc(h, &rest, (size_t)n_rows));
-    RS_TRY(rs_alloc(h, &d_num, 4));
-    HeavyPred yes{h->l_ptr, min_len, false}, no{h->l_ptr, min_len, true};
-    size_t need = 0;
-    RS_CUDA(cub::DeviceSelect::If(nullptr, need, order, h->row_heavy, d_num, (int)n_rows, yes, st));
-    void *tmp;
-    RS_TRY(rs_dev_alloc(h, &tmp, need + 256));
-    RS_CUDA(cub::DeviceSelect::If(tmp, need, order, h->row_heavy, d_num, (int)n_rows, yes, st));
-    RS_CUDA(cub::DeviceSelect::If(tmp, need, order, rest, d_num + 1, (int)n_rows, no, st));
-    int32_t cnt = 0;
-    RS_CUDA(cudaMemcpyAsync(&cnt, d_num, 4, cudaMemcpyDeviceToHost, st));
-    RS_CUDA(cudaStreamSynchronize(st));
-    h->n_heavy = cnt;
-    h->row_order = rest;
-    h->n_work_rows = n_rows - cnt;
-    return RS_OK;
-}
-
 // Popular columns: the rows of >= min_len entries (at most RS_POP_MAX, the longest).  `sorted`: ALL rows, longest
 // first (stable: ties by id), so a row's position in it is its rank; `len_sorted`: their lengths; `order` / n_rows:
 // the rows of this shard, longest first.  Splits the popular rows' ratings off the right CSR into the dense table,
@@ -800,13 +759,10 @@ int32_t rs_prep_rt(rs_knn *h) {
         RS_CUDA(cub::DeviceRadixSort::SortPairsDescending(tmp, need, len + rb, len_sorted + rb, ids + rb,
                                                           sorted, (int)rows, 0, 32, st));
         // Full-matrix Fits (one GPU, or cyclic shards) compute one triangle and mirror the other: there the longest
-        // rows can be taken out of the column walk.  RS_KNN_POP=0 keeps them in it (under cyclic sharding as
-        // producer / consumer CTAs: split_heavy_rows); RS_KNN_HEAVY_MIN sets the length threshold (tests).
+        // rows are taken out of the column walk as popular columns.  RS_KNN_POP_MIN sets the length threshold (tests).
         const bool full = h->row_begin == 0 && h->row_end == h->n_left;
         int64_t min_len = 8192;
-        if (const char *e = getenv("RS_KNN_HEAVY_MIN")) min_len = atoll(e);
-        bool pop = full && min_len >= 0;
-        if (const char *e = getenv("RS_KNN_POP")) pop = pop && atoi(e) != 0;
+        if (const char *e = getenv("RS_KNN_POP_MIN")) min_len = atoll(e);
         int32_t *order = sorted;
         int64_t n_order = rows;
         if (h->cyc_R > 1) {
@@ -823,12 +779,9 @@ int32_t rs_prep_rt(rs_knn *h) {
             order = owned;
             n_order = h->rows_local;
         }
-        h->n_heavy = 0;
-        h->row_heavy = nullptr;
         h->row_order = order;
         h->n_work_rows = n_order;
-        if (pop) RS_TRY(split_popular(h, sorted, len_sorted, order, n_order, min_len));
-        else RS_TRY(split_heavy_rows(h, order, n_order, full));
+        if (full) RS_TRY(split_popular(h, sorted, len_sorted, order, n_order, min_len));
         build_cp();
     }
     RS_CUDA(cudaGetLastError());

@@ -18,12 +18,7 @@
 // 12 B per triple; see DESIGN.md and profiles/.
 //
 // The longest rows ("popular columns") are taken out of that walk: their pairs are dense work items of the same
-// kernel and queue (pop_item below: lane = column, accumulators in registers), see the comment there.  The
-// producer / consumer kernel further down (sim_stream_heavy_kernel) is the earlier treatment of those rows, kept
-// behind RS_KNN_POP=0 and by the tests.
-#include <cstdlib>
-#include <cstring>
-
+// kernel and queue (pop_item below: lane = column, accumulators in registers), see the comment there.
 #include "common.cuh"
 #include "sim_terms.cuh"
 
@@ -87,7 +82,6 @@ struct PopArgs {
     int32_t n_blk, ld;        // blocks of 32 popular columns; row stride of the table
     const void *dense;
     int64_t n_first;          // dense items of the shard's popular rows: they open the work queue (longest chains)
-    int32_t skip;             // profiling only (RS_KNN_STREAM_SKIP, results are wrong): 1 popular rows' dense items, 2 walk items, 4 other rows' dense items
 };
 
 __device__ __forceinline__ void pop_cp_async16(void *dst, const void *src) {
@@ -270,7 +264,6 @@ __global__ void __launch_bounds__(SW * 32, 4) sim_stream_kernel(StreamArgs a, Po
             int64_t d = (int64_t)item;
             if (d >= pa.n_first) d = d >= pa.n_first + n_items ? d - n_items : -1;
             if (d >= pa.n_rows * pa.n_blk) break;
-            if (pa.skip && ((d >= 0 && d < pa.n_first && (pa.skip & 1)) || (d < 0 && (pa.skip & 2)) || (d >= pa.n_first && (pa.skip & 4)))) continue;
             if (d >= 0) {
                 __syncwarp();
                 if (POP == 1) pop_item<SIM, SHRINK, uint8_t>(a, pa, d, acc, lane);
@@ -395,235 +388,9 @@ __global__ void __launch_bounds__(SW * 32, 4) sim_stream_kernel(StreamArgs a, Po
     }
 }
 
-
-
-// ---------------------------------------------------------------------------------------------
-// Heavy rows: producer / consumer.  In the column walk above ONE warp owns a (row, chunk) item and
-// walks the row's entries serially, each step waiting for a gather that depends on the previous
-// lookup: ~600 cycles per entry under load, i.e. 25 ms for a blockbuster row of 78 k entries whatever
-// else the GPU does — invisible next to 41 ms of total work on one GPU, the critical path of a Fit
-// sharded over 8 (profiles/r02_stream_notes.md).  Here a whole CTA owns the item: eight PRODUCER
-// warps look the entries' runs up and copy them (cp.async: no registers, dozens of copies in flight)
-// into a ring of shared-memory slots, one entry per slot, in entry order; four CONSUMER warps, each
-// owning 64 of the chunk's 256 columns, apply the slots in order to the accumulators of their columns
-// — every accumulator receives the same terms in the same order with the same IEEE operations as in
-// the column walk, so the result is bit-identical; the memory latency is taken off the chain and the
-// chain itself is cut in four.
-constexpr int HV_CONS = 4, HV_PROD = 8, HV_WARPS = HV_CONS + HV_PROD;
-constexpr int HV_SLOTS = 32;      // entries in flight per CTA
-constexpr int HV_DEPTH = 3;       // copies a producer keeps in flight before it publishes the oldest
-constexpr int HV_JC = 256;        // same chunk width and chunk pointers as the column walk
-
-struct HeavyArgs {
-    const int32_t *rows;          // heavy rows, longest first
-    int32_t n_rows;
-    unsigned long long *counter;
-};
-
-__device__ __forceinline__ uint32_t hv_smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void hv_cp_async4(void *dst, const void *src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(hv_smem_u32(dst)), "l"(src) : "memory");
-}
-__device__ __forceinline__ void hv_cp_async8(void *dst, const void *src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(hv_smem_u32(dst)), "l"(src) : "memory");
-}
-__device__ __forceinline__ void hv_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void hv_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-template <int SIM, bool SHRINK>
-__global__ void __launch_bounds__(HV_WARPS * 32, 1) sim_stream_heavy_kernel(StreamArgs a, HeavyArgs hv) {
-    constexpr int NACC = SHRINK ? 4 : 3;
-    extern __shared__ double hv_smem[];
-    double *acc = hv_smem;                                              // [NACC][HV_JC]
-    double *s_rb = acc + NACC * HV_JC;                                  // [HV_SLOTS][HV_JC]
-    int32_t *s_jc = reinterpret_cast<int32_t *>(s_rb + HV_SLOTS * HV_JC);   // [HV_SLOTS][HV_JC]
-    double *s_ra = reinterpret_cast<double *>(s_jc + HV_SLOTS * HV_JC);     // [HV_SLOTS]
-    int32_t *s_n = reinterpret_cast<int32_t *>(s_ra + HV_SLOTS);            // [HV_SLOTS]
-    volatile int32_t *s_ready = s_n + HV_SLOTS;                             // [HV_SLOTS]  (entry index + 1) << 9 | raters, once the entry has landed
-    volatile int32_t *s_consumed = s_ready + HV_SLOTS;                      // [HV_CONS] entries applied so far, per consumer
-    volatile long long *s_item = reinterpret_cast<volatile long long *>(s_consumed + HV_CONS);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int64_t Q = a.n_chunks;
-    const int64_t n_items = (int64_t)hv.n_rows * Q;
-    const double nan_v = __longlong_as_double(0x7ff8000000000001ll);
-
-    for (;;) {
-        __syncthreads();                                     // the previous item is finished by every warp
-        if (threadIdx.x == 0) *s_item = (long long)atomicAdd(hv.counter, 1ull);
-        if (threadIdx.x < HV_SLOTS) s_ready[threadIdx.x] = 0;
-        if (threadIdx.x < HV_CONS) s_consumed[threadIdx.x] = 0;
-        __syncthreads();
-        const int64_t item = *s_item;
-        if (item >= n_items) break;
-        const int64_t q = item % Q;
-        const int32_t i = hv.rows[item / Q];
-        const int j0 = (int)(q * HV_JC);
-        if (a.symmetric == 1 && j0 + HV_JC <= i) continue;   // every column of the chunk is < i
-        if (a.symmetric == 2 && j0 > i) continue;            // every column of the chunk is > i
-        const bool diag_chunk = (i >= j0 && i < j0 + HV_JC);
-        const int64_t eb = a.l_ptr[i], ee = a.l_ptr[i + 1];
-        const int n_ent = (int)(ee - eb);
-
-        if (warp < HV_CONS) {
-            // ======================= consumers: apply the slots in entry order, 64 columns each =======================
-            const int cw = warp;                              // owns columns [64 cw, 64 cw + 64) of the chunk
-#pragma unroll
-            for (int z = 0; z < NACC; z++)
-                for (int x = lane; x < 64; x += 32) acc[z * HV_JC + 64 * cw + x] = 0.0;
-            __syncwarp();
-            for (int e = 0; e < n_ent; e++) {
-                const int slot = e % HV_SLOTS;
-                // one word says both "entry e has landed" and how many raters it brought: (e + 1) << 9 | n
-                int word;
-                while (((word = s_ready[slot]) >> 9) != e + 1) {}
-                __syncwarp();
-                const int n = word & 511;
-                if (n > 0) {
-                    const double ra = s_ra[slot];
-                    const double raa = ra * ra;                                   // core/sim.go:19 / :75
-                    const double *rbs = s_rb + slot * HV_JC;
-                    const int32_t *jcs = s_jc + slot * HV_JC;
-                    // the raters of ONE entry are distinct accumulators: their read-modify-writes are independent,
-                    // so up to 64 (or all 256) of them are loaded first and applied without ordering
-                    auto apply = [&](int j, double rb) {
-                        if (SIM == RS_SIM_MSD) {
-                            const double d = ra - rb;
-                            acc[j] += d * d;                                      // core/sim.go:37
-                            acc[HV_JC + j] += 1.0;                                // core/sim.go:38
-                        } else {
-                            acc[j] += raa;                                        // core/sim.go:19 / :75
-                            acc[HV_JC + j] += rb * rb;                            // core/sim.go:20 / :76
-                            acc[2 * HV_JC + j] += ra * rb;                        // core/sim.go:21 / :77
-                            if (SHRINK) acc[3 * HV_JC + j] += 1.0;
-                        }
-                    };
-                    if (n <= 64) {
-                        int jv[2];
-                        double rbv[2];
-#pragma unroll
-                        for (int u = 0; u < 2; u++) {
-                            const int t = lane + 32 * u;
-                            jv[u] = t < n ? jcs[t] - j0 : -1;
-                            rbv[u] = t < n ? rbs[t] : 0.0;
-                        }
-#pragma unroll
-                        for (int u = 0; u < 2; u++) if (jv[u] >= 0 && (jv[u] >> 6) == cw) apply(jv[u], rbv[u]);
-                    } else {
-                        int jv[8];
-                        double rbv[8];
-#pragma unroll
-                        for (int u = 0; u < 8; u++) {
-                            const int t = lane + 32 * u;
-                            jv[u] = t < n ? jcs[t] - j0 : -1;
-                            rbv[u] = t < n ? rbs[t] : 0.0;
-                        }
-#pragma unroll
-                        for (int u = 0; u < 8; u++) {
-                            const bool mine = jv[u] >= 0 && (jv[u] >> 6) == cw;
-                            if (!__any_sync(0xffffffffu, mine)) continue;          // the run is sorted: this consumer's columns are 1-2 of the 8 groups
-                            if (mine) apply(jv[u], rbv[u]);
-                        }
-                    }
-                }
-                __syncwarp();                                 // entry e is complete before e + 1 touches the same j
-                if (lane == 0) s_consumed[cw] = e + 1;        // the slot is free once all consumers are past it
-            }
-            __syncwarp();
-            double *out = a.sims + (a.cyc_R > 1 ? rs_cyc_local(i, a.cyc_R) : (int64_t)(i - a.row_begin)) * a.ld_s + j0;
-            for (int j = 64 * cw + lane; j < 64 * cw + 64; j += 32) {
-                const int64_t col = (int64_t)j0 + j;
-                if (col >= a.n_left) break;
-                if (a.symmetric == 1 && col < i) continue;                        // mirror pass writes it
-                if (a.symmetric == 2 && col > i) break;
-                double s = sim_value<SIM, SHRINK>(acc + j, HV_JC, a.shrinkage);      // core/sim.go:43 / :24 / :80
-                if (col == (int64_t)i) s = nan_v;                                 // diagonal stays NaN
-                out[j] = s;
-            }
-        } else {
-            // ======================= producers: entries e = p, p + HV_PROD, ... =======================
-            const int p = warp - HV_CONS;
-            double ai = 0.0;
-            if (SIM == RS_SIM_PEARSON) ai = a.pmeans[i];
-            if (SIM == RS_SIM_PEARSON_BASELINE) ai = a.global_bias + a.left_bias[i];
-            auto ent_of = [&](int k) { return p + k * HV_PROD; };   // entry index of this producer's k-th entry
-            int issued = 0, published = 0;                    // entries of this producer whose copies were committed / made visible
-            auto publish = [&](int k) {                       // the copies of entry k have landed (every lane waited)
-                __syncwarp();
-                __threadfence_block();
-                if (lane == 0) { const int e = ent_of(k); s_ready[e % HV_SLOTS] = ((e + 1) << 9) | s_n[e % HV_SLOTS]; }
-            };
-            const int my_total = n_ent > p ? (n_ent - p + HV_PROD - 1) / HV_PROD : 0;
-            for (int k0 = 0; k0 < my_total; k0 += 32) {
-                // each lane looks ONE of the next 32 entries up: a-side term and the run of c's list in the chunk
-                const int k_l = k0 + lane;
-                double ra_l = 0.0;
-                uint32_t lo_l = 0;
-                int n_l = 0;
-                if (k_l < my_total) {
-                    const int64_t e = eb + ent_of(k_l);
-                    const int32_t c = a.l_col[e];
-                    const double v = a.l_val[e];
-                    if (SIM == RS_SIM_PEARSON) ra_l = v - ai;                     // core/sim.go:73
-                    else if (SIM == RS_SIM_PEARSON_BASELINE) { const double bb = ai + a.right_bias[c]; ra_l = v - bb; }
-                    else ra_l = v;
-                    const int64_t rp = a.r_ptr[c];
-                    const int32_t *cpc = a.cp + (int64_t)c * (Q + 1) + q;
-                    int64_t lo64 = rp + cpc[0];
-                    int64_t hi = rp + cpc[1];
-                    if (diag_chunk) {
-                        const int64_t self64 = a.l2r[e];
-                        if (a.symmetric == 1) { if (self64 + 1 > lo64) lo64 = self64 + 1; }       // only j > i
-                        else { if (self64 < hi) hi = self64; }                                   // only j < i
-                    }
-                    n_l = hi > lo64 ? (int)(hi - lo64) : 0;
-                    lo_l = (uint32_t)lo64;
-                }
-                const int lim = my_total - k0 < 32 ? my_total - k0 : 32;
-                for (int u = 0; u < lim; u++) {
-                    const int k = k0 + u;
-                    const int e = ent_of(k);
-                    const int slot = e % HV_SLOTS;
-                    const double ra_u = __shfl_sync(0xffffffffu, ra_l, u);
-                    const uint32_t lo_u = __shfl_sync(0xffffffffu, lo_l, u);
-                    const int n_u = __shfl_sync(0xffffffffu, n_l, u);
-                    // the slot is free once the consumer has applied the entry that used it before
-                    for (bool first = true;; first = false) {
-                        int done = s_consumed[0];
-#pragma unroll
-                        for (int z = 1; z < HV_CONS; z++) { const int d = s_consumed[z]; done = d < done ? d : done; }
-                        if (done >= e - HV_SLOTS + 1) break;
-                        if (first) {
-                            // the ring is full: nothing can be issued, so everything this producer has in flight is
-                            // drained and made visible NOW — publishing must never wait for a slot, or the ring
-                            // runs at one memory latency per HV_SLOTS entries (226 ns per entry, measured)
-                            hv_wait<0>();
-                            while (published < issued) { publish(published); published++; }
-                        }
-                        __nanosleep(40);                      // (a busy poll steals the consumers' issue slots)
-                    }
-                    __syncwarp();
-                    for (int t = lane; t < n_u; t += 32) {
-                        hv_cp_async4(s_jc + slot * HV_JC + t, a.r_col + lo_u + t);
-                        hv_cp_async8(s_rb + slot * HV_JC + t, a.r_dev + lo_u + t);       // jr | jr - meanB (core/sim.go:74)
-                    }
-                    if (lane == 0) { s_ra[slot] = ra_u; s_n[slot] = n_u; }
-                    hv_commit();
-                    issued++;
-                    if (issued - published > HV_DEPTH) {      // the oldest outstanding entry has landed
-                        hv_wait<HV_DEPTH>();
-                        publish(published);
-                        published++;
-                    }
-                }
-            }
-            hv_wait<0>();
-            while (published < issued) { publish(published); published++; }
-        }
-    }
-}
-
-// does row r's own pass (column walk or sim_pop_kernel) compute cell (r, c)?  rr / rc: the rows' ranks.  The row
-// further down the longest-first order owns the pair; with the upper triangle two walked rows swap.
+// does row r's own pass (its column-walk or dense items in sim_stream_kernel) compute cell (r, c)?  rr / rc: the
+// rows' ranks.  The row further down the longest-first order owns the pair; with the upper triangle two walked rows
+// swap.
 __device__ __forceinline__ bool pop_owns(int32_t rr, int32_t rc, int32_t n_pop, int lower) {
     if (!lower && rr >= n_pop && rc >= n_pop) return rr < rc;
     return rr > rc;
@@ -771,34 +538,6 @@ static int32_t launch_stream(rs_knn *h, const StreamArgs &s, const PopArgs &pa, 
     return s.symmetric ? launch_stream_sym<SIM, SHRINK, 1>(h, s, pa, grid) : launch_stream_sym<SIM, SHRINK, 0>(h, s, pa, grid);
 }
 
-template <int SIM, bool SHRINK>
-static int32_t launch_heavy(rs_knn *h, const StreamArgs &a, const HeavyArgs &hv) {
-    constexpr int NACC = SHRINK ? 4 : 3;
-    const int smem = (NACC * HV_JC + HV_SLOTS * HV_JC) * 8 + HV_SLOTS * HV_JC * 4 + HV_SLOTS * 8 + HV_SLOTS * 4 * 2 + HV_CONS * 4 + 64;
-    auto kern = sim_stream_heavy_kernel<SIM, SHRINK>;
-    RS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-    int64_t grid = (int64_t)hv.n_rows * a.n_chunks;
-    if (grid > sms) grid = sms;
-    // on the auxiliary stream, beside the column walk of the other rows (one CTA per SM: ~104 KB of shared memory)
-    kern<<<(unsigned)grid, HV_WARPS * 32, smem, h->aux_stream>>>(a, hv);
-    h->prof.total_launches += 1;
-    return RS_OK;
-}
-
-static int32_t rs_heavy_rows_launch(rs_knn *h, const StreamArgs &a, const HeavyArgs &hv) {
-    switch (h->p.sim) {
-    case RS_SIM_COSINE: return launch_heavy<RS_SIM_COSINE, false>(h, a, hv);
-    case RS_SIM_MSD: return launch_heavy<RS_SIM_MSD, false>(h, a, hv);
-    case RS_SIM_PEARSON: return launch_heavy<RS_SIM_PEARSON, false>(h, a, hv);
-    case RS_SIM_PEARSON_BASELINE:
-        return h->p.shrinkage > 0.0 ? launch_heavy<RS_SIM_PEARSON_BASELINE, true>(h, a, hv)
-                                    : launch_heavy<RS_SIM_PEARSON_BASELINE, false>(h, a, hv);
-    default: rs_set_error("unknown similarity %d", h->p.sim); return RS_ERR_INVALID;
-    }
-}
-
 int32_t rs_sim_stream_launch(rs_knn *h) {
     StreamArgs a{};
     a.l_ptr = h->l_ptr; a.l_col = h->l_col; a.l_val = h->l_val; a.l2r = h->l2r;
@@ -832,25 +571,8 @@ int32_t rs_sim_stream_launch(rs_knn *h) {
         pa.n_blk = h->pop_ld / 32; pa.ld = h->pop_ld;
         pa.dense = h->pop_dense;
         pa.n_first = (h->n_all_rows - a.n_rows) * pa.n_blk;
-        if (const char *e = getenv("RS_KNN_STREAM_SKIP")) pa.skip = atoi(e);
     }
-    // heavy rows (rs_prep_rt split them off the order; JC = 256 only) run as producer / consumer CTAs on the
-    // auxiliary stream beside the column walk of the other rows
-    const bool heavy = !pop && h->n_heavy > 0 && a.symmetric != 0 && !h->force_sym && h->stream_jc == HV_JC;
-    if (heavy) {
-        HeavyArgs hv{};
-        hv.rows = h->row_heavy; hv.n_rows = h->n_heavy;
-        hv.counter = reinterpret_cast<unsigned long long *>(h->d_flags + 12);
-        RS_CUDA(cudaMemsetAsync(hv.counter, 0, 8, h->stream));
-        RS_CUDA(cudaEventRecord(h->ev_fork, h->stream));
-        RS_CUDA(cudaStreamWaitEvent(h->aux_stream, h->ev_fork, 0));
-        RS_TRY(rs_heavy_rows_launch(h, a, hv));
-        RS_CUDA(cudaEventRecord(h->ev_join, h->aux_stream));
-    }
-    if (a.n_rows <= 0 && !(pop && pa.n_rows > 0)) {
-        if (heavy) RS_CUDA(cudaStreamWaitEvent(h->stream, h->ev_join, 0));
-        return RS_OK;
-    }
+    if (a.n_rows <= 0 && !(pop && pa.n_rows > 0)) return RS_OK;
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
     const int64_t items = a.n_rows * (int64_t)h->n_chunks + (pop ? pa.n_rows * pa.n_blk : 0);
@@ -866,7 +588,6 @@ int32_t rs_sim_stream_launch(rs_knn *h) {
         break;
     default: rs_set_error("unknown similarity %d", h->p.sim); return RS_ERR_INVALID;
     }
-    if (heavy) RS_CUDA(cudaStreamWaitEvent(h->stream, h->ev_join, 0));
     h->prof.sim_launches++;
     h->prof.total_launches++;
     RS_CUDA(cudaGetLastError());

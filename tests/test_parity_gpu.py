@@ -83,14 +83,18 @@ def test_sims_bit_exact_both_triangles(ml100k, sim, user_based, tri, monkeypatch
 
 # ---- cyclic row shards (the multi-GPU Fit + Predict): every shard computes one triangle of its rows,
 # the mirror step pulls the other one from the peers; here all shards live on one GPU ----
-@pytest.mark.parametrize("pop", ["1", "0"])
+# pop_min "200": the longer rows are popular columns (mirror_pop_kernel); None: ML-100K has no row of the default
+# 8192 entries, so there are none and the plain column walk is mirrored by mirror_kernel
+@pytest.mark.parametrize("pop_min", ["200", None])
 @pytest.mark.parametrize("tri", ["upper", "lower"])
 @pytest.mark.parametrize("count", [2, 3])
-def test_cyclic_row_shards_equal_full(ml100k, count, tri, pop, monkeypatch):
+def test_cyclic_row_shards_equal_full(ml100k, count, tri, pop_min, monkeypatch):
     monkeypatch.setenv("RS_KNN_STREAM_TRI", tri)
     monkeypatch.setenv("RS_KNN_STREAM_JC", "256")
-    monkeypatch.setenv("RS_KNN_HEAVY_MIN", "200")      # the longer rows: popular columns (dense pass) / heavy-row kernel
-    monkeypatch.setenv("RS_KNN_POP", pop)
+    if pop_min is None:
+        monkeypatch.delenv("RS_KNN_POP_MIN", raising=False)
+    else:
+        monkeypatch.setenv("RS_KNN_POP_MIN", pop_min)
     u, i, r = split(ml100k["u1_base"])
     ts = rs.NewTrainSet(rs.NewRawSet(u, i, r))
     base = {"sim": rs.Pearson, "userBased": False, "k": 40}
@@ -254,34 +258,32 @@ def test_pinned_staging_of_large_batches(ml100k):
     assert L.rs_knn_trim_cache() == 0
 
 
-# ---- the longest rows of the exact sparse Fit.  mode "pop" (default): their ratings leave the CSR the column walk
-# reads and every pair with one of them comes from the dense pass (sim_pop_kernel: lane = popular column, register
-# accumulators); mode "heavy": they stay in the walk as producer / consumer CTAs.  Every row (min 0: the 512
-# longest become popular columns) and a mix (rows of >= 150 entries), both triangles, all similarities ----
-@pytest.mark.parametrize("mode", ["pop", "heavy"])
-@pytest.mark.parametrize("heavy_min", ["0", "150"])
+# ---- the longest rows of the exact sparse Fit: their ratings leave the CSR the column walk reads and every pair with
+# one of them comes from the dense items of sim_stream_kernel (lane = popular column, register accumulators).  Every
+# row (min 0: the 512 longest become popular columns) and a mix (rows of >= 150 entries), both triangles, all
+# similarities; 256-column chunks, the kernels of the ML-20M shape (ML-100K defaults to 128) ----
+@pytest.mark.parametrize("user_based", [True, False])
+@pytest.mark.parametrize("pop_min", ["0", "150"])
 @pytest.mark.parametrize("tri", ["upper", "lower"])
 @pytest.mark.parametrize("sim", ["cosine", "msd", "pearson"])
-def test_heavy_row_mode_bit_exact(ml100k, sim, tri, heavy_min, mode, monkeypatch):
+def test_popular_columns_bit_exact(ml100k, sim, tri, pop_min, user_based, monkeypatch):
     monkeypatch.setenv("RS_KNN_STREAM_TRI", tri)
-    monkeypatch.setenv("RS_KNN_STREAM_JC", "256")       # the heavy kernel shares the 256-column chunk pointers
-    monkeypatch.setenv("RS_KNN_HEAVY_MIN", heavy_min)
-    monkeypatch.setenv("RS_KNN_POP", "1" if mode == "pop" else "0")
-    for user_based in (True, False):
-        est, ref = fit_pair(ml100k["u2_base"], sim, "basic", user_based, extra={"simPath": "stream"})
-        got, want = est.Sims, ref.sims()
-        assert np.isnan(np.diag(got)).all()
-        assert bits_equal(got, want)
-        assert bits_equal(got, got.T)
+    monkeypatch.setenv("RS_KNN_STREAM_JC", "256")
+    monkeypatch.setenv("RS_KNN_POP_MIN", pop_min)
+    est, ref = fit_pair(ml100k["u2_base"], sim, "basic", user_based, extra={"simPath": "stream"})
+    got, want = est.Sims, ref.sims()
+    assert np.isnan(np.diag(got)).all()
+    assert bits_equal(got, want)
+    assert bits_equal(got, got.T)
 
 
 # ---- popular columns with the other table type and the other similarities: continuous ratings (the dense table
 # holds the b-side doubles instead of one byte per cell), PearsonBaseline with and without shrinkage (the b-side
 # term depends on both biases), a threshold that makes EVERY row popular (no column walk at all), and the
 # predictions that read the mirrored cells ----
-@pytest.mark.parametrize("heavy_min", ["0", "60"])
-def test_popular_columns_tables_and_baseline(ml100k, heavy_min, monkeypatch):
-    monkeypatch.setenv("RS_KNN_HEAVY_MIN", heavy_min)
+@pytest.mark.parametrize("pop_min", ["0", "60"])
+def test_popular_columns_tables_and_baseline(ml100k, pop_min, monkeypatch):
+    monkeypatch.setenv("RS_KNN_POP_MIN", pop_min)
     arr = ml100k["u3_base"]
     u, i, r = split(arr)
     rng = np.random.RandomState(11)

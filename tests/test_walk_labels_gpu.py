@@ -15,8 +15,7 @@ SIMS = {"cosine": rs.Cosine, "msd": rs.MSD, "pearson": rs.Pearson}
 
 @pytest.fixture(autouse=True)
 def _popular(monkeypatch):
-    monkeypatch.setenv("RS_KNN_HEAVY_MIN", str(POP_MIN))
-    monkeypatch.setenv("RS_KNN_POP", "1")
+    monkeypatch.setenv("RS_KNN_POP_MIN", str(POP_MIN))
 
 
 def data(user_based, continuous=False):

@@ -1,7 +1,7 @@
 """Seeded ratings whose walk labels are far from the row ids (tests/test_walk_labels*.py).
 
 Row r of the left dimension gets longer as r grows, in groups of 12 equal lengths (ties go by id), every seventh row
-takes one of three shared lengths instead, and the last five rows are rated by most right ids: with RS_KNN_HEAVY_MIN =
+takes one of three shared lengths instead, and the last five rows are rated by most right ids: with RS_KNN_POP_MIN =
 POP_MIN they are the popular columns.  The ratings are listed row by row, so row r's first-appearance inner id is r
 and the longest-first order runs against the ids."""
 import numpy as np

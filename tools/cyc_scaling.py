@@ -1,8 +1,7 @@
 #!/usr/bin/env python
 """Per-shard time of the exact sparse Fit under cyclic row sharding, measured on ONE GPU: fits shard 0
 of `count` shards (no peers needed for the similarity kernel itself) and prints the kernel time.
-usage: [CYC_INDEX=i] [CYC_POP=1,0] tools/cyc_scaling.py [workload] [counts...]
-CYC_POP: the values of RS_KNN_POP to run (1: popular columns as a dense pass, 0: heavy rows in the walk)."""
+usage: [CYC_INDEX=i] tools/cyc_scaling.py [workload] [counts...]"""
 import os
 import sys
 from pathlib import Path
@@ -25,12 +24,11 @@ right = train.innerItems if user_based else train.innerUsers
 dev = torch.device("cuda", 0)
 d_left, d_right = torch.from_numpy(left).to(dev), torch.from_numpy(right).to(dev)
 d_rating = torch.from_numpy(train.Ratings).to(dev)
-# CYC_SWEEP="min:max,min:max,...": popular-column thresholds (RS_KNN_HEAVY_MIN : RS_KNN_POP_MAX) to run in one process
+# CYC_SWEEP="min:max,min:max,...": popular-column thresholds (RS_KNN_POP_MIN : RS_KNN_POP_MAX) to run in one process
 sweep = [x.split(":") for x in os.environ["CYC_SWEEP"].split(",")] if "CYC_SWEEP" in os.environ else [None]
-for sw, pop, count in [(s_, p_, c_) for s_ in sweep for p_ in os.environ.get("CYC_POP", "1").split(",") for c_ in counts]:
-    os.environ["RS_KNN_POP"] = pop
+for sw, count in [(s_, c_) for s_ in sweep for c_ in counts]:
     if sw:
-        os.environ["RS_KNN_HEAVY_MIN"], os.environ["RS_KNN_POP_MAX"] = sw
+        os.environ["RS_KNN_POP_MIN"], os.environ["RS_KNN_POP_MAX"] = sw
         print("threshold", sw, end=" ")
     for index in ([int(os.environ["CYC_INDEX"])] if "CYC_INDEX" in os.environ else sorted({0, count - 1})):
         h = rs.core._Handle(sim=sim, knn_type=knn_type, k=k, device=0, shard_count=count if count > 1 else 0,
@@ -42,5 +40,5 @@ for sw, pop, count in [(s_, p_, c_) for s_ in sweep for p_ in os.environ.get("CY
                          train.GlobalMean)
             p = h.profile()
             ms.append(p["sim_kernel_ms"])
-        print(f"{wl} pop={pop} shards={count} index={index} sim_ms={min(ms[1:]):.2f} prep_ms={p['prep_ms']:.2f}", flush=True)
+        print(f"{wl} shards={count} index={index} sim_ms={min(ms[1:]):.2f} prep_ms={p['prep_ms']:.2f}", flush=True)
         h.close()

@@ -12,6 +12,6 @@ python tools/i8_peak.py --out $O/int8_peak.json > $O/i8.log 2>&1
 python bench.py --steps 2 --warmup 3 --no-cpu-baseline > $O/pre.log 2>&1 && \
 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file $O/launches_default.csv \
     python bench.py --steps 2 --warmup 3 --no-cpu-baseline > $O/ncu_list.log 2>&1
-ncu --set full --clock-control none --import-source on -k regex:'sim_stream_kernel|predict_select_kernel|sim_stream_heavy' -s 6 -c 3 \
+ncu --set full --clock-control none --import-source on -k regex:'sim_stream_kernel|predict_select_kernel' -s 6 -c 3 \
     -o $O/r02_default_full -f python bench.py --steps 2 --warmup 3 --no-cpu-baseline > $O/ncu_full.log 2>&1
 ls -la $O
