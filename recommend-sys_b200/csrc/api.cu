@@ -270,25 +270,11 @@ int32_t rs_knn_synchronize(rs_knn *h) {
     return RS_OK;
 }
 
-int32_t rs_knn_fit_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
-                          int64_t nnz, int32_t n_left, int32_t n_right, double global_mean,
-                          const double *d_left_bias, const double *d_right_bias, double global_bias) {
-    RS_ENTER(h);
-    if (!d_left || !d_right || !d_rating || nnz <= 0 || n_left <= 0 || n_right <= 0) {
-        rs_set_error("rs_knn_fit: empty or null input (nnz=%lld n_left=%d n_right=%d)", (long long)nnz, n_left,
-                     n_right);
-        return RS_ERR_INVALID;
-    }
-    if (h->p.knn_type == RS_KNN_BASELINE && !d_left_bias) {
-        rs_set_error("rs_knn_fit: RS_KNN_BASELINE needs left_bias (core/knn.go:179-187)");
-        return RS_ERR_INVALID;
-    }
-    if (h->p.sim == RS_SIM_PEARSON_BASELINE && (!d_left_bias || !d_right_bias)) {
-        rs_set_error("rs_knn_fit: RS_SIM_PEARSON_BASELINE needs both bias vectors");
-        return RS_ERR_INVALID;
-    }
-    RS_TRY(fold_profile(h));
-    free_fit_state(h);
+// Fit after the arguments were checked and the previous model was dropped: on failure the caller drops what was
+// built, so every error here may simply return.
+static int32_t fit(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating, int64_t nnz,
+                   int32_t n_left, int32_t n_right, double global_mean, const double *d_left_bias,
+                   const double *d_right_bias, double global_bias) {
     h->nnz = nnz;
     h->n_left = n_left;
     h->n_right = n_right;
@@ -325,8 +311,7 @@ int32_t rs_knn_fit_device(rs_knn *h, const int32_t *d_left, const int32_t *d_rig
     h->rows_local = h->cyc_R ? rs_cyc_rows(n_left, h->cyc_R, h->cyc_r) : rows;
 
     RS_CUDA(cudaEventRecord(h->ev_a, h->stream));
-    int32_t rc = rs_prep_build(h, d_left, d_right, d_rating, d_left_bias, d_right_bias);
-    if (rc != RS_OK) { free_fit_state(h); return rc; }
+    RS_TRY(rs_prep_build(h, d_left, d_right, d_rating, d_left_bias, d_right_bias));
 
     int path = h->p.sim_path;
     if (const char *force = getenv("RS_KNN_FORCE_PATH")) {  // debugging aid: "stream" | "tensor"
@@ -337,7 +322,6 @@ int32_t rs_knn_fit_device(rs_knn *h, const int32_t *d_left, const int32_t *d_rig
         // the deviation sums are integer contractions: tensor path only (integer ratings)
         if (!tensor_eligible(h) || path == RS_PATH_STREAM) {
             rs_set_error("RS_SIM_SLOPE_ONE needs integer ratings in [-11,11] (tensor path)");
-            free_fit_state(h);
             return RS_ERR_UNSUPPORTED;
         }
         path = RS_PATH_TENSOR;
@@ -347,7 +331,6 @@ int32_t rs_knn_fit_device(rs_knn *h, const int32_t *d_left, const int32_t *d_rig
         // triangle arrives by rs_knn_mirror: that schedule exists for the exact sparse path only
         if (path == RS_PATH_TENSOR) {
             rs_set_error("cyclic row shards run the stream path; shard the tensor path with row_begin/row_end");
-            free_fit_state(h);
             return RS_ERR_UNSUPPORTED;
         }
         path = RS_PATH_STREAM;
@@ -355,169 +338,52 @@ int32_t rs_knn_fit_device(rs_knn *h, const int32_t *d_left, const int32_t *d_rig
     if (path == RS_PATH_AUTO) path = tensor_eligible(h) && tensor_faster(h) ? RS_PATH_TENSOR : RS_PATH_STREAM;
     if (path == RS_PATH_TENSOR && !tensor_eligible(h)) {
         rs_set_error("tensor path needs integer ratings in [-11,11] and Cosine/MSD (or Pearson in SUMS mode)");
-        free_fit_state(h);
         return RS_ERR_UNSUPPORTED;
     }
     h->prof.sim_path_used = path;
     h->prof.corated_triples = h->triples;
-    rc = (path == RS_PATH_TENSOR) ? rs_prep_planes(h) : rs_prep_rt(h);
-    if (rc != RS_OK) { free_fit_state(h); return rc; }
+    RS_TRY(path == RS_PATH_TENSOR ? rs_prep_planes(h) : rs_prep_rt(h));
 
     h->ld_s = ((int64_t)n_left + 15) / 16 * 16;
     if (h->p.store == RS_STORE_MATRIX) {
-        rc = rs_alloc(h, &h->sims, (size_t)h->rows_local * (size_t)h->ld_s);
-        if (rc != RS_OK) { free_fit_state(h); return rc; }
+        RS_TRY(rs_alloc(h, &h->sims, (size_t)h->rows_local * (size_t)h->ld_s));
         RS_CUDA(cudaEventRecord(h->ev_b, h->stream));
-        rc = (path == RS_PATH_TENSOR) ? rs_sim_tensor_launch(h, nullptr, 0, 0) : rs_sim_stream_launch(h);
-        if (rc != RS_OK) { free_fit_state(h); return rc; }
+        RS_TRY(path == RS_PATH_TENSOR ? rs_sim_tensor_launch(h, nullptr, 0, 0) : rs_sim_stream_launch(h));
         RS_CUDA(cudaEventRecord(h->ev_c, h->stream));
-        if (path == RS_PATH_STREAM) {
-            rc = rs_symmetrize_launch(h);
-            if (rc != RS_OK) { free_fit_state(h); return rc; }
-        }
-    } else if (h->p.shard_count >= 1 && path == RS_PATH_TENSOR && rs_tensor_topk_fused(h)) {
-        // top-k only, FUSED: the tensor kernel's epilogue tests every similarity against the current k-th
-        // best of its two rows and appends the survivors to per-row candidate buffers; the buffers are merged
-        // into the running lists between the waves of the tile schedule (sim_tensor.cu).  No similarity row,
-        // slab or transpose is ever written: the only N-proportional buffers are the lists (N x k) and the
-        // candidate buffers (N x cap).  Every pair is computed once; a multi-GPU Fit deals the tiles of each
-        // wave to the shards, every shard ends with PARTIAL lists for all rows (united after an all-gather).
-        const int32_t k = h->p.topk > 0 ? h->p.topk : h->p.k;
-        const int64_t n = n_left;
-        h->cand_cap = 1792;                          // band 0 brings at most 2 * (512 + 256) entries per row
-        if (const char *e = getenv("RS_KNN_TOPK_CAP")) h->cand_cap = atoi(e);   // tests: force the overflow path
-        if (k > 256 || h->cand_cap + k > 2048 || h->cand_cap < 1) {
-            rs_set_error("fused top-k: k <= 256 and candidate capacity + k <= 2048 (k=%d cap=%d)", k, h->cand_cap);
-            free_fit_state(h);
-            return RS_ERR_UNSUPPORTED;
-        }
-        RS_TRY(rs_alloc(h, &h->topk_idx, (size_t)n * k));
-        RS_TRY(rs_alloc(h, &h->topk_sim, (size_t)n * k));
-        RS_TRY(rs_alloc(h, &h->thr_key, (size_t)n));
-        RS_TRY(rs_alloc(h, &h->thr_id, (size_t)n));
-        RS_TRY(rs_alloc(h, &h->cand_cnt, (size_t)n));
-        RS_TRY(rs_alloc(h, &h->row_flag, (size_t)n));
-        RS_TRY(rs_alloc(h, &h->cand_id, (size_t)n * h->cand_cap));
-        RS_TRY(rs_alloc(h, &h->cand_sim, (size_t)n * h->cand_cap));
-        h->topk_rows = n;
-        RS_CUDA(cudaMemsetAsync(h->topk_idx, 0xFF, (size_t)n * k * 4, h->stream));   // -1 = empty
-        RS_CUDA(cudaMemsetAsync(h->topk_sim, 0xFF, (size_t)n * k * 8, h->stream));   // NaN
-        RS_CUDA(cudaMemsetAsync(h->thr_key, 0, (size_t)n * 8, h->stream));           // accept every valid similarity
-        RS_CUDA(cudaMemsetAsync(h->thr_id, 0xFF, (size_t)n * 4, h->stream));
-        RS_CUDA(cudaMemsetAsync(h->cand_cnt, 0, (size_t)n * 4, h->stream));
-        RS_CUDA(cudaMemsetAsync(h->row_flag, 0, (size_t)n * 4, h->stream));
-        int32_t *d_over = h->d_flags + 14;
-        RS_CUDA(cudaEventRecord(h->ev_b, h->stream));
-        const int n_waves = rs_tensor_band_count(h);
-        for (int w = 0; w < n_waves && rc == RS_OK; w++) {
-            int rerun = 0;
-            for (;;) {
-                RS_CUDA(cudaMemsetAsync(d_over, 0, 4, h->stream));
-                rc = rs_sim_tensor_band_launch(h, w);
-                if (rc == RS_OK) rc = rs_topk_compact_launch(h, k, d_over, rerun);
-                if (rc != RS_OK) break;
-                int32_t over = 0;
-                RS_CUDA(cudaMemcpyAsync(&over, d_over, 4, cudaMemcpyDeviceToHost, h->stream));
-                RS_CUDA(cudaStreamSynchronize(h->stream));
-                if (rerun) rc = rs_topk_mask_launch(h, k, 1);      // thresholds of the rows that sat the pass out
-                if (over == 0 || rc != RS_OK) break;
-                rc = rs_topk_mask_launch(h, k, 0);                 // run the band again for the flagged rows only
-                rerun = 1;
-            }
-        }
-        if (rc != RS_OK) { free_fit_state(h); return rc; }
-        RS_CUDA(cudaEventRecord(h->ev_c, h->stream));
-    } else if (h->p.shard_count >= 1) {
-        // top-k only, SYMMETRIC SLABS (see rs_knn_params::shard_count): slab s = rows [s*m, s*m+m);
-        // of each slab only the part right of the diagonal is computed, the slab feeds the lists of
-        // its own rows, its transpose the lists of the rows below it.  Half the similarity work of
-        // full rows, and the slabs of a multi-GPU job are dealt round-robin so every rank gets the
-        // same share of the triangle.
-        const int32_t k = h->p.topk > 0 ? h->p.topk : h->p.k;
-        const int64_t n = n_left;
-        int64_t m = (int64_t)(6ll << 30) / (h->ld_s * 8);        // ~6 GiB slab + the same for its transpose
-        if (h->p.shard_count > 1) {
-            // enough slabs for an even deal: at least 4 per shard (down to 1024 rows each)
-            int64_t want = (n + 4ll * h->p.shard_count - 1) / (4ll * h->p.shard_count);
-            want = (want + 255) / 256 * 256;
-            if (want < 1024) want = 1024;
-            if (want < m) m = want;
-        }
-        if (const char *e = getenv("RS_KNN_SLAB_ROWS")) m = atoll(e);   // tests: many slabs on a small matrix
-        if (m < 256) m = 256;
-        m = m / 256 * 256;
-        if (m > n) m = (n + 15) / 16 * 16;
-        const int64_t ld_t = m;
-        double *tbuf = nullptr;
-        RS_TRY(rs_alloc(h, &h->sims, (size_t)m * (size_t)h->ld_s));
-        RS_TRY(rs_alloc(h, &tbuf, (size_t)n * (size_t)ld_t));
-        RS_TRY(rs_alloc(h, &h->topk_idx, (size_t)n * k));
-        RS_TRY(rs_alloc(h, &h->topk_sim, (size_t)n * k));
-        h->topk_rows = n;
-        RS_CUDA(cudaMemsetAsync(h->topk_idx, 0xFF, (size_t)n * k * 4, h->stream));   // -1 = empty
-        RS_CUDA(cudaMemsetAsync(h->topk_sim, 0xFF, (size_t)n * k * 8, h->stream));   // NaN
-        RS_CUDA(cudaEventRecord(h->ev_b, h->stream));
-        const int64_t n_slabs = (n + m - 1) / m;
-        h->force_sym = true;
-        for (int64_t sl = 0; sl < n_slabs; sl++) {
-            // snake deal: slab sl costs ~ (n_slabs - sl); rounds alternate direction so that every
-            // shard gets the same share of the triangle (8 GPUs, 25 slabs dealt plainly: max/mean 1.28)
-            const int64_t round = sl / h->p.shard_count, posn = sl % h->p.shard_count;
-            const int64_t owner = (round & 1) ? h->p.shard_count - 1 - posn : posn;
-            if (owner != h->p.shard_index) continue;
-            const int64_t r0 = sl * m, r1 = r0 + m < n ? r0 + m : n;
-            h->row_begin = r0;
-            h->row_end = r1;
-            h->col_begin = r0;
-            if (path == RS_PATH_STREAM) {
-                // the stream kernel skips whole column chunks left of the diagonal: unset = NaN
-                rc = cudaMemsetAsync(h->sims, 0xFF, (size_t)(r1 - r0) * (size_t)h->ld_s * 8, h->stream) == cudaSuccess
-                         ? RS_OK : RS_ERR_CUDA;
-                if (rc == RS_OK) rc = rs_sim_stream_launch(h);
-            } else {
-                rc = rs_sim_tensor_launch(h, nullptr, 0, 0);
-            }
-            if (rc == RS_OK) rc = rs_topk_slab_launch(h, r0, (int32_t)(r1 - r0), tbuf, ld_t, k);
-            if (rc != RS_OK) break;
-        }
-        h->force_sym = false;
-        h->col_begin = 0;
-        h->row_begin = 0;
-        h->row_end = n;
-        if (rc != RS_OK) { free_fit_state(h); return rc; }
-        RS_CUDA(cudaEventRecord(h->ev_c, h->stream));
+        if (path == RS_PATH_STREAM) RS_TRY(rs_symmetrize_launch(h));
     } else {
-        // top-k only: similarity rows are produced slab by slab and reduced to neighbour
-        // lists; the N x N matrix never exists in HBM.
-        const int32_t k = h->p.topk > 0 ? h->p.topk : h->p.k;
-        int64_t slab = (int64_t)(2ull << 30) / ((int64_t)h->ld_s * 8);  // ~2 GiB of rows at a time
-        if (slab < 128) slab = 128;
-        slab = slab / 128 * 128;
-        if (slab > rows) slab = rows;
-        RS_TRY(rs_alloc(h, &h->sims, (size_t)slab * (size_t)h->ld_s));
-        RS_TRY(rs_alloc(h, &h->topk_idx, (size_t)rows * k));
-        RS_TRY(rs_alloc(h, &h->topk_sim, (size_t)rows * k));
-        h->topk_rows = rows;
-        RS_CUDA(cudaEventRecord(h->ev_b, h->stream));
-        const int64_t rb = h->row_begin, re = h->row_end;
-        for (int64_t r0 = rb; r0 < re; r0 += slab) {
-            h->row_begin = r0;
-            h->row_end = r0 + slab < re ? r0 + slab : re;
-            rc = (path == RS_PATH_TENSOR) ? rs_sim_tensor_launch(h, nullptr, 0, 0) : rs_sim_stream_launch(h);
-            if (rc == RS_OK && path == RS_PATH_STREAM) rc = rs_symmetrize_launch(h);
-            if (rc == RS_OK)
-                rc = rs_topk_launch(h, k, h->topk_idx + (r0 - rb) * k, h->topk_sim + (r0 - rb) * k);
-            if (rc != RS_OK) break;
-        }
-        h->row_begin = rb;
-        h->row_end = re;
-        if (rc != RS_OK) { free_fit_state(h); return rc; }
+        RS_TRY(rs_fit_lists(h, path));        // records ev_b when its similarity work starts
         RS_CUDA(cudaEventRecord(h->ev_c, h->stream));
     }
     h->prep_pending = true;
     h->sim_pending = true;
     h->fitted = true;
     return RS_OK;
+}
+
+int32_t rs_knn_fit_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
+                          int64_t nnz, int32_t n_left, int32_t n_right, double global_mean,
+                          const double *d_left_bias, const double *d_right_bias, double global_bias) {
+    RS_ENTER(h);
+    if (!d_left || !d_right || !d_rating || nnz <= 0 || n_left <= 0 || n_right <= 0) {
+        rs_set_error("rs_knn_fit: empty or null input (nnz=%lld n_left=%d n_right=%d)", (long long)nnz, n_left,
+                     n_right);
+        return RS_ERR_INVALID;
+    }
+    if (h->p.knn_type == RS_KNN_BASELINE && !d_left_bias) {
+        rs_set_error("rs_knn_fit: RS_KNN_BASELINE needs left_bias (core/knn.go:179-187)");
+        return RS_ERR_INVALID;
+    }
+    if (h->p.sim == RS_SIM_PEARSON_BASELINE && (!d_left_bias || !d_right_bias)) {
+        rs_set_error("rs_knn_fit: RS_SIM_PEARSON_BASELINE needs both bias vectors");
+        return RS_ERR_INVALID;
+    }
+    RS_TRY(fold_profile(h));
+    free_fit_state(h);
+    const int32_t rc = fit(h, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean, d_left_bias, d_right_bias,
+                           global_bias);
+    if (rc != RS_OK) free_fit_state(h);       // a failed Fit leaves an unfitted handle, not a half-built model
+    return rc;
 }
 
 int32_t rs_scratch_get(rs_knn *h, int slot, size_t bytes, void **out) {
@@ -1012,7 +878,7 @@ int32_t rs_knn_topk_device(rs_knn *h, int32_t k, int32_t *d_idx, double *d_sim) 
     const int64_t rows = h->p.store == RS_STORE_TOPK ? h->topk_rows : h->rows_local;
     if (h->p.store == RS_STORE_MATRIX) RS_TRY(require_matrix(h, "rs_knn_topk"));
     if (h->p.store == RS_STORE_TOPK) {
-        const int32_t kk = h->p.topk > 0 ? h->p.topk : h->p.k;
+        const int32_t kk = rs_list_k(h);
         if (k != kk) {
             rs_set_error("rs_knn_topk: handle holds top-%d lists, asked for %d", kk, k);
             return RS_ERR_INVALID;
@@ -1021,7 +887,8 @@ int32_t rs_knn_topk_device(rs_knn *h, int32_t k, int32_t *d_idx, double *d_sim) 
         RS_CUDA(cudaMemcpyAsync(d_sim, h->topk_sim, (size_t)rows * k * 8, cudaMemcpyDeviceToDevice, h->stream));
         return RS_OK;
     }
-    return rs_topk_launch(h, k, d_idx, d_sim);
+    RS_TRY(rs_topk_check_k(k));
+    return rs_topk_rows_launch(h, h->sims, h->ld_s, h->n_left, h->rows_local, k, d_idx, d_sim);
 }
 
 int32_t rs_knn_topk(rs_knn *h, int32_t k, int32_t *idx, double *sim) {

@@ -323,13 +323,15 @@ int32_t rs_predict_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_rig
                           int32_t *d_nb_ids, double *d_nb_sims, int32_t *d_nb_count, int32_t nb_cap, int32_t foreign_zero = 0);
 int32_t rs_nb_cells_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_nb_ids, const int32_t *d_nb_count,
                            double *d_nb_sims);
-int32_t rs_topk_launch(rs_knn *h, int32_t k, int32_t *d_idx, double *d_sim);
 int32_t rs_slope_predict_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_right, int64_t n, double *d_out);
-int32_t rs_topk_slab_launch(rs_knn *h, int64_t g0, int32_t m, double *tbuf, int64_t ld_t, int32_t k);
-int32_t rs_topk_compact_launch(rs_knn *h, int32_t k, int32_t *d_overflow, int rerun);
-int32_t rs_topk_mask_launch(rs_knn *h, int32_t k, int restore);
+
+// ---- topk.cu ----
+// Neighbours per row of an RS_STORE_TOPK handle.
+inline int32_t rs_list_k(const rs_knn *h) { return h->p.topk > 0 ? h->p.topk : h->p.k; }
+int32_t rs_topk_check_k(int32_t k);
 int32_t rs_topk_rows_launch(rs_knn *h, const double *src, int64_t ld, int32_t n, int64_t rows, int32_t k, int32_t *d_idx,
                             double *d_sim);
+int32_t rs_fit_lists(rs_knn *h, int path);
 
 // ---- recommend.cu ----
 // One call of a recommendation entry point (include/rs_knn.h), checked by api.cu; every pointer is device memory.

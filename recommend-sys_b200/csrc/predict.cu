@@ -1,4 +1,4 @@
-// predict.cu — batched KNN.Predict (core/knn.go:75-141) and per-row top-k.
+// predict.cu — batched KNN.Predict (core/knn.go:75-141) and SlopeOne.Predict.
 //
 // Predict: one warp per (left,right) test pair.
 //   1. candidates = entries of the right row (core/knn.go:95-99), similarity gathered from
@@ -70,322 +70,6 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) predict_select_kernel(PredArgs
         return true;
     };
     select_loop<R>(a, a.work, n_eff, item, lane, hist, ckey, cpos, s_av[warp], sbuf, gbuf, scap);
-}
-
-
-// ---------------- per-row top-k from the resident matrix ----------------
-// +-0 share one key: they tie and are ordered by id, as the reference's float comparison does.  The block
-// top-k kernels carry the sign of a zero in bit 31 of the id word, so that a list reports the exact
-// similarity (-0.0 included) while the order stays that of (key, id).
-constexpr uint32_t NEG0 = 0x80000000u;
-__device__ __forceinline__ uint32_t neg0_bit(double s) {
-    return (unsigned long long)__double_as_longlong(s) == 0x8000000000000000ull ? NEG0 : 0u;
-}
-__device__ __forceinline__ bool ent_before(uint64_t ka, uint32_t pa, uint64_t kb, uint32_t pb) {
-    return rec_before(ka, pa & ~NEG0, kb, pb & ~NEG0);
-}
-__device__ __forceinline__ double ent_sim(uint64_t k, uint32_t p) { return (p & NEG0) ? -0.0 : rs_key_sim(k); }
-
-constexpr int TOPK_THREADS = 256;
-constexpr int TOPK_CAP = 2048;
-
-__device__ void block_bitonic(uint64_t *keys, uint32_t *pos, int n_pad) {
-    for (int size = 2; size <= n_pad; size <<= 1) {
-        for (int stride = size >> 1; stride > 0; stride >>= 1) {
-            __syncthreads();
-            for (int t = threadIdx.x; t < (n_pad >> 1); t += blockDim.x) {
-                int lo = 2 * t - (t & (stride - 1));
-                int hi = lo + stride;
-                bool up = ((lo & size) == 0);
-                uint64_t ka = keys[lo], kb = keys[hi];
-                uint32_t pa = pos[lo], pb = pos[hi];
-                bool swap = up ? ent_before(kb, pb, ka, pa) : ent_before(ka, pa, kb, pb);
-                if (swap) { keys[lo] = kb; keys[hi] = ka; pos[lo] = pb; pos[hi] = pa; }
-            }
-        }
-    }
-    __syncthreads();
-}
-
-__global__ void __launch_bounds__(TOPK_THREADS) topk_rows_kernel(const double *__restrict__ sims, int64_t ld_s,
-                                                                 int32_t n, int32_t k, int32_t *__restrict__ idx,
-                                                                 double *__restrict__ sim) {
-    __shared__ uint64_t keys[TOPK_CAP];
-    __shared__ uint32_t pos[TOPK_CAP];
-    __shared__ int s_have;
-    __shared__ uint64_t s_thr_key;
-    __shared__ uint32_t s_thr_pos;
-    const int64_t r = blockIdx.x;
-    const double *row = sims + r * ld_s;
-    if (threadIdx.x == 0) { s_have = 0; s_thr_key = 0; s_thr_pos = 0xffffffffu; }
-    __syncthreads();
-    bool have_thr = false;
-    for (int32_t base = 0; base < n; base += TOPK_THREADS) {
-        const int32_t j = base + threadIdx.x;
-        bool take = false;
-        uint64_t key = 0;
-        uint32_t neg0 = 0;
-        if (j < n) {
-            const double s = row[j];
-            if (s == s) {
-                key = rs_sim_key(s);
-                take = !have_thr || ent_before(key, (uint32_t)j, s_thr_key, s_thr_pos);
-                neg0 = neg0_bit(s);
-            }
-        }
-        if (take) {
-            int slot = atomicAdd(&s_have, 1);
-            keys[slot] = key;
-            pos[slot] = (uint32_t)j | neg0;
-        }
-        __syncthreads();
-        // every thread must see the SAME count: read it, then a second barrier before anybody's next
-        // atomicAdd can change it (otherwise a slow thread may take the branch below alone)
-        const int have_now = s_have;
-        __syncthreads();
-        if (have_now > TOPK_CAP - TOPK_THREADS) {
-            const int have = have_now;
-            for (int t = have + threadIdx.x; t < TOPK_CAP; t += blockDim.x) { keys[t] = 0; pos[t] = 0xffffffffu; }
-            block_bitonic(keys, pos, TOPK_CAP);
-            if (threadIdx.x == 0) {
-                s_have = k;
-                s_thr_key = keys[k - 1];
-                s_thr_pos = pos[k - 1];
-            }
-            have_thr = true;
-            __syncthreads();
-        }
-    }
-    const int have = s_have;
-    int n_pad = 32;
-    while (n_pad < have) n_pad <<= 1;
-    for (int t = have + threadIdx.x; t < n_pad; t += blockDim.x) { keys[t] = 0; pos[t] = 0xffffffffu; }
-    block_bitonic(keys, pos, n_pad);
-    for (int t = threadIdx.x; t < k; t += blockDim.x) {
-        const int64_t o = r * k + t;
-        if (t < have) { idx[o] = (int32_t)(pos[t] & ~NEG0); sim[o] = ent_sim(keys[t], pos[t]); }
-        else { idx[o] = -1; sim[o] = __longlong_as_double(0x7ff8000000000001ll); }
-    }
-}
-
-
-// ---------------------------------------------------------------------------------------------
-// Symmetric top-k slabs (RS_STORE_TOPK with shard_count >= 1).  A slab holds the rows
-// [g0, g0+m) of the similarity matrix, of which only the entries right of the diagonal are used;
-// each unordered pair {i, j} therefore feeds TWO neighbour lists: row i (through the slab) and row j
-// (through the slab's transpose), and no pair is computed twice.
-//   mode 0: src = slab,      block r <-> global row g0 + r, columns (g, n_cols), id = column
-//   mode 1: src = transpose, block r <-> global row g0 + r, columns [0, min(m, r)), id = g0 + column
-// The running list of the row (k entries, -1 = empty) is merged in: it seeds the candidate buffer.
-__global__ void __launch_bounds__(TOPK_THREADS) topk_merge_kernel(const double *__restrict__ src, int64_t ld,
-                                                                  int64_t g0, int32_t n_cols, int32_t m, int mode,
-                                                                  int32_t k, int32_t *__restrict__ idx,
-                                                                  double *__restrict__ sim) {
-    __shared__ uint64_t keys[TOPK_CAP];
-    __shared__ uint32_t pos[TOPK_CAP];
-    __shared__ int s_have;
-    __shared__ uint64_t s_thr_key;
-    __shared__ uint32_t s_thr_pos;
-    const int64_t r = blockIdx.x;
-    const int64_t g = g0 + r;
-    const double *row = src + r * ld;
-    int32_t clo, chi;
-    uint32_t id_off;
-    if (mode == 0) { clo = (int32_t)g + 1; chi = n_cols; id_off = 0; }
-    else { clo = 0; chi = r < m ? (int32_t)r : m; id_off = (uint32_t)g0; }
-    if (chi <= clo) return;                                   // nothing new for this row: the list stays
-    if (threadIdx.x == 0) { s_have = 0; s_thr_key = 0; s_thr_pos = 0xffffffffu; }
-    __syncthreads();
-    // seed with the running list; it is stored best first, so a FULL list gives the threshold right
-    // away (its last entry): almost every new candidate of a later slab is rejected by one compare
-    for (int t = threadIdx.x; t < k; t += blockDim.x) {
-        const int32_t id = idx[g * k + t];
-        if (id >= 0) {
-            const int slot = atomicAdd(&s_have, 1);
-            keys[slot] = rs_sim_key(sim[g * k + t]);
-            pos[slot] = (uint32_t)id | neg0_bit(sim[g * k + t]);
-        }
-    }
-    bool have_thr = idx[g * k + (k - 1)] >= 0;
-    if (have_thr && threadIdx.x == 0) {
-        s_thr_key = rs_sim_key(sim[g * k + (k - 1)]);
-        s_thr_pos = (uint32_t)idx[g * k + (k - 1)];
-    }
-    __syncthreads();
-    for (int32_t base = clo; base < chi; base += TOPK_THREADS) {
-        const int32_t j = base + threadIdx.x;
-        bool take = false;
-        uint64_t key = 0;
-        uint32_t neg0 = 0;
-        if (j < chi) {
-            const double s = row[j];
-            if (s == s) {
-                key = rs_sim_key(s);
-                take = !have_thr || ent_before(key, (uint32_t)j + id_off, s_thr_key, s_thr_pos);
-                neg0 = neg0_bit(s);
-            }
-        }
-        if (take) {
-            int slot = atomicAdd(&s_have, 1);
-            keys[slot] = key;
-            pos[slot] = ((uint32_t)j + id_off) | neg0;
-        }
-        __syncthreads();
-        // every thread must see the SAME count: read it, then a second barrier before anybody's next
-        // atomicAdd can change it (otherwise a slow thread may take the branch below alone)
-        const int have_now = s_have;
-        __syncthreads();
-        if (have_now > TOPK_CAP - TOPK_THREADS) {
-            const int have = have_now;
-            for (int t = have + threadIdx.x; t < TOPK_CAP; t += blockDim.x) { keys[t] = 0; pos[t] = 0xffffffffu; }
-            block_bitonic(keys, pos, TOPK_CAP);
-            if (threadIdx.x == 0) {
-                s_have = k;
-                s_thr_key = keys[k - 1];
-                s_thr_pos = pos[k - 1];
-            }
-            have_thr = true;
-            __syncthreads();
-        }
-    }
-    const int have = s_have;
-    int n_pad = 32;
-    while (n_pad < have) n_pad <<= 1;
-    for (int t = have + threadIdx.x; t < n_pad; t += blockDim.x) { keys[t] = 0; pos[t] = 0xffffffffu; }
-    block_bitonic(keys, pos, n_pad);
-    for (int t = threadIdx.x; t < k; t += blockDim.x) {
-        const int64_t o = g * k + t;
-        if (t < have) { idx[o] = (int32_t)(pos[t] & ~NEG0); sim[o] = ent_sim(keys[t], pos[t]); }
-        else { idx[o] = -1; sim[o] = __longlong_as_double(0x7ff8000000000001ll); }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// Fused top-k (sim_tensor.cu appends the survivors of each band to per-row candidate buffers): merge a
-// row's buffer into its running list — top k of (list U candidates) under (similarity desc, id asc) —,
-// publish the new k-th best as the row's threshold and empty the buffer.  A buffer that overflowed
-// (more than `cap` survivors since the last merge: impossible unless the similarities are ordered
-// adversarially along the diagonal distance) is NOT merged: what it holds only raises the threshold —
-// every entry is a real similarity of the row, so the k-th best of (list U buffer) is a valid lower
-// bound of the final one —, the row is flagged, and the band is run again for the flagged rows.
-__global__ void __launch_bounds__(TOPK_THREADS) topk_compact_kernel(
-    const int32_t *__restrict__ cand_id, const double *__restrict__ cand_sim, int32_t *__restrict__ cand_cnt,
-    int32_t cap, int32_t k, int32_t *__restrict__ idx, double *__restrict__ sim, unsigned long long *__restrict__ thr_key,
-    int32_t *__restrict__ thr_id, int32_t *__restrict__ row_flag, int32_t *__restrict__ overflow, int rerun) {
-    __shared__ uint64_t keys[TOPK_CAP];
-    __shared__ uint32_t pos[TOPK_CAP];
-    const int64_t g = blockIdx.x;
-    if (rerun && !row_flag[g]) return;                         // second pass of a band: flagged rows only
-    const int cnt_all = cand_cnt[g];
-    const bool over = cnt_all > cap;
-    const int cnt = over ? cap : cnt_all;
-    if (cnt == 0 && !rerun) return;                            // nothing new: list and threshold stay
-    int have = 0;                                              // the list is stored best first: its entries are a prefix
-    for (int t = threadIdx.x; t < k; t += blockDim.x) {
-        const int32_t id = idx[g * k + t];
-        keys[t] = id >= 0 ? rs_sim_key(sim[g * k + t]) : 0ull;
-        pos[t] = id >= 0 ? (uint32_t)id | neg0_bit(sim[g * k + t]) : 0xffffffffu;
-    }
-    __syncthreads();
-    // number of list entries (prefix length)
-    __shared__ int s_have;
-    if (threadIdx.x == 0) s_have = 0;
-    __syncthreads();
-    for (int t = threadIdx.x; t < k; t += blockDim.x)
-        if (pos[t] != 0xffffffffu) atomicAdd(&s_have, 1);
-    __syncthreads();
-    have = s_have;
-    for (int t = threadIdx.x; t < cnt; t += blockDim.x) {
-        keys[have + t] = rs_sim_key(cand_sim[g * cap + t]);
-        pos[have + t] = (uint32_t)cand_id[g * cap + t] | neg0_bit(cand_sim[g * cap + t]);
-    }
-    const int total = have + cnt;
-    int n_pad = 32;
-    while (n_pad < total) n_pad <<= 1;
-    __syncthreads();
-    for (int t = total + threadIdx.x; t < n_pad; t += blockDim.x) { keys[t] = 0; pos[t] = 0xffffffffu; }
-    block_bitonic(keys, pos, n_pad);
-    if (!over) {
-        for (int t = threadIdx.x; t < k; t += blockDim.x) {
-            const int64_t o = g * k + t;
-            if (t < total) { idx[o] = (int32_t)(pos[t] & ~NEG0); sim[o] = ent_sim(keys[t], pos[t]); }
-            else { idx[o] = -1; sim[o] = __longlong_as_double(0x7ff8000000000001ll); }
-        }
-    }
-    if (threadIdx.x == 0) {
-        // merged: the k-th best is IN the list, only strictly better entries matter from here on.  Overflowed:
-        // the buffer is discarded, so the k-th best of (list U buffer) itself — a real entry that may belong
-        // to the final list — and everything above it must be admitted again: threshold = just below it
-        // (same key, id + 1).
-        if (total >= k) { thr_key[g] = keys[k - 1]; thr_id[g] = (int32_t)(pos[k - 1] & ~NEG0) + (over ? 1 : 0); }
-        else { thr_key[g] = 0ull; thr_id[g] = -1; }            // list not full: accept every valid similarity
-        cand_cnt[g] = 0;
-        row_flag[g] = over ? 1 : 0;
-        if (over) atomicAdd(overflow, 1);
-    }
-}
-
-// Second pass of a band: rows that did NOT overflow already hold the band's entries — their threshold is
-// raised to "accept nothing" for the pass (restore = 0) and recomputed from their list afterwards (restore = 1).
-__global__ void topk_mask_kernel(const int32_t *__restrict__ row_flag, const int32_t *__restrict__ idx,
-                                 const double *__restrict__ sim, int32_t k, int64_t n, int restore,
-                                 unsigned long long *__restrict__ thr_key, int32_t *__restrict__ thr_id) {
-    const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= n || row_flag[g]) return;
-    if (!restore) { thr_key[g] = ~0ull; thr_id[g] = 0; return; }
-    const int32_t id = idx[g * k + (k - 1)];
-    if (id >= 0) { thr_key[g] = rs_sim_key(sim[g * k + (k - 1)]); thr_id[g] = id; }
-    else { thr_key[g] = 0ull; thr_id[g] = -1; }
-}
-
-// T[(c - c0)][r] = S[r][c] for r in [0, m), c in [c0, n): 32 x 32 tiles through shared memory
-__global__ void transpose_slab_kernel(const double *__restrict__ s, int64_t ld_s, int32_t m, int64_t c0, int32_t n,
-                                      double *__restrict__ t, int64_t ld_t) {
-    __shared__ double tile[32][33];
-    const int64_t r0 = (int64_t)blockIdx.y * 32, c_base = c0 + (int64_t)blockIdx.x * 32;
-    for (int y = threadIdx.y; y < 32; y += blockDim.y) {
-        const int64_t r = r0 + y, c = c_base + threadIdx.x;
-        tile[y][threadIdx.x] = (r < m && c < n) ? s[r * ld_s + c] : 0.0;
-    }
-    __syncthreads();
-    for (int y = threadIdx.y; y < 32; y += blockDim.y) {
-        const int64_t c = c_base + y, r = r0 + threadIdx.x;
-        if (c < n && r < m) t[(c - c0) * ld_t + r] = tile[threadIdx.x][y];
-    }
-}
-
-// Final neighbour lists from the partial lists of several ranks: out[row] = top k of the union of
-// lists[l][row][*] (every (row, neighbour) pair occurs in exactly one partial list).
-__global__ void __launch_bounds__(TOPK_THREADS) topk_union_kernel(const int32_t *__restrict__ idx_all,
-                                                                  const double *__restrict__ sim_all, int32_t n_lists,
-                                                                  int64_t n_rows, int32_t k, int32_t *__restrict__ idx,
-                                                                  double *__restrict__ sim) {
-    __shared__ uint64_t keys[TOPK_CAP];
-    __shared__ uint32_t pos[TOPK_CAP];
-    __shared__ int s_have;
-    const int64_t g = blockIdx.x;
-    if (threadIdx.x == 0) s_have = 0;
-    __syncthreads();
-    for (int t = threadIdx.x; t < n_lists * k; t += blockDim.x) {
-        const int64_t o = ((int64_t)(t / k) * n_rows + g) * k + (t % k);
-        const int32_t id = idx_all[o];
-        if (id >= 0) {
-            const int slot = atomicAdd(&s_have, 1);
-            keys[slot] = rs_sim_key(sim_all[o]);
-            pos[slot] = (uint32_t)id | neg0_bit(sim_all[o]);
-        }
-    }
-    __syncthreads();
-    const int have = s_have;
-    int n_pad = 32;
-    while (n_pad < have) n_pad <<= 1;
-    for (int t = have + threadIdx.x; t < n_pad; t += blockDim.x) { keys[t] = 0; pos[t] = 0xffffffffu; }
-    block_bitonic(keys, pos, n_pad);
-    for (int t = threadIdx.x; t < k; t += blockDim.x) {
-        const int64_t o = g * k + t;
-        if (t < have) { idx[o] = (int32_t)(pos[t] & ~NEG0); sim[o] = ent_sim(keys[t], pos[t]); }
-        else { idx[o] = -1; sim[o] = __longlong_as_double(0x7ff8000000000001ll); }
-    }
 }
 
 
@@ -600,90 +284,6 @@ int32_t rs_nb_cells_launch(rs_knn *h, const int32_t *d_left, const int32_t *d_nb
     nb_cells_kernel<<<1, 256, 0, h->stream>>>(h->sims, h->ld_s, h->row_begin, h->cyc_R, d_left, d_nb_ids, d_nb_count,
                                               d_nb_sims);
     h->prof.total_launches++;
-    RS_CUDA(cudaGetLastError());
-    return RS_OK;
-}
-
-int32_t rs_topk_launch(rs_knn *h, int32_t k, int32_t *d_idx, double *d_sim) {
-    const int64_t rows = h->cyc_R > 1 ? h->rows_local : h->row_end - h->row_begin;
-    if (rows <= 0) return RS_OK;
-    if (k < 1 || k > TOPK_CAP / 4) {
-        rs_set_error("top-k supports 1 <= k <= %d (got %d)", TOPK_CAP / 4, k);
-        return RS_ERR_UNSUPPORTED;
-    }
-    topk_rows_kernel<<<(unsigned)rows, TOPK_THREADS, 0, h->stream>>>(h->sims, h->ld_s, h->n_left, k, d_idx, d_sim);
-    h->prof.total_launches++;
-    RS_CUDA(cudaGetLastError());
-    return RS_OK;
-}
-
-// Top-k of `rows` rows of any row-major matrix of similarities or scores (ld = row pitch, n columns).
-int32_t rs_topk_rows_launch(rs_knn *h, const double *src, int64_t ld, int32_t n, int64_t rows, int32_t k, int32_t *d_idx,
-                            double *d_sim) {
-    if (rows <= 0) return RS_OK;
-    topk_rows_kernel<<<(unsigned)rows, TOPK_THREADS, 0, h->stream>>>(src, ld, n, k, d_idx, d_sim);
-    h->prof.total_launches++;
-    RS_CUDA(cudaGetLastError());
-    return RS_OK;
-}
-
-// Symmetric slab: merge the slab rows [g0, g0+m) (entries right of the diagonal) and their transpose
-// into the running neighbour lists of all rows >= g0 (see topk_merge_kernel).
-int32_t rs_topk_slab_launch(rs_knn *h, int64_t g0, int32_t m, double *tbuf, int64_t ld_t, int32_t k) {
-    if (k < 1 || k > TOPK_CAP / 4) {
-        rs_set_error("top-k supports 1 <= k <= %d (got %d)", TOPK_CAP / 4, k);
-        return RS_ERR_UNSUPPORTED;
-    }
-    const int32_t n = h->n_left;
-    topk_merge_kernel<<<(unsigned)m, TOPK_THREADS, 0, h->stream>>>(h->sims, h->ld_s, g0, n, m, 0, k, h->topk_idx,
-                                                                 h->topk_sim);
-    const int64_t rest = (int64_t)n - g0;                     // rows g0 .. n-1 receive transposed contributions
-    if (rest > 1) {
-        dim3 grid((unsigned)((rest + 31) / 32), (unsigned)((m + 31) / 32)), block(32, 8);
-        transpose_slab_kernel<<<grid, block, 0, h->stream>>>(h->sims, h->ld_s, m, g0, n, tbuf, ld_t);
-        topk_merge_kernel<<<(unsigned)rest, TOPK_THREADS, 0, h->stream>>>(tbuf, ld_t, g0, n, m, 1, k, h->topk_idx,
-                                                                        h->topk_sim);
-        h->prof.total_launches += 2;
-    }
-    h->prof.total_launches += 1;
-    RS_CUDA(cudaGetLastError());
-    return RS_OK;
-}
-
-int32_t rs_topk_compact_launch(rs_knn *h, int32_t k, int32_t *d_overflow, int rerun) {
-    if (k < 1 || k > TOPK_CAP / 4 || h->cand_cap + k > TOPK_CAP) {
-        rs_set_error("fused top-k supports k <= %d and cap + k <= %d (got k=%d cap=%d)", TOPK_CAP / 4, TOPK_CAP, k, h->cand_cap);
-        return RS_ERR_UNSUPPORTED;
-    }
-    topk_compact_kernel<<<(unsigned)h->n_left, TOPK_THREADS, 0, h->stream>>>(
-        h->cand_id, h->cand_sim, h->cand_cnt, h->cand_cap, k, h->topk_idx, h->topk_sim, h->thr_key, h->thr_id,
-        h->row_flag, d_overflow, rerun);
-    h->prof.total_launches++;
-    RS_CUDA(cudaGetLastError());
-    return RS_OK;
-}
-
-int32_t rs_topk_mask_launch(rs_knn *h, int32_t k, int restore) {
-    topk_mask_kernel<<<(unsigned)((h->n_left + 255) / 256), 256, 0, h->stream>>>(h->row_flag, h->topk_idx, h->topk_sim, k,
-                                                                                h->n_left, restore, h->thr_key, h->thr_id);
-    h->prof.total_launches++;
-    RS_CUDA(cudaGetLastError());
-    return RS_OK;
-}
-
-extern "C" int32_t rs_knn_topk_union_device(int32_t n_lists, int64_t n_rows, int32_t k, const int32_t *d_idx_all,
-                                            const double *d_sim_all, int32_t *d_idx, double *d_sim,
-                                            void *cuda_stream) {
-    if (n_lists < 1 || n_rows < 1 || k < 1 || !d_idx_all || !d_sim_all || !d_idx || !d_sim) {
-        rs_set_error("rs_knn_topk_union: bad argument");
-        return RS_ERR_INVALID;
-    }
-    if ((int64_t)n_lists * k > TOPK_CAP) {
-        rs_set_error("rs_knn_topk_union: n_lists * k = %lld exceeds %d", (long long)n_lists * k, TOPK_CAP);
-        return RS_ERR_UNSUPPORTED;
-    }
-    topk_union_kernel<<<(unsigned)n_rows, TOPK_THREADS, 0, reinterpret_cast<cudaStream_t>(cuda_stream)>>>(
-        d_idx_all, d_sim_all, n_lists, n_rows, k, d_idx, d_sim);
     RS_CUDA(cudaGetLastError());
     return RS_OK;
 }

@@ -12,7 +12,7 @@
 //   left query q (user-based: q is a user, the targets are the items t, score(t) = Predict(left = q, right = t)):
 //     all gathers of the query come from ONE matrix row, S[q][.]; the scores are handed out query-major, so the
 //     warps in flight share that row in L2.
-// Rated targets are then overwritten with NaN and topk_rows_kernel (predict.cu) picks the N best of each row.
+// Rated targets are then overwritten with NaN and topk_rows_kernel (topk.cu) picks the N best of each row.
 //
 // Row shards (rs_knn_*_sharded_device): a shard holds complete rows of the similarity matrix and both CSRs.
 //   right queries: the targets are the left rows, so a shard scores the targets it owns (local row t, global id

@@ -257,7 +257,7 @@ struct TcArgs {
     int sync_chunk, sync_slack, sync_timeout;
     // Fused top-k (pair kernel, RS_STORE_TOPK): no similarity is stored.  Every pair {i, j}, j > i, is tested
     // against the current k-th best of row i and of row j (thr_*; key 0 = list not full, accept) and the
-    // survivors are appended to the rows' candidate buffers, merged between waves (predict.cu).
+    // survivors are appended to the rows' candidate buffers, merged between waves (topk.cu).
     int topk_mode;
     const unsigned long long *thr_key;
     const int32_t *thr_id;
@@ -1144,7 +1144,7 @@ int32_t rs_sim_tensor_band_launch(rs_knn *h, int32_t wave) {
 }
 
 // Is the fused top-k path available for this Fit?  (Cosine / MSD on integer ratings, large enough for the
-// pair kernel; everything else reduces bounded slabs of similarity rows, see api.cu.)
+// pair kernel; everything else reduces bounded slabs of similarity rows, see topk.cu.)
 bool rs_tensor_topk_fused(const rs_knn *h) {
     if (h->p.sim != RS_SIM_COSINE && h->p.sim != RS_SIM_MSD) return false;
     if (const char *e = getenv("RS_KNN_TOPK_FUSED")) return atoi(e) != 0;

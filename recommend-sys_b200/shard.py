@@ -47,7 +47,7 @@ def allgather_topk(idx_local, sim_local, n: int, k: int, group=None, align: int 
 
 def slab_owner(slab: int, world: int) -> int:
     """Which shard computes slab `slab` under symmetric-slab sharding: slabs are dealt in snake order
-    (0..world-1, world-1..0, ...) because slab s costs ~ (n_slabs - s) — the same rule as csrc/api.cu."""
+    (0..world-1, world-1..0, ...) because slab s costs ~ (n_slabs - s) — the same rule as csrc/topk.cu."""
     rnd, pos = divmod(slab, world)
     return world - 1 - pos if rnd & 1 else pos
 

@@ -429,17 +429,39 @@ def test_topk_rows(ml100k):
         assert bits_equal(gs, ws)
 
 
-def test_topk_only_store_matches_matrix_store(ml100k):
+def topk_only_vs_matrix(ml100k, base, rows=None):
+    """The lists of an RS_STORE_TOPK handle (k = 100) against rs_knn_topk of the matrix handle, bit for bit; with
+    `rows`, a rowBegin/rowEnd top-k handle against those rows of the matrix."""
     u, i, r = split(ml100k["u1_base"])
     ts = rs.NewTrainSet(rs.NewRawSet(u, i, r))
-    full = rs.NewKNN(rs.Parameters({"sim": rs.MSD, "userBased": True}))
+    full = rs.NewKNN(rs.Parameters(base))
     full.Fit(ts)
-    only = rs.NewKNN(rs.Parameters({"sim": rs.MSD, "userBased": True, "store": "topk", "topk": 100}))
+    extra = {"rowBegin": rows[0], "rowEnd": rows[1]} if rows else {}
+    only = rs.NewKNN(rs.Parameters(dict(base, store="topk", topk=100, **extra)))
     only.Fit(ts)
     a, b = full.TopK(100), only.TopK(100)
+    if rows:
+        a = (a[0][rows[0]:rows[1]], a[1][rows[0]:rows[1]])
+    assert b[0].shape == a[0].shape
     assert np.array_equal(a[0], b[0]) and bits_equal(a[1], b[1])
+    return only, u, i
+
+
+def test_topk_only_store_matches_matrix_store(ml100k):
+    only, u, i = topk_only_vs_matrix(ml100k, {"sim": rs.MSD, "userBased": True})
     with pytest.raises(rs.core.RsError):
         only.PredictBatch(u[:4], i[:4])
+
+
+@pytest.mark.parametrize("path,rows", [
+    ("tensor", None),                     # 943 rows -> 8 slabs
+    ("stream", None),
+    ("stream", (128, 768)),               # a row shard of the top-k store: 5 slabs
+])
+def test_topk_only_store_row_slabs(ml100k, path, rows, monkeypatch):
+    """The full-row slab loop of RS_STORE_TOPK (shard_count 0) run several times: 128-row slabs."""
+    monkeypatch.setenv("RS_KNN_SLAB_ROWS", "128")
+    topk_only_vs_matrix(ml100k, {"sim": rs.MSD, "userBased": True, "simPath": path}, rows)
 
 
 @pytest.mark.parametrize("sim,path", [("msd", "tensor"), ("cosine", "tensor"), ("msd", "stream"),

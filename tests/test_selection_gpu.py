@@ -1,4 +1,4 @@
-"""Neighbour selection against the oracle in every regime of the selection code (csrc/predict.cu).
+"""Neighbour selection against the oracle in every regime of the selection code (csrc/select.cuh, csrc/topk.cu).
 
 predict_select_kernel<R> picks the top min(k, valid) candidates of a prediction with a radix selection on
 32-bit keys, falls back to exact 64-bit passes when one key32 value overfills the boundary bucket, takes
