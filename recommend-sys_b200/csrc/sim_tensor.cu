@@ -279,6 +279,12 @@ __device__ __forceinline__ unsigned long long ld_relaxed_gpu(const unsigned long
 //   l  = L/(ca*cb),                  L  = ca*cb*Sxy - ca*sb*Sx - cb*sa*Sy + n*sa*sb
 //   l/(sqrt(m)*sqrt(nn)) = L/(sqrt(Mi)*sqrt(Ni))   — the counts cancel; Mi==0 <=> m==0 exactly,
 // so NaN-ness matches the reference's 0/0 (core/sim.go:80) with no cancellation noise.
+// Range: Mi = ca^2 * sum (x - sa/ca)^2 over the co-rated x <= ca^3 * h^2 for ratings spanning 2h (largest when the
+// pair is co-rated over the whole row), so Mi, Ni and L fit int64 for left rows of up to ~4.2e5 ratings of [-11, 11]
+// (h = 11) or ~1.3e6 ratings of 1..5 (h = 2); a left row is at most as long as the other side has ids.  Partial
+// terms such as ca*ca*sxx and 2*ca*sa*sx are larger (up to 242 ca^3 for +-11) and leave int64 sooner: below the
+// bound the sums still come out right only because the device's 64-bit signed arithmetic wraps (two's complement),
+// which C++ leaves undefined.  Beyond the bound the result is wrong and nothing refuses it.
 __device__ __forceinline__ double pearson_from_sums(long long n, long long sx, long long sy, long long sxx,
                                                     long long syy, long long sxy, long long ca, long long sa,
                                                     long long cb, long long sb) {
