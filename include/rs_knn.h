@@ -332,6 +332,23 @@ int32_t rs_knn_update(rs_knn *h, const int32_t *left, const int32_t *right, cons
                       int32_t n_left, int32_t n_right, double global_mean);
 int32_t rs_knn_update_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
                              int64_t nnz, int32_t n_left, int32_t n_right, double global_mean);
+/* ADDING RATINGS TO A CYCLIC ROW SHARD (after rs_knn_mirror).  rs_knn_update and rs_knn_update_device refuse every row
+ * shard; this is their form for cyclic shards.  Every shard of the model is called with the same ratings, counts and
+ * global_mean, and no data moves between them: each merges the ratings into its copies of both CSRs and of every row's
+ * statistics, and recomputes the cells it stores — the full rows of the touched ids it owns, and the columns of the
+ * touched ids other shards own in each of its rows.  Afterwards every shard holds, bit for bit, the rows that a cyclic
+ * Fit of the union plus rs_knn_mirror gives it under the same block rule (blocks of 32 rows, block b on shard
+ * b % shard_count); a new left id lands on the shard that rule names, so a shard that held no rows may gain some.
+ * Inputs, return and memory as rs_knn_update_device.  Refused, leaving the shard exactly as it was:
+ *   RS_ERR_INVALID     not a cyclic row shard (a handle with every row), a cyclic shard before rs_knn_mirror, and
+ *                      every RS_ERR_INVALID case of rs_knn_update;
+ *   RS_ERR_UNSUPPORTED a row_begin/row_end shard (its range is fixed at create and cannot take new ids), and every
+ *                      RS_ERR_UNSUPPORTED case of rs_knn_update other than row shards;
+ *   RS_ERR_DUPLICATE, RS_ERR_OOM as rs_knn_update.
+ * The checks read only what every shard holds alike, so a refusal other than RS_ERR_OOM is the same on every shard.
+ * After an update, rs_knn_mirror returns RS_ERR_INVALID until the next Fit: the shard's rows are complete. */
+int32_t rs_knn_update_sharded_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
+                                     int64_t nnz, int32_t n_left, int32_t n_right, double global_mean);
 
 /* Parameters["k"] / ["mink"] are read at Predict time by the reference (core/knn.go:80-81): change
  * them on a fitted handle without refitting.  The predict kernel supports k <= 256. */
@@ -349,7 +366,8 @@ int32_t rs_knn_set_k(rs_knn *h, int32_t k, int32_t min_k);
  *                         loads over NVLink, transposed through shared memory).  The caller orders it
  *                         after every peer's Fit has finished (rs_knn_synchronize + a barrier) and
  *                         keeps the peers' matrices alive until it has finished.
- * Until rs_knn_mirror has run, Predict / sims_rows / topk on a cyclic shard fail with RS_ERR_INVALID. */
+ * Until rs_knn_mirror has run, Predict / sims_rows / topk on a cyclic shard fail with RS_ERR_INVALID, and after
+ * rs_knn_update_sharded_device it returns RS_ERR_INVALID until the next Fit. */
 /* Predict on a cyclic row shard for an all-reduce: the FULL test set goes to every shard; a pair whose left row
  * another shard owns yields +0.0 (all bits zero) instead of NaN, and a cold-start pair (left = -1) is answered by
  * shard (index % shard_count) only — so an integer SUM all-reduce of the 64-bit patterns over the shards assembles

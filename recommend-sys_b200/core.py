@@ -72,7 +72,7 @@ ABI_SYMBOLS = [
     "rs_knn_host_free", "rs_knn_score_all", "rs_knn_score_all_device", "rs_knn_recommend", "rs_knn_recommend_device",
     "rs_knn_score_all_sharded_device", "rs_knn_recommend_sharded_device", "rs_knn_score_all_given",
     "rs_knn_score_all_given_device", "rs_knn_recommend_given", "rs_knn_recommend_given_device", "rs_knn_update",
-    "rs_knn_update_device",
+    "rs_knn_update_device", "rs_knn_update_sharded_device",
 ]
 
 _knn_lib = None
@@ -135,6 +135,7 @@ def knn_lib():
     L.rs_knn_recommend_given_device.argtypes = [vp, i32, vp, vp, vp, i64, i32, vp, vp]
     L.rs_knn_update.argtypes = [vp, vp, vp, vp, i64, i32, i32, dbl]
     L.rs_knn_update_device.argtypes = [vp, vp, vp, vp, i64, i32, i32, dbl]
+    L.rs_knn_update_sharded_device.argtypes = [vp, vp, vp, vp, i64, i32, i32, dbl]
     _knn_lib = L
     return L
 
@@ -658,6 +659,13 @@ class _Handle:
 
     def update_device(self, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean):
         _check(knn_lib().rs_knn_update_device(self.h, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean))
+        self._after_fit(n_left, n_right)
+
+    def update_sharded_device(self, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean):
+        """update_device on a mirrored cyclic row shard: every shard gets the same ratings and afterwards holds its rows
+        of the Fit of the union (rs_knn_update_sharded_device)."""
+        _check(knn_lib().rs_knn_update_sharded_device(self.h, d_left, d_right, d_rating, nnz, n_left, n_right,
+                                                      global_mean))
         self._after_fit(n_left, n_right)
 
     def predict_batch(self, left, right):

@@ -162,7 +162,7 @@ int32_t init_handle(rs_knn *h) {
 extern "C" {
 
 const char *rs_last_error(void) { return g_err; }
-int32_t rs_knn_abi_version(void) { return 5; }
+int32_t rs_knn_abi_version(void) { return 6; }
 
 int32_t rs_knn_device_count(void) {
     int n = 0;
@@ -450,11 +450,11 @@ int32_t rs_knn_fit(rs_knn *h, const int32_t *left, const int32_t *right, const d
 }
 
 // Every check of rs_knn_update, in the order they fire: the handle is fitted; its model is one that an update can
-// extend exactly (a matrix of all rows, no Slope One, no bias of a global fit, the exact Pearson replay); the counts
-// do not shrink; the pointers are there when there are ratings.  The ratings themselves are checked on the device.
-static int32_t check_update(rs_knn *h, const int32_t *left, const int32_t *right, const double *rating, int64_t nnz,
-                            int32_t n_left, int32_t n_right) {
-    const char *who = "rs_knn_update";
+// extend exactly (a matrix of all rows — sharded: a mirrored cyclic row shard —, no Slope One, no bias of a global
+// fit, the exact Pearson replay); the counts do not shrink; the pointers are there when there are ratings.  The
+// ratings themselves are checked on the device.
+static int32_t check_update(rs_knn *h, const char *who, bool sharded, const int32_t *left, const int32_t *right,
+                            const double *rating, int64_t nnz, int32_t n_left, int32_t n_right) {
     if (!h->fitted) {
         rs_set_error("%s: Fit has not been called", who);
         return RS_ERR_INVALID;
@@ -463,9 +463,21 @@ static int32_t check_update(rs_knn *h, const int32_t *left, const int32_t *right
         rs_set_error("%s needs RS_STORE_MATRIX (the handle keeps top-k lists only)", who);
         return RS_ERR_UNSUPPORTED;
     }
-    if (h->cyc_R > 1 || h->p.shard_count > 1 || h->row_begin != 0 || h->row_end != h->n_left) {
+    if (!sharded && (h->cyc_R > 1 || h->p.shard_count > 1 || h->row_begin != 0 || h->row_end != h->n_left)) {
         rs_set_error("%s needs a handle that holds every row (no row_begin/row_end shard, shard_count <= 1)", who);
         return RS_ERR_UNSUPPORTED;
+    }
+    if (sharded && (h->row_begin != 0 || h->row_end != h->n_left)) {
+        rs_set_error("%s: a row_begin/row_end shard holds a fixed range of rows and cannot take new ids", who);
+        return RS_ERR_UNSUPPORTED;
+    }
+    if (sharded && h->cyc_R < 2) {
+        rs_set_error("%s: the handle is not a cyclic row shard (use rs_knn_update)", who);
+        return RS_ERR_INVALID;
+    }
+    if (sharded && !h->peers_ready) {
+        rs_set_error("%s: cyclic row shards hold one triangle of their rows until rs_knn_mirror has run", who);
+        return RS_ERR_INVALID;
     }
     if (h->p.sim == RS_SIM_SLOPE_ONE) {
         rs_set_error("%s: Slope One is not supported", who);
@@ -499,14 +511,21 @@ static int32_t check_update(rs_knn *h, const int32_t *left, const int32_t *right
 int32_t rs_knn_update_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
                              int64_t nnz, int32_t n_left, int32_t n_right, double global_mean) {
     RS_ENTER(h);
-    RS_TRY(check_update(h, d_left, d_right, d_rating, nnz, n_left, n_right));
+    RS_TRY(check_update(h, "rs_knn_update", false, d_left, d_right, d_rating, nnz, n_left, n_right));
+    return rs_update_run(h, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean);
+}
+
+int32_t rs_knn_update_sharded_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
+                                     int64_t nnz, int32_t n_left, int32_t n_right, double global_mean) {
+    RS_ENTER(h);
+    RS_TRY(check_update(h, "rs_knn_update_sharded", true, d_left, d_right, d_rating, nnz, n_left, n_right));
     return rs_update_run(h, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean);
 }
 
 int32_t rs_knn_update(rs_knn *h, const int32_t *left, const int32_t *right, const double *rating, int64_t nnz,
                       int32_t n_left, int32_t n_right, double global_mean) {
     RS_ENTER(h);
-    RS_TRY(check_update(h, left, right, rating, nnz, n_left, n_right));
+    RS_TRY(check_update(h, "rs_knn_update", false, left, right, rating, nnz, n_left, n_right));
     void *d_left = nullptr, *d_right = nullptr, *d_rating = nullptr;
     if (nnz > 0) {
         RS_TRY(rs_scratch_get(h, RS_SCR_FIT_LEFT, (size_t)nnz * 4, &d_left));
@@ -1031,6 +1050,11 @@ int32_t rs_knn_mirror(rs_knn *h) {
     RS_ENTER(h);
     if (!h->fitted || h->cyc_R < 2) {
         rs_set_error("rs_knn_mirror: the handle is not a fitted cyclic row shard");
+        return RS_ERR_INVALID;
+    }
+    if (h->updated) {
+        // the shard's rows are complete, and the peers' matrices may have moved or grown since they were attached
+        rs_set_error("rs_knn_mirror: the shard has been updated since its Fit; its rows are complete");
         return RS_ERR_INVALID;
     }
     for (int q = 0; q < h->cyc_R; q++)

@@ -368,10 +368,11 @@ struct rs_given_lists {
 int32_t rs_given_prepare(rs_knn *h, int32_t n_targets, const int64_t *d_ptr, const int32_t *d_ids,
                          const double *d_vals, int64_t n, rs_given_lists *out);
 // The similarity rows S*[b][v] = Sim(list b, left row v) of the lists ptr[0 .. nq) (ids: right ids), into out[nq][ld].
-// With `rows`, list b is list rows[b] of ptr and its Pearson mean qpmeans[rows[b]].
+// With `rows`, list b is list rows[b] of ptr and its Pearson mean qpmeans[rows[b]].  With `own` (a cyclic row shard),
+// only the rows the shard owns, at their local rows: out[nq][ld], ld >= rows_local.
 int32_t rs_given_sims_launch(rs_knn *h, const int64_t *ptr, const int32_t *ids, const double *vals,
                              const double *qpmeans, int64_t nq, double *out, int64_t ld,
-                             const int32_t *rows = nullptr);
+                             const int32_t *rows = nullptr, bool own = false);
 
 // ---- update.cu ----
 int32_t rs_update_run(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating, int64_t nnz,

@@ -13,6 +13,10 @@
 //   list in the right CSR, found by two binary searches (one lane per entry, 32 entries at a time), and the lanes
 //   update the accumulators of those raters — every v at most once per c, c strictly in order.
 //   It reads r_ptr / r_col / r_val and pmeans, which every RS_STORE_MATRIX handle holds (tensor-path Fits too).
+// given_sims_kernel<SIM, true>: the same values for the rows a cyclic row shard owns only, S*[b][loc] = Sim(list b,
+// L(v)) at v's local row loc (rs_knn_update_sharded_device: the columns a shard stores of rows it does not own).  A
+// work item is a block of GS_JC consecutive local rows; its raters are found over the global id range the block
+// spans, and the raters of other shards are skipped.  Every v still sees its entries c in ascending order.
 #include <cub/cub.cuh>
 
 #include "common.cuh"
@@ -71,9 +75,11 @@ struct GivenSimArgs {
     double *out;              // [nq][ld]
     int64_t ld;
     unsigned long long *counter;
+    int32_t cyc_R, cyc_r;     // OWN: the shard; n_left / n_blk count its local rows
+    uint32_t cyc_div;         // ceil(2^32 / cyc_R): __umulhi(blk, cyc_div) = blk / cyc_R for every block blk < 2^26
 };
 
-template <int SIM>
+template <int SIM, bool OWN = false>
 __global__ void __launch_bounds__(GS_WARPS * 32) given_sims_kernel(GivenSimArgs a) {
     extern __shared__ double s_gs[];                  // [GS_WARPS][3][GS_JC] accumulators, then [GS_WARPS][32] a-side terms
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -86,8 +92,11 @@ __global__ void __launch_bounds__(GS_WARPS * 32) given_sims_kernel(GivenSimArgs 
         item = __shfl_sync(0xffffffffu, item, 0);
         if ((int64_t)item >= n_items) break;
         const int64_t b = (int64_t)item / a.n_blk;    // list-major: the warps in flight walk the same list
-        const int32_t v0 = (int32_t)((int64_t)item % a.n_blk) * GS_JC;
-        const int32_t v1 = v0 + GS_JC < a.n_left ? v0 + GS_JC : a.n_left;
+        // OWN: local rows [l0, l1) of the shard, the global ids v0 .. v1-1 they span; else v0 .. v1-1 themselves
+        const int32_t l0 = (int32_t)((int64_t)item % a.n_blk) * GS_JC;
+        const int32_t l1 = l0 + GS_JC < a.n_left ? l0 + GS_JC : a.n_left;
+        const int32_t v0 = OWN ? (int32_t)rs_cyc_global(l0, a.cyc_R, a.cyc_r) : l0;
+        const int32_t v1 = OWN ? (int32_t)rs_cyc_global(l1 - 1, a.cyc_R, a.cyc_r) + 1 : l1;
         __syncwarp();                                 // the previous item has finished with acc
         for (int x = lane; x < 3 * GS_JC; x += 32) acc[x] = 0.0;
         const int64_t lb = a.rows ? a.rows[b] : b;
@@ -119,24 +128,32 @@ __global__ void __launch_bounds__(GS_WARPS * 32) given_sims_kernel(GivenSimArgs 
                 const double raa_u = ra_u * ra_u;                                 // core/sim.go:19 / :75
                 for (int t = lane; t < nn; t += 32) {
                     const int32_t v = a.r_col[lo_u + t];
-                    double rb = a.r_val[lo_u + t];
-                    if (SIM == RS_SIM_PEARSON) rb = rb - a.pmeans[v];             // core/sim.go:74, as build_rdev_kernel
-                    stream_update<SIM, false, GS_JC>(acc, v - v0, ra_u, raa_u, rb);
+                    int32_t j = v - v0;
+                    if (OWN) {                                                    // rs_cyc_owns / rs_cyc_local
+                        const uint32_t blk = (uint32_t)v / RS_CYC_B, q = __umulhi(blk, a.cyc_div);
+                        j = blk - q * a.cyc_R == (uint32_t)a.cyc_r ? (int32_t)(q * RS_CYC_B + (uint32_t)v % RS_CYC_B) - l0
+                                                                   : -1;
+                    }
+                    if (!OWN || j >= 0) {
+                        double rb = a.r_val[lo_u + t];
+                        if (SIM == RS_SIM_PEARSON) rb = rb - a.pmeans[v];         // core/sim.go:74, as build_rdev_kernel
+                        stream_update<SIM, false, GS_JC>(acc, j, ra_u, raa_u, rb);
+                    }
                 }
                 __syncwarp();   // entry c is complete before entry c+1 touches the same v
             }
         }
         __syncwarp();
         double *out = a.out + b * a.ld;
-        for (int j = lane; j < v1 - v0; j += 32)
-            out[v0 + j] = sim_value<SIM, false>(acc + j, GS_JC, 0.0);
+        for (int j = lane; j < l1 - l0; j += 32)
+            out[l0 + j] = sim_value<SIM, false>(acc + j, GS_JC, 0.0);
     }
 }
 
 template <int SIM>
-int32_t launch_given_sims(rs_knn *h, const GivenSimArgs &a) {
+int32_t launch_given_sims(rs_knn *h, const GivenSimArgs &a, bool own) {
     const size_t smem = (size_t)GS_WARPS * (3 * GS_JC + 32) * sizeof(double);
-    auto kern = given_sims_kernel<SIM>;
+    auto kern = own ? given_sims_kernel<SIM, true> : given_sims_kernel<SIM>;
     RS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
@@ -215,21 +232,25 @@ int32_t rs_given_prepare(rs_knn *h, int32_t n_targets, const int64_t *d_ptr, con
 }
 
 int32_t rs_given_sims_launch(rs_knn *h, const int64_t *ptr, const int32_t *ids, const double *vals,
-                             const double *qpmeans, int64_t nq, double *out, int64_t ld, const int32_t *rows) {
-    if (nq <= 0) return RS_OK;
+                             const double *qpmeans, int64_t nq, double *out, int64_t ld, const int32_t *rows,
+                             bool own) {
+    const int64_t width = own ? h->rows_local : h->n_left;
+    if (nq <= 0 || width <= 0) return RS_OK;
     void *counter;
     RS_TRY(rs_scratch_get(h, RS_SCR_GIVEN_COUNTER, 8, &counter));
     RS_CUDA(cudaMemsetAsync(counter, 0, 8, h->stream));
     GivenSimArgs a{};
     a.ptr = ptr; a.ids = ids; a.vals = vals; a.qpmeans = qpmeans; a.rows = rows; a.nq = nq;
     a.r_ptr = h->r_ptr; a.r_col = h->r_col; a.r_val = h->r_val; a.pmeans = h->pmeans;
-    a.n_left = h->n_left;
-    a.n_blk = (h->n_left + GS_JC - 1) / GS_JC;
+    a.n_left = (int32_t)width;
+    a.n_blk = (int32_t)((width + GS_JC - 1) / GS_JC);
     a.out = out; a.ld = ld;
     a.counter = reinterpret_cast<unsigned long long *>(counter);
-    if (h->p.sim == RS_SIM_COSINE) RS_TRY(launch_given_sims<RS_SIM_COSINE>(h, a));
-    else if (h->p.sim == RS_SIM_MSD) RS_TRY(launch_given_sims<RS_SIM_MSD>(h, a));
-    else if (h->p.sim == RS_SIM_PEARSON) RS_TRY(launch_given_sims<RS_SIM_PEARSON>(h, a));
+    a.cyc_R = h->cyc_R; a.cyc_r = h->cyc_r;
+    if (own) a.cyc_div = (uint32_t)(((1ull << 32) + h->cyc_R - 1) / h->cyc_R);
+    if (h->p.sim == RS_SIM_COSINE) RS_TRY(launch_given_sims<RS_SIM_COSINE>(h, a, own));
+    else if (h->p.sim == RS_SIM_MSD) RS_TRY(launch_given_sims<RS_SIM_MSD>(h, a, own));
+    else if (h->p.sim == RS_SIM_PEARSON) RS_TRY(launch_given_sims<RS_SIM_PEARSON>(h, a, own));
     else {
         rs_set_error("rs_knn_*_given: no similarity row for sim %d", h->p.sim);
         return RS_ERR_UNSUPPORTED;

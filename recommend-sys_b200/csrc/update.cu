@@ -12,6 +12,9 @@
 //     sparse Fit's terms, order and IEEE operations) and written into their rows and columns, diagonal NaN.  A cell
 //     between two untouched rows sums the same terms in the same order as before and their statistics do not change:
 //     it is kept.
+// A cyclic row shard (rs_knn_update_sharded_device) merges the same ratings into its copies of the CSRs and the
+// statistics, and recomputes the cells it stores: the full rows of the touched ids it owns, and, for a touched id i that
+// another shard owns, the column S[v][i] of each row v it owns (given_sims_kernel<SIM, true>, about N / R cells).
 // Everything up to the one read-back of the checks goes to scratch; the model's merged arrays go to spare blocks
 // (rs_knn::upd), and the model is written only when every check has passed and every block is allocated, so a
 // refused update, or one that runs out of memory, leaves the model as it was.
@@ -65,18 +68,22 @@ __global__ void upd_dup_kernel(const int32_t *__restrict__ row, const int32_t *_
     if (p < end && l_col[p] == c) atomicOr(flags, FLAG_DUP);
 }
 
-// The touched left rows, each keyed by its merged length + 1 (0: untouched) for a longest-first sort; flags[1] counts
-// them.  d_ptr: the added ratings' row pointers.
+// The touched left rows, each keyed by its merged length + 1 (0: untouched) and, above that, bit 31 for the rows the
+// handle owns (every row unless it is a cyclic shard), for a sort that puts the owned rows first, each group longest
+// first; flags[1] counts them, flags[3] the owned ones.  d_ptr: the added ratings' row pointers.
 __global__ void upd_touched_kernel(const int64_t *__restrict__ l_ptr, int32_t nl0, const int64_t *__restrict__ d_ptr,
-                                   int32_t nl, uint32_t *__restrict__ key, int32_t *__restrict__ ids,
-                                   int32_t *__restrict__ flags) {
+                                   int32_t nl, int32_t cyc_R, int32_t cyc_r, uint32_t *__restrict__ key,
+                                   int32_t *__restrict__ ids, int32_t *__restrict__ flags) {
     const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= nl) return;
     const int64_t dl = d_ptr[i + 1] - d_ptr[i];
     const bool touched = dl > 0 || i >= nl0;
-    key[i] = touched ? (uint32_t)((i < nl0 ? l_ptr[i + 1] - l_ptr[i] : 0) + dl + 1) : 0u;
+    const bool owned = cyc_R < 2 || rs_cyc_owns(i, cyc_R, cyc_r);
+    const int64_t len = (i < nl0 ? l_ptr[i + 1] - l_ptr[i] : 0) + dl + 1;
+    key[i] = touched ? (owned ? 0x80000000u : 0u) | (uint32_t)(len < 0x7fffffff ? len : 0x7fffffff) : 0u;
     ids[i] = i;
     if (touched) atomicAdd(flags + 1, 1);
+    if (touched && owned) atomicAdd(flags + 3, 1);
 }
 
 // The longest merged right row (Predict's candidate bound) into flags[2].
@@ -148,17 +155,34 @@ __global__ void upd_merge_new_kernel(const int32_t *__restrict__ key, const int3
 
 // Row i = rows[b] of the matrix and its column from the recomputed row slab[b]: S[i][v] = S[v][i] = slab[b][v], the
 // diagonal NaN as Fit leaves it.  Two touched rows write the same bits into their common cells: Sim(i, j) and
-// Sim(j, i) sum the same terms in the same order.
+// Sim(j, i) sum the same terms in the same order.  A cyclic shard (cyc_R >= 2) owns row i, stores it at its local row,
+// and writes the column into the rows v it owns.
 __global__ void upd_scatter_kernel(const double *__restrict__ slab, int64_t ld, const int32_t *__restrict__ rows,
-                                   int64_t nb, int32_t n, double *__restrict__ sims) {
+                                   int64_t nb, int32_t n, int32_t cyc_R, int32_t cyc_r, double *__restrict__ sims) {
     const int64_t x = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (x >= nb * n) return;
     const int64_t b = x / n;
     const int32_t v = (int32_t)(x - b * n);
     const int32_t i = rows[b];
     const double s = v == i ? __longlong_as_double(0x7ff8000000000001ll) : slab[b * ld + v];
-    sims[(int64_t)i * ld + v] = s;
-    sims[(int64_t)v * ld + i] = s;
+    if (cyc_R < 2) {
+        sims[(int64_t)i * ld + v] = s;
+        sims[(int64_t)v * ld + i] = s;
+    } else {
+        sims[rs_cyc_local(i, cyc_R) * ld + v] = s;
+        if (rs_cyc_owns(v, cyc_R, cyc_r)) sims[rs_cyc_local(v, cyc_R) * ld + i] = s;
+    }
+}
+
+// A cyclic shard's column i = rows[b] of a row another shard owns, from its own-row slab[b] (given_sims_kernel<SIM,
+// true>): S[loc][i] = slab[b][loc] for each of its n_own local rows.  Where it meets an owned touched row j, the two
+// writes carry the same bits, as above.
+__global__ void upd_scatter_own_kernel(const double *__restrict__ slab, int64_t n_own, const int32_t *__restrict__ rows,
+                                       int64_t nb, int64_t ld, double *__restrict__ sims) {
+    const int64_t x = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (x >= nb * n_own) return;
+    const int64_t b = x / n_own, loc = x - b * n_own;
+    sims[loc * ld + rows[b]] = slab[b * n_own + loc];
 }
 
 // Carves the update's scratch arrays out of one block.
@@ -174,7 +198,7 @@ struct Carve {
 };
 
 struct Work {
-    int32_t *flags;           // [0] FLAG_*, [1] touched rows, [2] longest merged right row
+    int32_t *flags;           // [0] FLAG_*, [1] touched rows, [2] longest merged right row, [3] touched rows owned
     int32_t *idx, *ls, *rs, *keys_a, *keys_b, *keys_l, *keys_r;
     int32_t *perm_l, *perm_r, *perm_lr, *perm_rl, *col_lr, *col_rl;
     int64_t *ptr_l, *ptr_r;
@@ -242,6 +266,8 @@ int32_t rs_update_run(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
     const int32_t nl0 = h->n_left, nr0 = h->n_right;
     const int64_t nnz0 = h->nnz, nnz = nnz0 + nd;
     const bool int8 = h->rating_class == RS_CLASS_INT8;
+    const int32_t cyc_R = h->cyc_R > 1 ? h->cyc_R : 0, cyc_r = h->cyc_r;
+    const int64_t rows0 = h->rows_local, rows = cyc_R ? rs_cyc_rows(nl, cyc_R, cyc_r) : nl;   // the matrix's rows
     // Fit keeps the dataset-order values only where a statistic is summed in that order (prep.cu)
     const bool dataset_order = !int8 || h->p.knn_type == RS_KNN_ZSCORE;
 
@@ -285,16 +311,17 @@ int32_t rs_update_run(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
         RS_CUDA(cudaMemsetAsync(w.ptr_l, 0, ((size_t)nl + 1) * 8, st));
         RS_CUDA(cudaMemsetAsync(w.ptr_r, 0, ((size_t)nr + 1) * 8, st));
     }
-    // the touched rows, longest merged row first (stable: ties by id), and the longest merged right row
-    upd_touched_kernel<<<blocks_for(nl), T, 0, st>>>(h->l_ptr, nl0, w.ptr_l, nl, w.len, w.ids, w.flags);
+    // the touched rows, owned first, each group longest merged row first (stable: ties by id), and the longest merged
+    // right row
+    upd_touched_kernel<<<blocks_for(nl), T, 0, st>>>(h->l_ptr, nl0, w.ptr_l, nl, cyc_R, cyc_r, w.len, w.ids, w.flags);
     upd_right_len_kernel<<<blocks_for(nr), T, 0, st>>>(h->r_ptr, nr0, w.ptr_r, nr, w.flags);
     RS_UPD_SORT([&](void *t, size_t &b) {
         return cub::DeviceRadixSort::SortPairsDescending(t, b, w.len, w.len_sorted, w.ids, w.rows, (int)nl, 0, 32, st);
     });
     h->prof.total_launches += 2;
     RS_CUDA(cudaGetLastError());
-    int32_t f[3];
-    RS_CUDA(cudaMemcpyAsync(f, w.flags, 12, cudaMemcpyDeviceToHost, st));
+    int32_t f[4];
+    RS_CUDA(cudaMemcpyAsync(f, w.flags, 16, cudaMemcpyDeviceToHost, st));
     RS_CUDA(cudaStreamSynchronize(st));
     if (f[0] & FLAG_BAD_ID) {
         rs_set_error("rs_knn_update: rating rows contain inner ids outside [0,%d) x [0,%d)", nl, nr);
@@ -313,7 +340,8 @@ int32_t rs_update_run(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
         rs_set_error("rs_knn_update: a (left,right) pair the model holds already, or twice among the added ratings");
         return RS_ERR_DUPLICATE;
     }
-    const int64_t n_touched = f[1];
+    const int64_t n_touched = f[1], n_owned = f[3];
+    const int64_t n_foreign = rows > 0 ? n_touched - n_owned : 0;   // the touched rows of other shards
     const int32_t max_right_len = f[2] > h->max_right_len ? f[2] : h->max_right_len;
 
     // ---- every block the update writes, before the model is written ----
@@ -337,19 +365,24 @@ int32_t rs_update_run(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
         RS_TRY(spare_of(h, RS_UPD_ROW_SUM, (int64_t)nl + 1, &row_sum));
     }
     // the matrix: new rows fit in place while ld_s = ceil(n_left / 16) * 16 keeps its value and the block has the
-    // rows; otherwise a block of ld_s rows in the new layout takes the old rows
+    // rows; otherwise a block of the rows the handle holds at n_left = ld_s, in the new layout, takes the old rows
     const int64_t ld = ((int64_t)nl + 15) / 16 * 16;
     double *sims = h->sims;
     void *grown = nullptr;
     size_t grown_bytes = 0;
-    if (nl > nl0 && !(ld == h->ld_s && h->upd_sims && h->upd_sims_bytes >= (size_t)nl * ld * 8)) {
-        RS_TRY(rs_cached_malloc(h->device, &grown, (size_t)ld * ld * 8, &grown_bytes));
+    if ((rows > rows0 || ld != h->ld_s) &&
+        !(ld == h->ld_s && h->upd_sims && h->upd_sims_bytes >= (size_t)rows * ld * 8)) {
+        const int64_t cap = cyc_R ? rs_cyc_rows(ld, cyc_R, cyc_r) : ld;
+        RS_TRY(rs_cached_malloc(h->device, &grown, cap > 0 ? (size_t)cap * ld * 8 : 256, &grown_bytes));
         sims = static_cast<double *>(grown);
     }
-    const int64_t batch = n_touched > 0 ? slab_batch(ld, n_touched) : 0;
+    // owned rows: full rows of ld; other shards' rows: columns of the handle's rows
+    const int64_t batch = n_owned > 0 ? slab_batch(ld, n_owned) : 0;
+    const int64_t batch_own = n_foreign > 0 ? slab_batch(rows, n_foreign) : 0;
+    const size_t slab_bytes = (size_t)(batch * ld > batch_own * rows ? batch * ld : batch_own * rows) * 8;
     void *slab = nullptr, *counter = nullptr;
-    if (n_touched > 0) {
-        int32_t rc = rs_scratch_get(h, RS_SCR_UPD_SLAB, (size_t)batch * ld * 8, &slab);
+    if (n_owned + n_foreign > 0) {
+        int32_t rc = rs_scratch_get(h, RS_SCR_UPD_SLAB, slab_bytes, &slab);
         if (rc == RS_OK) rc = rs_scratch_get(h, RS_SCR_GIVEN_COUNTER, 8, &counter);   // rs_given_sims_launch's
         if (rc != RS_OK) {
             rs_cached_free(h->device, grown, grown_bytes);
@@ -380,8 +413,8 @@ int32_t rs_update_run(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
                                                                 nullptr, nl0, w.ptr_l, l_ptr, nullptr, ld_val, nullptr);
         h->prof.total_launches += dataset_order ? 3 : 2;
     }
-    if (grown) {
-        RS_CUDA(cudaMemcpy2DAsync(sims, (size_t)ld * 8, h->sims, (size_t)h->ld_s * 8, (size_t)nl0 * 8, (size_t)nl0,
+    if (grown && rows0 > 0) {
+        RS_CUDA(cudaMemcpy2DAsync(sims, (size_t)ld * 8, h->sims, (size_t)h->ld_s * 8, (size_t)nl0 * 8, (size_t)rows0,
                                   cudaMemcpyDeviceToDevice, st));
     }
 
@@ -408,7 +441,7 @@ int32_t rs_update_run(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
     h->n_left = nl;
     h->n_right = nr;
     h->row_end = nl;
-    h->rows_local = nl;
+    h->rows_local = rows;
     h->ld_s = ld;
     h->max_right_len = max_right_len;
     h->global_mean = global_mean;
@@ -418,10 +451,20 @@ int32_t rs_update_run(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
     // the statistics are final when the call returns, as Fit's are: rs_knn_means / rs_knn_stddevs read them on the
     // auxiliary stream, which does not wait for this one
     RS_CUDA(cudaStreamSynchronize(st));
-    for (int64_t b0 = 0; b0 < n_touched; b0 += batch) {
-        const int64_t nb = n_touched - b0 < batch ? n_touched - b0 : batch;
+    for (int64_t b0 = 0; b0 < n_owned; b0 += batch) {
+        const int64_t nb = n_owned - b0 < batch ? n_owned - b0 : batch;
         RS_TRY(rs_given_sims_launch(h, h->l_ptr, h->l_col, h->l_val, h->pmeans, nb, (double *)slab, ld, w.rows + b0));
-        upd_scatter_kernel<<<blocks_for(nb * nl), T, 0, st>>>((const double *)slab, ld, w.rows + b0, nb, nl, sims);
+        upd_scatter_kernel<<<blocks_for(nb * nl), T, 0, st>>>((const double *)slab, ld, w.rows + b0, nb, nl, cyc_R,
+                                                               cyc_r, sims);
+        h->prof.total_launches++;
+    }
+    const int32_t *foreign = w.rows + n_owned;
+    for (int64_t b0 = 0; b0 < n_foreign; b0 += batch_own) {
+        const int64_t nb = n_foreign - b0 < batch_own ? n_foreign - b0 : batch_own;
+        RS_TRY(rs_given_sims_launch(h, h->l_ptr, h->l_col, h->l_val, h->pmeans, nb, (double *)slab, rows, foreign + b0,
+                                    true));
+        upd_scatter_own_kernel<<<blocks_for(nb * rows), T, 0, st>>>((const double *)slab, rows, foreign + b0, nb, ld,
+                                                                     sims);
         h->prof.total_launches++;
     }
     RS_CUDA(cudaGetLastError());

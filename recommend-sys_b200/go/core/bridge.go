@@ -145,6 +145,14 @@ func (d *deviceKNN) update(left, right []int32, rating []float64, nLeft, nRight 
 	runtime.KeepAlive(rating)
 }
 
+// updateShardedDevice adds ratings to a mirrored cyclic row shard (rs_knn_update_sharded_device): every shard of the
+// model gets the same device arrays, counts and GlobalMean, and afterwards holds its rows of the Fit of the union.
+func (d *deviceKNN) updateShardedDevice(dLeft, dRight, dRating unsafe.Pointer, nnz int64, nLeft, nRight int,
+	globalMean float64) {
+	check(C.rs_knn_update_sharded_device(d.h, (*C.int32_t)(dLeft), (*C.int32_t)(dRight), (*C.double)(dRating),
+		C.int64_t(nnz), C.int32_t(nLeft), C.int32_t(nRight), C.double(globalMean)))
+}
+
 // baselineALS is the EXTENSION behind Parameters["baseline"] = "als" (BASELINE.json config 3): ALS
 // baseline estimates computed on the device instead of BaseLine.Fit's sequential SGD
 // (core/base.go:135-163).  Returns (userBias, itemBias); the global bias is the global mean.

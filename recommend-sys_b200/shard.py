@@ -171,6 +171,7 @@ class ShardedKNN:
         est = ShardedKNN(rs.NewKNNWithMean(params))      # same constructors, same Parameters
         est.Fit(train)                                   # every rank passes the same TrainSet
         preds = est.PredictBatch(users, items)           # full prediction vector on every rank
+        est.Update(new_ratings)                          # every rank passes the same DataSet
 
     Fit uploads 1/world of the ratings per rank from (pinned) host memory and all-gathers them over
     NVLink, so the host->device traffic is divided by the number of GPUs."""
@@ -183,6 +184,7 @@ class ShardedKNN:
         self.world = dist.get_world_size(group)
         self.rank = dist.get_rank(group)
         self._need_mirror = False
+        self._split = False         # an Update succeeded on some ranks only: every call refuses until the next Fit
 
     def Fit(self, trainSet):
         import numpy as np
@@ -218,9 +220,22 @@ class ShardedKNN:
         # it, here and on every peer) is deferred to the first call that needs the whole rows, so the host
         # work in between — converting and routing the test set's ids — overlaps the kernel
         self._need_mirror = True
+        self._split = False
         return self
 
+    def _device(self):
+        """This rank's GPU: the update's inputs and the all-reduce of its return codes."""
+        import torch
+
+        return torch.device("cuda", torch.cuda.current_device())
+
+    def _refuse_if_split(self):
+        if self._split:
+            raise RuntimeError("ShardedKNN: an Update succeeded on some ranks and failed on others, so the shards no "
+                               "longer hold one model; Fit again")
+
     def _finish_fit(self):
+        self._refuse_if_split()
         if self._need_mirror:
             attach_peers_and_mirror(self.knn._h, self.group)
             self.knn._after_fit()
@@ -231,6 +246,7 @@ class ShardedKNN:
         import torch
         import torch.distributed as dist
 
+        self._refuse_if_split()
         k = self.knn
         n = len(userIDs)
         if n == 0:
@@ -262,6 +278,53 @@ class ShardedKNN:
         import numpy as np
 
         return float(self.PredictBatch(np.array([userID]), np.array([itemID]))[0])
+
+    def Update(self, rowSet):
+        """KNN.Update on the row shards: every rank passes the same `rowSet`, extends Data with it and adds it to its
+        shard (rs_knn_update_sharded_device), with no exchange of data; afterwards every rank holds its rows of the Fit
+        of Data.Extend(rowSet), bit for bit.  The ranks then agree on the outcome: a refusal (the same on every rank,
+        since every check reads replicated data) raises on every rank and leaves the model as it was everywhere; an
+        update that succeeded on some ranks and failed on others (out of memory, a CUDA error) raises on every rank,
+        and every later call raises until the next Fit."""
+        import numpy as np
+        import torch
+        import torch.distributed as dist
+
+        from . import core
+
+        self._finish_fit()
+        k = self.knn
+        data = k.Data.Extend(rowSet)
+        n0 = k.Data.Length()
+        iu, ii = data.innerUsers[n0:], data.innerItems[n0:]
+        if k._userBased:
+            left, right, n_left, n_right = iu, ii, data.UserCount, data.ItemCount
+        else:
+            left, right, n_left, n_right = ii, iu, data.ItemCount, data.UserCount
+        dev = self._device()
+        d_l = torch.from_numpy(np.ascontiguousarray(left, dtype=np.int32)).to(dev)
+        d_r = torch.from_numpy(np.ascontiguousarray(right, dtype=np.int32)).to(dev)
+        d_v = torch.from_numpy(np.ascontiguousarray(data.Ratings[n0:], dtype=np.float64)).to(dev)
+        err = None
+        try:
+            k._h.update_sharded_device(d_l.data_ptr(), d_r.data_ptr(), d_v.data_ptr(), len(d_v), n_left, n_right,
+                                       data.GlobalMean)
+        except core.RsError as e:
+            err = e
+        code = err.code if err is not None else 0
+        agree = torch.tensor([code, -code], dtype=torch.int64, device=dev)
+        dist.all_reduce(agree, op=dist.ReduceOp.MIN, group=self.group)
+        lo, hi = int(agree[0]), -int(agree[1])
+        if lo != hi:
+            self._split = True
+            raise core.RsError(lo, f"ShardedKNN.Update: the ranks disagree (return codes {lo} .. {hi}, this rank "
+                                   f"{code}{': ' + str(err) if err is not None else ''}); every call refuses until "
+                                   "the next Fit")
+        if err is not None:
+            raise err
+        k.Data = data
+        k.GlobalMean = data.GlobalMean
+        k._after_fit()
 
     def _device_queries(self, userIDs):
         """The query side and the inner-id queries on this rank's GPU (every rank passes the same users)."""
