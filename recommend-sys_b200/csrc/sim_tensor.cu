@@ -158,16 +158,6 @@ __device__ __forceinline__ void tma_load_box(uint32_t dst, const CUtensorMap *ma
         "l"(map), "r"(k & (RS_TC_KBLK - 1)), "r"(row), "r"(k / RS_TC_KBLK), "r"(plane), "r"(bar)
         : "memory");
 }
-__device__ __forceinline__ void tma_load_box_mc(uint32_t dst, const CUtensorMap *map, int row, int k, int plane,
-                                                uint32_t bar, uint16_t cta_mask) {
-    // the box lands at the same CTA-relative offset in every CTA of `cta_mask`, and each of them
-    // gets the complete_tx on its own mbarrier at the same offset
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.multicast::cluster "
-        "[%0], [%1, {%2, %3, %4, %5}], [%6], %7;" ::"r"(dst),
-        "l"(map), "r"(k & (RS_TC_KBLK - 1)), "r"(row), "r"(k / RS_TC_KBLK), "r"(plane), "r"(bar), "h"(cta_mask)
-        : "memory");
-}
 __device__ __forceinline__ uint32_t cluster_ctarank() {
     uint32_t r;
     asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -203,13 +193,6 @@ __device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t adesc, uint64_
 // mbarrier arrive once every previously issued tcgen05.mma of this thread has completed
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// same, arriving on the barrier at this offset in every CTA of `cta_mask`
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t cta_mask) {
-    asm volatile(
-        "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-        "h"(cta_mask)
-        : "memory");
 }
 __device__ __forceinline__ void tmem_ld8(uint32_t addr, int32_t (&v)[8]) {
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
@@ -250,7 +233,6 @@ struct TcArgs {
     const int32_t *row_sum;
     int32_t *cosums;        // TC_COSUMS: raw sums of rows [cos_row0, cos_row0+cos_nrows)
     int64_t cos_row0, cos_nrows;
-    int debug;              // RS_KNN_TC_DEBUG (timing experiments only): 1 = no TMA loads, 2 = no MMAs
     // K-lockstep throttle (performance hint only, see the TMA producer): chunks of `sync_chunk` K
     // blocks, a CTA may run at most `sync_slack` chunks ahead of the grid's average progress.
     unsigned long long *progress;
@@ -294,12 +276,107 @@ __device__ __forceinline__ double pearson_from_sums(long long n, long long sx, l
     return (double)L / (sqrt((double)Mi) * sqrt((double)Ni));
 }
 
-// CI x CJ = thread-block cluster shape.  The CTAs of a cluster work on CI x CJ adjacent tiles in
-// lockstep and share their operand loads: the A tile of a row block is needed by the CJ CTAs of
-// that cluster row, so each of them TMA-loads 1/CJ of it and MULTICASTS the slice to all CJ; the B
-// tile of a column block is shared the same way by the CI CTAs of a cluster column.  Per tile and
-// K block this cuts the L2/HBM operand traffic from 72 KB to 48/CJ + 24/CI KB.
-template <int MODE, int CI, int CJ>
+// K-lockstep throttle of the TMA producers.  Tiles that run at the same time share operand rows (supertile
+// rasterisation), but a row block is tens of MB long in K, so the sharing only hits in L2 while the CTAs stream
+// through K at the same position; left alone they drift apart and the DRAM traffic is 3-4x the ideal
+// (profiles/r01_tensor_cos_v2_summary.txt).  Every producer counts the K chunks it has issued in one global
+// counter and does not start chunk g before the grid as a whole has issued (g - slack) chunks per CTA.  The wait
+// is bounded and carries no data dependence: on a timeout the CTA just proceeds.
+// throttle_wait runs before K block kb; g counts the chunks this CTA has started.
+__device__ __forceinline__ void throttle_wait(const TcArgs &a, int kb, long long &g) {
+    const int chunk = a.sync_chunk;
+    if (chunk > 0 && kb % chunk == 0) {
+        if (g > 0) atomicAdd(a.progress, 1ull);          // chunk g-1 is issued
+        const long long need = (g - a.sync_slack) * (long long)gridDim.x;
+        if (need > 0 && (long long)ld_relaxed_gpu(a.progress) < need) {
+            const long long t0 = clock64();
+            while ((long long)ld_relaxed_gpu(a.progress) < need && clock64() - t0 < a.sync_timeout) {}
+        }
+        g++;
+    }
+}
+// Done: credit every chunk a CTA with the longest tile list would still issue.  The grid takes one tile per
+// cluster of CS CTAs.
+template <int CS>
+__device__ __forceinline__ void throttle_credit(const TcArgs &a, long long g) {
+    if (a.sync_chunk > 0) {
+        const int n_units = (int)(gridDim.x / CS);
+        const long long cpt = (a.k_blocks + a.sync_chunk - 1) / a.sync_chunk;
+        const long long max_chunks = (long long)((a.num_tiles + n_units - 1) / n_units) * cpt;
+        atomicAdd(a.progress, (unsigned long long)(max_chunks - g + 1));
+    }
+}
+
+// A thread's integer sums against 8 consecutive columns, read from the accumulator columns Cfg<MODE> assigns;
+// the sums a mode does not accumulate are left unset.
+struct Sums8 {
+    int32_t syy[8], sxy[8], sxx[8], cnt[8], sx[8], sy[8];
+};
+template <int MODE>
+__device__ __forceinline__ void tmem_ld_sums(uint32_t taddr, Sums8 &v) {
+    using C = Cfg<MODE>;
+    if constexpr (C::C_SYY >= 0) tmem_ld8(taddr + C::C_SYY, v.syy);
+    if constexpr (C::C_SXY >= 0) tmem_ld8(taddr + C::C_SXY, v.sxy);
+    if constexpr (C::C_SXX >= 0) tmem_ld8(taddr + C::C_SXX, v.sxx);
+    if constexpr (C::C_CNT >= 0) tmem_ld8(taddr + C::C_CNT, v.cnt);
+    if constexpr (C::C_SX >= 0) tmem_ld8(taddr + C::C_SX, v.sx);
+    if constexpr (C::C_SY >= 0) tmem_ld8(taddr + C::C_SY, v.sy);
+    tmem_ld_wait();
+}
+
+// S[i][j] from the sums of column c, for Cosine, MSD and Slope One (Pearson: pearson_from_sums)
+template <int MODE>
+__device__ __forceinline__ double sim_from_sums(const Sums8 &v, int c, int64_t i, int64_t j) {
+    if constexpr (MODE == TC_SLOPE) {
+        // core/slope_one.go:74-88: for i > j  dev[i][j] = sum(r_i - r_j) / count and
+        // dev[j][i] = -dev[i][j]; untouched cells (no co-rating, the diagonal) stay +0
+        const int32_t dbig = i > j ? v.sx[c] - v.sy[c] : v.sy[c] - v.sx[c];   // larger index minus smaller
+        const double q = (double)dbig / (double)v.cnt[c];
+        return (v.cnt[c] == 0 || i == j) ? 0.0 : (i > j ? q : -q);
+    } else {
+        static_assert(MODE == TC_COSINE || MODE == TC_MSD, "sim_from_sums: Cosine / MSD / Slope One");
+        double s;
+        if constexpr (MODE == TC_COSINE) {
+            // core/sim.go:24  l / (sqrt(m) * sqrt(n)),  m = Sxx, n = Syy, l = Sxy
+            s = (double)v.sxy[c] / (sqrt((double)v.sxx[c]) * sqrt((double)v.syy[c]));
+        } else {
+            // core/sim.go:43  1 / (sum/count + 1),  sum = (Sxx + Syy) - 2 Sxy (exact integer)
+            const int32_t sum = v.syy[c] - 2 * v.sxy[c];
+            s = 1.0 / ((double)sum / (double)v.cnt[c] + 1.0);
+        }
+        return j == i ? __longlong_as_double(0x7ff8000000000001ll) : s;   // diagonal stays unset (core/knn.go:202)
+    }
+}
+
+// Stores a thread's 8 similarities S[i][j0 .. j0+8): 64 contiguous bytes, if the handle holds row i (row_ok).
+// With a.mirror it also stores the mirrored S[j][i]: for a fixed j the 32 lanes write 32 consecutive doubles.
+template <int MODE>
+__device__ __forceinline__ void store8(const TcArgs &a, int64_t i, int64_t j0, bool row_ok, const double (&s)[8],
+                                       const Sums8 &v) {
+    if (row_ok) {
+        double *o = a.sims + (i - a.row_begin) * a.ld_s + j0;
+        if (j0 + 8 <= a.n_left) {
+#pragma unroll
+            for (int c = 0; c < 8; c += 2) *reinterpret_cast<double2 *>(o + c) = make_double2(s[c], s[c + 1]);
+        } else {
+#pragma unroll
+            for (int c = 0; c < 8; c++) if (j0 + c < a.n_left) o[c] = s[c];
+        }
+    }
+    if (a.mirror && i < a.n_left) {
+#pragma unroll
+        for (int c = 0; c < 8; c++) {
+            const int64_t j = j0 + c;
+            // Slope One is antisymmetric: dev[j][i] = -dev[i][j], signed zeros included, but cells
+            // that were never assigned (no co-rating) stay +0 on both sides
+            double sm = s[c];
+            if constexpr (MODE == TC_SLOPE) { if (v.cnt[c] != 0 && i != j) sm = -s[c]; }
+            if (j < a.n_left) a.sims[j * a.ld_s + i] = sm;
+        }
+    }
+}
+
+template <int MODE>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, TcArgs a) {
     using C = Cfg<MODE>;
@@ -307,15 +384,7 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
     constexpr int BN = G::BN, BK = G::BK, STAGES = G::STAGES;
     constexpr int A_PLANE_BYTES = G::A_PLANE_BYTES, B_PLANE_BYTES = G::B_PLANE_BYTES;
     constexpr int A_STAGE_BYTES = G::A_STAGE_BYTES, STAGE_BYTES = G::STAGE_BYTES;
-    constexpr int CS = CI * CJ;
-    const int crank = CS > 1 ? (int)cluster_ctarank() : 0;
-    const int ci = crank / CJ, cj = crank % CJ;
-    const int cluster_id = blockIdx.x / CS, n_clusters = gridDim.x / CS;
-    uint16_t mask_a = 0, mask_b = 0;        // CTAs sharing my A tile (cluster row) / my B tile (cluster column)
-#pragma unroll
-    for (int x = 0; x < CJ; x++) mask_a |= (uint16_t)(1u << (ci * CJ + x));
-#pragma unroll
-    for (int y = 0; y < CI; y++) mask_b |= (uint16_t)(1u << (y * CJ + cj));
+    const int cta_id = blockIdx.x, n_ctas = gridDim.x;
     extern __shared__ uint8_t smem_raw[];
     // SWIZZLE_128B needs 1024-byte aligned tiles
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -336,7 +405,7 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
         tma_prefetch_desc(&map_b);
         for (int s = 0; s < STAGES; s++) {
             mbar_init(full_bar + 8 * s, 1);
-            mbar_init(empty_bar + 8 * s, CI + CJ - 1);   // released by every CTA I multicast into
+            mbar_init(empty_bar + 8 * s, 1);
         }
         for (int s = 0; s < 2; s++) {
             mbar_init(tfull_bar + 8 * s, 1);
@@ -347,7 +416,6 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
     if (warp == 1) tmem_alloc(tmem_slot, TMEM_COLS);
     tc_fence_before();
     __syncthreads();
-    if (CS > 1) cluster_sync_all();   // every CTA's barriers exist before a peer can signal them
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot_ptr;
 
@@ -356,53 +424,27 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
         if (lane == 0) {
             int stage = 0;
             uint32_t phase = 0;
-            constexpr int A_SLICE = BM / CJ, B_SLICE = BN / CI;   // rows this CTA loads (and multicasts)
-            // K-lockstep throttle.  Tiles that run at the same time share operand rows (supertile
-            // rasterisation), but a row block is tens of MB long in K, so the sharing only hits in
-            // L2 while the CTAs stream through K at the same position; left alone they drift apart
-            // and the DRAM traffic is 3-4x the ideal (profiles/r01_tensor_cos_v2_summary.txt).
-            // Every producer counts the K chunks it has issued in one global counter and does not
-            // start chunk g before the grid as a whole has issued (g - slack) chunks per CTA.  The
-            // wait is bounded and carries no data dependence: on a timeout the CTA just proceeds.
-            const int chunk = a.sync_chunk;
-            const unsigned long long n_ctas = gridDim.x;
             long long g = 0;
-            for (int t = cluster_id; t < a.num_tiles; t += n_clusters) {
+            for (int t = cta_id; t < a.num_tiles; t += n_ctas) {
                 const int2 tile = a.tiles[t];
-                const int row_a = (tile.x * CI + ci) * BM + cj * A_SLICE;
-                const int row_b = (tile.y * CJ + cj) * BN + ci * B_SLICE;
+                const int row_a = tile.x * BM;
+                const int row_b = tile.y * BN;
                 for (int kb = 0; kb < a.k_blocks; kb++) {
-                    if (chunk > 0 && kb % chunk == 0) {
-                        if (g > 0) atomicAdd(a.progress, 1ull);          // chunk g-1 is issued
-                        const long long need = (g - a.sync_slack) * (long long)n_ctas;
-                        if (need > 0 && (long long)ld_relaxed_gpu(a.progress) < need) {
-                            const long long t0 = clock64();
-                            while ((long long)ld_relaxed_gpu(a.progress) < need && clock64() - t0 < a.sync_timeout) {}
-                        }
-                        g++;
-                    }
-                    mbar_wait(empty_bar + 8 * stage, phase ^ 1u, 0);   // all my destinations freed the stage
-                    const uint32_t sa = smem_base + stage * STAGE_BYTES + cj * A_SLICE * BK;
-                    const uint32_t sb = smem_base + stage * STAGE_BYTES + A_STAGE_BYTES + ci * B_SLICE * BK;
+                    throttle_wait(a, kb, g);
+                    mbar_wait(empty_bar + 8 * stage, phase ^ 1u, 0);   // the MMAs freed the stage
+                    const uint32_t sa = smem_base + stage * STAGE_BYTES;
+                    const uint32_t sb = sa + A_STAGE_BYTES;
                     const uint32_t fb = full_bar + 8 * stage;
-                    if (a.debug & 1) { mbar_arrive(fb); if (++stage == STAGES) { stage = 0; phase ^= 1u; } continue; }
-                    mbar_arrive_expect_tx(fb, STAGE_BYTES);            // my own stage: slices from all peers
+                    mbar_arrive_expect_tx(fb, STAGE_BYTES);
 #pragma unroll
                     for (int p = 0; p < 3; p++) {
-                        if (CJ > 1) tma_load_box_mc(sa + p * A_PLANE_BYTES, &map_a, row_a, kb * BK, p, fb, mask_a);
-                        else tma_load_box(sa + p * A_PLANE_BYTES, &map_a, row_a, kb * BK, p, fb);
-                        if (CI > 1) tma_load_box_mc(sb + p * B_PLANE_BYTES, &map_b, row_b, kb * BK, p, fb, mask_b);
-                        else tma_load_box(sb + p * B_PLANE_BYTES, &map_b, row_b, kb * BK, p, fb);
+                        tma_load_box(sa + p * A_PLANE_BYTES, &map_a, row_a, kb * BK, p, fb);
+                        tma_load_box(sb + p * B_PLANE_BYTES, &map_b, row_b, kb * BK, p, fb);
                     }
                     if (++stage == STAGES) { stage = 0; phase ^= 1u; }
                 }
             }
-            if (chunk > 0) {
-                // done: credit every chunk a CTA with the longest tile list would still issue
-                const long long cpt = (a.k_blocks + chunk - 1) / chunk;
-                const long long max_chunks = (long long)((a.num_tiles + n_clusters - 1) / n_clusters) * cpt;
-                atomicAdd(a.progress, (unsigned long long)(max_chunks - g + 1));
-            }
+            throttle_credit<1>(a, g);
         }
     } else if (warp == 1) {
         // ======================= MMA issuer =======================
@@ -411,7 +453,7 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
             uint32_t phase = 0;
             int acc = 0;
             uint32_t acc_phase = 0;
-            for (int t = cluster_id; t < a.num_tiles; t += n_clusters) {
+            for (int t = cta_id; t < a.num_tiles; t += n_ctas) {
                 mbar_wait(tempty_bar + 8 * acc, acc_phase ^ 1u, 1);   // epilogue drained this buffer
                 tc_fence_after();
                 const uint32_t d0 = tmem_base + (uint32_t)(acc * C::ACC_COLS);
@@ -421,7 +463,7 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
                     const uint32_t sa = smem_base + stage * STAGE_BYTES;
                     const uint32_t sb = sa + A_STAGE_BYTES;
 #pragma unroll
-                    for (int k = 0; k < ((a.debug & 2) ? 0 : BK / 32); k++) {
+                    for (int k = 0; k < BK / 32; k++) {
                         const uint32_t accum = (kb > 0 || k > 0) ? 1u : 0u;
                         const uint32_t ko = (uint32_t)k * 32u;
                         const uint64_t a_x2 = make_desc<BK>(sa + PL_X2 * A_PLANE_BYTES + ko);
@@ -447,9 +489,7 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
                             umma_i8(d0 + C::C_SXX, a_x2, b_m, make_idesc(BN), accum);
                         }
                     }
-                    // frees the smem stage (in every CTA that multicasts into it) once the MMAs are done
-                    if (CS > 1) umma_commit_mc(empty_bar + 8 * stage, (uint16_t)(mask_a | mask_b));
-                    else umma_commit(empty_bar + 8 * stage);
+                    umma_commit(empty_bar + 8 * stage);               // frees the smem stage once the MMAs are done
                     if (kb == a.k_blocks - 1) umma_commit(tfull_bar + 8 * acc);
                     if (++stage == STAGES) { stage = 0; phase ^= 1u; }
                 }
@@ -463,11 +503,10 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
         const int r_in_tile = q * 32 + lane;
         int acc = 0;
         uint32_t acc_phase = 0;
-        const double nan_v = __longlong_as_double(0x7ff8000000000001ll);
-        for (int t = cluster_id; t < a.num_tiles; t += n_clusters) {
+        for (int t = cta_id; t < a.num_tiles; t += n_ctas) {
             const int2 tile = a.tiles[t];
-            const int64_t i = ((int64_t)tile.x * CI + ci) * BM + r_in_tile;
-            const int64_t j0 = ((int64_t)tile.y * CJ + cj) * BN;
+            const int64_t i = (int64_t)tile.x * BM + r_in_tile;
+            const int64_t j0 = (int64_t)tile.y * BN;
             mbar_wait(tfull_bar + 8 * acc, acc_phase, 3);
             tc_fence_after();
             const uint32_t tbase = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * C::ACC_COLS);
@@ -476,16 +515,8 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
             const bool row_ok = (i < a.n_left) && (i >= a.row_begin) && (i < a.row_end);
 #pragma unroll 1
             for (int c0 = chalf * (BN / 2); c0 < (chalf + 1) * (BN / 2); c0 += 8) {
-                int32_t v_syy[8], v_sxy[8], v_sxx[8], v_cnt[8], v_sx[8], v_sy[8];
-                if (C::C_SYY >= 0) tmem_ld8(tbase + (C::C_SYY >= 0 ? C::C_SYY : 0) + c0, v_syy);
-                if (C::C_SXY >= 0) tmem_ld8(tbase + (C::C_SXY >= 0 ? C::C_SXY : 0) + c0, v_sxy);
-                if (C::C_SXX >= 0) tmem_ld8(tbase + (C::C_SXX >= 0 ? C::C_SXX : 0) + c0, v_sxx);
-                if (C::C_CNT >= 0) tmem_ld8(tbase + (C::C_CNT >= 0 ? C::C_CNT : 0) + c0, v_cnt);
-                if (C::C_SX >= 0) {
-                    tmem_ld8(tbase + (C::C_SX >= 0 ? C::C_SX : 0) + c0, v_sx);
-                    tmem_ld8(tbase + (C::C_SY >= 0 ? C::C_SY : 0) + c0, v_sy);
-                }
-                tmem_ld_wait();
+                Sums8 v;
+                tmem_ld_sums<MODE>(tbase + c0, v);
                 if constexpr (MODE == TC_COSUMS) {
                     const int64_t r = i - a.cos_row0;
                     if (i < a.n_left && r >= 0 && r < a.cos_nrows) {
@@ -494,61 +525,28 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
                             const int64_t j = j0 + c0 + c;
                             if (j < a.n_left) {
                                 int32_t *o = a.cosums + (r * a.n_left + j) * 6;
-                                o[0] = v_cnt[c]; o[1] = v_sx[c]; o[2] = v_sy[c];
-                                o[3] = v_sxx[c]; o[4] = v_syy[c]; o[5] = v_sxy[c];
+                                o[0] = v.cnt[c]; o[1] = v.sx[c]; o[2] = v.sy[c];
+                                o[3] = v.sxx[c]; o[4] = v.syy[c]; o[5] = v.sxy[c];
                             }
                         }
                     }
                 } else {
-                double s[8];
-#pragma unroll
-                for (int c = 0; c < 8; c++) {
-                    const int64_t j = j0 + c0 + c;
-                    if constexpr (MODE == TC_SLOPE) {
-                        // core/slope_one.go:74-88: for i > j  dev[i][j] = sum(r_i - r_j) / count and
-                        // dev[j][i] = -dev[i][j]; untouched cells (no co-rating, the diagonal) stay +0
-                        const int32_t dbig = i > j ? v_sx[c] - v_sy[c] : v_sy[c] - v_sx[c];   // larger index minus smaller
-                        const double q = (double)dbig / (double)v_cnt[c];
-                        s[c] = (v_cnt[c] == 0 || i == j) ? 0.0 : (i > j ? q : -q);
-                    } else if constexpr (MODE == TC_COSINE) {
-                        // core/sim.go:24  l / (sqrt(m) * sqrt(n)),  m = Sxx, n = Syy, l = Sxy
-                        s[c] = (double)v_sxy[c] / (sqrt((double)v_sxx[c]) * sqrt((double)v_syy[c]));
-                    } else if constexpr (MODE == TC_MSD) {
-                        // core/sim.go:43  1 / (sum/count + 1),  sum = (Sxx + Syy) - 2 Sxy (exact integer)
-                        const int32_t sum = v_syy[c] - 2 * v_sxy[c];
-                        s[c] = 1.0 / ((double)sum / (double)v_cnt[c] + 1.0);
-                    } else {
-                        long long cb = 0, sb = 0;
-                        if (j < a.n_left) { cb = a.row_cnt[j]; sb = a.row_sum[j]; }
-                        s[c] = pearson_from_sums(v_cnt[c], v_sx[c], v_sy[c], v_sxx[c], v_syy[c], v_sxy[c], ca, sa,
-                                                 cb, sb);
-                    }
-                    if (MODE != TC_SLOPE && j == i) s[c] = nan_v;   // diagonal stays unset (core/knn.go:202)
-                }
-                // S[i][j0+c0 .. +8): 64 contiguous bytes per thread
-                if (row_ok) {
-                    double *o = a.sims + (i - a.row_begin) * a.ld_s + j0 + c0;
-                    if (j0 + c0 + 8 <= a.n_left) {
-#pragma unroll
-                        for (int c = 0; c < 8; c += 2) *reinterpret_cast<double2 *>(o + c) = make_double2(s[c], s[c + 1]);
-                    } else {
-#pragma unroll
-                        for (int c = 0; c < 8; c++) if (j0 + c0 + c < a.n_left) o[c] = s[c];
-                    }
-                }
-                // mirrored S[j][i]: for a fixed j the 32 lanes write 32 consecutive doubles
-                if (a.mirror && i < a.n_left) {
+                    double s[8];
 #pragma unroll
                     for (int c = 0; c < 8; c++) {
                         const int64_t j = j0 + c0 + c;
-                        // Slope One is antisymmetric: dev[j][i] = -dev[i][j], signed zeros included, but cells
-                        // that were never assigned (no co-rating) stay +0 on both sides
-                        double sm = s[c];
-                        if constexpr (MODE == TC_SLOPE) { if (v_cnt[c] != 0 && i != j) sm = -s[c]; }
-                        if (j < a.n_left) a.sims[j * a.ld_s + i] = sm;
+                        if constexpr (MODE == TC_PEARSON) {
+                            long long cb = 0, sb = 0;
+                            if (j < a.n_left) { cb = a.row_cnt[j]; sb = a.row_sum[j]; }
+                            s[c] = pearson_from_sums(v.cnt[c], v.sx[c], v.sy[c], v.sxx[c], v.syy[c], v.sxy[c], ca, sa,
+                                                     cb, sb);
+                            if (j == i) s[c] = __longlong_as_double(0x7ff8000000000001ll);   // diagonal stays unset
+                        } else {
+                            s[c] = sim_from_sums<MODE>(v, c, i, j);
+                        }
                     }
+                    store8<MODE>(a, i, j0 + c0, row_ok, s, v);
                 }
-                }  // !COSUMS
             }
             tc_fence_before();
             mbar_arrive(tempty_bar + 8 * acc);     // 256 arrivals release the accumulator buffer
@@ -558,7 +556,6 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
 
     tc_fence_before();
     __syncthreads();
-    if (CS > 1) cluster_sync_all();   // no CTA leaves while a peer may still write into it
     tc_fence_after();
     if (warp == 1) {
         __syncwarp();
@@ -580,8 +577,9 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
 //             empty[s] : one per CTA; tcgen05.commit.cta_group::2 multicast to both
 //             tfull    : one per CTA (commit multicast) -> each CTA's epilogue reads ITS 128 TMEM lanes
 //             tempty   : even CTA only, 512 arrivals (both epilogues; the odd one arrives remotely)
-// Accumulator columns: Cosine [Syy | Sxy | Sxx], MSD [Syy+Sxx | count | Sxy] (N = 128 each; the wide
-// N = 256 combination of the single-CTA kernel is not available because the pair splits B by rows).
+// Accumulator columns are those of Cfg<MODE>: Cosine [Syy | Sxy | Sxx], MSD [Syy+Sxx | count | Sxy], Slope One
+// [count | Sy | Sx] (N = 128 each; the wide N = 256 combination of the single-CTA kernel is not available because
+// the pair splits B by rows).
 namespace pair {
 
 constexpr int P_BN = 128, P_BK = 64, P_STAGES = 6;
@@ -637,7 +635,7 @@ template <int MODE>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 sim_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, TcArgs a) {
     static_assert(MODE == TC_COSINE || MODE == TC_MSD || MODE == TC_SLOPE, "pair kernel: Cosine / MSD / Slope One");
-    constexpr int C_SYY = 0, C_B = 128, C_C = 256;   // Cosine: Syy, Sxy, Sxx   MSD: Syy+Sxx, count, Sxy   Slope: count, Sy, Sx
+    using C = Cfg<MODE>;
     const int rank = (int)cluster_ctarank();         // 0 = even CTA = MMA issuer
     const int pair_id = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
     extern __shared__ uint8_t smem_raw[];
@@ -676,23 +674,13 @@ sim_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
         if (lane == 0) {
             int stage = 0;
             uint32_t phase = 0;
-            const int chunk = a.sync_chunk;
-            const unsigned long long n_ctas = gridDim.x;
             long long g = 0;
             for (int t = pair_id; t < a.num_tiles; t += n_pairs) {
                 const int2 tile = a.tiles[t];
                 const int row_a = (tile.x * 2 + rank) * BM;                  // my 128 of the tile's 256 A rows
                 const int row_b = tile.y * P_BN + rank * (P_BN / 2);          // my 64 of the tile's 128 B rows
                 for (int kb = 0; kb < a.k_blocks; kb++) {
-                    if (chunk > 0 && kb % chunk == 0) {                       // K-lockstep throttle (see above)
-                        if (g > 0) atomicAdd(a.progress, 1ull);
-                        const long long need = (g - a.sync_slack) * (long long)n_ctas;
-                        if (need > 0 && (long long)ld_relaxed_gpu(a.progress) < need) {
-                            const long long t0 = clock64();
-                            while ((long long)ld_relaxed_gpu(a.progress) < need && clock64() - t0 < a.sync_timeout) {}
-                        }
-                        g++;
-                    }
+                    throttle_wait(a, kb, g);
                     mbar_wait(empty_bar + 8 * stage, phase ^ 1u, 0);
                     const uint32_t sa = smem_base + stage * P_STAGE;
                     const uint32_t sb = sa + P_A_STAGE;
@@ -706,11 +694,7 @@ sim_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
                     if (++stage == P_STAGES) { stage = 0; phase ^= 1u; }
                 }
             }
-            if (chunk > 0) {
-                const long long cpt = (a.k_blocks + chunk - 1) / chunk;
-                const long long max_chunks = (long long)((a.num_tiles + n_pairs - 1) / n_pairs) * cpt;
-                atomicAdd(a.progress, (unsigned long long)(max_chunks - g + 1));
-            }
+            throttle_credit<2>(a, g);
         }
     } else if (warp == 1) {
         // ======================= MMA issuer (even CTA only) =======================
@@ -737,18 +721,18 @@ sim_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
                         const uint64_t b_m = make_desc<P_BK>(sb + PL_M * P_B_PLANE + ko);
                         const uint64_t b_x = make_desc<P_BK>(sb + PL_X * P_B_PLANE + ko);
                         if constexpr (MODE == TC_SLOPE) {
-                            umma_i8_2sm(d0 + C_SYY, a_m, b_m, make_idesc_2sm(P_BN), accum);    // count
-                            umma_i8_2sm(d0 + C_B, a_m, b_x, make_idesc_2sm(P_BN), accum);      // Sy
-                            umma_i8_2sm(d0 + C_C, a_x, b_m, make_idesc_2sm(P_BN), accum);      // Sx
+                            umma_i8_2sm(d0 + C::C_CNT, a_m, b_m, make_idesc_2sm(P_BN), accum);
+                            umma_i8_2sm(d0 + C::C_SY, a_m, b_x, make_idesc_2sm(P_BN), accum);
+                            umma_i8_2sm(d0 + C::C_SX, a_x, b_m, make_idesc_2sm(P_BN), accum);
                         } else if constexpr (MODE == TC_COSINE) {
-                            umma_i8_2sm(d0 + C_SYY, a_m, b_x2, make_idesc_2sm(P_BN), accum);   // Syy
-                            umma_i8_2sm(d0 + C_B, a_x, b_x, make_idesc_2sm(P_BN), accum);      // Sxy
-                            umma_i8_2sm(d0 + C_C, a_x2, b_m, make_idesc_2sm(P_BN), accum);     // Sxx
+                            umma_i8_2sm(d0 + C::C_SYY, a_m, b_x2, make_idesc_2sm(P_BN), accum);
+                            umma_i8_2sm(d0 + C::C_SXY, a_x, b_x, make_idesc_2sm(P_BN), accum);
+                            umma_i8_2sm(d0 + C::C_SXX, a_x2, b_m, make_idesc_2sm(P_BN), accum);
                         } else {
-                            umma_i8_2sm(d0 + C_SYY, a_m, b_x2, make_idesc_2sm(P_BN), accum);   // Syy
-                            umma_i8_2sm(d0 + C_SYY, a_x2, b_m, make_idesc_2sm(P_BN), 1u);      //  += Sxx
-                            umma_i8_2sm(d0 + C_B, a_m, b_m, make_idesc_2sm(P_BN), accum);      // count
-                            umma_i8_2sm(d0 + C_C, a_x, b_x, make_idesc_2sm(P_BN), accum);      // Sxy
+                            umma_i8_2sm(d0 + C::C_SYY, a_m, b_x2, make_idesc_2sm(P_BN), accum);
+                            umma_i8_2sm(d0 + C::C_SYY, a_x2, b_m, make_idesc_2sm(P_BN), 1u);   // Syy += Sxx
+                            umma_i8_2sm(d0 + C::C_CNT, a_m, b_m, make_idesc_2sm(P_BN), accum);
+                            umma_i8_2sm(d0 + C::C_SXY, a_x, b_x, make_idesc_2sm(P_BN), accum);
                         }
                     }
                     umma_commit_2sm(empty_bar + 8 * stage);          // frees the stage in both CTAs
@@ -764,7 +748,6 @@ sim_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
         const int chalf = (warp - 2) >> 2;          // which half of the tile's columns this warp converts
         const int r_in_tile = q * 32 + lane;
         uint32_t acc_phase = 0;
-        const double nan_v = __longlong_as_double(0x7ff8000000000001ll);
         const uint32_t tempty_leader = tempty_bar & PEER_MASK;
         unsigned long long *s_thrk = reinterpret_cast<unsigned long long *>(smem_gen + P_STAGES * P_STAGE + 256);
         uint32_t *s_thri = reinterpret_cast<uint32_t *>(s_thrk + 2 * P_BN);
@@ -793,30 +776,11 @@ sim_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
             const bool row_ok = (i < a.n_left) && (i >= a.row_begin) && (i < a.row_end);
 #pragma unroll 1
             for (int c0 = chalf * (P_BN / 2); c0 < (chalf + 1) * (P_BN / 2); c0 += 8) {
-                int32_t v_a[8], v_b[8], v_c[8];
-                tmem_ld8(tbase + C_SYY + c0, v_a);
-                tmem_ld8(tbase + C_B + c0, v_b);
-                tmem_ld8(tbase + C_C + c0, v_c);
-                tmem_ld_wait();
+                Sums8 v;
+                tmem_ld_sums<MODE>(tbase + c0, v);
                 double s[8];
 #pragma unroll
-                for (int c = 0; c < 8; c++) {
-                    const int64_t j = j0 + c0 + c;
-                    if constexpr (MODE == TC_SLOPE) {
-                        // core/slope_one.go:74-88 (see the single-CTA epilogue): v_a = count, v_b = Sy, v_c = Sx
-                        const int32_t dbig = i > j ? v_c[c] - v_b[c] : v_b[c] - v_c[c];
-                        const double q = (double)dbig / (double)v_a[c];
-                        s[c] = (v_a[c] == 0 || i == j) ? 0.0 : (i > j ? q : -q);
-                    } else if constexpr (MODE == TC_COSINE) {
-                        // core/sim.go:24  l / (sqrt(m) * sqrt(n)),  m = Sxx, n = Syy, l = Sxy
-                        s[c] = (double)v_b[c] / (sqrt((double)v_c[c]) * sqrt((double)v_a[c]));
-                    } else {
-                        // core/sim.go:43  1 / (sum/count + 1),  sum = (Sxx + Syy) - 2 Sxy (exact integer)
-                        const int32_t sum = v_a[c] - 2 * v_c[c];
-                        s[c] = 1.0 / ((double)sum / (double)v_b[c] + 1.0);
-                    }
-                    if (MODE != TC_SLOPE && j == i) s[c] = nan_v;   // diagonal stays unset (core/knn.go:202)
-                }
+                for (int c = 0; c < 8; c++) s[c] = sim_from_sums<MODE>(v, c, i, j0 + c0 + c);
                 if (a.topk_mode) {
                     // selection fused into the epilogue: one compare against each of the two rows' thresholds,
                     // the rare survivor is appended to that row's candidate buffer
@@ -845,25 +809,7 @@ sim_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
                     }
                     continue;
                 }
-                if (row_ok) {
-                    double *o = a.sims + (i - a.row_begin) * a.ld_s + j0 + c0;
-                    if (j0 + c0 + 8 <= a.n_left) {
-#pragma unroll
-                        for (int c = 0; c < 8; c += 2) *reinterpret_cast<double2 *>(o + c) = make_double2(s[c], s[c + 1]);
-                    } else {
-#pragma unroll
-                        for (int c = 0; c < 8; c++) if (j0 + c0 + c < a.n_left) o[c] = s[c];
-                    }
-                }
-                if (a.mirror && i < a.n_left) {
-#pragma unroll
-                    for (int c = 0; c < 8; c++) {
-                        const int64_t j = j0 + c0 + c;
-                        double sm = s[c];
-                        if constexpr (MODE == TC_SLOPE) { if (v_a[c] != 0 && i != j) sm = -s[c]; }   // antisymmetric
-                        if (j < a.n_left) a.sims[j * a.ld_s + i] = sm;
-                    }
-                }
+                store8<MODE>(a, i, j0 + c0, row_ok, s, v);
             }
             tc_fence_before();
             mbar_arrive_cluster(tempty_leader);    // 2 x 256 arrivals release the accumulators of the pair
@@ -924,92 +870,81 @@ int32_t make_map(const rs_knn *h, int box_k, int box_rows, CUtensorMap *map) {
     return RS_OK;
 }
 
-template <int MODE, int CI, int CJ>
-int32_t launch_mode(rs_knn *h, const TcArgs &a) {
-    constexpr int CS = CI * CJ;
-    using G = Geo<MODE>;
-    constexpr int SMEM_BYTES = G::SMEM_BYTES;
+typedef void (*TcKernel)(CUtensorMap, CUtensorMap, TcArgs);
+
+// Launches one persistent wave of `kern` (`smem` bytes of dynamic shared memory) in clusters of `cs` CTAs: 1, or 2
+// for the CTA pair.  Each CTA loads operand boxes of bk bytes of K by a_rows rows of A and b_rows rows of B.
+int32_t launch_tc(rs_knn *h, TcKernel kern, int smem, int cs, int bk, int a_rows, int b_rows, TcArgs a) {
+    a.k_blocks = (int32_t)(h->tc_kpad / bk);
+    // K-lockstep throttle: only worth it when a row block does not fit in L2 many times over
+    a.progress = reinterpret_cast<unsigned long long *>(h->d_flags + 4);
+    a.sync_chunk = (a.k_blocks >= 256 && a.num_tiles > 148) ? 32 : 0;
+    a.sync_slack = 1;
+    a.sync_timeout = 40000;   // clocks (~20 us): a hint, never a dependence
+    if (a.sync_chunk > 0) RS_CUDA(cudaMemsetAsync(a.progress, 0, 8, h->stream));
     CUtensorMap ma, mb;
-    RS_TRY(make_map(h, G::BK, BM / CJ, &ma));
-    RS_TRY(make_map(h, G::BK, G::BN / CI, &mb));
-    auto kern = sim_tensor_kernel<MODE, CI, CJ>;
-    RS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    RS_TRY(make_map(h, bk, a_rows, &ma));
+    RS_TRY(make_map(h, bk, b_rows, &mb));
+    RS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
     cudaLaunchConfig_t cfg{};
     cfg.blockDim = dim3(NUM_THREADS);
-    cfg.dynamicSmemBytes = SMEM_BYTES;
+    cfg.dynamicSmemBytes = smem;
     cfg.stream = h->stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CS;
+    attr[0].val.clusterDim.x = cs;
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    int n_clusters = sms / CS;
-    if (CS > 1) {
-        cfg.gridDim = dim3((unsigned)(n_clusters * CS));
+    int n_clusters = sms / cs;
+    if (cs > 1) {
+        cfg.gridDim = dim3((unsigned)(n_clusters * cs));
         int max_clusters = 0;
         RS_CUDA(cudaOccupancyMaxActiveClusters(&max_clusters, kern, &cfg));
         if (max_clusters < 1) {
-            rs_set_error("a %d-CTA cluster of the tensor kernel does not fit on this device", CS);
+            rs_set_error("a CTA pair of the tensor kernel does not fit on this device");
             return RS_ERR_CUDA;
         }
         if (n_clusters > max_clusters) n_clusters = max_clusters;   // persistent: one resident wave
     }
     if (n_clusters > a.num_tiles) n_clusters = a.num_tiles;
-    cfg.gridDim = dim3((unsigned)(n_clusters * CS));
+    cfg.gridDim = dim3((unsigned)(n_clusters * cs));
     RS_CUDA(cudaLaunchKernelEx(&cfg, kern, ma, mb, a));
     RS_CUDA(cudaGetLastError());
     return RS_OK;
 }
 
 template <int MODE>
-int32_t launch_pair(rs_knn *h, const TcArgs &a) {
-    CUtensorMap ma, mb;
-    RS_TRY(make_map(h, pair::P_BK, BM, &ma));
-    RS_TRY(make_map(h, pair::P_BK, pair::P_BN / 2, &mb));
-    auto kern = pair::sim_tensor_pair_kernel<MODE>;
-    RS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, pair::P_SMEM));
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-    cudaLaunchConfig_t cfg{};
-    cfg.blockDim = dim3(NUM_THREADS);
-    cfg.dynamicSmemBytes = pair::P_SMEM;
-    cfg.stream = h->stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    int n_pairs = sms / 2;
-    cfg.gridDim = dim3((unsigned)(n_pairs * 2));
-    int max_clusters = 0;
-    RS_CUDA(cudaOccupancyMaxActiveClusters(&max_clusters, kern, &cfg));
-    if (max_clusters < 1) {
-        rs_set_error("a CTA pair of the tensor kernel does not fit on this device");
-        return RS_ERR_CUDA;
-    }
-    if (n_pairs > max_clusters) n_pairs = max_clusters;   // persistent: one resident wave
-    if (n_pairs > a.num_tiles) n_pairs = a.num_tiles;
-    cfg.gridDim = dim3((unsigned)(n_pairs * 2));
-    RS_CUDA(cudaLaunchKernelEx(&cfg, kern, ma, mb, a));
-    RS_CUDA(cudaGetLastError());
-    return RS_OK;
+int32_t launch_single(rs_knn *h, const TcArgs &a) {
+    using G = Geo<MODE>;
+    return launch_tc(h, sim_tensor_kernel<MODE>, G::SMEM_BYTES, 1, G::BK, BM, G::BN, a);
 }
 
-template <int CI, int CJ>
-int32_t launch_shape(rs_knn *h, const TcArgs &a, bool cosums) {
-    if (cosums) return launch_mode<TC_COSUMS, CI, CJ>(h, a);
-    if (h->p.sim == RS_SIM_SLOPE_ONE) return launch_mode<TC_SLOPE, CI, CJ>(h, a);
-    if (h->p.sim == RS_SIM_COSINE) return launch_mode<TC_COSINE, CI, CJ>(h, a);
-    if (h->p.sim == RS_SIM_MSD) return launch_mode<TC_MSD, CI, CJ>(h, a);
-    if (h->p.sim == RS_SIM_PEARSON) return launch_mode<TC_PEARSON, CI, CJ>(h, a);
-    rs_set_error("tensor path supports Cosine, MSD and Pearson (sums mode) only");
-    return RS_ERR_UNSUPPORTED;
+template <int MODE>
+int32_t launch_pair(rs_knn *h, const TcArgs &a) {
+    return launch_tc(h, pair::sim_tensor_pair_kernel<MODE>, pair::P_SMEM, 2, pair::P_BK, BM, pair::P_BN / 2, a);
+}
+
+// Copies a tile list into the grow-only device buffer *buf of *cap bytes.  Returns once the copy is done:
+// `tiles` is a pageable temporary.
+int32_t upload_tiles(rs_knn *h, const std::vector<int2> &tiles, void **buf, size_t *cap) {
+    const size_t bytes = tiles.size() * sizeof(int2);
+    if (bytes > *cap) {
+        RS_CUDA(cudaStreamSynchronize(h->stream));
+        if (*buf) cudaFree(*buf);
+        *buf = nullptr;
+        *cap = 0;
+        RS_CUDA(cudaMalloc(buf, bytes + 256));
+        *cap = bytes + 256;
+    }
+    if (bytes) {
+        RS_CUDA(cudaMemcpyAsync(*buf, tiles.data(), bytes, cudaMemcpyHostToDevice, h->stream));
+        RS_CUDA(cudaStreamSynchronize(h->stream));
+    }
+    return RS_OK;
 }
 
 }  // namespace
@@ -1102,19 +1037,7 @@ int32_t rs_sim_tensor_band_launch(rs_knn *h, int32_t wave) {
             flat.insert(flat.end(), bands[w].begin(), bands[w].end());
         }
         h->band_off[n_waves] = (int64_t)flat.size();
-        const size_t bytes = flat.size() * sizeof(int2);
-        if (bytes > h->band_buf_bytes) {
-            RS_CUDA(cudaStreamSynchronize(h->stream));
-            if (h->band_buf) cudaFree(h->band_buf);
-            h->band_buf = nullptr;
-            h->band_buf_bytes = 0;
-            RS_CUDA(cudaMalloc(&h->band_buf, bytes + 256));
-            h->band_buf_bytes = bytes + 256;
-        }
-        if (bytes) {
-            RS_CUDA(cudaMemcpyAsync(h->band_buf, flat.data(), bytes, cudaMemcpyHostToDevice, h->stream));
-            RS_CUDA(cudaStreamSynchronize(h->stream));  // `flat` is a pageable temporary
-        }
+        RS_TRY(upload_tiles(h, flat, &h->band_buf, &h->band_buf_bytes));
         memcpy(h->band_key, key, sizeof(key));
     }
     const int64_t t0 = h->band_off[wave], t1 = h->band_off[wave + 1];
@@ -1122,7 +1045,6 @@ int32_t rs_sim_tensor_band_launch(rs_knn *h, int32_t wave) {
     TcArgs a{};
     a.tiles = reinterpret_cast<const int2 *>(h->band_buf) + t0;
     a.num_tiles = (int32_t)(t1 - t0);
-    a.k_blocks = (int32_t)(h->tc_kpad / pair::P_BK);
     a.n_left = h->n_left;
     a.row_begin = 0;
     a.row_end = h->n_left;
@@ -1136,13 +1058,6 @@ int32_t rs_sim_tensor_band_launch(rs_knn *h, int32_t wave) {
     a.cand_id = h->cand_id;
     a.cand_sim = h->cand_sim;
     a.cand_cap = h->cand_cap;
-    if (const char *e = getenv("RS_KNN_TC_DEBUG")) a.debug = atoi(e);
-    a.progress = reinterpret_cast<unsigned long long *>(h->d_flags + 4);
-    a.sync_chunk = (a.k_blocks >= 256 && a.num_tiles > 148) ? 32 : 0;
-    a.sync_slack = 1;
-    a.sync_timeout = 40000;
-    if (const char *e = getenv("RS_KNN_TC_SYNC")) sscanf(e, "%d,%d,%d", &a.sync_chunk, &a.sync_slack, &a.sync_timeout);
-    if (a.sync_chunk > 0) RS_CUDA(cudaMemsetAsync(a.progress, 0, 8, h->stream));
     RS_TRY(mode == TC_COSINE ? launch_pair<TC_COSINE>(h, a) : launch_pair<TC_MSD>(h, a));
     h->prof.sim_launches++;
     h->prof.total_launches++;
@@ -1168,71 +1083,47 @@ int32_t rs_sim_tensor_launch(rs_knn *h, int32_t *d_cosums, int64_t cos_row0, int
     const int64_t re = cosums ? cos_row0 + cos_nrows : h->row_end;
     if (re <= rb) return RS_OK;
     const bool mirror = !cosums && rb == 0 && re == h->n_left;
-    // cluster shape: the CI x CJ CTAs of a cluster share operand loads by TMA multicast.  Measured on
-    // the ML-20M item shape (profiles/r01_tensor_calibration.md): with the K-lockstep throttle the
-    // L2 already serves the sharing, 2x1 (B tile multicast) is worth ~6 % for Cosine / MSD, larger
-    // clusters lose to their own lockstep coupling, and Pearson is fastest unclustered.  Small
-    // problems run unclustered so every SM gets a tile.  RS_KNN_TC_CLUSTER=1x1|1x2|2x1|... overrides.
     const int mode = cosums ? TC_COSUMS
-                            : (h->p.sim == RS_SIM_COSINE ? TC_COSINE
-                               : h->p.sim == RS_SIM_MSD ? TC_MSD : h->p.sim == RS_SIM_SLOPE_ONE ? TC_SLOPE : TC_PEARSON);
+                            : h->p.sim == RS_SIM_COSINE ? TC_COSINE
+                            : h->p.sim == RS_SIM_MSD ? TC_MSD
+                            : h->p.sim == RS_SIM_SLOPE_ONE ? TC_SLOPE
+                            : h->p.sim == RS_SIM_PEARSON ? TC_PEARSON : -1;
+    if (mode < 0) {
+        rs_set_error("tensor path supports Cosine, MSD and Pearson (sums mode) only");
+        return RS_ERR_UNSUPPORTED;
+    }
     const bool wide = mode == TC_COSINE || mode == TC_MSD || mode == TC_SLOPE;       // 128 x 128 tiles, 64-byte K blocks
     const int BN = wide ? Cfg<TC_COSINE>::BN : Cfg<TC_PEARSON>::BN;
-    const int BK = wide ? Cfg<TC_COSINE>::BK : Cfg<TC_PEARSON>::BK;
-    static_assert(Cfg<TC_COSINE>::BN == Cfg<TC_MSD>::BN && Cfg<TC_COSINE>::BK == Cfg<TC_MSD>::BK &&
-                  Cfg<TC_COSINE>::BN == Cfg<TC_SLOPE>::BN && Cfg<TC_COSINE>::BK == Cfg<TC_SLOPE>::BK, "host tile geometry");
+    static_assert(Cfg<TC_COSINE>::BN == Cfg<TC_MSD>::BN && Cfg<TC_COSINE>::BN == Cfg<TC_SLOPE>::BN, "host tile geometry");
     const int64_t plain_tiles = ((re - rb + BM - 1) / BM) * ((h->n_left + BN - 1) / BN) / (mirror ? 2 : 1);
-    int ci = wide ? 2 : 1, cj = 1;
-    if (plain_tiles < 4 * 148) { ci = 1; cj = 1; }
-    // Cosine / MSD on large problems: the cta_group::2 pair kernel (256 x 128 tiles = the 2x1 cluster
-    // tile of the list below).  RS_KNN_TC_PAIR=0|1 overrides.
-    bool use_pair = wide && ci == 2 && cj == 1;
+    // Which kernel: Cosine / MSD / Slope One problems of at least four tiles per SM run the cta_group::2 pair kernel
+    // (256 x 128 tiles; measured on the ML-20M item shape in profiles/r01_tensor_calibration.md), everything else the
+    // single-CTA kernel, so that small problems give every SM a tile.  RS_KNN_TC_PAIR=0|1 overrides.
+    bool use_pair = wide && plain_tiles >= 4 * 148;
     if (const char *e = getenv("RS_KNN_TC_PAIR")) use_pair = wide && atoi(e) != 0;
-    if (use_pair) { ci = 2; cj = 1; }
-    if (const char *e = getenv("RS_KNN_TC_CLUSTER")) {
-        if (use_pair) {}
-        else if (!strcmp(e, "1x1")) { ci = 1; cj = 1; }
-        else if (!strcmp(e, "1x2")) { ci = 1; cj = 2; }
-        else if (!strcmp(e, "2x2")) { ci = 2; cj = 2; }
-        else if (!strcmp(e, "2x1")) { ci = 2; cj = 1; }
-    }
-    int sup_i = 8, sup_j = 1024 / BN;   // supertile (1024 x 1024 similarities), in plain tiles
-    if (const char *e = getenv("RS_KNN_TC_SUP")) sscanf(e, "%d,%d", &sup_i, &sup_j);
-    // tile list in units of cluster tiles (ci x cj plain tiles each)
+    const int ci = use_pair ? 2 : 1;   // row blocks per tile: the pair kernel's tiles are 256 x 128
     const int nbj = (int)((h->n_left + BN - 1) / BN);
     const int bi0 = (int)(rb / BM), bi1 = (int)((re + BM - 1) / BM);
-    const int64_t key[5] = {h->n_left, rb, re,
-                            (mirror ? 1 : 0) + 2 * (ci * 16 + cj) + 1024 * (int64_t)(sup_i * 4096 + sup_j) + ((int64_t)BN << 40),
+    const int64_t key[5] = {h->n_left, rb, re, (mirror ? 1 : 0) + (use_pair ? 2 : 0) + 4 * (int64_t)BN,
                             cosums ? 0 : h->col_begin};
     if (memcmp(key, h->tile_key, sizeof(key)) != 0) {
-        // Rasterised in supertiles so concurrently running clusters touch few distinct row blocks.
-        const int SUP_I = sup_i / ci > 0 ? sup_i / ci : 1, SUP_J = sup_j / cj > 0 ? sup_j / cj : 1;
-        const int cbi0 = bi0 / ci, cbi1 = (bi1 + ci - 1) / ci, ncbj = (nbj + cj - 1) / cj;
+        // Rasterised in supertiles of 1024 x 1024 similarities so concurrently running CTAs touch few
+        // distinct row blocks.
+        const int SUP_I = 8 / ci, SUP_J = 1024 / BN;
+        const int cbi0 = bi0 / ci, cbi1 = (bi1 + ci - 1) / ci;
         std::vector<int2> tiles;
-        auto needed = [&](int cbi, int cbj) {
-            // mirror mode keeps a cluster tile iff it holds a pair (i, j) with j >= i; a symmetric slab
+        auto needed = [&](int cbi, int bj) {
+            // mirror mode keeps a tile iff it holds a pair (i, j) with j >= i; a symmetric slab
             // (col_begin > 0) needs nothing left of its first row
-            if (!cosums && (int64_t)(cbj * cj + cj) * BN <= h->col_begin) return false;
-            return !mirror || (int64_t)(cbj * cj + cj) * BN > (int64_t)(cbi * ci) * BM;
+            if (!cosums && (int64_t)(bj + 1) * BN <= h->col_begin) return false;
+            return !mirror || (int64_t)(bj + 1) * BN > (int64_t)(cbi * ci) * BM;
         };
         for (int sbi = cbi0; sbi < cbi1; sbi += SUP_I)
-            for (int sbj = 0; sbj < ncbj; sbj += SUP_J)
+            for (int sbj = 0; sbj < nbj; sbj += SUP_J)
                 for (int cbi = sbi; cbi < sbi + SUP_I && cbi < cbi1; cbi++)
-                    for (int cbj = sbj; cbj < sbj + SUP_J && cbj < ncbj; cbj++)
-                        if (needed(cbi, cbj)) tiles.push_back(make_int2(cbi, cbj));
-        const size_t bytes = tiles.size() * sizeof(int2);
-        if (bytes > h->tile_buf_bytes) {
-            RS_CUDA(cudaStreamSynchronize(h->stream));
-            if (h->tile_buf) cudaFree(h->tile_buf);
-            h->tile_buf = nullptr;
-            h->tile_buf_bytes = 0;
-            RS_CUDA(cudaMalloc(&h->tile_buf, bytes + 256));
-            h->tile_buf_bytes = bytes + 256;
-        }
-        if (bytes) {
-            RS_CUDA(cudaMemcpyAsync(h->tile_buf, tiles.data(), bytes, cudaMemcpyHostToDevice, h->stream));
-            RS_CUDA(cudaStreamSynchronize(h->stream));  // `tiles` is a pageable temporary
-        }
+                    for (int bj = sbj; bj < sbj + SUP_J && bj < nbj; bj++)
+                        if (needed(cbi, bj)) tiles.push_back(make_int2(cbi, bj));
+        RS_TRY(upload_tiles(h, tiles, &h->tile_buf, &h->tile_buf_bytes));
         memcpy(h->tile_key, key, sizeof(key));
         h->tile_count = (int32_t)tiles.size();
     }
@@ -1241,7 +1132,6 @@ int32_t rs_sim_tensor_launch(rs_knn *h, int32_t *d_cosums, int64_t cos_row0, int
     TcArgs a{};
     a.tiles = reinterpret_cast<const int2 *>(h->tile_buf);
     a.num_tiles = h->tile_count;
-    a.k_blocks = (int32_t)(h->tc_kpad / BK);
     a.n_left = h->n_left;
     a.row_begin = rb;
     a.row_end = re;
@@ -1253,21 +1143,14 @@ int32_t rs_sim_tensor_launch(rs_knn *h, int32_t *d_cosums, int64_t cos_row0, int
     a.cosums = d_cosums;
     a.cos_row0 = cos_row0;
     a.cos_nrows = cos_nrows;
-    if (const char *e = getenv("RS_KNN_TC_DEBUG")) a.debug = atoi(e);
-    // K-lockstep throttle: only worth it when a row block does not fit in L2 many times over
-    a.progress = reinterpret_cast<unsigned long long *>(h->d_flags + 4);
-    a.sync_chunk = (a.k_blocks >= 256 && h->tile_count > 148) ? 32 : 0;
-    a.sync_slack = 1;
-    a.sync_timeout = 40000;   // clocks (~20 us): a hint, never a dependence
-    if (const char *e = getenv("RS_KNN_TC_SYNC")) sscanf(e, "%d,%d,%d", &a.sync_chunk, &a.sync_slack, &a.sync_timeout);
-    if (a.sync_chunk > 0) RS_CUDA(cudaMemsetAsync(a.progress, 0, 8, h->stream));
     int32_t rc;
-    if (use_pair) rc = mode == TC_COSINE ? launch_pair<TC_COSINE>(h, a)
-                       : mode == TC_MSD ? launch_pair<TC_MSD>(h, a) : launch_pair<TC_SLOPE>(h, a);
-    else if (ci == 1 && cj == 1) rc = launch_shape<1, 1>(h, a, cosums);
-    else if (ci == 1 && cj == 2) rc = launch_shape<1, 2>(h, a, cosums);
-    else if (ci == 2 && cj == 1) rc = launch_shape<2, 1>(h, a, cosums);
-    else rc = launch_shape<2, 2>(h, a, cosums);
+    switch (mode) {
+    case TC_COSINE: rc = use_pair ? launch_pair<TC_COSINE>(h, a) : launch_single<TC_COSINE>(h, a); break;
+    case TC_MSD: rc = use_pair ? launch_pair<TC_MSD>(h, a) : launch_single<TC_MSD>(h, a); break;
+    case TC_SLOPE: rc = use_pair ? launch_pair<TC_SLOPE>(h, a) : launch_single<TC_SLOPE>(h, a); break;
+    case TC_PEARSON: rc = launch_single<TC_PEARSON>(h, a); break;
+    default: rc = launch_single<TC_COSUMS>(h, a); break;   // TC_COSUMS
+    }
     RS_TRY(rc);
     if (!cosums) h->prof.sim_launches++;
     h->prof.total_launches++;

@@ -241,9 +241,7 @@ def _path(est):
     return {v: k for k, v in rs.core.RS_SIM_PATH.items()}[est.Profile()["sim_path_used"]]
 
 
-VARIANTS = {"single": {"RS_KNN_TC_PAIR": "0", "RS_KNN_TC_CLUSTER": "1x1"},
-            "cluster2x1": {"RS_KNN_TC_PAIR": "0", "RS_KNN_TC_CLUSTER": "2x1"},
-            "cluster1x2": {"RS_KNN_TC_PAIR": "0", "RS_KNN_TC_CLUSTER": "1x2"},
+VARIANTS = {"single": {"RS_KNN_TC_PAIR": "0"},
             "pair": {"RS_KNN_TC_PAIR": "1"}}
 
 

@@ -42,11 +42,9 @@ def test_cosums_bit_exact(ml100k, user_based):
                 assert np.array_equal(got[r, c].astype(np.int64), want), (row0 + r, int(c))
 
 
-# kernel variants: the single-CTA kernel (small problems), 2x1 / 1x2 multicast clusters, and the
-# cta_group::2 CTA-pair kernel (the default on large Cosine / MSD problems) — forced here on ml-100k
-VARIANTS = {"single": {"RS_KNN_TC_PAIR": "0", "RS_KNN_TC_CLUSTER": "1x1"},
-            "cluster2x1": {"RS_KNN_TC_PAIR": "0", "RS_KNN_TC_CLUSTER": "2x1"},
-            "cluster1x2": {"RS_KNN_TC_PAIR": "0", "RS_KNN_TC_CLUSTER": "1x2"},
+# kernel variants: the single-CTA kernel (small problems) and the cta_group::2 CTA-pair kernel (the default on
+# large Cosine / MSD problems) — forced here on ml-100k
+VARIANTS = {"single": {"RS_KNN_TC_PAIR": "0"},
             "pair": {"RS_KNN_TC_PAIR": "1"}}
 
 

@@ -29,8 +29,7 @@ def same(a, b):
 
 
 cases = [("msd", "basic", True, {"simPath": "tensor"}, {"RS_KNN_TC_PAIR": "1"}),
-         ("cosine", "basic", False, {"simPath": "tensor"}, {"RS_KNN_TC_PAIR": "0", "RS_KNN_TC_CLUSTER": "2x1"}),
-         ("cosine", "basic", False, {"simPath": "tensor"}, {"RS_KNN_TC_PAIR": "0", "RS_KNN_TC_CLUSTER": "1x1"}),
+         ("cosine", "basic", False, {"simPath": "tensor"}, {"RS_KNN_TC_PAIR": "0"}),
          ("pearson", "centered", False, {}, {}),
          ("msd", "zscore", True, {"simPath": "stream"}, {"RS_KNN_STREAM_JC": "256"}),
          ("pearson_baseline", "baseline", False, {"baseline": "als", "shrinkage": 50.0}, {})]
