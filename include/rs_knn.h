@@ -332,6 +332,36 @@ int32_t rs_knn_update(rs_knn *h, const int32_t *left, const int32_t *right, cons
                       int32_t n_left, int32_t n_right, double global_mean);
 int32_t rs_knn_update_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
                              int64_t nnz, int32_t n_left, int32_t n_right, double global_mean);
+/* REMOVING OR CHANGING RATINGS OF A FITTED MODEL (an extension, the other half of rs_knn_update).  The pairs
+ * (left[i], right[i]) are inner-id pairs the model holds.  rs_knn_remove drops them: the remaining ratings keep their
+ * relative dataset order.  rs_knn_change gives pair i the rating rating[i] at its place in the dataset order (the same
+ * value is allowed).  Afterwards the model is, bit for bit, what rs_knn_fit returns for the edited ratings in the edited
+ * dataset order with the SAME n_left x n_right and GlobalMean global_mean: matrix, means, stddevs, Predict,
+ * rs_knn_predict_neighbors, rs_knn_topk, score rows, recommendation lists, fold-in (_given) and rs_knn_cosums.  Inner
+ * ids are never renumbered or dropped: an id left without ratings keeps the empty row a Fit gives it (NaN everywhere;
+ * Predict falls back to GlobalMean).  Only the similarity rows (and columns) of the left ids the pairs name are
+ * recomputed, as in rs_knn_update.  n may be 0 (a new GlobalMean only).  Host pointers are consumed when the call
+ * returns; the _device variants read their arrays on the handle's stream.  The call returns once the pairs are
+ * validated and the work is queued.
+ * Refused before anything of the model is written, leaving it exactly as it was:
+ *   RS_ERR_INVALID     the handle is not fitted, an id outside [0, n_left) x [0, n_right), a pair the model does not
+ *                      hold, a null pointer with n > 0, a removal that would leave no rating (rs_knn_fit refuses
+ *                      nnz = 0);
+ *   RS_ERR_DUPLICATE   a pair named twice in one call;
+ *   RS_ERR_UNSUPPORTED every model rs_knn_update refuses (RS_STORE_TOPK, row shards of both kinds, RS_SIM_SLOPE_ONE,
+ *                      RS_KNN_BASELINE, RS_SIM_PEARSON_BASELINE, Pearson in RS_PEARSON_SUMS mode); a NaN change; a
+ *                      change to a value outside the integers in [-11, 11] on a model fitted on that class;
+ *   RS_ERR_OOM         as rs_knn_update.
+ * The counts never change; rs_knn_profile's corated_triples stays the last Fit's, and the candidate bound of Predict
+ * (the longest right row) is not lowered.  Memory as rs_knn_update: the edited arrays go to the same two blocks per
+ * array.  To find a pair's place in the dataset order, a Fit that keeps the dataset-order values (non-integer ratings,
+ * RS_KNN_ZSCORE) also keeps their right ids, 4 bytes per rating. */
+int32_t rs_knn_remove(rs_knn *h, const int32_t *left, const int32_t *right, int64_t n, double global_mean);
+int32_t rs_knn_remove_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, int64_t n, double global_mean);
+int32_t rs_knn_change(rs_knn *h, const int32_t *left, const int32_t *right, const double *rating, int64_t n,
+                      double global_mean);
+int32_t rs_knn_change_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
+                             int64_t n, double global_mean);
 /* ADDING RATINGS TO A CYCLIC ROW SHARD (after rs_knn_mirror).  rs_knn_update and rs_knn_update_device refuse every row
  * shard; this is their form for cyclic shards.  Every shard of the model is called with the same ratings, counts and
  * global_mean, and no data moves between them: each merges the ratings into its copies of both CSRs and of every row's

@@ -34,6 +34,7 @@ _LIB_KNN = Path(os.environ.get("RS_KNN_LIB", _PKG / "librs_knn_b200.so"))   # RS
 _LIB_HOST = _PKG / "librs_host.so"
 
 RS_OK = 0
+RS_ERR_INVALID, RS_ERR_DUPLICATE = -1, -5
 newID = -1  # core/data.go:129
 
 # enum values of include/rs_knn.h
@@ -72,7 +73,8 @@ ABI_SYMBOLS = [
     "rs_knn_host_free", "rs_knn_score_all", "rs_knn_score_all_device", "rs_knn_recommend", "rs_knn_recommend_device",
     "rs_knn_score_all_sharded_device", "rs_knn_recommend_sharded_device", "rs_knn_score_all_given",
     "rs_knn_score_all_given_device", "rs_knn_recommend_given", "rs_knn_recommend_given_device", "rs_knn_update",
-    "rs_knn_update_device", "rs_knn_update_sharded_device",
+    "rs_knn_update_device", "rs_knn_update_sharded_device", "rs_knn_remove", "rs_knn_remove_device", "rs_knn_change",
+    "rs_knn_change_device",
 ]
 
 _knn_lib = None
@@ -136,6 +138,10 @@ def knn_lib():
     L.rs_knn_update.argtypes = [vp, vp, vp, vp, i64, i32, i32, dbl]
     L.rs_knn_update_device.argtypes = [vp, vp, vp, vp, i64, i32, i32, dbl]
     L.rs_knn_update_sharded_device.argtypes = [vp, vp, vp, vp, i64, i32, i32, dbl]
+    L.rs_knn_remove.argtypes = [vp, vp, vp, i64, dbl]
+    L.rs_knn_remove_device.argtypes = [vp, vp, vp, i64, dbl]
+    L.rs_knn_change.argtypes = [vp, vp, vp, vp, i64, dbl]
+    L.rs_knn_change_device.argtypes = [vp, vp, vp, vp, i64, dbl]
     _knn_lib = L
     return L
 
@@ -368,15 +374,49 @@ class TrainSet(DataSet):
         # core/data.go:137-151 — inner id = order of first appearance
         self.innerUsers, self.UserCount = _inner_ids(self.Users)
         self.innerItems, self.ItemCount = _inner_ids(self.Items)
+        self._uraw = self._iraw = None
         self._umap = None
         self._imap = None
         self._ulook = None
         self._ilook = None
 
+    @classmethod
+    def _of(cls, rows: DataSet, inner_users, inner_items, user_count, item_count, uraw, iraw):
+        """A TrainSet of `rows` under given inner ids and counts.  uraw / iraw: the raw id of every inner id, needed
+        once an id may have no row left (None: every id has one)."""
+        ts = cls.__new__(cls)
+        DataSet.__init__(ts, rows.Users, rows.Items, rows.Ratings)
+        ts.GlobalMean = _global_mean(ts.Ratings)
+        ts.innerUsers = np.ascontiguousarray(inner_users, dtype=np.int32)
+        ts.innerItems = np.ascontiguousarray(inner_items, dtype=np.int32)
+        ts.UserCount, ts.ItemCount = int(user_count), int(item_count)
+        ts._uraw, ts._iraw = uraw, iraw
+        ts._umap = ts._imap = ts._ulook = ts._ilook = None
+        return ts
+
+    def _known(self):
+        """(raw ids, inner ids) of every user and of every item the set numbers: its rows' own, or after a removal the
+        raw id of each inner id (an id whose rows are all removed keeps its number)."""
+        if self._uraw is None:
+            return (self.Users, self.innerUsers), (self.Items, self.innerItems)
+        return ((self._uraw, np.arange(self.UserCount, dtype=np.int32)),
+                (self._iraw, np.arange(self.ItemCount, dtype=np.int32)))
+
+    def _raw_ids(self):
+        """The raw id of every inner id, users and items."""
+        if self._uraw is not None:
+            return self._uraw, self._iraw
+        uraw = np.zeros(self.UserCount, dtype=np.int64)
+        iraw = np.zeros(self.ItemCount, dtype=np.int64)
+        uraw[self.innerUsers] = self.Users
+        iraw[self.innerItems] = self.Items
+        return uraw, iraw
+
     def _maps(self):
         if self._umap is None:
-            self._umap = dict(zip(self.Users.tolist(), self.innerUsers.tolist()))
-            self._imap = dict(zip(self.Items.tolist(), self.innerItems.tolist()))
+            (ur, ui), (ir, ii) = self._known()
+            self._umap = dict(zip(ur.tolist(), ui.tolist()))
+            self._imap = dict(zip(ir.tolist(), ii.tolist()))
 
     def ConvertUserID(self, userID):
         self._maps()
@@ -389,23 +429,75 @@ class TrainSet(DataSet):
     def convert_users(self, raw, out=None):
         """Vectorised ConvertUserID for a batch (newID = -1 for unseen ids)."""
         if self._ulook is None:
-            self._ulook = _lookup_table(self.Users, self.innerUsers)
+            self._ulook = _lookup_table(*self._known()[0])
         return _convert(self._ulook, raw, out)
 
     def convert_items(self, raw, out=None):
         if self._ilook is None:
-            self._ilook = _lookup_table(self.Items, self.innerItems)
+            self._ilook = _lookup_table(*self._known()[1])
         return _convert(self._ilook, raw, out)
 
     def RatingRange(self):
         return float(self.Ratings.min()), float(self.Ratings.max())
 
     def Extend(self, rowSet: DataSet) -> "TrainSet":
-        """The TrainSet of this one's rows followed by `rowSet`'s: NewTrainSet of the concatenation, so the inner ids
-        continue the order of first appearance (known ids keep theirs, new ones come after) and GlobalMean is that
-        TrainSet's, bit for bit."""
-        return TrainSet(DataSet(np.concatenate([self.Users, rowSet.Users]), np.concatenate([self.Items, rowSet.Items]),
-                                np.concatenate([self.Ratings, rowSet.Ratings])))
+        """The TrainSet of this one's rows followed by `rowSet`'s.  The inner ids continue this set's numbering: known
+        ids keep theirs (also an id whose rows were all removed), new ones are numbered from UserCount / ItemCount in
+        order of first appearance in `rowSet`.  GlobalMean is that of the concatenated ratings.  For a set that was
+        never edited this is NewTrainSet of the concatenation, bit for bit."""
+        iu, user_count, new_users = _continue_ids(self.convert_users(rowSet.Users), rowSet.Users, self.UserCount)
+        ii, item_count, new_items = _continue_ids(self.convert_items(rowSet.Items), rowSet.Items, self.ItemCount)
+        rows = DataSet(np.concatenate([self.Users, rowSet.Users]), np.concatenate([self.Items, rowSet.Items]),
+                       np.concatenate([self.Ratings, rowSet.Ratings]))
+        uraw = iraw = None
+        if self._uraw is not None:
+            uraw, iraw = np.concatenate([self._uraw, new_users]), np.concatenate([self._iraw, new_items])
+        return TrainSet._of(rows, np.concatenate([self.innerUsers, iu]), np.concatenate([self.innerItems, ii]),
+                            user_count, item_count, uraw, iraw)
+
+    def _rows_of(self, userIDs, itemIDs, who):
+        """The row of each (raw user, raw item) pair, refused as the device refuses an edit: RsError RS_ERR_INVALID
+        for an unknown id or a pair the set does not hold, RS_ERR_DUPLICATE for a pair named twice."""
+        users = np.ascontiguousarray(userIDs, dtype=np.int64)
+        items = np.ascontiguousarray(itemIDs, dtype=np.int64)
+        if len(users) != len(items):
+            raise ValueError(f"{who}: {len(users)} users and {len(items)} items")
+        iu, ii = self.convert_users(users), self.convert_items(items)
+        if (iu == newID).any() or (ii == newID).any():
+            raise RsError(RS_ERR_INVALID, f"{who}: a raw user or item id the set does not know")
+        want = iu.astype(np.int64) * self.ItemCount + ii
+        if len(np.unique(want)) < len(want):
+            raise RsError(RS_ERR_DUPLICATE, f"{who}: a (user, item) pair named twice")
+        have = self.innerUsers.astype(np.int64) * self.ItemCount + self.innerItems
+        order = np.argsort(have, kind="stable")
+        pos = np.clip(np.searchsorted(have[order], want), 0, max(len(have) - 1, 0))
+        if len(want) and (len(have) == 0 or (have[order][pos] != want).any()):
+            raise RsError(RS_ERR_INVALID, f"{who}: a (user, item) pair the set does not hold")
+        return order[pos]
+
+    def Remove(self, userIDs, itemIDs) -> "TrainSet":
+        """This set without the rows of the (raw user, raw item) pairs; the remaining rows keep their order.  The inner
+        ids and counts stay as they are, and an id whose rows are all removed still converts to its inner id.
+        GlobalMean is that of the remaining ratings.  Refused (RsError) for an unknown id, a pair the set does not hold
+        or names twice, and a removal that would leave no row."""
+        rows = self._rows_of(userIDs, itemIDs, "Remove")
+        keep = np.ones(self.Length(), dtype=bool)
+        keep[rows] = False
+        if not keep.any():
+            raise RsError(RS_ERR_INVALID, "Remove: the removal would leave no rating")
+        uraw, iraw = self._raw_ids()
+        return TrainSet._of(self.SubSet(keep), self.innerUsers[keep], self.innerItems[keep], self.UserCount,
+                            self.ItemCount, uraw, iraw)
+
+    def Change(self, rowSet: DataSet) -> "TrainSet":
+        """This set with the rating of each (raw user, raw item) pair of `rowSet` replaced by its rating there, at the
+        row's place; ids, counts and the order of the rows stay as they are.  GlobalMean is that of the changed
+        ratings.  Refused (RsError) for an unknown id and a pair the set does not hold or names twice."""
+        rows = self._rows_of(rowSet.Users, rowSet.Items, "Change")
+        ratings = self.Ratings.copy()
+        ratings[rows] = rowSet.Ratings
+        return TrainSet._of(DataSet(self.Users, self.Items, ratings), self.innerUsers, self.innerItems, self.UserCount,
+                            self.ItemCount, self._uraw, self._iraw)
 
 
 class _HostBlock:
@@ -472,6 +564,22 @@ def _convert(table, raw, out=None):
     pos = np.clip(np.searchsorted(uniq, raw), 0, len(uniq) - 1)
     out[:] = np.where(uniq[pos] == raw, inner[pos], newID)
     return out
+
+
+def _continue_ids(inner, raw, count):
+    """Inner ids of `raw` given those a set knows (`inner`, newID where unknown) and its count: the unknown ones are
+    numbered from `count` in order of first appearance.  Returns the ids, the new count and the raw id of each new
+    inner id."""
+    inner = np.array(inner, dtype=np.int32)
+    unknown = inner == newID
+    if not unknown.any():
+        return inner, count, np.zeros(0, dtype=np.int64)
+    raw_new = np.ascontiguousarray(raw, dtype=np.int64)[unknown]
+    new_inner, n_new = _inner_ids(raw_new)
+    inner[unknown] = new_inner + count
+    first = np.zeros(n_new, dtype=np.int64)
+    first[new_inner] = raw_new
+    return inner, count + n_new, first
 
 
 def NewTrainSet(rowSet: DataSet) -> TrainSet:
@@ -667,6 +775,27 @@ class _Handle:
         _check(knn_lib().rs_knn_update_sharded_device(self.h, d_left, d_right, d_rating, nnz, n_left, n_right,
                                                       global_mean))
         self._after_fit(n_left, n_right)
+
+    def remove(self, left, right, global_mean):
+        """Drops (left, right) pairs the model holds: it becomes the Fit of the remaining ratings under the same ids and
+        counts, bit for bit (rs_knn_remove)."""
+        left = np.ascontiguousarray(left, dtype=np.int32)
+        right = np.ascontiguousarray(right, dtype=np.int32)
+        _check(knn_lib().rs_knn_remove(self.h, _ptr(left), _ptr(right), len(left), global_mean))
+
+    def remove_device(self, d_left, d_right, n, global_mean):
+        _check(knn_lib().rs_knn_remove_device(self.h, d_left, d_right, n, global_mean))
+
+    def change(self, left, right, rating, global_mean):
+        """Gives (left, right) pairs the model holds new ratings at their places: it becomes the Fit of the changed
+        ratings, bit for bit (rs_knn_change)."""
+        left = np.ascontiguousarray(left, dtype=np.int32)
+        right = np.ascontiguousarray(right, dtype=np.int32)
+        rating = np.ascontiguousarray(rating, dtype=np.float64)
+        _check(knn_lib().rs_knn_change(self.h, _ptr(left), _ptr(right), _ptr(rating), len(rating), global_mean))
+
+    def change_device(self, d_left, d_right, d_rating, n, global_mean):
+        _check(knn_lib().rs_knn_change_device(self.h, d_left, d_right, d_rating, n, global_mean))
 
     def predict_batch(self, left, right):
         left = np.ascontiguousarray(left, dtype=np.int32)
@@ -1002,6 +1131,36 @@ class KNN(Base):
         self.GlobalMean = data.GlobalMean
         self._after_fit()
 
+    def _edit_pairs(self, userIDs, itemIDs):
+        iu, ii = self.Data.convert_users(userIDs), self.Data.convert_items(itemIDs)
+        return (iu, ii) if self._userBased else (ii, iu)
+
+    def Remove(self, userIDs, itemIDs):
+        """Removes the ratings of the (raw user, raw item) pairs from the fitted model without a refit: the model
+        becomes the Fit of Data.Remove(userIDs, itemIDs) under the same inner ids and counts, bit for bit —
+        similarities, Means, StdDevs, GlobalMean, Predict and Recommend (rs_knn_remove; only the rows of the users
+        (items) the pairs name are recomputed).  An id whose ratings are all removed keeps its number and gets an empty
+        row.  Refused (RsError) before any device work for an unknown id or a pair the model does not hold or names
+        twice, and by the device for the models rs_knn_update refuses; Data, GlobalMean, Means and StdDevs change
+        only on success."""
+        data = self.Data.Remove(userIDs, itemIDs)
+        left, right = self._edit_pairs(userIDs, itemIDs)
+        self._h.remove(left, right, data.GlobalMean)
+        self.Data = data
+        self.GlobalMean = data.GlobalMean
+        self._after_fit()
+
+    def Change(self, rowSet: DataSet):
+        """Gives the (raw user, raw item) pairs of `rowSet` its ratings, each at its place in the data, without a
+        refit: the model becomes the Fit of Data.Change(rowSet), bit for bit (rs_knn_change).  Refused as Remove, and
+        by the device for a NaN rating or, on a model fitted on integer ratings in [-11, 11], a rating outside them."""
+        data = self.Data.Change(rowSet)
+        left, right = self._edit_pairs(rowSet.Users, rowSet.Items)
+        self._h.change(left, right, rowSet.Ratings, data.GlobalMean)
+        self.Data = data
+        self.GlobalMean = data.GlobalMean
+        self._after_fit()
+
     @property
     def Sims(self):
         """core/knn.go:21 — the dense N x N matrix, NaN = unset (copied from HBM on demand)."""
@@ -1102,8 +1261,7 @@ class KNN(Base):
 
     def _raw_items(self, ids):
         """Inner item ids -> raw item ids; -1 (an unused slot) -> newID."""
-        raw = np.empty(self.Data.ItemCount, dtype=np.int64)    # inner -> raw: the order of first appearance
-        raw[self.Data.innerItems] = self.Data.Items
+        raw = self.Data._raw_ids()[1]                          # inner -> raw, also for items without ratings
         return np.where(ids >= 0, raw[np.maximum(ids, 0)], newID)
 
     def Profile(self):

@@ -45,6 +45,7 @@ void free_fit_state(rs_knn *h) {
     h->l_ptr = h->r_ptr = nullptr;
     h->l_col = h->r_col = nullptr;
     h->l_val = h->r_val = h->ld_val = nullptr;
+    h->ld_col = nullptr;
     h->l_code = nullptr;
     h->means = h->stddevs = h->pmeans = h->left_bias = h->right_bias = nullptr;
     h->r_dev = nullptr;
@@ -162,7 +163,7 @@ int32_t init_handle(rs_knn *h) {
 extern "C" {
 
 const char *rs_last_error(void) { return g_err; }
-int32_t rs_knn_abi_version(void) { return 6; }
+int32_t rs_knn_abi_version(void) { return 7; }
 
 int32_t rs_knn_device_count(void) {
     int n = 0;
@@ -451,10 +452,10 @@ int32_t rs_knn_fit(rs_knn *h, const int32_t *left, const int32_t *right, const d
 
 // Every check of rs_knn_update, in the order they fire: the handle is fitted; its model is one that an update can
 // extend exactly (a matrix of all rows — sharded: a mirrored cyclic row shard —, no Slope One, no bias of a global
-// fit, the exact Pearson replay); the counts do not shrink; the pointers are there when there are ratings.  The
-// ratings themselves are checked on the device.
+// fit, the exact Pearson replay); the counts do not shrink; the pointers are there when there are ratings (`rated`:
+// a rating pointer among them).  The ratings themselves are checked on the device.
 static int32_t check_update(rs_knn *h, const char *who, bool sharded, const int32_t *left, const int32_t *right,
-                            const double *rating, int64_t nnz, int32_t n_left, int32_t n_right) {
+                            const double *rating, int64_t nnz, int32_t n_left, int32_t n_right, bool rated = true) {
     if (!h->fitted) {
         rs_set_error("%s: Fit has not been called", who);
         return RS_ERR_INVALID;
@@ -497,7 +498,7 @@ static int32_t check_update(rs_knn *h, const char *who, bool sharded, const int3
                      (long long)nnz, h->n_left, h->n_right);
         return RS_ERR_INVALID;
     }
-    if (nnz > 0 && (!left || !right || !rating)) {
+    if (nnz > 0 && (!left || !right || (rated && !rating))) {
         rs_set_error("%s: null argument", who);
         return RS_ERR_INVALID;
     }
@@ -522,22 +523,75 @@ int32_t rs_knn_update_sharded_device(rs_knn *h, const int32_t *d_left, const int
     return rs_update_run(h, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean);
 }
 
+// The host ratings of an update or an edit, staged in the scratch slots of rs_knn_fit's inputs (rating null: a
+// removal).  The update and the edits read their inputs before their validation read-back: the host arrays are
+// consumed when they return.
+static int32_t stage_ratings(rs_knn *h, const int32_t *left, const int32_t *right, const double *rating, int64_t n,
+                             const int32_t **d_left, const int32_t **d_right, const double **d_rating) {
+    void *dl = nullptr, *dr = nullptr, *dv = nullptr;
+    if (n > 0) {
+        RS_TRY(rs_scratch_get(h, RS_SCR_FIT_LEFT, (size_t)n * 4, &dl));
+        RS_TRY(rs_scratch_get(h, RS_SCR_FIT_RIGHT, (size_t)n * 4, &dr));
+        RS_CUDA(cudaMemcpyAsync(dl, left, (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
+        RS_CUDA(cudaMemcpyAsync(dr, right, (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
+        if (rating) {
+            RS_TRY(rs_scratch_get(h, RS_SCR_FIT_RATING, (size_t)n * 8, &dv));
+            RS_CUDA(cudaMemcpyAsync(dv, rating, (size_t)n * 8, cudaMemcpyHostToDevice, h->stream));
+        }
+    }
+    *d_left = static_cast<const int32_t *>(dl);
+    *d_right = static_cast<const int32_t *>(dr);
+    *d_rating = static_cast<const double *>(dv);
+    return RS_OK;
+}
+
 int32_t rs_knn_update(rs_knn *h, const int32_t *left, const int32_t *right, const double *rating, int64_t nnz,
                       int32_t n_left, int32_t n_right, double global_mean) {
     RS_ENTER(h);
     RS_TRY(check_update(h, "rs_knn_update", false, left, right, rating, nnz, n_left, n_right));
-    void *d_left = nullptr, *d_right = nullptr, *d_rating = nullptr;
-    if (nnz > 0) {
-        RS_TRY(rs_scratch_get(h, RS_SCR_FIT_LEFT, (size_t)nnz * 4, &d_left));
-        RS_TRY(rs_scratch_get(h, RS_SCR_FIT_RIGHT, (size_t)nnz * 4, &d_right));
-        RS_TRY(rs_scratch_get(h, RS_SCR_FIT_RATING, (size_t)nnz * 8, &d_rating));
-        RS_CUDA(cudaMemcpyAsync(d_left, left, (size_t)nnz * 4, cudaMemcpyHostToDevice, h->stream));
-        RS_CUDA(cudaMemcpyAsync(d_right, right, (size_t)nnz * 4, cudaMemcpyHostToDevice, h->stream));
-        RS_CUDA(cudaMemcpyAsync(d_rating, rating, (size_t)nnz * 8, cudaMemcpyHostToDevice, h->stream));
-    }
-    // the update reads its inputs before its validation read-back: they are consumed when it returns
-    return rs_update_run(h, (const int32_t *)d_left, (const int32_t *)d_right, (const double *)d_rating, nnz, n_left,
-                         n_right, global_mean);
+    const int32_t *d_left, *d_right;
+    const double *d_rating;
+    RS_TRY(stage_ratings(h, left, right, rating, nnz, &d_left, &d_right, &d_rating));
+    return rs_update_run(h, d_left, d_right, d_rating, nnz, n_left, n_right, global_mean);
+}
+
+// Every check of rs_knn_remove / rs_knn_change: rs_knn_update's at the fitted counts (an edit is refused on every model
+// an update is), with a rating pointer for a change only.  The pairs themselves are checked on the device.
+static int32_t check_edit(rs_knn *h, const char *who, bool remove, const int32_t *left, const int32_t *right,
+                          const double *rating, int64_t n) {
+    return check_update(h, who, false, left, right, rating, n, h->n_left, h->n_right, !remove);
+}
+
+int32_t rs_knn_remove(rs_knn *h, const int32_t *left, const int32_t *right, int64_t n, double global_mean) {
+    RS_ENTER(h);
+    RS_TRY(check_edit(h, "rs_knn_remove", true, left, right, nullptr, n));
+    const int32_t *d_left, *d_right;
+    const double *d_rating;
+    RS_TRY(stage_ratings(h, left, right, nullptr, n, &d_left, &d_right, &d_rating));
+    return rs_edit_run(h, true, d_left, d_right, nullptr, n, global_mean);
+}
+
+int32_t rs_knn_remove_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, int64_t n, double global_mean) {
+    RS_ENTER(h);
+    RS_TRY(check_edit(h, "rs_knn_remove", true, d_left, d_right, nullptr, n));
+    return rs_edit_run(h, true, d_left, d_right, nullptr, n, global_mean);
+}
+
+int32_t rs_knn_change(rs_knn *h, const int32_t *left, const int32_t *right, const double *rating, int64_t n,
+                      double global_mean) {
+    RS_ENTER(h);
+    RS_TRY(check_edit(h, "rs_knn_change", false, left, right, rating, n));
+    const int32_t *d_left, *d_right;
+    const double *d_rating;
+    RS_TRY(stage_ratings(h, left, right, rating, n, &d_left, &d_right, &d_rating));
+    return rs_edit_run(h, false, d_left, d_right, d_rating, n, global_mean);
+}
+
+int32_t rs_knn_change_device(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
+                             int64_t n, double global_mean) {
+    RS_ENTER(h);
+    RS_TRY(check_edit(h, "rs_knn_change", false, d_left, d_right, d_rating, n));
+    return rs_edit_run(h, false, d_left, d_right, d_rating, n, global_mean);
 }
 
 static int32_t require_matrix(rs_knn *h, const char *who) {

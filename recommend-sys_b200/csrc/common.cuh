@@ -71,10 +71,10 @@ inline int64_t rs_cyc_rows(int64_t n, int count, int index) {
     return rows;
 }
 
-// The model arrays rs_knn_update rewrites (update.cu); rs_knn::upd holds their blocks.
+// The model arrays rs_knn_update, rs_knn_remove and rs_knn_change rewrite (update.cu); rs_knn::upd holds their blocks.
 enum rs_upd_array {
     RS_UPD_L_PTR, RS_UPD_L_COL, RS_UPD_L_VAL, RS_UPD_L_CODE, RS_UPD_LD_VAL, RS_UPD_R_PTR, RS_UPD_R_COL, RS_UPD_R_VAL,
-    RS_UPD_MEANS, RS_UPD_STDDEVS, RS_UPD_PMEANS, RS_UPD_ROW_CNT, RS_UPD_ROW_SUM, RS_UPD_ARRAYS
+    RS_UPD_MEANS, RS_UPD_STDDEVS, RS_UPD_PMEANS, RS_UPD_ROW_CNT, RS_UPD_ROW_SUM, RS_UPD_LD_COL, RS_UPD_ARRAYS
 };
 
 struct rs_knn {
@@ -135,6 +135,7 @@ struct rs_knn {
     double *l_val = nullptr;
     uint8_t *l_code = nullptr;
     double *ld_val = nullptr;  // left rows in DATASET order (means / std accumulate in it)
+    int32_t *ld_col = nullptr; // their right ids, where Fit keeps ld_val (an edit finds its entry in that order by id)
     // CSR of the right rows, entries ascending by left id (Predict candidates)
     int64_t *r_ptr = nullptr;
     int32_t *r_col = nullptr;
@@ -194,7 +195,7 @@ struct rs_knn {
     double *topk_sim = nullptr;
 
     int32_t *d_flags = nullptr;  // small device scratch for validation flags
-    // rs_knn_update: the model arrays an update rewrote live in blocks of their own (the arena only grows until the
+    // rs_knn_update (and the edits): the model arrays an update rewrote live in blocks of their own (the arena only grows until the
     // next Fit), two per array: the model's, p[cur], and the spare the next update merges into.  cur = -1 while
     // the model's array is the Fit's, in the arena.
     struct UpdArray { void *p[2] = {nullptr, nullptr}; size_t bytes[2] = {0, 0}; int cur = -1; };
@@ -299,7 +300,7 @@ int32_t rs_row_stats_launch(rs_knn *h, const int64_t *ptr, const double *ld_val,
                             int want_std, double *means, double *stddevs, double *pmeans);
 int32_t rs_prep_stats(rs_knn *h);
 // Kernels of the CSR build that rs_knn_update runs on the added ratings as Fit runs them on all ratings.
-enum rs_prep_flag { FLAG_BAD_ID = 1, FLAG_NOT_INT8 = 2, FLAG_DUP = 4, FLAG_NAN = 8 };
+enum rs_prep_flag { FLAG_BAD_ID = 1, FLAG_NOT_INT8 = 2, FLAG_DUP = 4, FLAG_NAN = 8, FLAG_MISSING = 16 };
 __global__ void ptr_from_sorted_kernel(const int32_t *__restrict__ keys, int64_t nnz, int32_t n_rows,
                                        int64_t *__restrict__ ptr);
 __global__ void gather_keys_kernel(const int32_t *__restrict__ src, const int32_t *__restrict__ perm, int64_t n,
@@ -377,6 +378,9 @@ int32_t rs_given_sims_launch(rs_knn *h, const int64_t *ptr, const int32_t *ids, 
 // ---- update.cu ----
 int32_t rs_update_run(rs_knn *h, const int32_t *d_left, const int32_t *d_right, const double *d_rating, int64_t nnz,
                       int32_t n_left, int32_t n_right, double global_mean);
+// rs_knn_remove (remove) / rs_knn_change: the pairs d_left[e], d_right[e] the model holds, dropped or given d_rating[e]
+int32_t rs_edit_run(rs_knn *h, bool remove, const int32_t *d_left, const int32_t *d_right, const double *d_rating,
+                    int64_t nd, double global_mean);
 void rs_update_release(rs_knn *h);
 
 // First position in [lo, hi) of an ascending id array whose id is >= v: the searches of given.cu and update.cu.

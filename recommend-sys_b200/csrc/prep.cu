@@ -554,8 +554,13 @@ int32_t rs_prep_build(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
     gather_csr_kernel<<<blocks_for(nnz), T, 0, st>>>(perm_lr, d_right, d_rating, nnz, h->l_col, h->l_val);
     gather_csr_kernel<<<blocks_for(nnz), T, 0, st>>>(perm_rl, d_left, d_rating, nnz, h->r_col, h->r_val);
     dup_check_kernel<<<blocks_for(nnz), T, 0, st>>>(keys_b, h->r_col, nnz, h->d_flags);   // keys_b: the right ids, sorted
-    if (need_dataset_order) gather_val_kernel<<<blocks_for(nnz), T, 0, st>>>(perm_l, d_rating, nnz, h->ld_val);
-    h->prof.total_launches += need_dataset_order ? 4 : 3;
+    if (need_dataset_order) {
+        // and their right ids, by which rs_knn_remove / rs_knn_change find a pair's place in that order
+        RS_TRY(rs_alloc(h, &h->ld_col, nnz));
+        gather_val_kernel<<<blocks_for(nnz), T, 0, st>>>(perm_l, d_rating, nnz, h->ld_val);
+        gather_keys_kernel<<<blocks_for(nnz), T, 0, st>>>(d_right, perm_l, nnz, h->ld_col);
+    }
+    h->prof.total_launches += need_dataset_order ? 5 : 3;
 
     // byte codes (rating + 12) of the integer class: operands of the tensor path and of the exact
     // integer row sums.  Any other float64 rating set runs on the stream path, which reads the

@@ -145,6 +145,23 @@ func (d *deviceKNN) update(left, right []int32, rating []float64, nLeft, nRight 
 	runtime.KeepAlive(rating)
 }
 
+// remove drops (left, right) pairs (inner ids) the model holds: it becomes the Fit of the remaining ratings under the
+// same ids and counts (rs_knn_remove).
+func (d *deviceKNN) remove(left, right []int32, globalMean float64) {
+	check(C.rs_knn_remove(d.h, i32(left), i32(right), C.int64_t(len(left)), C.double(globalMean)))
+	runtime.KeepAlive(left)
+	runtime.KeepAlive(right)
+}
+
+// change gives (left, right) pairs (inner ids) the model holds new ratings at their places: it becomes the Fit of the
+// changed ratings (rs_knn_change).
+func (d *deviceKNN) change(left, right []int32, rating []float64, globalMean float64) {
+	check(C.rs_knn_change(d.h, i32(left), i32(right), f64(rating), C.int64_t(len(rating)), C.double(globalMean)))
+	runtime.KeepAlive(left)
+	runtime.KeepAlive(right)
+	runtime.KeepAlive(rating)
+}
+
 // updateShardedDevice adds ratings to a mirrored cyclic row shard (rs_knn_update_sharded_device): every shard of the
 // model gets the same device arrays, counts and GlobalMean, and afterwards holds its rows of the Fit of the union.
 func (d *deviceKNN) updateShardedDevice(dLeft, dRight, dRating unsafe.Pointer, nnz int64, nLeft, nRight int,

@@ -83,14 +83,24 @@ struct TrainSet : DataSet {
     std::unordered_map<int64_t, int32_t> InnerUserIDs, InnerItemIDs;
     int ConvertUserID(int64_t u) const { auto it = InnerUserIDs.find(u); return it == InnerUserIDs.end() ? newID : it->second; }
     int ConvertItemID(int64_t i) const { auto it = InnerItemIDs.find(i); return it == InnerItemIDs.end() ? newID : it->second; }
+    // inner item id -> raw item id, for every item the maps number (also one whose ratings were all removed)
+    std::vector<int64_t> RawItems() const {
+        std::vector<int64_t> raw(ItemCount);
+        for (const auto &kv : InnerItemIDs) raw[kv.second] = kv.first;
+        return raw;
+    }
 };
+
+inline double MeanOf(const std::vector<double> &r) {   // stat.Mean, core/data.go:134
+    double sum = 0.0;
+    for (double x : r) sum += x;
+    return sum / (double)r.size();
+}
 
 inline TrainSet NewTrainSet(const DataSet &rowSet) {  // core/data.go:131-154
     TrainSet s;
     static_cast<DataSet &>(s) = rowSet;
-    double sum = 0.0;
-    for (double r : s.Ratings) sum += r;
-    s.GlobalMean = sum / (double)s.Ratings.size();  // stat.Mean, core/data.go:134
+    s.GlobalMean = MeanOf(s.Ratings);
     s.innerUsers.resize(s.Length());
     s.innerItems.resize(s.Length());
     s.UserCount = (int)rs_host_inner_ids(s.Users.data(), (int64_t)s.Length(), s.innerUsers.data());
@@ -102,14 +112,71 @@ inline TrainSet NewTrainSet(const DataSet &rowSet) {  // core/data.go:131-154
     return s;
 }
 
-// The TrainSet of t's rows followed by rowSet's: NewTrainSet of the concatenation (inner ids continue the order of
-// first appearance, GlobalMean is the concatenation's).
+// The TrainSet of t's rows followed by rowSet's.  The inner ids continue t's numbering: known ids keep theirs (also
+// one whose ratings were all removed), new ones follow UserCount / ItemCount in order of first appearance.  GlobalMean
+// is the concatenation's.  For a set never edited this is NewTrainSet of the concatenation.
 inline TrainSet Extend(const TrainSet &t, const DataSet &rowSet) {
-    DataSet d = t;
-    d.Users.insert(d.Users.end(), rowSet.Users.begin(), rowSet.Users.end());
-    d.Items.insert(d.Items.end(), rowSet.Items.begin(), rowSet.Items.end());
-    d.Ratings.insert(d.Ratings.end(), rowSet.Ratings.begin(), rowSet.Ratings.end());
-    return NewTrainSet(d);
+    TrainSet s = t;
+    for (size_t j = 0; j < rowSet.Length(); j++) {
+        const auto u = s.InnerUserIDs.emplace(rowSet.Users[j], s.UserCount);
+        if (u.second) s.UserCount++;
+        const auto i = s.InnerItemIDs.emplace(rowSet.Items[j], s.ItemCount);
+        if (i.second) s.ItemCount++;
+        s.Users.push_back(rowSet.Users[j]);
+        s.Items.push_back(rowSet.Items[j]);
+        s.Ratings.push_back(rowSet.Ratings[j]);
+        s.innerUsers.push_back(u.first->second);
+        s.innerItems.push_back(i.first->second);
+    }
+    s.GlobalMean = MeanOf(s.Ratings);
+    return s;
+}
+
+// The row of each (raw user, raw item) pair of t.  Refused as rs_knn_remove / rs_knn_change refuse: an unknown id, a
+// pair t does not hold, a pair named twice.
+inline std::vector<size_t> PairRows(const TrainSet &t, const std::vector<int64_t> &users,
+                                    const std::vector<int64_t> &items) {
+    std::unordered_map<int64_t, size_t> row;
+    for (size_t j = 0; j < t.Length(); j++)
+        row.emplace((int64_t)t.innerUsers[j] * t.ItemCount + t.innerItems[j], j);
+    std::vector<size_t> out;
+    std::unordered_map<int64_t, bool> seen;
+    for (size_t j = 0; j < users.size(); j++) {
+        const int iu = t.ConvertUserID(users[j]), ii = t.ConvertItemID(items[j]);
+        if (iu == newID || ii == newID) throw std::runtime_error("edit: a raw user or item id the set does not know");
+        const int64_t key = (int64_t)iu * t.ItemCount + ii;
+        const auto it = row.find(key);
+        if (it == row.end()) throw std::runtime_error("edit: a (user, item) pair the set does not hold");
+        if (!seen.emplace(key, true).second) throw std::runtime_error("edit: a (user, item) pair named twice");
+        out.push_back(it->second);
+    }
+    return out;
+}
+
+// t without the rows of the (raw user, raw item) pairs; the rest keep their order, and the ids, counts and maps stay
+// as they are (an id whose rows are all removed still converts).  GlobalMean is the remaining ratings'.
+inline TrainSet Remove(const TrainSet &t, const std::vector<int64_t> &users, const std::vector<int64_t> &items) {
+    std::vector<bool> drop(t.Length(), false);
+    for (size_t j : PairRows(t, users, items)) drop[j] = true;
+    TrainSet s = t;
+    s.Users.clear(); s.Items.clear(); s.Ratings.clear(); s.innerUsers.clear(); s.innerItems.clear();
+    for (size_t j = 0; j < t.Length(); j++) {
+        if (drop[j]) continue;
+        s.Users.push_back(t.Users[j]); s.Items.push_back(t.Items[j]); s.Ratings.push_back(t.Ratings[j]);
+        s.innerUsers.push_back(t.innerUsers[j]); s.innerItems.push_back(t.innerItems[j]);
+    }
+    if (s.Length() == 0) throw std::runtime_error("edit: the removal would leave no rating");
+    s.GlobalMean = MeanOf(s.Ratings);
+    return s;
+}
+
+// t with the rating of each (raw user, raw item) pair of rowSet replaced by rowSet's, at the row's place.
+inline TrainSet Change(const TrainSet &t, const DataSet &rowSet) {
+    const std::vector<size_t> rows = PairRows(t, rowSet.Users, rowSet.Items);
+    TrainSet s = t;
+    for (size_t j = 0; j < rows.size(); j++) s.Ratings[rows[j]] = rowSet.Ratings[j];
+    s.GlobalMean = MeanOf(s.Ratings);
+    return s;
 }
 
 // core/data.go:49-70 — the reference's permutation is unseeded (SURVEY.md hazard 3); here mt19937_64(seed).
@@ -260,6 +327,27 @@ struct KNN : Estimator {
         ReadStats();
     }
 
+    // Removes the ratings of the (raw user, raw item) pairs without a refit (rs_knn_remove): the model becomes the
+    // Fit of Remove(*Data, users, items) under the same inner ids and counts, bit for bit, and Data that TrainSet.
+    void Remove(const std::vector<int64_t> &users, const std::vector<int64_t> &items) {
+        auto t = std::make_shared<const TrainSet>(core::Remove(*Data, users, items));
+        std::vector<int32_t> left, right;
+        EditPairs(users, items, left, right);
+        rs_check(rs_knn_remove(h_, left.data(), right.data(), (int64_t)left.size(), t->GlobalMean));
+        Edited(t);
+    }
+
+    // Gives the (raw user, raw item) pairs of rowSet its ratings without a refit (rs_knn_change): the model becomes
+    // the Fit of Change(*Data, rowSet), bit for bit, and Data that TrainSet.
+    void Change(const DataSet &rowSet) {
+        auto t = std::make_shared<const TrainSet>(core::Change(*Data, rowSet));
+        std::vector<int32_t> left, right;
+        EditPairs(rowSet.Users, rowSet.Items, left, right);
+        rs_check(rs_knn_change(h_, left.data(), right.data(), rowSet.Ratings.data(), (int64_t)left.size(),
+                               t->GlobalMean));
+        Edited(t);
+    }
+
     std::vector<double> PredictBatch(const std::vector<int64_t> &users, const std::vector<int64_t> &items) override {
         std::vector<int32_t> l(users.size()), r(users.size());
         for (size_t j = 0; j < users.size(); j++) {
@@ -284,8 +372,7 @@ struct KNN : Estimator {
         if (!users.empty())
             rs_check(rs_knn_recommend(h_, userBased_ ? RS_SIDE_LEFT : RS_SIDE_RIGHT, q.data(), (int64_t)q.size(), n,
                                       ids.data(), scores.data()));
-        std::vector<int64_t> raw(Data->ItemCount);          // inner -> raw: the order of first appearance
-        for (size_t j = 0; j < Data->Length(); j++) raw[Data->innerItems[j]] = Data->Items[j];
+        const std::vector<int64_t> raw = Data->RawItems();   // inner -> raw
         items.resize(ids.size());
         for (size_t j = 0; j < ids.size(); j++) items[j] = ids[j] >= 0 ? raw[ids[j]] : newID;
     }
@@ -321,8 +408,7 @@ struct KNN : Estimator {
         if (!users.empty())
             rs_check(rs_knn_recommend_given(h_, userBased_ ? RS_SIDE_LEFT : RS_SIDE_RIGHT, ptr.data(), ids.data(),
                                             vals.data(), (int64_t)users.size(), n, top.data(), scores.data()));
-        std::vector<int64_t> raw(Data->ItemCount);          // inner -> raw: the order of first appearance
-        for (size_t j = 0; j < Data->Length(); j++) raw[Data->innerItems[j]] = Data->Items[j];
+        const std::vector<int64_t> raw = Data->RawItems();   // inner -> raw
         items.resize(top.size());
         for (size_t j = 0; j < top.size(); j++) items[j] = top[j] >= 0 ? raw[top[j]] : newID;
     }
@@ -337,6 +423,22 @@ struct KNN : Estimator {
     std::unique_ptr<Estimator> Clone() const override { return std::make_unique<KNN>(KNNType, Params); }
 
   private:
+    void EditPairs(const std::vector<int64_t> &users, const std::vector<int64_t> &items, std::vector<int32_t> &left,
+                   std::vector<int32_t> &right) const {
+        for (size_t j = 0; j < users.size(); j++) {
+            const int32_t iu = Data->ConvertUserID(users[j]), ii = Data->ConvertItemID(items[j]);
+            left.push_back(userBased_ ? iu : ii);
+            right.push_back(userBased_ ? ii : iu);
+        }
+    }
+
+    void Edited(const std::shared_ptr<const TrainSet> &t) {
+        extended_ = t;
+        Data = t.get();
+        GlobalMean = t->GlobalMean;
+        ReadStats();
+    }
+
     void ReadStats() {
         if (KNNType == "centered" || KNNType == "zscore") { Means.resize(nLeft_); rs_check(rs_knn_means(h_, Means.data())); }
         if (KNNType == "zscore") { StdDevs.resize(nLeft_); rs_check(rs_knn_stddevs(h_, StdDevs.data())); }

@@ -7,6 +7,10 @@
 //             ratings given there instead of the train set's; one line per user in order of first appearance)
 //   recommend ... <k> <n> --update <ratings file> <user> [<user> ...]   (KNN::Update with the second file's ratings,
 //             then KNN::Recommend)
+//   recommend ... <k> <n> --remove <ratings file> <user> [<user> ...]   (KNN::Remove of the second file's (user, item)
+//             pairs, its ratings ignored, then KNN::Recommend)
+//   recommend ... <k> <n> --change <ratings file> <user> [<user> ...]   (KNN::Change with the second file's ratings,
+//             then KNN::Recommend)
 //
 // The estimator is fitted with k = 40 and `k` is set afterwards (Predict reads k at call time, core/knn.go:80-81).
 // One output line per user: the user id, then n pairs "item score", the score as the 16 hex digits of its bits.
@@ -57,8 +61,15 @@ int main(int argc, char **argv) {
         knn.RecommendGiven(load_file(argv[8]), n, users, items, scores);
     } else {
         int a = 7;
-        if (!std::strcmp(argv[7], "--update") && argc >= 10) {
+        if (argc >= 10 && !std::strcmp(argv[7], "--update")) {
             knn.Update(load_file(argv[8]));
+            a = 9;
+        } else if (argc >= 10 && !std::strcmp(argv[7], "--remove")) {
+            const core::DataSet d = load_file(argv[8]);
+            knn.Remove(d.Users, d.Items);
+            a = 9;
+        } else if (argc >= 10 && !std::strcmp(argv[7], "--change")) {
+            knn.Change(load_file(argv[8]));
             a = 9;
         }
         for (; a < argc; a++) users.push_back(std::atoll(argv[a]));
