@@ -56,7 +56,9 @@ enum rs_knn_type { RS_KNN_BASIC = 0, RS_KNN_CENTERED = 1, RS_KNN_ZSCORE = 2, RS_
 /* How Pearson is evaluated.
  *   EXACT: FP64 replay of core/sim.go:65-80 in the reference's accumulation order
  *          (ascending right id) — bit-identical similarities and neighbour lists.
- *   SUMS : the six integer co-rating sums on int8 tensor cores + an FP64 epilogue;
+ *   SUMS : the six integer co-rating sums on int8 tensor cores + an FP64 epilogue that forms
+ *          L / (sqrt(Mi) * sqrt(Ni)) from exact integers: within 4 ulps of the exact value (6 once
+ *          |L|, Mi or Ni pass 2^53), NaN exactly where Mi * Ni == 0, +0.0 where L == 0, symmetric;
  *          equal to EXACT within 1e-9*max(1,|s|), not bit-identical (SURVEY.md hazard 2). */
 enum rs_pearson_mode { RS_PEARSON_EXACT = 0, RS_PEARSON_SUMS = 1 };
 /* Which device kernel computes the similarities.
@@ -66,7 +68,10 @@ enum rs_pearson_mode { RS_PEARSON_EXACT = 0, RS_PEARSON_SUMS = 1 };
  *           cost model: dense int8 work N(N-1)/2 * 2*G*K against the co-rated triples counted
  *           during Fit (csrc/api.cu tensor_faster; constants measured on B200).
  *   TENSOR: tcgen05.mma.kind::i8 masked contractions (fails with RS_ERR_UNSUPPORTED if
- *           the ratings are not small integers).
+ *           the ratings are not small integers, or if its int32 sums could overflow: with
+ *           m = the largest |rating| and n2 = the second-longest left row, 4 m^2 n2 > 2^31-1
+ *           for MSD, m^2 n2 for Cosine and Pearson SUMS, 2 m n2 for Slope One; AUTO then runs
+ *           STREAM).
  *   STREAM: FP64 CUDA-core sparse replay: work proportional to the co-rated triples,
  *           accumulation in the reference's order; accepts ANY float64 ratings (no limit on
  *           the number of distinct values; NaN ratings are refused). */
@@ -201,7 +206,9 @@ int32_t rs_knn_topk_device(rs_knn *h, int32_t k, int32_t *d_idx, double *d_sim);
 
 /* Integer co-rating sums {count, sum_x, sum_y, sum_xx, sum_yy, sum_xy} of left rows
  * [row0,row0+nrows) against all N rows, straight from the tensor-core contraction
- * (out: nrows*N*6 int32, host).  Parity surface for "integer co-rating sums bit-exact". */
+ * (out: nrows*N*6 int32, host).  Parity surface for "integer co-rating sums bit-exact".
+ * RS_ERR_UNSUPPORTED when the sums could leave int32: m^2 n1 > 2^31-1, m = the largest
+ * |rating|, n1 = the longest left row (the sums of a row with itself run over all of it). */
 int32_t rs_knn_cosums(rs_knn *h, int64_t row0, int64_t nrows, int32_t *out);
 
 /* KNN.Means / KNN.StdDevs (core/knn.go:24-25): n_left doubles each, host. */

@@ -98,11 +98,48 @@ int32_t fold_profile(rs_knn *h) {
     return RS_OK;
 }
 
-bool tensor_eligible(const rs_knn *h) {
+// Integer ratings and a similarity the tensor path computes.
+bool tensor_kind(const rs_knn *h) {
     if (h->rating_class != RS_CLASS_INT8) return false;
     if (h->p.sim == RS_SIM_COSINE || h->p.sim == RS_SIM_MSD || h->p.sim == RS_SIM_SLOPE_ONE) return true;
     if (h->p.sim == RS_SIM_PEARSON && h->p.pearson_mode == RS_PEARSON_SUMS) return true;
     return false;
+}
+
+// The tensor path accumulates in int32 (kind::i8 MMAs) and is exact only while no sum can leave it.  With m = the
+// largest |rating| and a pair co-rated over at most n2 ratings (its shorter row, so n2 = the second-longest left
+// row), the largest value an int32 of `sim` reaches: Sum (x - y)^2 <= 4 m^2 n2 for MSD, which its epilogue forms in
+// int32 from Sxx + Syy and Sxy; Sxx, Syy, |Sxy| <= m^2 n2 for Cosine and Pearson `sums`; |Sx - Sy| <= 2 m n2 for Slope
+// One, whose epilogue forms that difference in int32.  Pearson also reads the row sums, |sum| <= m n1 over the longest
+// row n1.  *what names the bound.
+int64_t tensor_peak(const rs_knn *h, int sim, const char **what) {
+    const int64_t m = h->int_abs_max, n1 = h->row_len1, n2 = h->row_len2;
+    switch (sim) {
+    case RS_SIM_MSD: *what = "4 m^2 n2"; return 4 * m * m * n2;
+    case RS_SIM_SLOPE_ONE: *what = "2 m n2"; return 2 * m * n2;
+    case RS_SIM_PEARSON:
+        if (m * n1 > m * m * n2) { *what = "m n1"; return m * n1; }
+        *what = "m^2 n2";
+        return m * m * n2;
+    default: *what = "m^2 n2"; return m * m * n2;
+    }
+}
+
+bool tensor_in_range(const rs_knn *h) {
+    const char *what;
+    return tensor_peak(h, h->p.sim, &what) <= INT32_MAX;
+}
+
+bool tensor_eligible(const rs_knn *h) { return tensor_kind(h) && tensor_in_range(h); }
+
+// The error of a Fit (or rs_knn_cosums, sim = RS_SIM_COSINE: the same sums) that the int32 accumulators cannot hold.
+int32_t tensor_range_error(const rs_knn *h, int sim, const char *who) {
+    const char *what;
+    const int64_t peak = tensor_peak(h, sim, &what);
+    rs_set_error("%s: the tensor path's int32 accumulators cannot hold this Fit's sums: %s = %lld > 2^31-1 (m = %d = "
+                 "largest |rating|, n1 = %lld and n2 = %lld = the longest and second-longest left row)", who, what,
+                 (long long)peak, h->int_abs_max, (long long)h->row_len1, (long long)h->row_len2);
+    return RS_ERR_UNSUPPORTED;
 }
 
 // Fit path model.  Both paths are bit-exact for Cosine / MSD, so RS_PATH_AUTO takes the faster one.
@@ -321,10 +358,11 @@ static int32_t fit(rs_knn *h, const int32_t *d_left, const int32_t *d_right, con
     }
     if (h->p.sim == RS_SIM_SLOPE_ONE) {
         // the deviation sums are integer contractions: tensor path only (integer ratings)
-        if (!tensor_eligible(h) || path == RS_PATH_STREAM) {
+        if (!tensor_kind(h) || path == RS_PATH_STREAM) {
             rs_set_error("RS_SIM_SLOPE_ONE needs integer ratings in [-11,11] (tensor path)");
             return RS_ERR_UNSUPPORTED;
         }
+        if (!tensor_in_range(h)) return tensor_range_error(h, h->p.sim, "RS_SIM_SLOPE_ONE");
         path = RS_PATH_TENSOR;
     }
     if (h->cyc_R) {
@@ -337,10 +375,11 @@ static int32_t fit(rs_knn *h, const int32_t *d_left, const int32_t *d_right, con
         path = RS_PATH_STREAM;
     }
     if (path == RS_PATH_AUTO) path = tensor_eligible(h) && tensor_faster(h) ? RS_PATH_TENSOR : RS_PATH_STREAM;
-    if (path == RS_PATH_TENSOR && !tensor_eligible(h)) {
+    if (path == RS_PATH_TENSOR && !tensor_kind(h)) {
         rs_set_error("tensor path needs integer ratings in [-11,11] and Cosine/MSD (or Pearson in SUMS mode)");
         return RS_ERR_UNSUPPORTED;
     }
+    if (path == RS_PATH_TENSOR && !tensor_in_range(h)) return tensor_range_error(h, h->p.sim, "rs_knn_fit");
     h->prof.sim_path_used = path;
     h->prof.corated_triples = h->triples;
     RS_TRY(path == RS_PATH_TENSOR ? rs_prep_planes(h) : rs_prep_rt(h));
@@ -989,6 +1028,14 @@ int32_t rs_knn_cosums(rs_knn *h, int64_t row0, int64_t nrows, int32_t *out) {
     }
     if (h->rating_class != RS_CLASS_INT8) {
         rs_set_error("rs_knn_cosums: integer co-rating sums need integer ratings in [-11,11]");
+        return RS_ERR_UNSUPPORTED;
+    }
+    // the six sums of a row with itself (the diagonal) run over the whole row: |Sxx| <= m^2 n1
+    const int64_t m = h->int_abs_max;
+    if (m * m * h->row_len1 > INT32_MAX) {
+        rs_set_error("rs_knn_cosums: the int32 sums cannot hold this Fit's: m^2 n1 = %lld > 2^31-1 (m = %d = largest "
+                     "|rating|, n1 = %lld = the longest left row)", (long long)(m * m * h->row_len1), h->int_abs_max,
+                     (long long)h->row_len1);
         return RS_ERR_UNSUPPORTED;
     }
     if (nrows == 0) return RS_OK;

@@ -6,6 +6,7 @@
 #include <cstdarg>
 #include <cstdint>
 #include <cstdio>
+#include <cstring>
 #include <mutex>
 #include <vector>
 
@@ -147,7 +148,10 @@ struct rs_knn {
     double *left_bias = nullptr;  // KNN.Bias
     int32_t *row_cnt = nullptr;   // ratings per left row and their integer sum (tensor path, Pearson)
     int32_t *row_sum = nullptr;
-    int64_t max_row_cnt = 0;
+    // integer class: the largest |rating| and the two longest left rows, which bound every int32 accumulator of the
+    // tensor path (tensor_eligible, api.cu)
+    int32_t int_abs_max = 0;
+    int64_t row_len1 = 0, row_len2 = 0;
     int32_t max_right_len = 0;    // longest right row = most candidates one prediction can have
     double triples = 0.0;         // co-rated triples of the full matrix: sum over right rows of cnt*(cnt-1)/2
     double *right_bias = nullptr;
@@ -299,6 +303,16 @@ int32_t rs_prep_planes(rs_knn *h);
 int32_t rs_row_stats_launch(rs_knn *h, const int64_t *ptr, const double *ld_val, const double *l_val, int64_t n,
                             int want_std, double *means, double *stddevs, double *pmeans);
 int32_t rs_prep_stats(rs_knn *h);
+// Words of h->d_flags (16 x int32) where rs_prep_stats leaves the tensor path's limits for integer ratings: the largest
+// |rating|, and at the 8-byte aligned pair RS_FL_LEN_TOP2 the longest (high word) and second-longest (low) left row.
+constexpr int RS_FL_ABS_MAX = 1, RS_FL_LEN_TOP2 = 12;
+inline void rs_tensor_limits_read(rs_knn *h, const int32_t fl[16]) {
+    unsigned long long t;
+    std::memcpy(&t, fl + RS_FL_LEN_TOP2, 8);
+    h->int_abs_max = fl[RS_FL_ABS_MAX];
+    h->row_len1 = (int64_t)(t >> 32);
+    h->row_len2 = (int64_t)(t & 0xFFFFFFFFull);
+}
 // Kernels of the CSR build that rs_knn_update runs on the added ratings as Fit runs them on all ratings.
 enum rs_prep_flag { FLAG_BAD_ID = 1, FLAG_NOT_INT8 = 2, FLAG_DUP = 4, FLAG_NAN = 8, FLAG_MISSING = 16 };
 __global__ void ptr_from_sorted_kernel(const int32_t *__restrict__ keys, int64_t nnz, int32_t n_rows,

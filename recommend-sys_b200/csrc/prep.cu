@@ -113,17 +113,58 @@ __global__ void code_int8_kernel(const double *__restrict__ val, int64_t nnz, ui
     if (i < nnz) code[i] = (uint8_t)((int)val[i] + RS_INT8_BIAS);
 }
 
+// (longest, second longest) packed as (hi << 32 | lo): inserts a row length.  A stale read only costs a retry, and
+// `lo` never shrinks, so a length at or below a stale `lo` is below the current one too.
+__device__ __forceinline__ void top2_insert(unsigned long long *p, uint32_t c) {
+    unsigned long long old = *reinterpret_cast<volatile unsigned long long *>(p);
+    while (c > (uint32_t)old) {
+        const uint32_t hi = (uint32_t)(old >> 32);
+        const unsigned long long nw = c > hi ? ((unsigned long long)c << 32) | hi : ((unsigned long long)hi << 32) | c;
+        const unsigned long long seen = atomicCAS(p, old, nw);
+        if (seen == old) return;
+        old = seen;
+    }
+}
+
+// Row counts and integer sums; with `limits` also what the tensor path's int32 accumulators depend on (tensor_eligible,
+// api.cu): the largest |rating| into limits[RS_FL_ABS_MAX], the two longest rows into limits[RS_FL_LEN_TOP2 ..].  One
+// warp per row; the block's rows are reduced in shared memory first, so the global words see one update per block.
 __global__ void row_isum_kernel(const int64_t *__restrict__ l_ptr, const uint8_t *__restrict__ l_code,
-                                int32_t n_left, int32_t *__restrict__ row_cnt, int32_t *__restrict__ row_sum) {
+                                int32_t n_left, int32_t *__restrict__ row_cnt, int32_t *__restrict__ row_sum,
+                                int32_t *limits) {
+    __shared__ int32_t s_mx;
+    __shared__ unsigned long long s_top2;
+    if (threadIdx.x == 0) { s_mx = 0; s_top2 = 0ull; }
+    if (limits) __syncthreads();
     int32_t row = (int32_t)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
     int lane = threadIdx.x & 31;
-    if (row >= n_left) return;
-    int s = 0;
-    for (int64_t x = l_ptr[row] + lane; x < l_ptr[row + 1]; x += 32) s += (int)l_code[x] - RS_INT8_BIAS;
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    if (lane == 0) {
-        row_cnt[row] = (int32_t)(l_ptr[row + 1] - l_ptr[row]);
-        row_sum[row] = s;
+    if (row < n_left) {
+        int s = 0, mx = 0;
+        for (int64_t x = l_ptr[row] + lane; x < l_ptr[row + 1]; x += 32) {
+            const int v = (int)l_code[x] - RS_INT8_BIAS;
+            s += v;
+            mx = max(mx, abs(v));
+        }
+        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        mx = __reduce_max_sync(0xffffffffu, mx);
+        if (lane == 0) {
+            const int32_t c = (int32_t)(l_ptr[row + 1] - l_ptr[row]);
+            row_cnt[row] = c;
+            row_sum[row] = s;
+            if (limits) {
+                atomicMax(&s_mx, mx);
+                top2_insert(&s_top2, (uint32_t)c);
+            }
+        }
+    }
+    if (limits) {
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            if (s_mx > *reinterpret_cast<volatile int32_t *>(limits + RS_FL_ABS_MAX)) atomicMax(limits + RS_FL_ABS_MAX, s_mx);
+            unsigned long long *g = reinterpret_cast<unsigned long long *>(limits + RS_FL_LEN_TOP2);
+            top2_insert(g, (uint32_t)(s_top2 >> 32));
+            top2_insert(g, (uint32_t)s_top2);
+        }
     }
 }
 
@@ -360,13 +401,15 @@ int bits_for(int32_t n) {
 }  // namespace
 
 // The statistics of every left row from the left CSR, into the buffers h points to: means, stddevs (z-score) and
-// pmeans, and for integer ratings row_cnt / row_sum.  Fit's, and rs_knn_update's for the merged rows.
+// pmeans, and for integer ratings row_cnt / row_sum and the tensor path's limits in h->d_flags (zeroed by the caller,
+// read back with rs_tensor_limits_read).  Fit's, and rs_knn_update's for the merged rows.
 int32_t rs_prep_stats(rs_knn *h) {
     cudaStream_t st = h->stream;
     const int32_t nl = h->n_left;
     const int want_std = h->p.knn_type == RS_KNN_ZSCORE;
     if (h->rating_class == RS_CLASS_INT8) {
-        row_isum_kernel<<<blocks_for((int64_t)nl * 32), T, 0, st>>>(h->l_ptr, h->l_code, nl, h->row_cnt, h->row_sum);
+        row_isum_kernel<<<blocks_for((int64_t)nl * 32), T, 0, st>>>(h->l_ptr, h->l_code, nl, h->row_cnt, h->row_sum,
+                                                                     h->d_flags);
         means_from_isum_kernel<<<blocks_for(nl), T, 0, st>>>(h->row_cnt, h->row_sum, nl, h->means, h->pmeans);
         h->prof.total_launches += 2;
     }
@@ -602,6 +645,7 @@ int32_t rs_prep_build(rs_knn *h, const int32_t *d_left, const int32_t *d_right, 
     { unsigned long long t; memcpy(&t, fl8 + 6, 8); h->triples = (double)t; }
     h->max_right_len = fl8[15];
     { unsigned long long t[2]; memcpy(t, fl8 + 8, 16); h->inc_upper = (double)t[0]; h->inc_lower = (double)t[1]; }
+    rs_tensor_limits_read(h, fl8);
     pick_triangle(h);
     if (flags & FLAG_DUP) {
         rs_set_error("duplicate (left,right) rating pairs are not supported (the reference's merge-join "

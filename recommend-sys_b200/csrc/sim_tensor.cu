@@ -5,11 +5,15 @@
 // rows a, b is a dot product of int8 planes of the left matrix (X = rating, X2 = rating^2,
 // M = 1 where rated):
 //     count = M_a.M_b   Sx = X_a.M_b   Sy = M_a.X_b   Sxx = X2_a.M_b   Syy = M_a.X2_b   Sxy = X_a.X_b
-// The int32 accumulation is exact, so the FP64 epilogue reproduces the reference bit for bit
+// The int32 accumulation is exact while no sum leaves int32: with m = the largest |rating| and n2 = the
+// second-longest left row (a pair is co-rated over at most its shorter row), 4 m^2 n2 for MSD (its epilogue
+// forms Sxx + Syy - 2 Sxy in int32), m^2 n2 for Cosine and Pearson, 2 m n2 for Slope One (Sx - Sy); tensor_eligible
+// (api.cu) refuses a Fit beyond them.  Inside them the FP64 epilogue reproduces the reference bit for bit
 // for Cosine (core/sim.go:10-25) and MSD (core/sim.go:28-44), whose Go sums are sums of small
-// integers.  Pearson from the sums is exact arithmetic on integers (see pearson_from_sums),
-// i.e. the correctly rounded value, but NOT the reference's rounding sequence; the bit-exact
-// Pearson is the stream path (sim_stream.cu).
+// integers.  Pearson from the sums is exact integer arithmetic followed by four roundings (see
+// pearson_from_sums): within 4 ulps of the exact value (6 once an integer passes 2^53), but NOT the
+// reference's rounding sequence; the
+// bit-exact Pearson is the stream path (sim_stream.cu).
 //
 // Kernel shape (one CTA per SM, persistent over a static tile list):
 //   tile      = 128 left rows (MMA M, TMEM lanes) x BN left rows (MMA N) x all K;
@@ -60,7 +64,8 @@ constexpr int TMEM_COLS = 512;
 // plane order in global and shared memory
 constexpr int PL_X2 = 0, PL_M = 1, PL_X = 2;
 
-enum { TC_COSINE = 0, TC_MSD = 1, TC_PEARSON = 2, TC_COSUMS = 3, TC_SLOPE = 4 };
+// TC_PEARSON128: Pearson with the __int128 epilogue (pearson_from_sums), for rows too long for the int64 one
+enum { TC_COSINE = 0, TC_MSD = 1, TC_PEARSON = 2, TC_COSUMS = 3, TC_SLOPE = 4, TC_PEARSON128 = 5 };
 
 // Per-mode tile shape.  Every tcgen05.mma reads its A slab (128 x 32 B) and B slab (N x 32 B) from
 // shared memory, so narrow instructions are shared-memory bound: 3 x N=64 (the first Cosine
@@ -86,6 +91,7 @@ template <> struct Cfg<TC_PEARSON> {
     static constexpr int C_SYY = 0, C_CNT = 64, C_SY = 128, C_SX = 192, C_SXY = 256, C_SXX = 320;
 };
 template <> struct Cfg<TC_COSUMS> : Cfg<TC_PEARSON> {};
+template <> struct Cfg<TC_PEARSON128> : Cfg<TC_PEARSON> {};
 template <> struct Cfg<TC_SLOPE> {
     // Slope One deviations (core/slope_one.go:71-90): count, Sy = M_I x [M|X]_J (N = 256), Sx = X_I x M_J
     static constexpr int BN = 128, BK = 64, STAGES = 4;
@@ -261,19 +267,50 @@ __device__ __forceinline__ unsigned long long ld_relaxed_gpu(const unsigned long
 //   l  = L/(ca*cb),                  L  = ca*cb*Sxy - ca*sb*Sx - cb*sa*Sy + n*sa*sb
 //   l/(sqrt(m)*sqrt(nn)) = L/(sqrt(Mi)*sqrt(Ni))   — the counts cancel; Mi==0 <=> m==0 exactly,
 // so NaN-ness matches the reference's 0/0 (core/sim.go:80) with no cancellation noise.
-// Range: Mi = ca^2 * sum (x - sa/ca)^2 over the co-rated x <= ca^3 * h^2 for ratings spanning 2h (largest when the
-// pair is co-rated over the whole row), so Mi, Ni and L fit int64 for left rows of up to ~4.2e5 ratings of [-11, 11]
-// (h = 11) or ~1.3e6 ratings of 1..5 (h = 2); a left row is at most as long as the other side has ids.  Partial
-// terms such as ca*ca*sxx and 2*ca*sa*sx are larger (up to 242 ca^3 for +-11) and leave int64 sooner: below the
-// bound the sums still come out right only because the device's 64-bit signed arithmetic wraps (two's complement),
-// which C++ leaves undefined.  Beyond the bound the result is wrong and nothing refuses it.
+// Range: Mi = ca^2 * sum (x - sa/ca)^2 over the co-rated x, and every partial term and partial sum of the three
+// integers is at most 4 m^2 n1^3 for ratings |x| <= m and rows of at most n1 ratings (ca*ca*sxx, 2*ca*sa*sx up to
+// 242 ca^3 for +-11).  Two instantiations (the host picks one per Fit, rs_sim_tensor_launch):
+//   I128 = false  int64, exact and free of signed overflow while 4 m^2 n1^3 < 2^63 (rows of up to ~2.67e5 ratings of
+//                 +-11, ~4.5e5 of 1..5: every MovieLens shape);
+//   I128 = true   __int128 beyond: with the co-rated sums and the row sums inside int32 (tensor_eligible in api.cu)
+//                 and rows of fewer than 2^31 ratings every term is below 2^100.
+// Rounding: L, Mi and Ni convert exactly below 2^53 and correctly rounded (to nearest) above; then two square roots,
+// a product and a quotient, each correctly rounded.  Relative error below 4 * 2^-53 (to first order) while |L|, Mi
+// and Ni are below 2^53, i.e. within 4 ulps of the exact L / sqrt(Mi * Ni); past 2^53 the conversion of L adds
+// 2^-53 and those of Mi and Ni 2^-53 each, halved by the square root: 6 ulps.  It is not the correctly rounded value,
+// and not the reference's rounding sequence.
+// (double) of a __int128 is lowered in software without a documented rounding; this one rounds to nearest: below
+// 2^63 cvt.rn.f64.s64, above a right shift to 62 bits that ORs the dropped bits into the last one (the sticky bit
+// lies below the rounding position, so rounding the shifted value to 53 bits rounds the original), then an exact
+// power-of-two scaling.
+__device__ __forceinline__ double i128_to_double_rn(__int128 v) {
+    const long long lo = (long long)v;
+    if ((__int128)lo == v) return (double)lo;
+    const unsigned __int128 u = v < 0 ? (unsigned __int128)(-v) : (unsigned __int128)v;   // >= 2^63
+    const unsigned long long uh = (unsigned long long)(u >> 64);
+    const int bits = uh ? 128 - __clzll((long long)uh) : 64;
+    const int shift = bits - 62;
+    const unsigned long long w = (unsigned long long)(u >> shift) | ((u & (((unsigned __int128)1 << shift) - 1)) != 0);
+    const double d = ldexp((double)(long long)w, shift);
+    return v < 0 ? -d : d;
+}
+
+template <bool I128>
 __device__ __forceinline__ double pearson_from_sums(long long n, long long sx, long long sy, long long sxx,
                                                     long long syy, long long sxy, long long ca, long long sa,
                                                     long long cb, long long sb) {
-    const long long Mi = ca * ca * sxx - 2 * ca * sa * sx + n * sa * sa;
-    const long long Ni = cb * cb * syy - 2 * cb * sb * sy + n * sb * sb;
-    const long long L = ca * cb * sxy - ca * sb * sx - cb * sa * sy + n * sa * sb;
-    return (double)L / (sqrt((double)Mi) * sqrt((double)Ni));
+    if constexpr (!I128) {
+        const long long Mi = ca * ca * sxx - 2 * ca * sa * sx + n * sa * sa;
+        const long long Ni = cb * cb * syy - 2 * cb * sb * sy + n * sb * sb;
+        const long long L = ca * cb * sxy - ca * sb * sx - cb * sa * sy + n * sa * sb;
+        return (double)L / (sqrt((double)Mi) * sqrt((double)Ni));
+    } else {
+        using i128 = __int128;
+        const i128 Mi = (i128)ca * ca * sxx - (i128)(2 * ca) * sa * sx + (i128)n * sa * sa;
+        const i128 Ni = (i128)cb * cb * syy - (i128)(2 * cb) * sb * sy + (i128)n * sb * sb;
+        const i128 L = (i128)ca * cb * sxy - (i128)ca * sb * sx - (i128)cb * sa * sy + (i128)n * sa * sb;
+        return i128_to_double_rn(L) / (sqrt(i128_to_double_rn(Mi)) * sqrt(i128_to_double_rn(Ni)));
+    }
 }
 
 // K-lockstep throttle of the TMA producers.  Tiles that run at the same time share operand rows (supertile
@@ -511,7 +548,7 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
             tc_fence_after();
             const uint32_t tbase = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * C::ACC_COLS);
             long long ca = 0, sa = 0;
-            if (MODE == TC_PEARSON && i < a.n_left) { ca = a.row_cnt[i]; sa = a.row_sum[i]; }
+            if ((MODE == TC_PEARSON || MODE == TC_PEARSON128) && i < a.n_left) { ca = a.row_cnt[i]; sa = a.row_sum[i]; }
             const bool row_ok = (i < a.n_left) && (i >= a.row_begin) && (i < a.row_end);
 #pragma unroll 1
             for (int c0 = chalf * (BN / 2); c0 < (chalf + 1) * (BN / 2); c0 += 8) {
@@ -535,11 +572,11 @@ sim_tensor_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
 #pragma unroll
                     for (int c = 0; c < 8; c++) {
                         const int64_t j = j0 + c0 + c;
-                        if constexpr (MODE == TC_PEARSON) {
+                        if constexpr (MODE == TC_PEARSON || MODE == TC_PEARSON128) {
                             long long cb = 0, sb = 0;
                             if (j < a.n_left) { cb = a.row_cnt[j]; sb = a.row_sum[j]; }
-                            s[c] = pearson_from_sums(v.cnt[c], v.sx[c], v.sy[c], v.sxx[c], v.syy[c], v.sxy[c], ca, sa,
-                                                     cb, sb);
+                            s[c] = pearson_from_sums<MODE == TC_PEARSON128>(v.cnt[c], v.sx[c], v.sy[c], v.sxx[c],
+                                                                            v.syy[c], v.sxy[c], ca, sa, cb, sb);
                             if (j == i) s[c] = __longlong_as_double(0x7ff8000000000001ll);   // diagonal stays unset
                         } else {
                             s[c] = sim_from_sums<MODE>(v, c, i, j);
@@ -947,6 +984,15 @@ int32_t upload_tiles(rs_knn *h, const std::vector<int2> &tiles, void **buf, size
     return RS_OK;
 }
 
+// Pearson: the int64 epilogue is exact and free of signed overflow while every term of pearson_from_sums, at most
+// 4 m^2 n1^3 (m = the largest |rating|, n1 = the longest left row), is below 2^63; past that the __int128 one runs.
+// RS_KNN_PEARSON_I128=1 forces the __int128 epilogue (tests: both are exact integers, so both give the same bits).
+bool pearson_i128(const rs_knn *h) {
+    if (const char *e = getenv("RS_KNN_PEARSON_I128")) if (atoi(e) != 0) return true;
+    const unsigned __int128 m = (unsigned __int128)h->int_abs_max, n1 = (unsigned __int128)h->row_len1;
+    return 4 * m * m * n1 * n1 * n1 >= ((unsigned __int128)1 << 63);
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------
@@ -1148,7 +1194,7 @@ int32_t rs_sim_tensor_launch(rs_knn *h, int32_t *d_cosums, int64_t cos_row0, int
     case TC_COSINE: rc = use_pair ? launch_pair<TC_COSINE>(h, a) : launch_single<TC_COSINE>(h, a); break;
     case TC_MSD: rc = use_pair ? launch_pair<TC_MSD>(h, a) : launch_single<TC_MSD>(h, a); break;
     case TC_SLOPE: rc = use_pair ? launch_pair<TC_SLOPE>(h, a) : launch_single<TC_SLOPE>(h, a); break;
-    case TC_PEARSON: rc = launch_single<TC_PEARSON>(h, a); break;
+    case TC_PEARSON: rc = pearson_i128(h) ? launch_single<TC_PEARSON128>(h, a) : launch_single<TC_PEARSON>(h, a); break;
     default: rc = launch_single<TC_COSUMS>(h, a); break;   // TC_COSUMS
     }
     RS_TRY(rc);

@@ -493,10 +493,16 @@ int32_t upd_recompute(rs_knn *h, const int32_t *touched, int64_t n_owned, int64_
     double *sims = h->sims;
     h->planes = nullptr;                         // rs_knn_cosums rebuilds the int8 planes of the new ratings ...
     h->updated = true;                           // ... into a block of their own (rs_prep_planes)
+    // the tensor path's limits of the new ratings (rs_knn_cosums), read back with the synchronisation below
+    int32_t fl[16];
+    RS_CUDA(cudaMemsetAsync(h->d_flags + RS_FL_ABS_MAX, 0, 4, st));
+    RS_CUDA(cudaMemsetAsync(h->d_flags + RS_FL_LEN_TOP2, 0, 8, st));
     RS_TRY(rs_prep_stats(h));
+    RS_CUDA(cudaMemcpyAsync(fl, h->d_flags, sizeof(fl), cudaMemcpyDeviceToHost, st));
     // the statistics are final when the call returns, as Fit's are: rs_knn_means / rs_knn_stddevs read them on the
     // auxiliary stream, which does not wait for this one
     RS_CUDA(cudaStreamSynchronize(st));
+    rs_tensor_limits_read(h, fl);
     for (int64_t b0 = 0; b0 < n_owned; b0 += s.batch) {
         const int64_t nb = n_owned - b0 < s.batch ? n_owned - b0 : s.batch;
         RS_TRY(rs_given_sims_launch(h, h->l_ptr, h->l_col, h->l_val, h->pmeans, nb, s.p, ld, touched + b0));

@@ -183,34 +183,40 @@ def test_fixtures_reach_the_signed_range():
 
 
 # ---------------------------------------------------------------------------------------------------------
-# Pearson `sums`: the int64 bound of pearson_from_sums (host only)
+# the tensor path's integer limits (host only)
 # ---------------------------------------------------------------------------------------------------------
-def pearson_sums_max_len(half_range):
-    """The longest left row for which Mi = ca^2 Sxx - 2 ca sa Sx + n sa^2 of pearson_from_sums (csrc/sim_tensor.cu)
-    fits int64: Mi = ca^2 * sum (x - sa / ca)^2 <= L^3 * half_range^2 for a row of L ratings, largest when a row is
-    co-rated over its whole length."""
-    lo, hi = 1, 1 << 22
-    while lo < hi:
-        mid = (lo + hi + 1) // 2
-        if mid ** 3 * half_range ** 2 <= (1 << 63) - 1:
-            lo = mid
-        else:
-            hi = mid - 1
-    return lo
+INT32_MAX = (1 << 31) - 1
 
 
-def test_pearson_sums_int64_bound():
-    """+-11 ratings: rows up to ~4.2e5; ratings 1..5: up to ~1.3e6.  A left row can be as long as the other side has
-    ids, so every workload of bench.py (ratings 1..5) is inside the bound; item-based Pearson `sums` at the Netflix
-    shape (480,189 users) would not be with +-11 ratings."""
+def tensor_max_n2(sim, m):
+    """The longest second-longest left row n2 whose co-rated sums the tensor path's int32 accumulators hold, for ratings
+    of |x| <= m (tensor_eligible, csrc/api.cu): 4 m^2 n2 (MSD's Sum (x - y)^2), m^2 n2 (Cosine, Pearson `sums`:
+    Sxx, Syy, |Sxy|), 2 m n2 (Slope One: its epilogue forms Sx - Sy)."""
+    return INT32_MAX // {"msd": 4 * m * m, "cosine": m * m, "pearson": m * m, "slope_one": 2 * m}[sim]
+
+
+def test_tensor_int32_limits():
+    """+-11: MSD up to n2 = 4,436,949, Cosine and Pearson `sums` up to 17,747,798, Slope One up to 97,612,893.  Pearson
+    forms Mi, Ni and L in int64 while 4 m^2 n1^3 < 2^63 (rows of up to 267,104 ratings of +-11), else in __int128:
+    with every sum below 2^31 (and its row sums, |sa| <= m n1 < 2^31) the largest partial term n sa^2 stays below
+    2^93.  Every workload of bench.py (ratings 1..5) is inside the limits of its
+    similarity on the longest possible rows (a left row is at most as long as the other side has ids)."""
     import bench
 
-    wide, narrow = pearson_sums_max_len(11), pearson_sums_max_len(2)
-    assert 420_000 < wide < 430_000 and 1_300_000 < narrow < 1_330_000
+    assert tensor_max_n2("msd", 11) == 4_436_949 and tensor_max_n2("cosine", 11) == 17_747_798
+    assert tensor_max_n2("slope_one", 11) == 97_612_893
+    assert 4 * 121 * 4_436_950 > INT32_MAX and 121 * 17_747_799 > INT32_MAX and 22 * 97_612_894 > INT32_MAX
+    # Slope One's |Sx - Sy| reaches 2 m n2: one row all +11, the other all -11
+    assert 11 * 97_612_894 - (-11) * 97_612_894 > INT32_MAX >= 11 * 97_612_893 - (-11) * 97_612_893
+    # the int64 Pearson epilogue: every term is at most 4 m^2 n1^3
+    assert 4 * 121 * 267_104 ** 3 < 1 << 63 <= 4 * 121 * 267_105 ** 3
+    assert INT32_MAX * INT32_MAX ** 2 < 1 << 93
     for name, (users, items, *_rest, user_based, _k) in bench.WORKLOADS.items():
         longest = items if user_based else users
-        assert longest < narrow, name
-    assert bench.WORKLOADS["netflix_item_cosine_k50"][0] > wide
+        for sim in ("msd", "cosine", "pearson", "slope_one"):
+            assert longest <= tensor_max_n2(sim, 5), (name, sim)
+    # with ratings of +-11 the Netflix item shape (480,189 users) would still be inside every limit
+    assert bench.WORKLOADS["netflix_item_cosine_k50"][0] <= tensor_max_n2("msd", 11)
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -331,20 +337,92 @@ def test_topk_schedules_negative_neighbours(name, user_based, schedule, monkeypa
         assert bits_equal(got[1], want_s), count
 
 
+def _exact(data, user_based):
+    """The exact sums of a fixture (tests/exact_sums.py) over the inner ids the device sees, and Pearson's (L, Mi, Ni)."""
+    import exact_sums as ex
+
+    rs = _rs()
+    ts = rs.NewTrainSet(rs.NewRawSet(*data[:3]))
+    left, right = _left(ts.innerUsers, ts.innerItems, user_based)
+    n_left, n_right = (ts.UserCount, ts.ItemCount) if user_based else (ts.ItemCount, ts.UserCount)
+    s = ex.Sums(left, right, ts.Ratings, n_left, n_right)
+    return s, s.pearson_terms()
+
+
+# Pearson's tiles are 128 x 64 left rows with 128-byte K blocks: rows of the compared side around 64 and 192
+PEARSON_SHAPES = ((63, 193), (64, 192), (65, 191), (191, 65), (192, 64), (193, 63))
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("user_based", [True, False])
-@pytest.mark.parametrize("name", ["uniform", "extremes"])
+@pytest.mark.parametrize("name", ["uniform", "extremes", "shapes"])
 def test_pearson_sums_signed(name, user_based):
-    data = FIXTURES[name]()
-    est = _fit(data, "pearson", user_based, simPath="tensor", pearsonMode="sums")
-    assert _path(est) == "tensor"
-    got, want = est.Sims, oracle(name, data, "pearson", user_based).sims(copy=False)
-    assert np.array_equal(np.isnan(got), np.isnan(want))
-    ok = ~np.isnan(want)
-    err = np.abs(got[ok] - want[ok])
-    assert (err <= 1e-9 * np.maximum(1.0, np.abs(want[ok]))).all(), err.max()
-    assert bits_equal(got, got.T)
-    est.Close()
+    """Pearson `sums` within 1e-9 of the oracle's exact replay and, against the exact integers, with NaN exactly where
+    Mi Ni == 0, +0.0 exactly where L == 0, bit-symmetric and within 4 ulps (6 past 2^53) of the exact value.  "shapes":
+    the int-range shapes and Pearson's own tile edges."""
+    import exact_sums as ex
+
+    if name == "shapes":
+        cases = [(f"shape{nu}x{ni}", make_shape(nu, ni)) for nu, ni in SHAPES + PEARSON_SHAPES]
+    else:
+        cases = [(name, FIXTURES[name]())]
+    worst = [-1.0, -1.0]
+    for case, data in cases:
+        est = _fit(data, "pearson", user_based, simPath="tensor", pearsonMode="sums")
+        assert _path(est) == "tensor"
+        got, want = est.Sims, oracle(case, data, "pearson", user_based).sims(copy=False)
+        assert np.array_equal(np.isnan(got), np.isnan(want)), case
+        ok = ~np.isnan(want)
+        err = np.abs(got[ok] - want[ok])
+        assert (err <= 1e-9 * np.maximum(1.0, np.abs(want[ok]))).all(), (case, err.max())
+        assert bits_equal(got, got.T), case
+        _, (L, Mi, Ni) = _exact(data, user_based)
+        w = ex.check_ratio(got, L, Mi, Ni, who=case)
+        worst = [max(a, b) for a, b in zip(worst, w)]
+        est.Close()
+    print(f"\nPearson sums {name} user_based={user_based}: max ulps (<2^53, >=2^53) = {tuple(worst)}")
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("user_based", [True, False])
+def test_pearson_sums_i128_epilogue(user_based, monkeypatch):
+    """The __int128 instantiation of pearson_from_sums (the one Fits with rows past 267,104 ratings of +-11 run) forced
+    on short rows gives the int64 one's bits: both form the same exact integers and round them the same way."""
+    cases = [(name, FIXTURES[name]()) for name in ("uniform", "extremes")]
+    cases += [(f"shape{nu}x{ni}", make_shape(nu, ni)) for nu, ni in PEARSON_SHAPES]
+    for case, data in cases:
+        got = []
+        for force in ("0", "1"):
+            monkeypatch.setenv("RS_KNN_PEARSON_I128", force)
+            est = _fit(data, "pearson", user_based, simPath="tensor", pearsonMode="sums")
+            assert _path(est) == "tensor"
+            got.append(est.Sims)
+            est.Close()
+        assert bits_equal(got[0], got[1]), case
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("user_based", [True, False])
+def test_pearson_sums_row_shards(user_based):
+    """Contiguous row shards in `sums` mode (the non-mirrored tile list, row_begin > 0): each shard is its rows of the
+    full-handle Fit bit for bit and meets the exact rules; aligned and unaligned boundaries."""
+    import exact_sums as ex
+
+    data = FIXTURES["uniform"]()
+    full = _fit(data, "pearson", user_based, simPath="tensor", pearsonMode="sums")
+    S = full.Sims
+    full.Close()
+    n = S.shape[0]
+    _, (L, Mi, Ni) = _exact(data, user_based)
+    for bounds in ((0, 384, n), (0, 100, 333, n), (0, 63, 65, n)):
+        for b, e in zip(bounds[:-1], bounds[1:]):
+            est = _fit(data, "pearson", user_based, simPath="tensor", pearsonMode="sums", rowBegin=b, rowEnd=e)
+            assert _path(est) == "tensor"
+            got = est.Sims
+            est.Close()
+            assert got.shape == (e - b, n)
+            assert bits_equal(got, S[b:e]), (b, e)
+            ex.check_ratio(got, L, Mi, Ni, row0=b, who=f"rows {b}:{e}")
 
 
 @pytest.mark.gpu

@@ -3,7 +3,7 @@
 Integer co-rating sums must be bit-exact; Cosine and MSD similarities computed from them must be
 bit-identical to the oracle (their Go sums are sums of small integers, exact in float64);
 Pearson in `sums` mode is held to |d| <= 1e-9 * max(1, |ref|) (SURVEY.md §7.3 item 2) with an
-exactly matching NaN pattern."""
+exactly matching NaN pattern, and to 4 ulps of the exact value of its integer sums (tests/exact_sums.py)."""
 import numpy as np
 import pytest
 
@@ -97,14 +97,24 @@ def test_tensor_row_shard(ml100k, pair, monkeypatch):
 
 
 def test_pearson_sums_mode_tolerance(ml100k):
-    est, ref, _ = _fit(ml100k["u1_base"], "pearson", False, pearsonMode="sums")
-    assert est.Profile()["sim_path_used"] == rs.core.RS_SIM_PATH["tensor"]
-    got, want = est.Sims, ref.sims()
-    assert np.array_equal(np.isnan(got), np.isnan(want))        # NaN-ness decided on exact integers
-    ok = ~np.isnan(want)
-    err = np.abs(got[ok] - want[ok])
-    assert (err <= 1e-9 * np.maximum(1.0, np.abs(want[ok]))).all(), err.max()
-    assert bits_equal(got, got.T)
+    """Both orientations: within 1e-9 of the oracle's replay, and against the exact integer sums (tests/exact_sums.py)
+    NaN exactly where Mi Ni == 0, +0.0 exactly where L == 0, bit-symmetric, within 4 ulps of the exact value."""
+    import exact_sums as ex
+
+    for user_based in (False, True):
+        est, ref, ts = _fit(ml100k["u1_base"], "pearson", user_based, pearsonMode="sums")
+        assert est.Profile()["sim_path_used"] == rs.core.RS_SIM_PATH["tensor"]
+        got, want = est.Sims, ref.sims()
+        assert np.array_equal(np.isnan(got), np.isnan(want))        # NaN-ness decided on exact integers
+        ok = ~np.isnan(want)
+        err = np.abs(got[ok] - want[ok])
+        assert (err <= 1e-9 * np.maximum(1.0, np.abs(want[ok]))).all(), err.max()
+        assert bits_equal(got, got.T)
+        left, right = (ts.innerUsers, ts.innerItems) if user_based else (ts.innerItems, ts.innerUsers)
+        n_left, n_right = (ts.UserCount, ts.ItemCount) if user_based else (ts.ItemCount, ts.UserCount)
+        L, Mi, Ni = ex.Sums(left, right, ts.Ratings, n_left, n_right).pearson_terms()
+        worst = ex.check_ratio(got, L, Mi, Ni, who=f"user_based={user_based}")
+        print(f"\nML-100K Pearson sums user_based={user_based}: max ulps (<2^53, >=2^53) = {worst}")
 
 
 def test_tensor_rejects_non_integer_ratings():
